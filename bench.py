@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B]           # this repo's CUDA path
     python bench.py --impl reference [--steps K] [--warmup W]                  # CPU reference arm
+    python bench.py ... --dump-outputs DIR     # also write a seeded sample of the last timed step's result to DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of synthetic input: B independent hmult
 (config_4.cfg, maxLevel 45, currentLevel 35, alpha 15) per GPU, all B ciphertext pairs distinct and resident
@@ -86,6 +87,24 @@ class ClockSampler(threading.Thread):
                 "samples": len(sm)}
 
 
+DUMP_BYTES = 32 << 20  # one step's result is 9.1 GB (256 x 2 x 34 x 65536 words); --dump-outputs writes a sample of this size
+DUMP_SEED = 0x64756D70
+
+
+def dump_outputs(dirname, name, out, budget, torch):
+    """Write a seeded sample of `out` (int64 [..., N] residues below 2^36, exact in float64) as dirname/name.npy: per row
+    (every ciphertext, component and limb) the same pseudo-random coefficient positions on every run, so that two builds of
+    the project can be compared output for output.  Shape [..., k] with k = budget / (8 bytes x rows)."""
+    import numpy as np
+    rows, n = out.numel() // out.shape[-1], out.shape[-1]
+    k = max(1, min(n, budget // (8 * rows)))
+    g = torch.Generator().manual_seed(DUMP_SEED)
+    idx = torch.randint(0, n, (*out.shape[:-1], k), generator=g).to(out.device)
+    sample = torch.gather(out, -1, idx).cpu().numpy().astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, name + ".npy"), sample)
+
+
 def cpu_port_sample(n_ops, threads):
     """Time the scalar oracle port (oracle/oracle.c) on the same workload: n_ops hmult, `threads` host threads."""
     from orc import Oracle, uniform_limbs
@@ -113,7 +132,7 @@ def run_reference(args, real_stdout):
     threads = os.cpu_count() or 1
     for _ in range(max(0, min(args.warmup, 1))):
         cpu_port_sample(1, threads)
-    steps = max(1, args.steps)
+    steps = args.steps
     us, used = cpu_port_sample(steps, threads)
     sim = {}
     run = os.path.join(ROOT, "oracle", "_ref", "count.run")
@@ -270,7 +289,12 @@ def main():
                     help="with --gpus N > 1 the bench also times ONE ciphertext's key switch and the op sequence limb-sharded over the "
                          "N GPUs (peer-direct NVLink exchanges vs NCCL all-gathers vs one GPU) -> extra.limb_sharded; this skips it")
     ap.add_argument("--sharded", action="store_true", help="(default for N > 1; kept for compatibility)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded %d MB sample of the last step's hmult results (float64) to "
+                         "DIR/hmult_out.npy (DIR/hmult_out_rank<r>.npy per rank with several GPUs)" % (DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args, real_stdout)
 
@@ -295,7 +319,7 @@ def main():
     except Exception as e:  # not fatal: the run proceeds with the inherited affinity
         numa = "unchanged (%s)" % type(e).__name__
     W = max(3, args.warmup)
-    K, L = max(1, args.steps), LEVEL
+    K, L = args.steps, LEVEL
     B = args.batch if args.batch > 0 else max(1, 256 // world)
 
     ctx = hml.Context(CFG, MAX_LEVEL, ALPHA, device=local)
@@ -443,6 +467,8 @@ def main():
     n_ops = K * B * world
     us_per_op = ms_total * 1e3 / n_ops
     sampler.join(timeout=2)
+    if args.dump_outputs:  # `out` holds the last timed step's results until the profile below rewrites its first chunk
+        dump_outputs(args.dump_outputs, "hmult_out" if world == 1 else "hmult_out_rank%d" % rank, out, DUMP_BYTES // world, torch)
 
     # ---------------- end to end through the host-buffer C-ABI call (pinned host memory, H2D + D2H inside)
     Be = args.e2e_batch

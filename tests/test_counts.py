@@ -117,3 +117,23 @@ def test_bench_reference_arm_prints_exactly_one_json_line():
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
     r1 = subprocess.run(cmd, capture_output=True, text=True, timeout=600, env=dict(os.environ, RANK="1", WORLD_SIZE="2"))
     assert r1.returncode == 0 and r1.stdout.strip() == ""
+
+
+def test_bench_dump_outputs_and_steps(tmp_path):
+    """bench.py --dump-outputs samples the same positions of every row on every run, exactly and within its byte budget;
+    --steps below 1 is refused rather than rounded up"""
+    import subprocess
+    import sys
+    import numpy as np
+    import torch
+    import bench
+    out = torch.randint(0, 1 << 36, (3, 2, 5, 4096), dtype=torch.int64)
+    for name in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / "d"), name, out, 1 << 16, torch)
+    a, b = np.load(tmp_path / "d" / "a.npy"), np.load(tmp_path / "d" / "b.npy")
+    assert a.dtype == np.float64 and a.shape == (3, 2, 5, (1 << 16) // (8 * 30)) and a.nbytes <= 1 << 16
+    assert np.array_equal(a, b)
+    rows, got = out.reshape(30, -1).numpy(), a.reshape(30, -1)
+    assert all(np.isin(got[i], rows[i]).all() for i in range(30))
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 2 and "--steps" in r.stderr
