@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libhomulator_b200.so")
 CLI = os.path.join(HERE, "Homulator.run")
-CU = ["ntt.cu", "ntt_fused.cu", "ewe.cu", "bconv_umma.cu", "context.cu", "hostpath.cu", "shard.cu", "replay.cu", "cli.cu"]
+CU = ["ntt.cu", "ewe.cu", "bconv_umma.cu", "context.cu", "hostpath.cu", "shard.cu", "replay.cu", "cli.cu"]
 CPP = ["config.cpp", "params.cpp", "planner.cpp"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

@@ -533,15 +533,6 @@ k_bconv_umma(const ModConst *__restrict__ mc, LimbMap src_lm, LimbMap dst_lm, BC
   }
 }
 
-// HML_UMMA_CTAS = 1 | 2: CTAs per SM for 16-source conversions (tuning knob, see the kernel's NT parameter)
-static int umma_ctas_per_sm() {
-  static const int v = [] {
-    const char *e = getenv("HML_UMMA_CTAS");
-    return e && atoi(e) == 1 ? 1 : 2;
-  }();
-  return v;
-}
-
 template <int N16, bool FOLD, bool F64, int W, int NT>
 static void launch_umma_t(const ModConst *mc, const LimbMap &src_lm, const LimbMap &dst_lm, const BConvArgs &a, const BConvImage &im, cudaStream_t s) {
   const int tiles_per_batch = a.N / UMMA_TM, n_tiles = tiles_per_batch * a.n_batches;
@@ -586,8 +577,7 @@ static void launch_umma_multi_t(const ModConst *mc, const BConvJob *d_jobs, int 
 
 bool launch_bconv_umma_multi(const ModConst *mc, const BConvJob *d_jobs, const BConvImage *ims, const int *n_dst, int n_jobs, const BConvArgs &a,
                              cudaStream_t s) {
-  if (n_jobs < 2 || n_jobs > 8 || !d_jobs || a.N < 128 || a.N % 128 != 0 || a.step1 || a.fold || a.src_off || !bconv_umma_enabled() ||
-      umma_ctas_per_sm() != 2)
+  if (n_jobs < 2 || n_jobs > 8 || !d_jobs || a.N < 128 || a.N % 128 != 0 || a.step1 || a.fold || a.src_off || !bconv_umma_enabled())
     return false;
   int K = 0, NP = 0, ND = 0, waste3 = 0, waste4 = 0;
   for (int j = 0; j < n_jobs; ++j) {
@@ -605,15 +595,15 @@ bool launch_bconv_umma_multi(const ModConst *mc, const BConvJob *d_jobs, const B
 template <int N16, bool FOLD, bool F64>
 static void launch_umma_w(const ModConst *mc, const LimbMap &src_lm, const LimbMap &dst_lm, const BConvArgs &a, const BConvImage &im, cudaStream_t s) {
   // targets per epilogue warp; trips of 3 or 4, whichever leaves fewer masked slots
-  if (N16 == 1 && umma_ctas_per_sm() == 2) {
+  if constexpr (N16 == 1) {
     const int c = (a.n_dst + 1) / 2;
     if (((c + 2) / 3) * 3 < ((c + 3) / 4) * 4) launch_umma_t<1, FOLD, F64, 3, 256>(mc, src_lm, dst_lm, a, im, s);
     else launch_umma_t<1, FOLD, F64, 4, 256>(mc, src_lm, dst_lm, a, im, s);
-    return;
+  } else {
+    const int c = (a.n_dst + 3) / 4;
+    if (((c + 2) / 3) * 3 < ((c + 3) / 4) * 4) launch_umma_t<N16, FOLD, F64, 3, 512>(mc, src_lm, dst_lm, a, im, s);
+    else launch_umma_t<N16, FOLD, F64, 4, 512>(mc, src_lm, dst_lm, a, im, s);
   }
-  const int c = (a.n_dst + 3) / 4;
-  if (((c + 2) / 3) * 3 < ((c + 3) / 4) * 4) launch_umma_t<N16, FOLD, F64, 3, 512>(mc, src_lm, dst_lm, a, im, s);
-  else launch_umma_t<N16, FOLD, F64, 4, 512>(mc, src_lm, dst_lm, a, im, s);
 }
 
 template <int N16>

@@ -31,9 +31,6 @@ int fail(hml_ctx *ctx, int code, const std::string &msg) {
   return code;
 }
 
-// the transform tables as seen from stream s: the batch path's second lane has its own queue counters (ntt_fused.cu)
-static const NttTables &tabs_for(hml_ctx *ctx, cudaStream_t s) { return (ctx->s_lane && s == ctx->s_lane) ? ctx->tabs_lane : ctx->tabs; }
-
 namespace hml {
 void ws_enter(hml_ctx *ctx, cudaStream_t s) {
   if (ctx->have_last && ctx->last_stream != s) {
@@ -186,19 +183,10 @@ static int ctx_init_device(hml_ctx *ctx) {
   if ((rc = upload(ctx, mc, &ctx->mc))) return rc;
   ctx->tabs.fwd_rows = ctx->tw_fwd_rows; ctx->tabs.inv_rows = ctx->tw_inv_rows;
   ctx->tabs.fwd = ctx->tw_fwd; ctx->tabs.inv = ctx->tw_inv; ctx->tabs.mc = ctx->mc;
-  if (two_pass) {  // queue + dependency counters of the single-launch transform, one block per stream lane
-    const size_t words = ntt_fused_ctrl_words();
-    CU_TRY(ctx, cudaMalloc((void **)&ctx->ntt_ctrl, (2 * words + 8) * sizeof(unsigned)));
-    CU_TRY(ctx, cudaMemset(ctx->ntt_ctrl, 0, (2 * words + 8) * sizeof(unsigned)));
-    ctx->tabs.fused_ctrl = ctx->ntt_ctrl;
-    ctx->tabs.col_ctr = ctx->ntt_ctrl + 2 * words;
-    ctx->tabs_lane = ctx->tabs;
-    ctx->tabs_lane.fused_ctrl = ctx->ntt_ctrl + words;
-    ctx->tabs_lane.col_ctr = ctx->ntt_ctrl + 2 * words + 4;
-  } else {
-    ctx->tabs.fused_ctrl = nullptr;
-    ctx->tabs.col_ctr = nullptr;
-    ctx->tabs_lane = ctx->tabs;
+  if (two_pass) {
+    CU_TRY(ctx, cudaMalloc((void **)&ctx->col_ctr, 2 * sizeof(unsigned)));
+    CU_TRY(ctx, cudaMemset(ctx->col_ctr, 0, 2 * sizeof(unsigned)));
+    ctx->tabs.col_ctr = ctx->col_ctr;
   }
   return HML_OK;
 }
@@ -259,13 +247,10 @@ extern "C" void hml_ctx_destroy(hml_ctx *ctx) {
     for (auto *o : kv.second.d_off1) cudaFree(o);
     for (auto &u : kv.second.up) { cudaFree(u.d_mat); cudaFree(u.d_img); }
   }
-  cudaFree(ctx->tw_fwd); cudaFree(ctx->tw_inv); cudaFree(ctx->tw_fwd_rows); cudaFree(ctx->tw_inv_rows); cudaFree(ctx->mc); cudaFree(ctx->ws); cudaFree(ctx->stage); cudaFree(ctx->ntt_ctrl);
+  cudaFree(ctx->tw_fwd); cudaFree(ctx->tw_inv); cudaFree(ctx->tw_fwd_rows); cudaFree(ctx->tw_inv_rows); cudaFree(ctx->mc); cudaFree(ctx->ws); cudaFree(ctx->stage); cudaFree(ctx->col_ctr);
   if (ctx->s_in) cudaStreamDestroy(ctx->s_in);
   if (ctx->s_comp) cudaStreamDestroy(ctx->s_comp);
   if (ctx->s_out) cudaStreamDestroy(ctx->s_out);
-  if (ctx->s_lane) cudaStreamDestroy(ctx->s_lane);
-  if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
-  if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
   if (ctx->ev_ws) cudaEventDestroy(ctx->ev_ws);
   if (ctx->prof.start) cudaEventDestroy(ctx->prof.start);
   for (auto &m : ctx->prof.marks) cudaEventDestroy(m.second);
@@ -490,8 +475,8 @@ static int ntt_api(hml_ctx *ctx, bool inverse, const uint64_t *in, uint64_t *out
     l.n_batch = 1;
     l.in = (const u64 *)in + off * N; l.out = (u64 *)out + off * N;
     l.in_limb_stride = l.out_limb_stride = N; l.n_limbs = n; l.n_polys = 1; l.post_scale = nullptr;
-    if (inverse) launch_ntt_inverse(tabs_for(ctx, (cudaStream_t)stream), ctx->p.logN, lm, l, (cudaStream_t)stream);
-    else launch_ntt_forward(tabs_for(ctx, (cudaStream_t)stream), ctx->p.logN, lm, l, (cudaStream_t)stream);
+    if (inverse) launch_ntt_inverse(ctx->tabs, ctx->p.logN, lm, l, (cudaStream_t)stream);
+    else launch_ntt_forward(ctx->tabs, ctx->p.logN, lm, l, (cudaStream_t)stream);
     prof_mark(ctx, inverse ? HML_CLS_INTT : HML_CLS_NTT, (cudaStream_t)stream);
     ctx->exec.kernel_launches += ctx->p.logN <= NTT_SMALL_LOG ? 1 : 2;
   }
@@ -524,8 +509,8 @@ static int ntt_batch_api(hml_ctx *ctx, bool inverse, const uint64_t *in, uint64_
     l.in = (const u64 *)in + (size_t)b0 * n_limbs * N; l.out = (u64 *)out + (size_t)b0 * n_limbs * N;
     l.in_limb_stride = l.out_limb_stride = N; l.n_limbs = n_limbs; l.n_polys = 1; l.post_scale = nullptr;
     l.n_batch = std::min(per, n_batch - b0); l.in_batch_stride = l.out_batch_stride = (long long)n_limbs * N;
-    if (inverse) launch_ntt_inverse(tabs_for(ctx, (cudaStream_t)stream), ctx->p.logN, lm, l, (cudaStream_t)stream);
-    else launch_ntt_forward(tabs_for(ctx, (cudaStream_t)stream), ctx->p.logN, lm, l, (cudaStream_t)stream);
+    if (inverse) launch_ntt_inverse(ctx->tabs, ctx->p.logN, lm, l, (cudaStream_t)stream);
+    else launch_ntt_forward(ctx->tabs, ctx->p.logN, lm, l, (cudaStream_t)stream);
     prof_mark(ctx, inverse ? HML_CLS_INTT : HML_CLS_NTT, (cudaStream_t)stream);
     ctx->exec.kernel_launches += ctx->p.logN <= NTT_SMALL_LOG ? 1 : 2;
   }
@@ -622,19 +607,12 @@ size_t ks_ws_words(const Params &p, uint32_t L) {
 
 
 // K1..K4: ModUp (INTT + digit scaling, base conversion, NTT of the converted limbs).  Buffers: yb [nb][L] | ext [nb][beta][E].
-// HML_HPIP=0 keeps the inner product in its own kernel (k_inner) everywhere
-static bool hpip_enabled() {
-  static const bool v = [] { const char *e = getenv("HML_HPIP"); return !(e && atoi(e) == 0); }();
-  return v;
-}
 // The fusion pays for ONE ciphertext per launch (measured at the north-star shape: ModUp transform + inner product 112 -> 95 us,
 // hmult 245 -> 233 us, hrotate 249 -> 227 us): there the stand-alone inner product is latency-bound on the 150 MB key.  In a
 // 32-ciphertext chunk the key is read once per chunk and k_inner streams at the HBM rate, while the row pass is bound by the
-// FP64 pipe and the fused multiply-accumulates (+45 % FP64 work) land exactly there: 168 -> 178 us per hmult.  HML_HPIP=2 forces
-// the fusion for every batch size.
+// FP64 pipe and the fused multiply-accumulates (+45 % FP64 work) land exactly there: 168 -> 178 us per hmult.
 bool ks_uses_hpip(const hml_ctx *ctx, uint32_t L, uint32_t nb) {
-  static const int mode = [] { const char *e = getenv("HML_HPIP"); return e ? atoi(e) : 1; }();
-  return hpip_enabled() && ctx->p.logN > NTT_SMALL_LOG && ctx->p.beta(L) >= 2 && (nb == 1 || mode == 2);
+  return ctx->p.logN > NTT_SMALL_LOG && ctx->p.beta(L) >= 2 && nb == 1;
 }
 
 int ks_modup(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, u64 *yb, u64 *ext, cudaStream_t s, const NttMac *mac, const KsAuto *au) {
@@ -654,7 +632,7 @@ int ks_modup(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d,
       l.in_galois = (unsigned)(au->g & (2ull * N - 1)); l.in_ginv8 = gi & 255u;
       l.side_out = au->sigma_d; l.side_batch_stride = au->sigma_stride;
     }
-    launch_ntt_inverse(tabs_for(ctx, s), logN, lc->q_lm, l, s);
+    launch_ntt_inverse(ctx->tabs, logN, lc->q_lm, l, s);
     prof_mark(ctx, HML_CLS_INTT, s);
     ctx->exec.intt_limbs += (uint64_t)nb * L; ctx->exec.kernel_launches += npass;
   }
@@ -695,7 +673,7 @@ int ks_modup(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d,
       l.mac = *mac;
       ctx->exec.ewe_limbs += 2ull * nb * E * beta;
     }
-    launch_ntt_forward(tabs_for(ctx, s), logN, lc->ext_lm, l, s);
+    launch_ntt_forward(ctx->tabs, logN, lc->ext_lm, l, s);
     prof_mark(ctx, HML_CLS_NTT, s);
     ctx->exec.ntt_limbs += (uint64_t)nb * ((uint64_t)beta * E - L); ctx->exec.kernel_launches += npass;
   }
@@ -758,7 +736,7 @@ int ks_inner(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d,
     l.in = acc; l.out = acc; l.in_limb_stride = l.out_limb_stride = N; l.in_poly_stride = l.out_poly_stride = (long long)AL * N;
     l.n_limbs = A + (mu ? 1 : 0); l.n_polys = 2 * nb; l.post_scale = mu ? lc->moddown_scale_u : lc->moddown_scale;  // acc is [nb][2][AL][N]
     l.n_batch = 1;
-    launch_ntt_inverse(tabs_for(ctx, s), logN, mu ? lc->pu_lm : lc->p_lm, l, s);
+    launch_ntt_inverse(ctx->tabs, logN, mu ? lc->pu_lm : lc->p_lm, l, s);
     prof_mark(ctx, HML_CLS_INTT, s);
     ctx->exec.intt_limbs += 2ull * nb * l.n_limbs; ctx->exec.kernel_launches += npass;
   }
@@ -831,7 +809,7 @@ int ks_tail(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, u64 *acc, u6
       f.cst = lc->pinv; f.n_c = 2;
       f.z_galois = (unsigned)(add0_galois & (2ull * N - 1));
     }
-    launch_ntt_forward(tabs_for(ctx, s), logN, lc->q_lm, l, s);
+    launch_ntt_forward(ctx->tabs, logN, lc->q_lm, l, s);
     prof_mark(ctx, HML_CLS_NTT, s);
     ctx->exec.ntt_limbs += 2ull * nb * L; ctx->exec.kernel_launches += npass;
     if (fuse) ctx->exec.ewe_limbs += (uint64_t)nb * (2 * L + (add0.ptr ? L : 0) + (add1.ptr ? L : 0));
@@ -1036,7 +1014,7 @@ extern "C" int hml_keyswitch_shard_begin(hml_ctx *ctx, uint32_t L, uint32_t rank
     l.n_batch = 1;
     l.in = (const u64 *)d_own; l.out = (u64 *)gather1 + (size_t)rank * sp->gq * N;
     l.in_limb_stride = l.out_limb_stride = N; l.n_limbs = nq; l.n_polys = 1; l.post_scale = sp->scale1;
-    launch_ntt_inverse(tabs_for(ctx, (cudaStream_t)stream), ctx->p.logN, sp->q_lm, l, (cudaStream_t)stream);
+    launch_ntt_inverse(ctx->tabs, ctx->p.logN, sp->q_lm, l, (cudaStream_t)stream);
     prof_mark(ctx, HML_CLS_INTT, (cudaStream_t)stream);
     ctx->exec.intt_limbs += nq; ctx->exec.kernel_launches += ctx->p.logN <= NTT_SMALL_LOG ? 1 : 2;
   }
@@ -1066,7 +1044,7 @@ static int shard_mid_tail(hml_ctx *ctx, ShardPlan *sp, uint32_t rank, const u64 
       for (uint32_t k = 0; k < ne; ++k) m.key_pos[k] = (uint16_t)k;
       ctx->exec.ewe_limbs += 2ull * ne * beta;
     }
-    launch_ntt_forward(tabs_for(ctx, s), logN, sp->e_lm, l, s);
+    launch_ntt_forward(ctx->tabs, logN, sp->e_lm, l, s);
     prof_mark(ctx, HML_CLS_NTT, s);
     ctx->exec.ntt_limbs += (uint64_t)beta * ne - nq; ctx->exec.kernel_launches += npass;
   }
@@ -1086,7 +1064,7 @@ static int shard_mid_tail(hml_ctx *ctx, ShardPlan *sp, uint32_t rank, const u64 
     l.in = acc; l.in_limb_stride = N; l.in_poly_stride = (long long)ne * N;
     l.out = gather2 + (size_t)rank * 2 * sp->gp * N - (size_t)nq * N; l.out_limb_stride = N; l.out_poly_stride = (long long)sp->gp * N;
     l.n_limbs = np; l.n_polys = 2; l.post_scale = sp->scale2;
-    launch_ntt_inverse(tabs_for(ctx, s), logN, sp->p_lm, l, s);
+    launch_ntt_inverse(ctx->tabs, logN, sp->p_lm, l, s);
     prof_mark(ctx, HML_CLS_INTT, s);
     ctx->exec.intt_limbs += 2 * np; ctx->exec.kernel_launches += npass;
   }
@@ -1152,7 +1130,7 @@ static int shard_end_run(hml_ctx *ctx, ShardPlan *sp, const u64 *gather2, const 
       f.cst = sp->pinv; f.n_c = 2;
       ctx->exec.ewe_limbs += 2 * nq;
     }
-    launch_ntt_forward(tabs_for(ctx, s), logN, sp->q_lm, l, s);
+    launch_ntt_forward(ctx->tabs, logN, sp->q_lm, l, s);
     prof_mark(ctx, HML_CLS_NTT, s);
     ctx->exec.ntt_limbs += 2 * nq; ctx->exec.kernel_launches += npass;
   }
@@ -1473,7 +1451,7 @@ int rescale_run(hml_ctx *ctx, uint32_t L, const u64 *in, long long in_poly_strid
     l.n_batch = 1;
     l.in = in + (size_t)(L - 1) * N; l.out = rb; l.in_limb_stride = l.out_limb_stride = N;
     l.in_poly_stride = in_poly_stride; l.out_poly_stride = N; l.n_limbs = 1; l.n_polys = n_polys;
-    launch_ntt_inverse(tabs_for(ctx, s), logN, lm, l, s);
+    launch_ntt_inverse(ctx->tabs, logN, lm, l, s);
     prof_mark(ctx, HML_CLS_INTT, s);
     ctx->exec.intt_limbs += n_polys; ctx->exec.kernel_launches += npass;
   }
@@ -1489,7 +1467,7 @@ int rescale_run(hml_ctx *ctx, uint32_t L, const u64 *in, long long in_poly_strid
       f.x = in; f.x_c_stride = in_poly_stride; f.x_b_stride = 0; f.z = nullptr; f.z_mask = 0;
       f.dst = out; f.dst_c_stride = out_poly_stride; f.dst_b_stride = 0; f.cst = lc->qlinv; f.n_c = (int)n_polys;
     }
-    launch_ntt_forward(tabs_for(ctx, s), logN, lc->q_lm, l, s);
+    launch_ntt_forward(ctx->tabs, logN, lc->q_lm, l, s);
     prof_mark(ctx, HML_CLS_NTT, s);
     ctx->exec.ntt_limbs += (uint64_t)n_polys * (L - 1); ctx->exec.kernel_launches += npass;
   }
@@ -1542,7 +1520,7 @@ extern "C" int hml_rescale_shard_begin(hml_ctx *ctx, uint32_t L, uint32_t rank, 
   l.in = (const u64 *)x_own; l.in_limb_stride = N; l.in_poly_stride = (long long)nq * N;
   l.out = (u64 *)r_own - (size_t)(nq - 1) * N; l.out_limb_stride = N; l.out_poly_stride = N;  // position nq-1 lands on r_own
   l.n_limbs = 1; l.n_polys = 2;
-  launch_ntt_inverse(tabs_for(ctx, (cudaStream_t)stream), ctx->p.logN, lm, l, (cudaStream_t)stream);
+  launch_ntt_inverse(ctx->tabs, ctx->p.logN, lm, l, (cudaStream_t)stream);
   prof_mark(ctx, HML_CLS_INTT, (cudaStream_t)stream);
   ctx->exec.intt_limbs += 2; ctx->exec.kernel_launches += ctx->p.logN <= NTT_SMALL_LOG ? 1 : 2;
   return check_launch(ctx, "rescale shard begin");
@@ -1580,7 +1558,7 @@ extern "C" int hml_rescale_shard_end(hml_ctx *ctx, uint32_t L, uint32_t rank, ui
       f.x = (const u64 *)x_own; f.x_c_stride = (long long)nq * N; f.x_b_stride = 0; f.z = nullptr; f.z_mask = 0;
       f.dst = (u64 *)out_own; f.dst_c_stride = (long long)nk * N; f.dst_b_stride = 0; f.cst = sp->qlinv_own; f.n_c = 2;
     }
-    launch_ntt_forward(tabs_for(ctx, s), logN, lm, l, s);
+    launch_ntt_forward(ctx->tabs, logN, lm, l, s);
     prof_mark(ctx, HML_CLS_NTT, s);
     ctx->exec.ntt_limbs += 2ull * nk; ctx->exec.kernel_launches += npass;
   }
@@ -1669,7 +1647,7 @@ int hmult_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct_a, const u64 
     f.z = d0; f.z_c_stride = (long long)(d1 - d0); f.z_b_stride = (long long)PL; f.z_mask = 3;
     f.dst = ct_out; f.dst_c_stride = (long long)(L - 1) * N; f.dst_b_stride = 2ll * (L - 1) * N;
     f.cst = lc->pinv; f.cst2 = lc->qlinv; f.n_c = 2; f.x_packed = ks_uses_hpip(ctx, L, nb) ? 0 : 1; f.z_packed = 1;
-    launch_ntt_forward(tabs_for(ctx, s), logN, lc->q_lm, l, s);
+    launch_ntt_forward(ctx->tabs, logN, lc->q_lm, l, s);
     prof_mark(ctx, HML_CLS_NTT, s);
     ctx->exec.ntt_limbs += 2ull * nb * (L - 1); ctx->exec.kernel_launches += 2;
     ctx->exec.ewe_limbs += 2ull * nb * 4 * (L - 1);
@@ -1695,9 +1673,8 @@ int hrot_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct, const u64 *rk
                     u64 *ws, cudaStream_t s) {
   const size_t N = ctx->p.N, PL = N * L;
   u64 *sb = ws, *rest = sb + 2 * nb * PL;  // sb [nb][2][L][N]
-  static const bool fuse_auto = [] { const char *e = getenv("HML_AUTO_FUSE"); return !(e && atoi(e) == 0); }();
   const bool in_place = ct_out < ct + 2 * nb * PL && ct < ct_out + 2 * nb * PL;  // the epilogue would gather c0 rows it has overwritten
-  if (fuse_auto && !in_place && ctx->p.logN > NTT_SMALL_LOG && (g & (2 * N - 1)) != 1) {
+  if (!in_place && ctx->p.logN > NTT_SMALL_LOG && (g & (2 * N - 1)) != 1) {
     // two-pass rings: no kernel for the automorphism (reference :1302-1319).  In evaluation order sigma_g maps every 256-slot
     // row onto one source row (ntt_core.cuh RowSigma), so the ModUp INTT permutes c1 while it loads it (and leaves sigma(c1)
     // in sb for the inner product's own-digit term) and the ModDown epilogue gathers sigma(c0) from the raw c0
@@ -1748,10 +1725,9 @@ int hrot_hoisted_run(hml_ctx *ctx, uint32_t L, const u64 *ct, uint32_t n_rot, co
   u64 *sb = ws, *yb = sb + 2 * PL, *ext = yb + PL, *acc = ext + (size_t)beta * E * N, *vb = acc + 2 * (size_t)E * N;
   const BatchPtr c1{ct + PL, 0};
   if ((rc = ks_modup(ctx, lc, L, 1, c1, yb, ext, s, nullptr))) return rc;
-  static const bool fuse_auto = [] { const char *e = getenv("HML_AUTO_FUSE"); return !(e && atoi(e) == 0); }();
   for (uint32_t r = 0; r < n_rot; ++r) {
     // sigma_r(c0), the addend of the ModDown epilogue: gathered by the epilogue itself on two-pass rings (hrot_run), else a kernel
-    const bool gather = fuse_auto && p.logN > NTT_SMALL_LOG && (galois[r] & (2 * N - 1)) != 1;
+    const bool gather = p.logN > NTT_SMALL_LOG && (galois[r] & (2 * N - 1)) != 1;
     if (!gather) {
       launch_automorph(p.logN, L, ct, sb, galois[r], s);
       prof_mark(ctx, HML_CLS_AUTO, s);
@@ -1834,46 +1810,15 @@ extern "C" int hml_padd(hml_ctx *ctx, uint32_t L, const uint64_t *ct, const uint
 }
 
 // ------------------------------------------------------------------------------------------------ batched
-// Optionally (HML_BATCH_LANES=2) chunks alternate between two lanes — the caller's stream + an internal one, each with its
-// own workspace half, fork / join with events — so that the HBM-bound element-wise kernels of one chunk may overlap the
-// FP64-bound transforms of the other.  Measured on B200: two lanes of 16 = one lane of 32 (209.9 vs 209.7 us per hmult;
-// every kernel already fills the machine, only launch tails overlap), so one lane is the default.
-static uint32_t batch_lanes() {
-  static const uint32_t v = [] {
-    const char *e = getenv("HML_BATCH_LANES");  // tuning knob: 1 or 2
-    return (uint32_t)(e && atoi(e) == 2 ? 2 : 1);
-  }();
-  return v;
-}
-
+// chunks of at most HML_BATCH_CHUNK ciphertexts, one after the other on the caller's stream, sharing one workspace
 template <class RunChunk>
-static int run_batch_lanes(hml_ctx *ctx, uint32_t n, size_t ws_per_ct, cudaStream_t user, RunChunk run) {
-  const uint32_t lanes = n > 1 ? batch_lanes() : 1;
-  // chunks no larger than HML_BATCH_CHUNK, and at least `lanes` of them when the batch allows it
-  uint32_t chunk = std::min<uint32_t>(HML_BATCH_CHUNK, (n + lanes - 1) / lanes);
-  int rc = ensure_ws(ctx, (size_t)lanes * chunk * ws_per_ct);
+static int run_batch_chunks(hml_ctx *ctx, uint32_t n, size_t ws_per_ct, cudaStream_t user, RunChunk run) {
+  const uint32_t chunk = std::min<uint32_t>(HML_BATCH_CHUNK, n);
+  int rc = ensure_ws(ctx, (size_t)chunk * ws_per_ct);
   if (rc) return rc;
   ws_enter(ctx, user);
-  const bool two = lanes == 2 && n > chunk;
-  if (two) {
-    if (!ctx->s_lane) {
-      CU_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_lane, cudaStreamNonBlocking));
-      CU_TRY(ctx, cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
-      CU_TRY(ctx, cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
-    }
-    CU_TRY(ctx, cudaEventRecord(ctx->ev_fork, user));
-    CU_TRY(ctx, cudaStreamWaitEvent(ctx->s_lane, ctx->ev_fork, 0));
-  }
-  uint32_t k = 0;
-  for (uint32_t i = 0; i < n; i += chunk, ++k) {
-    const uint32_t nb = std::min(chunk, n - i);
-    const bool side = two && (k & 1);
-    if ((rc = run(i, nb, ctx->ws + (side ? (size_t)chunk * ws_per_ct : 0), side ? ctx->s_lane : user))) break;
-  }
-  if (two) {
-    cudaEventRecord(ctx->ev_join, ctx->s_lane);
-    cudaStreamWaitEvent(user, ctx->ev_join, 0);
-  }
+  for (uint32_t i = 0; i < n; i += chunk)
+    if ((rc = run(i, std::min(chunk, n - i), ctx->ws, user))) break;
   return rc;
 }
 
@@ -1885,7 +1830,7 @@ extern "C" int hml_hmult_batch(hml_ctx *ctx, uint32_t L, uint32_t n, const uint6
   if (!ct_a || !ct_b || !evk || !ct_out) return fail(ctx, HML_ERR_INVALID, "null buffer");
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   const size_t N = ctx->p.N, in_w = 2 * N * L, out_w = 2 * N * (L - 1);
-  return run_batch_lanes(ctx, n, hmult_ws_words(ctx->p, L, 1), (cudaStream_t)stream, [&](uint32_t i, uint32_t nb, u64 *ws, cudaStream_t s) {
+  return run_batch_chunks(ctx, n, hmult_ws_words(ctx->p, L, 1), (cudaStream_t)stream, [&](uint32_t i, uint32_t nb, u64 *ws, cudaStream_t s) {
     return hmult_run(ctx, L, nb, (const u64 *)ct_a + i * in_w, (const u64 *)ct_b + i * in_w, (const u64 *)evk, evk_q_limbs,
                      (u64 *)ct_out + i * out_w, ws, s);
   });
@@ -1900,7 +1845,7 @@ extern "C" int hml_hrotate_batch(hml_ctx *ctx, uint32_t L, uint32_t n, const uin
   if (!(galois_elt & 1)) return fail(ctx, HML_ERR_INVALID, "galois element must be odd");
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   const size_t w = 2 * (size_t)ctx->p.N * L;
-  return run_batch_lanes(ctx, n, hrot_ws_words(ctx->p, L, 1), (cudaStream_t)stream, [&](uint32_t i, uint32_t nb, u64 *ws, cudaStream_t s) {
+  return run_batch_chunks(ctx, n, hrot_ws_words(ctx->p, L, 1), (cudaStream_t)stream, [&](uint32_t i, uint32_t nb, u64 *ws, cudaStream_t s) {
     return hrot_run(ctx, L, nb, (const u64 *)ct + i * w, (const u64 *)rotkey, evk_q_limbs, galois_elt, (u64 *)ct_out + i * w, ws, s);
   });
 }

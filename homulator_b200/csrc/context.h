@@ -104,8 +104,8 @@ struct hml_ctx {
 
   double *tw_fwd = nullptr, *tw_inv = nullptr, *tw_fwd_rows = nullptr, *tw_inv_rows = nullptr;
   hml::ModConst *mc = nullptr;
-  hml::NttTables tabs{}, tabs_lane{};   // tabs_lane: the same tables with the second stream lane's queue counters
-  unsigned *ntt_ctrl = nullptr;         // 2 x ntt_fused_ctrl_words()
+  hml::NttTables tabs{};
+  unsigned *col_ctr = nullptr;  // tabs.col_ctr: the column passes' tile queue (two-pass rings)
 
   std::map<uint32_t, hml::LevelConsts> levels;
   std::map<std::vector<uint32_t>, hml::DevBConv> bconv_cache;
@@ -118,10 +118,6 @@ struct hml_ctx {
 
   // host-buffer API: staging buffers + streams
   cudaStream_t s_in = nullptr, s_comp = nullptr, s_out = nullptr;
-  // batched ops: a second lane (stream + workspace half) so that the HBM-bound kernels of one chunk overlap the
-  // FP64-bound kernels of the other
-  cudaStream_t s_lane = nullptr;
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   hml::u64 *stage = nullptr;
   size_t stage_words = 0;
 

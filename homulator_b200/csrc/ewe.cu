@@ -493,16 +493,11 @@ void launch_bconv(const ModConst *mc, const LimbMap &src_lm, const LimbMap &dst_
     return;
   }
   const int n_src_pad = bconv_pad_src(a.n_src), n_dst_pad = bconv_pad_dst(a.n_dst);
-  static const int tm_env = [] {
-    const char *e = getenv("HML_BCONV_TM");  // tuning knob: coefficients per CTA (<= 16 sources); 0 = adaptive
-    const int v = e ? atoi(e) : 0;
-    return (v == 64 || v == 128 || v == 256) ? v : 0;
-  }();
   // big tiles amortise the per-CTA set-up (matrix fragments, moduli); small launches need more, shorter CTAs to fill 148 SMs
   int tm = 64;
   if (n_src_pad <= 16) {
-    tm = tm_env ? tm_env : 256;
-    while (!tm_env && tm > 64 && (long long)(a.N / tm) * a.n_batches < 1480) tm >>= 1;
+    tm = 256;
+    while (tm > 64 && (long long)(a.N / tm) * a.n_batches < 1480) tm >>= 1;
   }
   while (tm > a.N) tm >>= 1;  // tiny rings (tests): N >= 16
   switch (n_src_pad <= 16 ? n_src_pad / 4 : 0) {

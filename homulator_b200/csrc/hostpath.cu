@@ -7,7 +7,6 @@
 // streams (copy-in, compute, copy-out) and two staging slots, so the H2D of chunk i+1 and the D2H of chunk i-1 overlap the
 // kernels of chunk i, and every chunk runs through the BATCHED schedule (one launch per stage for the whole chunk).
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 
 #include "launch.h"
@@ -17,16 +16,8 @@ using namespace hml;
 
 // Ciphertexts per pipeline step.  The path is PCIe-bound (73 MB in and 36 MB out per hmult in the uint64 layout against
 // ~0.2 ms of kernels), so what a larger chunk buys in kernel efficiency is invisible while the pipeline's tail — the last
-// chunk's kernels and copy-out, which nothing overlaps — grows with it.  HML_HOST_CHUNK overrides (1..64).
-static uint32_t host_chunk() {
-  static const uint32_t v = [] {
-    const char *e = getenv("HML_HOST_CHUNK");
-    const int n = e ? atoi(e) : 2;
-    return (uint32_t)std::min(std::max(n, 1), 64);
-  }();
-  return v;
-}
-#define HOST_CHUNK host_chunk()
+// chunk's kernels and copy-out, which nothing overlaps — grows with it.
+constexpr uint32_t HOST_CHUNK = 2;
 
 // packed [n_limbs][5N] <-> words [n_limbs][N]; two coefficients per thread
 __global__ void __launch_bounds__(256) k_unpack(const unsigned char *__restrict__ in, u64 *__restrict__ out, size_t N) {

@@ -1,7 +1,6 @@
 // See ntt.cuh for the algorithm.  sm_100a only.
 #include "ntt_core.cuh"
 
-#include <cstdlib>
 #include <cstring>
 #include <type_traits>
 
@@ -776,27 +775,11 @@ static void allow_smem(KERNEL k, int bytes) {
 
 // items of a row CTA: short CTAs keep the tail of the launch small (a CTA is dispatched whenever a slot frees up, so the
 // launch ends about one CTA-time after the ideal), long CTAs amortise the 32 KB twiddle blob
-static int row_items_target() {
-  static const int v = [] {
-    const char *e = getenv("HML_ROW_ITEMS");  // tuning knob
-    const int n = e ? atoi(e) : 8;
-    return n < 1 ? 1 : n;
-  }();
-  return v;
-}
+constexpr int ROW_ITEMS = 8;
 static int row_split(int n_items, int ctas_xy) {
-  const int tgt = row_items_target();
-  int z = (n_items + tgt - 1) / tgt;
+  int z = (n_items + ROW_ITEMS - 1) / ROW_ITEMS;
   while (z > 1 && (long long)ctas_xy * z > 64ll * sm_count()) --z;
   return z < 1 ? 1 : z;
-}
-
-static int col_dynamic_env() {
-  static const int v = [] {
-    const char *e = getenv("HML_COL_DYN");  // 0: static split of the column-pass tiles over the persistent CTAs (round-1 schedule)
-    return e ? atoi(e) : 1;
-  }();
-  return v;
 }
 
 template <int LOGR1, int NT>
@@ -814,7 +797,7 @@ static void launch_cols_t(bool inverse, const NttTables &t, int logN, const Limb
   }
   // the queue enumerates the members of the launch without the skipped ones: the limbs that skip a poly must come first
   ColQueue qu{t.col_ctr, 0, 0};
-  bool dyn = t.col_ctr != nullptr && col_dynamic_env();
+  bool dyn = t.col_ctr != nullptr;
   for (int i = 0; i < l.n_limbs; ++i) {
     const bool sk = lm.skip[i] < l.n_polys;
     if (sk && i != qu.n_skip) dyn = false;
@@ -839,20 +822,11 @@ static void launch_cols_t(bool inverse, const NttTables &t, int logN, const Limb
   else launch_pdl(ntt_fwd_cols<LOGR1, NT, false, false>, grid, NT, 2 * K::STAGE_BYTES, s, t, logN, lm, l, total, qu);
 }
 
-static int col_threads_env() {
-  static const int v = [] {
-    const char *e = getenv("HML_COL_NT");  // tuning knob: force 128 or 256 threads per column-pass CTA (default: by launch size)
-    const int n = e ? atoi(e) : 0;
-    return n == 128 || n == 256 ? n : 0;
-  }();
-  return v;
-}
-
 static void launch_cols(bool inverse, const NttTables &t, int logN, const LimbMap &lm, const NttLaunch &l, cudaStream_t s) {
   // one ciphertext's worth of limbs is only a few 32 KB tiles per resident CTA: 16 KB tiles (128 threads, six CTAs per SM) fill
   // the machine more evenly there (measured: 55.9 vs 60.1 us for the 115-limb ModUp launch); big batches prefer 32 KB tiles
   const long long tiles32 = (long long)l.n_limbs * l.n_polys * l.n_batch << (logN - 12);
-  const bool big = col_threads_env() ? col_threads_env() == 256 : tiles32 >= 6ll * 3 * sm_count();
+  const bool big = tiles32 >= 6ll * 3 * sm_count();
   switch (logN - NTT_ROW_LOG) {
     case 5: big ? launch_cols_t<5, 256>(inverse, t, logN, lm, l, s) : launch_cols_t<5, 128>(inverse, t, logN, lm, l, s); break;
     case 6: big ? launch_cols_t<6, 256>(inverse, t, logN, lm, l, s) : launch_cols_t<6, 128>(inverse, t, logN, lm, l, s); break;
@@ -872,7 +846,7 @@ static void launch_rows(bool inverse, const NttTables &t, int logN, const LimbMa
   }
   const int tiles = 1 << (logN - NTT_ROW_LOG - 4);
   if (!inverse && l.mac.evk) {  // the grid splits the ciphertexts; every CTA walks all digits of its (ciphertext, limb, tile)
-    const int per = std::max(1, row_items_target() / std::max(1, l.n_polys));
+    const int per = std::max(1, ROW_ITEMS / std::max(1, l.n_polys));
     int z = (l.n_batch + per - 1) / per;
     while (z > 1 && (long long)tiles * l.n_limbs * z > 64ll * sm_count()) --z;
     if (l.mac.evk_packed) launch_pdl(ntt_rows<false, 3>, dim3(tiles * std::max(1, z), l.n_limbs), NTT_THREADS, ROW_SMEM_BYTES, s, t, logN, lm, l);
@@ -890,7 +864,6 @@ void launch_ntt_forward(const NttTables &t, int logN, const LimbMap &lm, const N
     launch_pdl(ntt_small, dim3(1, l.n_limbs * l.n_polys * l.n_batch), 256, sizeof(double) << logN, s, t, logN, lm, l, 0);
     return;
   }
-  if (!l.mac.evk && launch_ntt_fused(false, t, logN, lm, l, t.fused_ctrl, s)) return;
   launch_cols(false, t, logN, lm, l, s);
   launch_rows(false, t, logN, lm, l, s);
 }
@@ -900,7 +873,6 @@ void launch_ntt_inverse(const NttTables &t, int logN, const LimbMap &lm, const N
     launch_pdl(ntt_small, dim3(1, l.n_limbs * l.n_polys * l.n_batch), 256, sizeof(double) << logN, s, t, logN, lm, l, 1);
     return;
   }
-  if (launch_ntt_fused(true, t, logN, lm, l, t.fused_ctrl, s)) return;
   launch_rows(true, t, logN, lm, l, s);
   launch_cols(true, t, logN, lm, l, s);
 }

@@ -42,10 +42,8 @@ struct NttTables {
   const double *fwd, *inv;            // [n_mod][N]
   const double *fwd_rows, *inv_rows;  // [n_mod][N / 4096][4096]
   const ModConst *mc;                 // [n_mod]
-  // queue and dependency counters of the single-launch transform (ntt_fused.cu), ntt_fused_ctrl_words() zero-initialised words;
-  // null: two-kernel transforms.  Launches that may run CONCURRENTLY need distinct blocks.
-  unsigned *fused_ctrl;
-  // tile queue of the column passes (ntt.cu, ColQueue): two zero-initialised words, same concurrency rule; null: static split
+  // tile queue of the column passes (ntt.cu, ColQueue): two zero-initialised words; null: static split.  Launches that may run
+  // CONCURRENTLY need distinct counters.
   unsigned *col_ctr;
 };
 
@@ -126,11 +124,6 @@ struct NttLaunch {
   int out_f64;                // forward only, two-pass rings, no fused epilogue: leave the raw lazy sums (|v| < 10 q) as doubles
                               // in `out` instead of canonical words (consumer: InnerArgs::ext_f64)
 };
-
-// single-launch transform (ntt_fused.cu); returns false when the shape is outside it (the caller runs the two-kernel path)
-bool launch_ntt_fused(bool inverse, const NttTables &t, int logN, const LimbMap &lm, const NttLaunch &l, unsigned *ctrl, cudaStream_t s);
-size_t ntt_fused_ctrl_words();
-int ntt_fused_enabled();
 
 void launch_ntt_forward(const NttTables &t, int logN, const LimbMap &lm, const NttLaunch &l, cudaStream_t s);
 void launch_ntt_inverse(const NttTables &t, int logN, const LimbMap &lm, const NttLaunch &l, cudaStream_t s);

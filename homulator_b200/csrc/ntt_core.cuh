@@ -1,5 +1,5 @@
-// Device-side building blocks shared by the two-kernel transforms (ntt.cu) and the single-launch transform (ntt_fused.cu):
-// asynchronous copies, the 16-point butterfly network and the row pass's swizzled shared-memory addressing.
+// Device-side building blocks of the two-kernel transforms (ntt.cu): asynchronous copies, the 16-point butterfly network and
+// the row pass's swizzled shared-memory addressing.
 #pragma once
 #include "ntt.cuh"
 #include "launch.h"

@@ -1,5 +1,5 @@
 """Transform microbenchmark: microseconds per launch of hml_ntt / hml_intt at several limb counts (one ciphertext-sized
-launch each) and per limb on the batched ModUp shape (32 x 115 limbs).  Run once per setting of HML_NTT_FUSED / HML_COL_NT."""
+launch each) and per limb on the batched ModUp shape (32 x 115 limbs)."""
 import os, sys, torch
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 import homulator_b200 as hml
@@ -29,4 +29,4 @@ row = {"fwd_batched_us_per_limb": t(batched(False)) / (115 * 32), "inv_batched_u
 for n in (2, 7, 16, 35, 70, 115):
     row["fwd_%d" % n] = t(single(n, False), 20)
     row["inv_%d" % n] = t(single(n, True), 20)
-print("NTT_FUSED=%s COL_NT=%s " % (os.environ.get("HML_NTT_FUSED", "1"), os.environ.get("HML_COL_NT", "256")) + " ".join("%s=%.3f" % kv for kv in row.items()))
+print(" ".join("%s=%.3f" % kv for kv in row.items()))

@@ -1,5 +1,5 @@
 """Profiling driver for the forward transform on the launch shape bench.py's roofline times (32 ciphertexts x 115 limbs):
-    [HML_NTT_FUSED=1] python profiles/prof_ntt.py [n_warm] [n_prof]"""
+    python profiles/prof_ntt.py [n_warm] [n_prof]"""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)

@@ -1,6 +1,7 @@
-"""Child process of tests/test_gpu_ops.py::test_alternative_kernel_paths: the library reads its tuning switches once per process
-(HML_NTT_FUSED, HML_HPIP, HML_BCONV_UMMA, HML_COL_NT ...), so every alternative code path is proven in a process of its own:
-hmult / hrotate / keyswitch / rescale / batched ops against the oracle on a two-pass ring."""
+"""Child process of tests/test_gpu_ops.py::test_alternative_kernel_paths: the library reads its switches once per process
+(HML_BCONV_UMMA, HML_PDL, HML_BATCH_CHUNK), so every setting is proven in a process of its own: hmult / hrotate / keyswitch /
+rescale / batched ops against the oracle on a two-pass ring, and batched transforms small enough for the 128-thread column
+pass and large enough for the 256-thread one."""
 import os
 import sys
 
@@ -37,12 +38,15 @@ def main():
         assert np.array_equal(to_host(got[0]), want_m) and np.array_equal(to_host(got[1]), o.hmult(L, b, b, evk, L))
         rot = ctx.hrotate_batch(L, A3, K, 25)
         assert np.array_equal(to_host(rot[2]), want_r)
-        x = ctx.uniform(list(range(L)), 9, lead=(3,))
         idx = list(range(L))
-        fwd = ctx.ntt_batch(x, idx)
-        assert torch.equal(ctx.ntt_batch(fwd, idx, inverse=True), x)
-        for i in range(L):
-            assert np.array_equal(to_host(fwd[1, i]), o.ntt(i, to_host(x[1, i])))
+        # 3 x L limbs: 128-thread column CTAs.  256 x L limbs is at least 18 32 KB tiles per SM (3584 tiles at N = 8192,
+        # 5120 at N = 16384): 256-thread column CTAs
+        for lead, seed, j in (((3,), 9, 1), ((256,), 10, 200)):
+            x = ctx.uniform(idx, seed, lead=lead)
+            fwd = ctx.ntt_batch(x, idx)
+            assert torch.equal(ctx.ntt_batch(fwd, idx, inverse=True), x)
+            for i in range(L):
+                assert np.array_equal(to_host(fwd[j, i]), o.ntt(i, to_host(x[j, i])))
     print("ENV_PATHS_OK")
 
 

@@ -307,9 +307,9 @@ def test_parameter_sets_B_C_two_pass_rings(N, ML, A, L):
     Oracle.set_threads(1)
 
 
-def test_batch_lanes_and_small_chunks_in_a_subprocess():
-    """HML_BATCH_CHUNK / HML_BATCH_LANES are read once per process: run a 7-ciphertext batch with chunks of 2 on two lanes
-    (two streams, two workspace halves) in a child process and compare with single calls."""
+def test_small_chunks_in_a_subprocess():
+    """HML_BATCH_CHUNK is read once per process: run a 7-ciphertext batch with chunks of 2 in a child process and compare
+    with single calls."""
     import os
     import subprocess
     import sys
@@ -328,15 +328,15 @@ def test_batch_lanes_and_small_chunks_in_a_subprocess():
         "torch.cuda.synchronize()\n"
         "assert torch.equal(got, torch.stack([ctx.hmult(L, a[i], b[i], evk) for i in range(n)]))\n"
         "assert torch.equal(rot, torch.stack([ctx.hrotate(L, a[i], evk, 5) for i in range(n)]))\n"
-        "print('lanes ok')\n" % root)
-    env = dict(os.environ, HML_BATCH_CHUNK="2", HML_BATCH_LANES="2")
+        "print('chunks ok')\n" % root)
+    env = dict(os.environ, HML_BATCH_CHUNK="2")
     r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "lanes ok" in r.stdout, r.stdout + r.stderr
+    assert r.returncode == 0 and "chunks ok" in r.stdout, r.stdout + r.stderr
 
 
-@pytest.mark.parametrize("n", [1, 8, 35])
+@pytest.mark.parametrize("n", [1, 8, 35, 70])
 def test_batch_chunking_small(n):
-    """hml_*_batch runs up to 32 ciphertexts per launch: cover a partial chunk and a full + partial chunk."""
+    """hml_*_batch runs up to 64 ciphertexts per launch: cover partial chunks and a full + partial chunk."""
     N, ML, A, L = 2048, 7, 3, 7
     ctx, o = hml.Context(N=N, max_level=ML, alpha=A), Oracle(N, 36, ML, A)
     (a, b), evk = make_case(o, L, L, 1200)
@@ -491,14 +491,12 @@ def test_hrotate_in_place_and_identity(north_star):
     assert np.array_equal(to_host(ctx.hrotate(L, to_dev(a), K, 1)), o.hrotate(L, a, evk, L, 1))
 
 
-@pytest.mark.parametrize("env", [{"HML_NTT_FUSED": "1"}, {"HML_HPIP": "0"}, {"HML_HPIP": "2"}, {"HML_BCONV_UMMA": "0"},
-                                 {"HML_COL_NT": "256", "HML_PDL": "0"}, {"HML_NTT_FUSED": "1", "HML_NTT_G": "1", "HML_NTT_LAG": "1"},
-                                 {"HML_COL_DYN": "0", "HML_AUTO_FUSE": "0"}, {"HML_COL_NT": "128"}, {"HML_BATCH_CHUNK": "2"}],
+@pytest.mark.parametrize("env", [{"HML_BCONV_UMMA": "0"}, {"HML_PDL": "0"}, {"HML_BATCH_CHUNK": "2"}],
                          ids=lambda e: ",".join("%s=%s" % kv for kv in e.items()))
 def test_alternative_kernel_paths(env):
-    """Every kernel path behind a process-wide switch — the single-launch transform (ntt_fused.cu), the inner product fused
-    into the ModUp transform for every batch size / not at all, the FP64 tensor-core conversion, programmatic dependent launch
-    off — is bit-exact against the oracle too (tests/sp_env_paths.py, one child process per setting)."""
+    """Every setting of a process-wide switch — the FP64 tensor-core conversion everywhere, programmatic dependent launch
+    off, batches in chunks of two — is bit-exact against the oracle too (tests/sp_env_paths.py, one child process per
+    setting)."""
     import os
     import subprocess
     import sys
