@@ -69,6 +69,7 @@ EXPORTS = [
     "hml_shard_connect_local", "hml_shard_prepare", "hml_shard_check", "hml_shard_own_limbs", "hml_keyswitch_sharded",
     "hml_hrotate_sharded", "hml_hmult_sharded", "hml_rescale_sharded", "hml_ew_sharded", "hml_group_op", "hml_hrotate_hoisted",
     "hml_replay_create", "hml_replay_bind", "hml_replay_run", "hml_replay_slot", "hml_replay_slot_level", "hml_replay_destroy",
+    "hml_shard_create_ex", "hml_hrotate_hoisted_sharded", "hml_group_hrotate_hoisted",
 ]
 
 
@@ -147,6 +148,7 @@ def load_library():
     L.hml_ipc_close.argtypes = [vp, vp]
     L.hml_shard_status.argtypes = [vp, vp, u32, vp]
     L.hml_shard_create.argtypes = [vp, u32, u32, u32, C.POINTER(vp)]
+    L.hml_shard_create_ex.argtypes = [vp, u32, u32, u32, u32, C.POINTER(vp)]
     L.hml_shard_destroy.argtypes = [vp]
     L.hml_shard_handles.argtypes = [vp, C.c_char_p]
     L.hml_shard_connect_ipc.argtypes = [vp, C.c_char_p]
@@ -162,6 +164,9 @@ def load_library():
     L.hml_group_op.argtypes = [C.POINTER(vp), u32, i32, u32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), u64,
                                C.POINTER(vp)]
     L.hml_hrotate_hoisted.argtypes = [vp, u32, vp, u32, C.POINTER(vp), u32, C.POINTER(u64), C.POINTER(vp), vp]
+    L.hml_hrotate_hoisted_sharded.argtypes = [vp, u32, vp, u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(vp), vp]
+    L.hml_group_hrotate_hoisted.argtypes = [C.POINTER(vp), u32, u32, C.POINTER(vp), u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(vp),
+                                            C.POINTER(vp)]
     L.hml_replay_create.argtypes = [vp, vp, u32, C.POINTER(_TraceOp), u32, u32, C.POINTER(vp)]
     L.hml_replay_bind.argtypes = [vp, vp, C.POINTER(vp), u32, C.POINTER(u32), C.POINTER(vp), u32, vp, u32]
     L.hml_replay_run.argtypes = [vp, vp]
@@ -539,17 +544,18 @@ class Context:
 class Shard:
     """One rank's view of a limb-shard group (hml_shard, homulator_b200/csrc/shard.cu): every sharded op is ONE C-ABI call.
     Build with Shard.ipc(ctx, max_L, rank, world, exchange) (one process per GPU) or Shard.local_group(ctxs, max_L)
-    (one process driving all ranks; emulation on a single GPU when the ctxs share a device)."""
+    (one process driving all ranks; emulation on a single GPU when the ctxs share a device).  max_rot (1..16, the same on
+    every rank) is the number of hoisted rotations that share one exchange (hrotate_hoisted)."""
 
-    def __init__(self, ctx, max_L, rank, world):
-        self.ctx, self.max_L, self.rank, self.world = ctx, max_L, rank, world
+    def __init__(self, ctx, max_L, rank, world, max_rot=1):
+        self.ctx, self.max_L, self.rank, self.world, self.max_rot = ctx, max_L, rank, world, max_rot
         self.h = C.c_void_p()
-        ctx._chk(ctx.lib.hml_shard_create(ctx.h, max_L, rank, world, C.byref(self.h)))
+        ctx._chk(ctx.lib.hml_shard_create_ex(ctx.h, max_L, rank, world, max_rot, C.byref(self.h)))
 
     @classmethod
-    def ipc(cls, ctx, max_L, rank, world, exchange):
+    def ipc(cls, ctx, max_L, rank, world, exchange, max_rot=1):
         """`exchange(obj)` returns the list of every rank's obj (torch.distributed.all_gather_object)."""
-        sh = cls(ctx, max_L, rank, world)
+        sh = cls(ctx, max_L, rank, world, max_rot)
         buf = C.create_string_buffer(256)
         ctx._chk(ctx.lib.hml_shard_handles(sh.h, buf))
         allh = exchange(bytes(buf.raw))
@@ -558,9 +564,9 @@ class Shard:
         return sh
 
     @classmethod
-    def local_group(cls, ctxs, max_L):
+    def local_group(cls, ctxs, max_L, max_rot=1):
         world = len(ctxs)
-        group = [cls(c, max_L, r, world) for r, c in enumerate(ctxs)]
+        group = [cls(c, max_L, r, world, max_rot) for r, c in enumerate(ctxs)]
         if world > 1:
             arr = (C.c_void_p * world)(*[g.h for g in group])
             ctxs[0]._chk(ctxs[0].lib.hml_shard_connect_local(arr, world))
@@ -602,6 +608,21 @@ class Shard:
         out = c.empty(2, max(nq, 1), c.N) if out is None else out
         c._chk(c.lib.hml_hrotate_sharded(self.h, L, _ptr(ct_own), _ptr(rk_own), g, _ptr(out), c._stream()))
         return out
+
+    def hrotate_hoisted(self, L, ct_own, rk_owns, galois_elts, outs=None):
+        """Rotations of ONE sharded ciphertext sharing one ModUp (hml_hrotate_hoisted_sharded); rk_owns[i] is this rank's key
+        slice for galois_elts[i] (None on a rank that owns no extended limb).  Returns the list of outputs [2][nq][N]."""
+        c = self.ctx
+        nq, _ = self.own(L)
+        n = len(galois_elts)
+        if len(rk_owns) != n:
+            raise ValueError("one key slice per galois element")
+        outs = [c.empty(2, max(nq, 1), c.N) for _ in range(n)] if outs is None else outs
+        keys = (C.c_void_p * max(n, 1))(*[(_ptr(k) if k is not None else None) for k in rk_owns])
+        po = (C.c_void_p * max(n, 1))(*[_ptr(o) for o in outs])
+        gs = (C.c_uint64 * max(n, 1))(*[int(g) for g in galois_elts])
+        c._chk(c.lib.hml_hrotate_hoisted_sharded(self.h, L, _ptr(ct_own), n, keys, gs, po, c._stream()))
+        return outs
 
     def hmult(self, L, a_own, b_own, evk_own, out=None):
         c = self.ctx
@@ -646,6 +667,33 @@ def group_op(group, kind, L, a, b=None, key=None, out0=None, out1=None, galois_e
     if rc:
         msgs = [g.ctx.lib.hml_last_error(g.ctx.h).decode() for g in group]
         raise HmlError(rc, next((m for m in msgs if m), "group op failed"))
+
+
+def group_hrotate_hoisted(group, L, ct_own, keys, galois_elts, outs=None, streams=None):
+    """hml_group_hrotate_hoisted: Shard.hrotate_hoisted on every rank of a local group from one host thread.  ct_own[r] is rank
+    r's ciphertext slice, keys[r][i] its key slice for galois_elts[i] (None where the rank owns no extended limb); returns
+    outs[r][i] (allocated when not given)."""
+    import torch
+    world, n = len(group), len(galois_elts)
+    ctx = group[0].ctx
+    if len(ct_own) != world or len(keys) != world or any(len(k) != n for k in keys):
+        raise ValueError("ct_own needs one entry per rank, keys one list of len(galois_elts) key slices per rank")
+    if outs is None:
+        outs = [[g.ctx.empty(2, max(g.own(L)[0], 1), g.ctx.N) for _ in range(n)] for g in group]
+    if streams is None:
+        st = torch.cuda.current_stream(ctx.device).cuda_stream
+        streams = [st] * world
+    gh = (C.c_void_p * world)(*[g.h for g in group])
+    ca = (C.c_void_p * world)(*[_ptr(t) for t in ct_own])
+    ka = (C.c_void_p * max(world * n, 1))(*[(_ptr(k) if k is not None else None) for r in range(world) for k in keys[r]])
+    oa = (C.c_void_p * max(world * n, 1))(*[_ptr(o) for r in range(world) for o in outs[r]])
+    gs = (C.c_uint64 * max(n, 1))(*[int(g) for g in galois_elts])
+    sa = (C.c_void_p * world)(*streams)
+    rc = ctx.lib.hml_group_hrotate_hoisted(gh, world, L, ca, n, ka, gs, oa, sa)
+    if rc:
+        msgs = [g.ctx.lib.hml_last_error(g.ctx.h).decode() for g in group]
+        raise HmlError(rc, next((m for m in msgs if m), "group hoisted rotation failed"))
+    return outs
 
 
 class Replay:

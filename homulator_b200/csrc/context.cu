@@ -1021,6 +1021,30 @@ extern "C" int hml_keyswitch_shard_begin(hml_ctx *ctx, uint32_t L, uint32_t rank
   return check_launch(ctx, "keyswitch shard begin");
 }
 
+// forward NTT of the owned extended digits ext [beta][ne] in place; with hpip the inner product with evk_own rides in the row
+// pass (NttMac) and the transformed digits are never stored
+static void shard_ext_ntt(hml_ctx *ctx, ShardPlan *sp, u64 *ext, bool hpip, const u64 *d_own, const u64 *evk_own, u64 *acc, cudaStream_t s) {
+  const Params &p = ctx->p;
+  const size_t N = p.N;
+  const uint32_t nq = sp->own_q.size(), ne = nq + sp->own_p.size(), beta = sp->beta;
+  const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
+  NttLaunch l{};
+  l.n_batch = 1;
+  l.in = ext; l.out = ext; l.in_limb_stride = l.out_limb_stride = N; l.in_poly_stride = l.out_poly_stride = (long long)ne * N;
+  l.n_limbs = ne; l.n_polys = beta;
+  l.in_f64 = l.out_f64 = npass == 2;
+  if (hpip) {
+    NttMac &m = l.mac;
+    m.evk = evk_own; m.d = d_own; m.acc = acc; m.d_batch_stride = 0; m.acc_batch_stride = 0; m.acc_comp_stride = (long long)ne * N;
+    m.evk_limbs = (int)ne; m.u_limb = -1;
+    for (uint32_t k = 0; k < ne; ++k) m.key_pos[k] = (uint16_t)k;
+    ctx->exec.ewe_limbs += 2ull * ne * beta;
+  }
+  launch_ntt_forward(ctx->tabs, logN, sp->e_lm, l, s);
+  prof_mark(ctx, HML_CLS_NTT, s);
+  ctx->exec.ntt_limbs += (uint64_t)beta * ne - nq; ctx->exec.kernel_launches += npass;
+}
+
 // everything of the middle phase after the ModUp conversions: NTT of the extended digits, inner product with the owned key
 // slices, INTT (+ scaling) of the owned P-limbs, copied into this rank's slot of gather buffer 2
 static int shard_mid_tail(hml_ctx *ctx, ShardPlan *sp, uint32_t rank, const u64 *d_own, const u64 *evk_own, u64 *gather2, cudaStream_t s) {
@@ -1031,23 +1055,7 @@ static int shard_mid_tail(hml_ctx *ctx, ShardPlan *sp, uint32_t rank, const u64 
   u64 *ext = ctx->ws, *acc = ext + (size_t)beta * ne * N;
   // one ciphertext's slice per rank: the inner product rides in the ModUp transform's row pass (NttMac) whenever it can
   const bool hpip = ks_uses_hpip(ctx, sp->L, 1);
-  {
-    NttLaunch l{};
-    l.n_batch = 1;
-    l.in = ext; l.out = ext; l.in_limb_stride = l.out_limb_stride = N; l.in_poly_stride = l.out_poly_stride = (long long)ne * N;
-    l.n_limbs = ne; l.n_polys = beta;
-    l.in_f64 = l.out_f64 = npass == 2;
-    if (hpip) {
-      NttMac &m = l.mac;
-      m.evk = evk_own; m.d = d_own; m.acc = acc; m.d_batch_stride = 0; m.acc_batch_stride = 0; m.acc_comp_stride = (long long)ne * N;
-      m.evk_limbs = (int)ne; m.u_limb = -1;
-      for (uint32_t k = 0; k < ne; ++k) m.key_pos[k] = (uint16_t)k;
-      ctx->exec.ewe_limbs += 2ull * ne * beta;
-    }
-    launch_ntt_forward(ctx->tabs, logN, sp->e_lm, l, s);
-    prof_mark(ctx, HML_CLS_NTT, s);
-    ctx->exec.ntt_limbs += (uint64_t)beta * ne - nq; ctx->exec.kernel_launches += npass;
-  }
+  shard_ext_ntt(ctx, sp, ext, hpip, d_own, evk_own, acc, s);
   if (!hpip) {
     InnerArgs a{};
     a.d = d_own; a.ext = ext; a.evk = evk_own; a.acc = acc; a.N = N; a.n_ext = ne; a.beta = beta;
@@ -1096,9 +1104,12 @@ extern "C" int hml_keyswitch_shard_mid(hml_ctx *ctx, uint32_t L, uint32_t rank, 
   return shard_mid_tail(ctx, sp, rank, (const u64 *)d_own, (const u64 *)evk_own, (u64 *)gather2, s);
 }
 
-// last phase: BConv P -> owned Q-limbs (sources in `gather2`, or at src_off relative to it), NTT, (acc - v) * P^-1
+// last phase: BConv P -> owned Q-limbs (sources in `gather2`, or at src_off relative to it), NTT, (acc - v) * P^-1.
+// acc_in / vb_in: the accumulator pair [2][ne] and the conversion output [2][nq] (null: the workspace positions of the key
+// switch).  add0_galois != 0 reads add0 through that automorphism (fused epilogue, two-pass rings only).
 static int shard_end_run(hml_ctx *ctx, ShardPlan *sp, const u64 *gather2, const long long *src_off, u64 *out0_own, u64 *out1_own, cudaStream_t s,
-                         const u64 *add0_own = nullptr, const u64 *add1_own = nullptr) {
+                         const u64 *add0_own = nullptr, const u64 *add1_own = nullptr, const u64 *acc_in = nullptr, u64 *vb_in = nullptr,
+                         u64 add0_galois = 0) {
   int rc;
   if ((rc = ensure_ws(ctx, shard_ws_words(ctx->p, *sp)))) return rc;
   ws_enter(ctx, s);
@@ -1107,7 +1118,9 @@ static int shard_end_run(hml_ctx *ctx, ShardPlan *sp, const u64 *gather2, const 
   const uint32_t nq = sp->own_q.size(), np = sp->own_p.size(), ne = nq + np, beta = sp->beta;
   const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
   if (nq == 0) return HML_OK;
-  u64 *ext = ctx->ws, *acc = ext + (size_t)beta * ne * N, *vb = acc + 2 * (size_t)ne * N;
+  const u64 *acc = acc_in ? acc_in : ctx->ws + (size_t)beta * ne * N;
+  u64 *vb = vb_in ? vb_in : ctx->ws + (size_t)beta * ne * N + 2 * (size_t)ne * N;
+  if (add0_galois && (npass != 2 || !add0_own || add1_own)) return fail(ctx, HML_ERR_INVALID, "automorphism on the addend needs the fused ModDown epilogue");
   {
     BConvArgs a{};
     a.in = gather2; a.out = vb; a.in_batch_stride = (long long)sp->gp * N; a.out_batch_stride = (long long)nq * N;
@@ -1128,6 +1141,7 @@ static int shard_end_run(hml_ctx *ctx, ShardPlan *sp, const u64 *gather2, const 
       f.z_mask = (add0_own ? 1u : 0u) | (add1_own ? 2u : 0u);
       f.dst = out0_own; f.dst_c_stride = (long long)(out1_own - out0_own); f.dst_b_stride = 0;
       f.cst = sp->pinv; f.n_c = 2;
+      f.z_galois = (unsigned)(add0_galois & (2ull * N - 1));
       ctx->exec.ewe_limbs += 2 * nq;
     }
     launch_ntt_forward(ctx->tabs, logN, sp->q_lm, l, s);
@@ -1348,6 +1362,34 @@ static int shard_p2p_check(hml_ctx *ctx, const HostBConv &hb) {
   return HML_OK;
 }
 
+// the ModUp conversions of the peer-direct middle phase: every digit (its limbs read from the owners' gather buffers 1, at the
+// offsets built by shard_peer_offsets relative to this rank's own buffer g1_own) -> owned extended limbs, ext [beta][ne]
+static void shard_modup_p2p(hml_ctx *ctx, ShardPlan *sp, const uint64_t *g1_own, u64 *ext, cudaStream_t s) {
+  const size_t N = ctx->p.N;
+  const uint32_t ne = sp->own_q.size() + sp->own_p.size(), beta = sp->beta;
+  bool merged_up = false;
+  if (sp->up_jobs) {
+    BConvArgs a{};
+    a.in = (const u64 *)g1_own; a.out = ext; a.step1 = nullptr; a.N = N; a.n_batches = 1; a.out_f64 = ctx->p.logN > NTT_SMALL_LOG;
+    std::vector<BConvImage> ims(beta);
+    std::vector<int> nd(beta);
+    for (uint32_t j = 0; j < beta; ++j) { ims[j] = sp->up[j].im; nd[j] = sp->up[j].n_dst; }
+    merged_up = launch_bconv_umma_multi(ctx->mc, sp->up_jobs, ims.data(), nd.data(), (int)beta, a, s);
+    if (merged_up) {
+      prof_mark(ctx, HML_CLS_BCONV, s);
+      ctx->exec.kernel_launches++;
+      for (uint32_t j = 0; j < beta; ++j) ctx->exec.bconv_limb_macs += (uint64_t)sp->up[j].n_src * sp->up[j].n_dst;
+    }
+  }
+  for (uint32_t j = 0; j < beta && !merged_up; ++j) {
+    if (sp->up[j].empty()) continue;
+    BConvArgs a{};
+    a.in = (const u64 *)g1_own; a.out = ext + (size_t)j * ne * N; a.step1 = nullptr; a.N = N; a.n_batches = 1;
+    a.src_off = sp->d_off1[j]; a.out_f64 = ctx->p.logN > NTT_SMALL_LOG;
+    run_bconv(ctx, sp->up[j], sp->up_src[j], a, s);
+  }
+}
+
 extern "C" int hml_keyswitch_shard_mid_p2p(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *d_own,
                                            const uint64_t *const *peers1, const uint64_t *evk_own, uint64_t *gather2_own, void *stream) {
   int rc = shard_check(ctx, L, rank, world);
@@ -1361,31 +1403,9 @@ extern "C" int hml_keyswitch_shard_mid_p2p(hml_ctx *ctx, uint32_t L, uint32_t ra
   if ((rc = shard_peer_offsets(ctx, sp, peers1, false))) return rc;
   if ((rc = ensure_ws(ctx, shard_ws_words(ctx->p, *sp)))) return rc;
   ws_enter(ctx, (cudaStream_t)stream);
-  const size_t N = ctx->p.N;
-  const uint32_t ne = sp->own_q.size() + sp->own_p.size(), beta = sp->beta;
+  const uint32_t ne = sp->own_q.size() + sp->own_p.size();
   if (ne == 0) return HML_OK;
-  u64 *ext = ctx->ws;
-  bool merged_up = false;
-  if (sp->up_jobs) {
-    BConvArgs a{};
-    a.in = (const u64 *)peers1[rank]; a.out = ext; a.step1 = nullptr; a.N = N; a.n_batches = 1; a.out_f64 = ctx->p.logN > NTT_SMALL_LOG;
-    std::vector<BConvImage> ims(beta);
-    std::vector<int> nd(beta);
-    for (uint32_t j = 0; j < beta; ++j) { ims[j] = sp->up[j].im; nd[j] = sp->up[j].n_dst; }
-    merged_up = launch_bconv_umma_multi(ctx->mc, sp->up_jobs, ims.data(), nd.data(), (int)beta, a, (cudaStream_t)stream);
-    if (merged_up) {
-      prof_mark(ctx, HML_CLS_BCONV, (cudaStream_t)stream);
-      ctx->exec.kernel_launches++;
-      for (uint32_t j = 0; j < beta; ++j) ctx->exec.bconv_limb_macs += (uint64_t)sp->up[j].n_src * sp->up[j].n_dst;
-    }
-  }
-  for (uint32_t j = 0; j < beta && !merged_up; ++j) {
-    if (sp->up[j].empty()) continue;
-    BConvArgs a{};
-    a.in = (const u64 *)peers1[rank]; a.out = ext + (size_t)j * ne * N; a.step1 = nullptr; a.N = N; a.n_batches = 1;
-    a.src_off = sp->d_off1[j]; a.out_f64 = ctx->p.logN > NTT_SMALL_LOG;
-    run_bconv(ctx, sp->up[j], sp->up_src[j], a, (cudaStream_t)stream);
-  }
+  shard_modup_p2p(ctx, sp, peers1[rank], ctx->ws, (cudaStream_t)stream);
   return shard_mid_tail(ctx, sp, rank, (const u64 *)d_own, (const u64 *)evk_own, (u64 *)gather2_own, (cudaStream_t)stream);
 }
 
@@ -1415,9 +1435,101 @@ int shard_end_p2p_add(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, c
   return shard_end_run(ctx, sp, (const u64 *)peers2[rank], sp->d_off2, (u64 *)out0_own, (u64 *)out1_own, s, (const u64 *)add0_own, (const u64 *)add1_own);
 }
 
+// ---- hoisted rotations of one limb-sharded ciphertext (shard.cu, hml_hrotate_hoisted_sharded).  One ModUp of c1 serves every
+// rotation; a group of up to H rotations shares one inner-product launch, one P-limb INTT and one exchange.  Workspace:
+//   ext [beta][ne] | acc [H][2][ne] | vb [2][nq]        (H = 1: the key switch's layout)
+size_t shard_hoist_ws_words(const Params &p, const ShardPlan &sp, uint32_t H) {
+  const size_t ne = sp.own_q.size() + sp.own_p.size(), nq = sp.own_q.size();
+  return (size_t)p.N * ((size_t)sp.beta * ne + 2 * (size_t)H * ne + 2 * nq);
+}
+
+static int shard_plan_on_device(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, ShardPlan **sp) {
+  int rc = shard_check(ctx, L, rank, world);
+  if (rc) return rc;
+  HML_CU_TRY(ctx, cudaSetDevice(ctx->device));
+  return get_shard_plan(ctx, L, rank, world, sp);
+}
+
+// phase 1 of a group of n <= H rotations.  peers1 != null (the op's first group): the ModUp conversions from the owners' gather
+// buffers 1 and the forward NTT of the owned extended digits, stored for the later groups (no fused inner product).  Then ONE
+// launch of the inner product for all n rotations: acc[r] = sum_j sigma_r(t_j) * keys[r][j]; the own-digit term reads c1_own
+// through sigma_r as well.
+int shard_hoist_inner(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uint32_t H, const uint64_t *const *peers1, const uint64_t *c1_own,
+                      uint32_t n, const uint64_t *const *keys, const uint64_t *galois, cudaStream_t s) {
+  ShardPlan *sp;
+  int rc = shard_plan_on_device(ctx, L, rank, world, &sp);
+  if (rc) return rc;
+  if (n == 0 || n > H || H > IP_MAX_ROT) return fail(ctx, HML_ERR_INVALID, "hoisted group larger than the shard's rotation capacity");
+  if ((rc = ensure_ws(ctx, shard_hoist_ws_words(ctx->p, *sp, H)))) return rc;
+  ws_enter(ctx, s);
+  const Params &p = ctx->p;
+  const size_t N = p.N;
+  const uint32_t ne = sp->own_q.size() + sp->own_p.size(), beta = sp->beta;
+  if (ne == 0) return HML_OK;
+  u64 *ext = ctx->ws, *acc = ext + (size_t)beta * ne * N;
+  if (peers1) {
+    for (auto &u : sp->up) if ((rc = shard_p2p_check(ctx, u))) return rc;
+    if ((rc = shard_peer_offsets(ctx, sp, peers1, false))) return rc;
+    shard_modup_p2p(ctx, sp, peers1[rank], ext, s);
+    shard_ext_ntt(ctx, sp, ext, false, nullptr, nullptr, nullptr, s);
+  }
+  InnerRotArgs a{};
+  a.d = (const u64 *)c1_own; a.ext = ext; a.acc = acc; a.acc_rot_stride = 2ll * ne * N;
+  a.N = (int)N; a.n_ext = (int)ne; a.beta = (int)beta; a.evk_limbs = (int)ne; a.logN = p.logN; a.ext_f64 = p.logN > NTT_SMALL_LOG;
+  for (uint32_t r = 0; r < n; ++r) {
+    const unsigned g = (unsigned)(galois[r] & (2ull * N - 1));
+    a.evk[r] = (const u64 *)keys[r]; a.galois[r] = g == 1 ? 0 : g;
+  }
+  launch_inner_product_rot(ctx->mc, sp->e_lm, a, (int)n, s);
+  prof_mark(ctx, HML_CLS_EWE, s);
+  ctx->exec.ewe_limbs += 2ull * n * ne * beta; ctx->exec.kernel_launches++;
+  return check_launch(ctx, "hoisted shard inner product");
+}
+
+// the rest of phase 1: ONE inverse NTT (+ scaling) of the owned P-limbs of all 2n accumulators, rotation r into this rank's
+// contribution to slot r of its gather buffer 2 (slot_words apart; slot 0 is the key switch's layout)
+int shard_hoist_intt(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uint32_t n, uint64_t *g2_own, size_t slot_words, cudaStream_t s) {
+  ShardPlan *sp;
+  int rc = shard_plan_on_device(ctx, L, rank, world, &sp);
+  if (rc) return rc;
+  ws_enter(ctx, s);
+  const Params &p = ctx->p;
+  const size_t N = p.N;
+  const uint32_t nq = sp->own_q.size(), np = sp->own_p.size(), ne = nq + np;
+  const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
+  if (np == 0) return HML_OK;
+  NttLaunch l{};
+  l.in = ctx->ws + (size_t)sp->beta * ne * N; l.in_limb_stride = N; l.in_poly_stride = (long long)ne * N; l.in_batch_stride = 2ll * ne * N;
+  // as in shard_mid_tail: limb k of p_lm sits at position nq + k of an accumulator, so the output base is shifted back by nq limbs
+  l.out = (u64 *)g2_own + (size_t)rank * 2 * sp->gp * N - (size_t)nq * N; l.out_limb_stride = N; l.out_poly_stride = (long long)sp->gp * N;
+  l.out_batch_stride = (long long)slot_words;
+  l.n_limbs = np; l.n_polys = 2; l.n_batch = (int)n; l.post_scale = sp->scale2;
+  launch_ntt_inverse(ctx->tabs, logN, sp->p_lm, l, s);
+  prof_mark(ctx, HML_CLS_INTT, s);
+  ctx->exec.intt_limbs += 2ull * n * np; ctx->exec.kernel_launches += npass;
+  return check_launch(ctx, "hoisted shard P-limb INTT");
+}
+
+// phase 2 of rotation r of the group: ModDown from slot r of the owners' gather buffers 2, plus add0 (read through add0_galois
+// when it is not 0) on component 0
+int shard_hoist_end(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uint32_t H, const uint64_t *const *peers2, size_t slot_words,
+                    uint32_t r, const uint64_t *add0, uint64_t add0_galois, uint64_t *out0, uint64_t *out1, cudaStream_t s) {
+  ShardPlan *sp;
+  int rc = shard_plan_on_device(ctx, L, rank, world, &sp);
+  if (rc) return rc;
+  if ((rc = shard_p2p_check(ctx, sp->down))) return rc;
+  if ((rc = shard_peer_offsets(ctx, sp, peers2, true))) return rc;
+  const size_t N = ctx->p.N, ne = sp->own_q.size() + sp->own_p.size();
+  u64 *acc = ctx->ws + (size_t)sp->beta * ne * N;
+  return shard_end_run(ctx, sp, (const u64 *)peers2[rank] + (size_t)r * slot_words, sp->d_off2, (u64 *)out0, (u64 *)out1, s, (const u64 *)add0, nullptr,
+                       acc + 2 * (size_t)r * ne * N, acc + 2 * (size_t)H * ne * N, add0_galois);
+}
+
 // everything a sharded op at level L needs that costs host time or synchronises the device (plans, conversion images, offset
-// tables, workspace): done ahead of the first exchange so that no rank sits in a spin-wait while a peer is still preparing
-int shard_prepare(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *const *peers1, const uint64_t *const *peers2) {
+// tables, workspace for up to max_rot hoisted rotations): done ahead of the first exchange so that no rank sits in a spin-wait
+// while a peer is still preparing
+int shard_prepare(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *const *peers1, const uint64_t *const *peers2,
+                  uint32_t max_rot) {
   int rc = shard_check(ctx, L, rank, world);
   if (rc) return rc;
   HML_CU_TRY(ctx, cudaSetDevice(ctx->device));
@@ -1428,7 +1540,7 @@ int shard_prepare(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const
   if ((rc = shard_peer_offsets(ctx, sp, peers1, false))) return rc;
   if ((rc = shard_peer_offsets(ctx, sp, peers2, true))) return rc;
   const uint32_t nq = sp->own_q.size();
-  return ensure_ws(ctx, std::max(shard_ws_words(ctx->p, *sp), (size_t)2 * nq * ctx->p.N));
+  return ensure_ws(ctx, std::max(shard_hoist_ws_words(ctx->p, *sp, max_rot), (size_t)2 * nq * ctx->p.N));
 }
 
 // ------------------------------------------------------------------------------------------------ rescale

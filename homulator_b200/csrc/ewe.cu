@@ -248,6 +248,67 @@ void launch_inner_product(const ModConst *mc, const LimbMap &lm, const InnerArgs
   else launch_inner_t<false>(mc, lm, a, s);
 }
 
+// Hoisted rotations of one ciphertext (limb-sharded, shard.cu): k_inner's single-ciphertext body with the automorphism on
+// load, once per rotation (blockIdx.z), each with its own key and galois element.  Rotations are the slowest grid dimension,
+// so the digits stay in L2 while the later rotations re-read them.  Five to eight digits need 128 registers (two CTAs per SM)
+// to hold the 32 key words without spilling.
+template <int IP_MAX_BETA>
+__global__ void __launch_bounds__(EW_THREADS, IP_MAX_BETA > 4 ? 2 : 3) k_inner_rot(const ModConst *__restrict__ mc, LimbMap lm, InnerRotArgs a) {
+  pdl_wait();
+  const int i2 = blockIdx.x * EW_THREADS + threadIdx.x;
+  if (i2 >= a.N / 2) return;
+  const int e = blockIdx.y, r = blockIdx.z;
+  const ModConst m = mc[lm.mod[e]];
+  const int kl = lm.pos[e], own = lm.skip[e];
+  const size_t n2 = a.N / 2;
+  const unsigned g = a.galois[r];
+  const u64 *evk = a.evk[r];
+  unsigned s0 = 2u * i2, s1 = 2u * i2 + 1u;
+  if (g) {  // the index formula of k_inner
+    const unsigned sh = 32 - a.logN, m2n = (2u << a.logN) - 1u;
+    s0 = __brev((((g * (2u * (__brev(s0) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
+    s1 = __brev((((g * (2u * (__brev(s1) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
+  }
+  ulonglong2 t[IP_MAX_BETA];
+#pragma unroll
+  for (int j = 0; j < IP_MAX_BETA; ++j)
+    if (j < a.beta) {
+      const u64 *p = j == own ? a.d + (size_t)e * a.N : a.ext + ((size_t)j * a.n_ext + e) * a.N;
+      t[j] = g ? make_ulonglong2(__ldg(p + s0), __ldg(p + s1)) : ld2(p, i2);
+    }
+  ulonglong2 kraw[IP_MAX_BETA][2];  // every key word requested before the first use, as in k_inner
+#pragma unroll
+  for (int j = 0; j < IP_MAX_BETA; ++j)
+#pragma unroll
+    for (int c = 0; c < 2; ++c)
+      kraw[j][c] = j < a.beta ? ld2(evk, (((size_t)j * 2 + c) * a.evk_limbs + kl) * n2 + i2) : make_ulonglong2(0, 0);
+  pin_loads(kraw);
+  double s00 = 0, s01 = 0, s10 = 0, s11 = 0;  // [component][coefficient]
+#pragma unroll
+  for (int j = 0; j < IP_MAX_BETA; ++j)
+    if (j < a.beta) {
+      const bool f64 = a.ext_f64 && j != own;
+      const double t0 = f64 ? __longlong_as_double((long long)t[j].x) : u64_to_f64(t[j].x);
+      const double t1 = f64 ? __longlong_as_double((long long)t[j].y) : u64_to_f64(t[j].y);
+      s00 += mulmod_var(t0, u64_to_f64(kraw[j][0].x), m.q, m.qinv);
+      s01 += mulmod_var(t1, u64_to_f64(kraw[j][0].y), m.q, m.qinv);
+      s10 += mulmod_var(t0, u64_to_f64(kraw[j][1].x), m.q, m.qinv);
+      s11 += mulmod_var(t1, u64_to_f64(kraw[j][1].y), m.q, m.qinv);
+    }
+  u64 *acc = a.acc + (size_t)r * a.acc_rot_stride;
+  st2(acc, (size_t)e * n2 + i2, finish(s00, m), finish(s01, m));
+  st2(acc, (size_t)(a.n_ext + e) * n2 + i2, finish(s10, m), finish(s11, m));
+}
+
+void launch_inner_product_rot(const ModConst *mc, const LimbMap &lm, const InnerRotArgs &a, int n_rot, cudaStream_t s) {
+  const dim3 g = ew_grid(a.N, a.n_ext, n_rot);
+  if (a.beta <= 1) launch_pdl(k_inner_rot<1>, g, EW_THREADS, 0, s, mc, lm, a);
+  else if (a.beta <= 2) launch_pdl(k_inner_rot<2>, g, EW_THREADS, 0, s, mc, lm, a);
+  else if (a.beta <= 3) launch_pdl(k_inner_rot<3>, g, EW_THREADS, 0, s, mc, lm, a);
+  else if (a.beta <= 4) launch_pdl(k_inner_rot<4>, g, EW_THREADS, 0, s, mc, lm, a);
+  else launch_pdl(k_inner_rot<8>, g, EW_THREADS, 0, s, mc, lm, a);
+}
+
 // ------------------------------------------------------------------------------------------------ (x - y) * c (+ z)
 __global__ void __launch_bounds__(EW_THREADS) k_sub_mul_add(const ModConst *__restrict__ mc, LimbMap lm, SubMulArgs a) {
   pdl_wait();

@@ -54,6 +54,23 @@ struct InnerArgs {
 };
 void launch_inner_product(const ModConst *mc, const LimbMap &lm, const InnerArgs &a, cudaStream_t s);
 
+// The same inner product for up to IP_MAX_ROT hoisted rotations of one ciphertext in ONE launch (grid.z = rotation): every
+// rotation reads the same digits d / ext, through its own automorphism (as InnerArgs::galois), and multiplies them by its own
+// key (8-byte words).  Rotation r writes acc + r * acc_rot_stride, [2][n_ext][N] words.  The digits of one launch are read
+// from L2 after the first rotation.
+constexpr int IP_MAX_ROT = 16;
+struct InnerRotArgs {
+  const u64 *d;                    // [>= number of owned Q-limbs][N], read through the automorphism like ext
+  const u64 *ext;                  // [beta][n_ext][N]
+  u64 *acc;
+  long long acc_rot_stride;
+  int N, n_ext, beta, evk_limbs, logN;  // beta <= 8
+  int ext_f64;                     // as InnerArgs::ext_f64
+  const u64 *evk[IP_MAX_ROT];      // [beta][2][evk_limbs][N] per rotation
+  unsigned galois[IP_MAX_ROT];     // galois element mod 2N per rotation; 0 = identity
+};
+void launch_inner_product_rot(const ModConst *mc, const LimbMap &lm, const InnerRotArgs &a, int n_rot, cudaStream_t s);
+
 // out = (x - y) * c (+ z) per limb:  ModDownSub (+ HMULT add)  reference src/Operation.cpp:548-590, :967-1005
 // and Rescale sub+mul  reference src/Operation.cpp:825-911.  cst[limb] = (c, RN(c/q)).  n_polys via strides.
 struct SubMulArgs {

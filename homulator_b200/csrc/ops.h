@@ -79,4 +79,12 @@ int hrot_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const hml::u64 *ct, const hm
 // limb-sharded building blocks beyond the ABI's phase entry points (shard.cu)
 int shard_end_p2p_add(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *const *peers2, uint64_t *out0_own,
                       uint64_t *out1_own, const uint64_t *add0_own, const uint64_t *add1_own, cudaStream_t s);
-int shard_prepare(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *const *peers1, const uint64_t *const *peers2);
+int shard_prepare(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *const *peers1, const uint64_t *const *peers2,
+                  uint32_t max_rot);
+// hoisted rotations of one sharded ciphertext, H = the shard's rotation capacity (context.cu)
+size_t shard_hoist_ws_words(const hml::Params &p, const hml::ShardPlan &sp, uint32_t H);
+int shard_hoist_inner(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uint32_t H, const uint64_t *const *peers1, const uint64_t *c1_own,
+                      uint32_t n, const uint64_t *const *keys, const uint64_t *galois, cudaStream_t s);
+int shard_hoist_intt(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uint32_t n, uint64_t *g2_own, size_t slot_words, cudaStream_t s);
+int shard_hoist_end(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uint32_t H, const uint64_t *const *peers2, size_t slot_words,
+                    uint32_t r, const uint64_t *add0, uint64_t add0_galois, uint64_t *out0, uint64_t *out1, cudaStream_t s);

@@ -7,7 +7,7 @@
 // layout with evk_q_limbs >= L serve every level; a plaintext's first limbs serve the lower levels).  A trace runs on one GPU
 // (hml_ctx) or limb-sharded over a group (hml_shard), as plain launches or as ONE captured CUDA graph,
 // and optionally with hoisted rotations: consecutive hrotate ops that read the same slot share one ModUp
-// (hml_hrotate_hoisted; single-GPU traces only).
+// (hml_hrotate_hoisted on one GPU, hml_hrotate_hoisted_sharded over a shard group).
 #include <algorithm>
 #include <cstring>
 #include <map>
@@ -23,6 +23,8 @@ extern "C" int hml_hmult_sharded(hml_shard *sh, uint32_t L, const uint64_t *a_ow
 extern "C" int hml_ew_sharded(hml_shard *sh, uint32_t L, int kind, const uint64_t *a_own, const uint64_t *b_own, uint64_t *out_own, void *stream);
 extern "C" int hml_shard_own_limbs(const hml_shard *sh, uint32_t L, uint32_t *n_own_q, uint32_t *n_own_q_after_rescale);
 extern "C" int hml_shard_prepare(hml_shard *sh, uint32_t L);
+extern "C" int hml_hrotate_hoisted_sharded(hml_shard *sh, uint32_t L, const uint64_t *ct_own, uint32_t n_rot, const uint64_t *const *rotkeys_own,
+                                           const uint64_t *galois_elts, uint64_t *const *outs_own, void *stream);
 
 struct hml_replay {
   hml_ctx *ctx = nullptr;
@@ -55,7 +57,6 @@ extern "C" int hml_replay_create(hml_ctx *ctx, hml_shard *sh, uint32_t L, const 
   *out = nullptr;
   int rc = check_level(ctx, L, 1);
   if (rc) return rc;
-  if (sh && (flags & HML_REPLAY_HOIST)) return fail(ctx, HML_ERR_UNSUPPORTED, "hoisted rotations are implemented for single-GPU traces only");
   hml_replay *rp = new hml_replay();
   rp->ctx = ctx; rp->sh = sh; rp->L = L; rp->flags = flags;
   rp->ops.assign(ops, ops + n_ops);
@@ -164,7 +165,7 @@ static int enqueue(hml_replay *rp, cudaStream_t s) {
     const uint64_t *a = rp->slot[o.a];
     switch (o.kind) {
       case HML_OP_HROTATE: {
-        if ((rp->flags & HML_REPLAY_HOIST) && !rp->sh) {
+        if (rp->flags & HML_REPLAY_HOIST) {
           // the run of consecutive rotations of the same source (none of which overwrites it) shares one ModUp
           size_t j = i;
           std::vector<const uint64_t *> keys;
@@ -180,7 +181,8 @@ static int enqueue(hml_replay *rp, cudaStream_t s) {
             ++j;
           }
           if (outs.size() >= 2) {
-            rc = hml_hrotate_hoisted(ctx, L, a, (uint32_t)outs.size(), keys.data(), rp->evk_q_limbs, gs.data(), outs.data(), st);
+            rc = rp->sh ? hml_hrotate_hoisted_sharded(rp->sh, L, a, (uint32_t)outs.size(), keys.data(), gs.data(), outs.data(), st)
+                        : hml_hrotate_hoisted(ctx, L, a, (uint32_t)outs.size(), keys.data(), rp->evk_q_limbs, gs.data(), outs.data(), st);
             i = j - 1;
             break;
           }

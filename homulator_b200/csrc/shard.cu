@@ -28,7 +28,8 @@ using namespace hml;
 struct hml_shard {
   hml_ctx *ctx = nullptr;
   uint32_t rank = 0, world = 1, max_L = 0;
-  size_t n1 = 0, n2 = 0, nf = 0, nr = 0;   // words of the own buffers
+  uint32_t max_rot = 1;                    // hoisted rotations per group: gather buffer 2 holds max_rot slots of n2 words
+  size_t n1 = 0, n2 = 0, nf = 0, nr = 0;   // words of the own buffers (n2: one slot of gather buffer 2)
   uint64_t *g1 = nullptr, *g2 = nullptr, *fl = nullptr, *rb = nullptr;
   std::vector<uint64_t *> p1, p2, pf, pr;       // every rank's buffers as pointers valid on this device (own at [rank])
   uint64_t **pf_dev = nullptr;                  // device copy of pf
@@ -56,14 +57,15 @@ static int sfail(hml_shard *sh, int code, const std::string &msg) { return fail(
 static uint32_t own_q_count(uint32_t L, uint32_t rank, uint32_t world) { return L > rank ? (L - rank + world - 1) / world : 0; }
 
 // ------------------------------------------------------------------------------------------------ lifetime
-extern "C" int hml_shard_create(hml_ctx *ctx, uint32_t max_L, uint32_t rank, uint32_t world, hml_shard **out) {
+extern "C" int hml_shard_create_ex(hml_ctx *ctx, uint32_t max_L, uint32_t rank, uint32_t world, uint32_t max_rot, hml_shard **out) {
   if (!ctx || !out) return HML_ERR_INVALID;
   *out = nullptr;
   int rc = shard_check(ctx, max_L, rank, world);
   if (rc) return rc;
+  if (max_rot < 1 || max_rot > IP_MAX_ROT) return fail(ctx, HML_ERR_INVALID, "max_rot must be in [1, 16]");
   HML_CU_TRY(ctx, cudaSetDevice(ctx->device));
   hml_shard *sh = new hml_shard();
-  sh->ctx = ctx; sh->rank = rank; sh->world = world; sh->max_L = max_L;
+  sh->ctx = ctx; sh->rank = rank; sh->world = world; sh->max_L = max_L; sh->max_rot = max_rot;
   const size_t N = ctx->p.N, A = ctx->p.alpha;
   const size_t gq = (max_L + world - 1) / world, gp = (A + world - 1) / world;
   sh->n1 = (size_t)world * gq * N; sh->n2 = (size_t)world * 2 * gp * N; sh->nf = 3 * (size_t)world + 8; sh->nr = 2 * N;
@@ -72,7 +74,7 @@ extern "C" int hml_shard_create(hml_ctx *ctx, uint32_t max_L, uint32_t rank, uin
     return e == cudaSuccess ? cudaMemset(*p, 0, words * 8) : e;
   };
   cudaError_t e = alloc(&sh->g1, sh->n1);
-  if (e == cudaSuccess) e = alloc(&sh->g2, sh->n2);
+  if (e == cudaSuccess) e = alloc(&sh->g2, sh->n2 * max_rot);
   if (e == cudaSuccess) e = alloc(&sh->fl, sh->nf);
   if (e == cudaSuccess) e = alloc(&sh->rb, sh->nr);
   if (e == cudaSuccess) e = alloc(&sh->scratch, 5 * std::max<size_t>(1, own_q_count(max_L, rank, world)) * N);
@@ -92,6 +94,10 @@ extern "C" int hml_shard_create(hml_ctx *ctx, uint32_t max_L, uint32_t rank, uin
   }
   *out = sh;
   return HML_OK;
+}
+
+extern "C" int hml_shard_create(hml_ctx *ctx, uint32_t max_L, uint32_t rank, uint32_t world, hml_shard **out) {
+  return hml_shard_create_ex(ctx, max_L, rank, world, 1, out);
 }
 
 extern "C" int hml_shard_destroy(hml_shard *sh) {
@@ -144,6 +150,8 @@ extern "C" int hml_shard_connect_local(hml_shard *const *group, uint32_t world) 
   if (!group || world == 0) return HML_ERR_INVALID;
   for (uint32_t r = 0; r < world; ++r)
     if (!group[r] || group[r]->world != world || group[r]->rank != r) return HML_ERR_INVALID;
+  for (uint32_t r = 1; r < world; ++r)  // slot r of every gather buffer 2 sits r * n2 words in: all ranks need the same layout
+    if (group[r]->max_rot != group[0]->max_rot) return sfail(group[r], HML_ERR_INVALID, "every rank of a shard group must use the same max_rot");
   for (uint32_t r = 0; r < world; ++r) {
     hml_shard *sh = group[r];
     HML_CU_TRY(sh->ctx, cudaSetDevice(sh->ctx->device));
@@ -170,7 +178,7 @@ extern "C" int hml_shard_prepare(hml_shard *sh, uint32_t L) {
   if (!sh) return HML_ERR_INVALID;
   if (!sh->connected) return sfail(sh, HML_ERR_INVALID, "shard group not connected");
   if (L > sh->max_L) return sfail(sh, HML_ERR_INVALID, "level above the shard's maximum");
-  return shard_prepare(sh->ctx, L, sh->rank, sh->world, (const uint64_t *const *)sh->p1.data(), (const uint64_t *const *)sh->p2.data());
+  return shard_prepare(sh->ctx, L, sh->rank, sh->world, (const uint64_t *const *)sh->p1.data(), (const uint64_t *const *)sh->p2.data(), sh->max_rot);
 }
 
 extern "C" int hml_shard_status(hml_ctx *ctx, const uint64_t *flags, uint32_t world, void *stream);
@@ -309,63 +317,212 @@ extern "C" int hml_ew_sharded(hml_shard *sh, uint32_t L, int kind, const uint64_
   return HML_OK;
 }
 
+// ------------------------------------------------------------------------------------------------ hoisted rotations
+// n_rot rotations of ONE sharded ciphertext sharing one ModUp of c1 (the sharded form of hml_hrotate_hoisted, bit-identical to
+// it on the owned limbs).  The rotations run in groups of up to max_rot; a group shares one inner-product launch, one P-limb
+// INTT and one exchange, and uses slots 0.. of every rank's gather buffer 2:
+//   begin | X0 | ModUp, IP(0), INTT(0) | X1 | end(0) | IP(1) | X1 | INTT(1) | X1 | end(1) | ...
+// begin and X0 run once per op.  The extra X1 in front of a later group's INTT orders its writes to gather buffer 2 after every
+// peer's ModDown reads of the previous group.  end(k) is one ModDown per rotation of the group, with sigma_r(c0) as its addend:
+// gathered by the fused epilogue on two-pass rings, an automorphism kernel into the shard scratch on single-pass rings.
+enum HoistStepKind { HS_BEGIN, HS_INNER, HS_INTT, HS_END, HS_X0, HS_X1 };
+struct HoistStep {
+  int kind;
+  uint32_t group;
+};
+struct HoistOp {
+  uint32_t L, n_rot;
+  const uint64_t *ct;            // [2][nq][N]
+  const uint64_t *const *keys;   // [n_rot] owned key slices (may be null on a rank that owns no extended limb)
+  const uint64_t *galois;        // [n_rot]
+  uint64_t *const *outs;         // [n_rot] [2][nq][N]
+};
+
+static std::vector<HoistStep> hoist_steps(uint32_t n_rot, uint32_t H) {
+  std::vector<HoistStep> v{{HS_BEGIN, 0}, {HS_X0, 0}};
+  for (uint32_t k = 0; k * H < n_rot; ++k) {
+    v.push_back({HS_INNER, k});
+    if (k) v.push_back({HS_X1, k});
+    v.push_back({HS_INTT, k});
+    v.push_back({HS_X1, k});
+    v.push_back({HS_END, k});
+  }
+  return v;
+}
+
+static int hoist_check(hml_shard *sh, const HoistOp &op) {
+  hml_ctx *ctx = sh->ctx;
+  if (!sh->connected) return sfail(sh, HML_ERR_INVALID, "shard group not connected");
+  int rc = check_level(ctx, op.L, 1);
+  if (rc) return rc;
+  if (op.L > sh->max_L) return sfail(sh, HML_ERR_INVALID, "level above the shard's maximum");
+  if (!op.ct || !op.galois || !op.outs) return sfail(sh, HML_ERR_INVALID, "null buffer");
+  const uint32_t nq = own_q_count(op.L, sh->rank, sh->world);
+  const bool own_ext = nq > 0 || own_q_count(op.L + ctx->p.alpha, sh->rank, sh->world) > 0;
+  const size_t words = 2 * (size_t)std::max<uint32_t>(nq, 1) * ctx->p.N;
+  for (uint32_t r = 0; r < op.n_rot; ++r) {
+    const uint64_t *o = op.outs[r];
+    if (!o) return sfail(sh, HML_ERR_INVALID, "null output");
+    if (o < op.ct + words && op.ct < o + words) return sfail(sh, HML_ERR_INVALID, "an output aliases the input");
+    if (!(op.galois[r] & 1)) return sfail(sh, HML_ERR_INVALID, "galois element must be odd");
+    if (own_ext && (!op.keys || !op.keys[r])) return sfail(sh, HML_ERR_INVALID, "null rotation key on a rank that owns extended limbs");
+  }
+  return HML_OK;
+}
+
+static int hoist_prepare(hml_shard *sh, uint32_t L) {
+  HML_CU_TRY(sh->ctx, cudaSetDevice(sh->ctx->device));
+  return shard_prepare(sh->ctx, L, sh->rank, sh->world, (const uint64_t *const *)sh->p1.data(), (const uint64_t *const *)sh->p2.data(), sh->max_rot);
+}
+
+static int hoist_phase(hml_shard *sh, const HoistOp &op, const HoistStep &st, cudaStream_t s) {
+  hml_ctx *ctx = sh->ctx;
+  const uint32_t L = op.L, rank = sh->rank, world = sh->world, H = sh->max_rot;
+  const size_t N = ctx->p.N;
+  const uint32_t nq = own_q_count(L, rank, world);
+  const uint64_t *c1 = op.ct + (size_t)nq * N;
+  const uint32_t lo = st.group * H, n = std::min(H, op.n_rot - lo);
+  auto peers = [](const std::vector<uint64_t *> &v) { return (const uint64_t *const *)v.data(); };
+  switch (st.kind) {
+    case HS_BEGIN: return hml_keyswitch_shard_begin(ctx, L, rank, world, c1, sh->g1, (void *)s);
+    case HS_INNER:
+      return shard_hoist_inner(ctx, L, rank, world, H, st.group == 0 ? peers(sh->p1) : nullptr, c1, n, op.keys ? op.keys + lo : nullptr,
+                               op.galois + lo, s);
+    case HS_INTT: return shard_hoist_intt(ctx, L, rank, world, n, sh->g2, sh->n2, s);
+    case HS_END:
+      for (uint32_t r = 0; r < n && nq; ++r) {
+        const uint64_t g = op.galois[lo + r] & (2 * N - 1);
+        uint64_t *o = op.outs[lo + r];
+        const uint64_t *add = op.ct;  // g = 1: sigma(c0) is c0 itself
+        uint64_t add_g = 0;
+        if (g != 1 && ctx->p.logN > NTT_SMALL_LOG) {
+          add_g = g;
+          ctx->exec.automorph_limbs += nq;
+        } else if (g != 1) {
+          int rc = hml_automorph(ctx, op.ct, sh->scratch, g, nq, (void *)s);
+          if (rc) return rc;
+          add = sh->scratch;
+        }
+        int rc = shard_hoist_end(ctx, L, rank, world, H, peers(sh->p2), sh->n2, r, add, add_g, o, o + (size_t)nq * N, s);
+        if (rc) return rc;
+      }
+      return HML_OK;
+  }
+  return HML_ERR_INVALID;
+}
+
+extern "C" int hml_hrotate_hoisted_sharded(hml_shard *sh, uint32_t L, const uint64_t *ct_own, uint32_t n_rot, const uint64_t *const *rotkeys_own,
+                                           const uint64_t *galois_elts, uint64_t *const *outs_own, void *stream) {
+  if (!sh) return HML_ERR_INVALID;
+  if (n_rot == 0) return HML_OK;
+  const HoistOp op{L, n_rot, ct_own, rotkeys_own, galois_elts, outs_own};
+  int rc = hoist_check(sh, op);
+  if (rc || (rc = hoist_prepare(sh, L))) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  for (const HoistStep &st : hoist_steps(n_rot, sh->max_rot)) {
+    rc = st.kind == HS_X0 ? fused_sync(sh, 0, s) : st.kind == HS_X1 ? fused_sync(sh, 1, s) : hoist_phase(sh, op, st, s);
+    if (rc) return rc;
+  }
+  sh->rb_dirty = false;  // no rescale buffer written; X0 ordered this op after every peer's earlier reads of it
+  return HML_OK;
+}
+
 // ------------------------------------------------------------------------------------------------ group driver
-// All ranks of a group driven from one host thread, phase by phase.  op: 0 keyswitch (a = d_own, out0/out1), 1 hrotate
-// (a = ct_own, out0), 2 hmult (a, b, out0), 3 rescale (a, out0).  Arrays are indexed by rank; streams[r] is rank r's stream.
+// All ranks of a group driven from one host thread, phase by phase.  Arrays are indexed by rank; streams[r] is rank r's stream.
 // Ranks that share a device MUST share one stream; they are then ordered by that stream and use separate signal / wait
 // launches (host-side epochs) instead of the fused exchange.
-extern "C" int hml_group_op(hml_shard *const *group, uint32_t world, int op_kind, uint32_t L, const uint64_t *const *a, const uint64_t *const *b,
-                            const uint64_t *const *key, uint64_t *const *out0, uint64_t *const *out1, uint64_t galois_elt, void *const *streams) {
-  if (!group || world == 0 || !a || !out0 || op_kind < 0 || op_kind > 3) return HML_ERR_INVALID;
-  bool emulate = false;
+static int group_setup(hml_shard *const *group, uint32_t world, void *const *streams, bool *emulate) {
+  *emulate = false;
   for (uint32_t r = 0; r < world; ++r) {
     if (!group[r] || group[r]->world != world || group[r]->rank != r) return HML_ERR_INVALID;
     for (uint32_t q = 0; q < r; ++q)
       if (group[q]->ctx->device == group[r]->ctx->device) {
-        emulate = true;
+        *emulate = true;
         if ((streams ? streams[q] : nullptr) != (streams ? streams[r] : nullptr))
           return fail(group[r]->ctx, HML_ERR_INVALID, "ranks that share a device must share one stream");
       }
   }
+  return HML_OK;
+}
+
+static cudaStream_t group_stream(void *const *streams, uint32_t r) { return (cudaStream_t)(streams ? streams[r] : nullptr); }
+
+static int group_exchange(hml_shard *const *group, uint32_t world, bool emulate, void *const *streams, int grp) {
+  int rc;
+  if (!emulate) {
+    for (uint32_t r = 0; r < world; ++r) {
+      cudaSetDevice(group[r]->ctx->device);
+      if ((rc = fused_sync(group[r], grp, group_stream(streams, r)))) return rc;
+    }
+    return HML_OK;
+  }
+  for (uint32_t r = 0; r < world; ++r) {
+    hml_shard *sh = group[r];
+    cudaSetDevice(sh->ctx->device);
+    if ((rc = hml_shard_signal(sh->ctx, (uint64_t *const *)sh->pf_dev, grp * world + r, ++sh->host_epoch[grp], world, (void *)group_stream(streams, r)))) return rc;
+  }
+  for (uint32_t r = 0; r < world; ++r) {
+    hml_shard *sh = group[r];
+    cudaSetDevice(sh->ctx->device);
+    if ((rc = hml_shard_wait(sh->ctx, sh->fl, grp * world, sh->host_epoch[grp], world, (void *)group_stream(streams, r)))) return rc;
+  }
+  return HML_OK;
+}
+
+// op: 0 keyswitch (a = d_own, out0/out1), 1 hrotate (a = ct_own, out0), 2 hmult (a, b, out0), 3 rescale (a, out0).
+extern "C" int hml_group_op(hml_shard *const *group, uint32_t world, int op_kind, uint32_t L, const uint64_t *const *a, const uint64_t *const *b,
+                            const uint64_t *const *key, uint64_t *const *out0, uint64_t *const *out1, uint64_t galois_elt, void *const *streams) {
+  if (!group || world == 0 || !a || !out0 || op_kind < 0 || op_kind > 3) return HML_ERR_INVALID;
+  bool emulate;
+  int rc = group_setup(group, world, streams, &emulate);
+  if (rc) return rc;
   std::vector<ShardOp> ops(world);
   for (uint32_t r = 0; r < world; ++r) {
     ops[r] = ShardOp{op_kind, L, (const uint64_t *)a[r], b ? (const uint64_t *)b[r] : nullptr, key ? (const uint64_t *)key[r] : nullptr, (uint64_t *)out0[r],
                      out1 ? (uint64_t *)out1[r] : nullptr, galois_elt};
-    int rc = op_check(group[r], ops[r]);
-    if (rc) return rc;
+    if ((rc = op_check(group[r], ops[r]))) return rc;
   }
-  auto stream_of = [&](uint32_t r) { return (cudaStream_t)(streams ? streams[r] : nullptr); };
-  auto exchange = [&](int grp) -> int {
-    int rc;
-    if (!emulate) {
-      for (uint32_t r = 0; r < world; ++r) {
-        cudaSetDevice(group[r]->ctx->device);
-        if ((rc = fused_sync(group[r], grp, stream_of(r)))) return rc;
-      }
-      return HML_OK;
-    }
-    for (uint32_t r = 0; r < world; ++r) {
-      hml_shard *sh = group[r];
-      cudaSetDevice(sh->ctx->device);
-      if ((rc = hml_shard_signal(sh->ctx, (uint64_t *const *)sh->pf_dev, grp * world + r, ++sh->host_epoch[grp], world, (void *)stream_of(r)))) return rc;
-    }
-    for (uint32_t r = 0; r < world; ++r) {
-      hml_shard *sh = group[r];
-      cudaSetDevice(sh->ctx->device);
-      if ((rc = hml_shard_wait(sh->ctx, sh->fl, grp * world, sh->host_epoch[grp], world, (void *)stream_of(r)))) return rc;
-    }
-    return HML_OK;
-  };
-  int rc;
-  if (op_kind == SOP_RESCALE && group[0]->rb_dirty && (rc = exchange(2))) return rc;
+  if (op_kind == SOP_RESCALE && group[0]->rb_dirty && (rc = group_exchange(group, world, emulate, streams, 2))) return rc;
   const int n = op_phases(op_kind);
   for (int ph = 0; ph < n; ++ph) {
     for (uint32_t r = 0; r < world; ++r) {
       cudaSetDevice(group[r]->ctx->device);
-      if ((rc = run_phase(group[r], ops[r], ph, stream_of(r)))) return rc;
+      if ((rc = run_phase(group[r], ops[r], ph, group_stream(streams, r)))) return rc;
     }
-    if (ph + 1 < n && (rc = exchange(op_exchange(op_kind, ph)))) return rc;
+    if (ph + 1 < n && (rc = group_exchange(group, world, emulate, streams, op_exchange(op_kind, ph)))) return rc;
   }
   for (uint32_t r = 0; r < world; ++r) group[r]->rb_dirty = op_kind == SOP_RESCALE;
+  return HML_OK;
+}
+
+// hml_hrotate_hoisted_sharded for every rank of a local group; rotkeys_own / outs_own are rank-major ([rank * n_rot + i])
+extern "C" int hml_group_hrotate_hoisted(hml_shard *const *group, uint32_t world, uint32_t L, const uint64_t *const *ct_own, uint32_t n_rot,
+                                         const uint64_t *const *rotkeys_own, const uint64_t *galois_elts, uint64_t *const *outs_own,
+                                         void *const *streams) {
+  if (!group || world == 0 || !ct_own) return HML_ERR_INVALID;
+  bool emulate;
+  int rc = group_setup(group, world, streams, &emulate);
+  if (rc) return rc;
+  if (n_rot == 0) return HML_OK;
+  if (!outs_own) return fail(group[0]->ctx, HML_ERR_INVALID, "null output");
+  std::vector<HoistOp> ops(world);
+  for (uint32_t r = 0; r < world; ++r) {
+    if (group[r]->max_rot != group[0]->max_rot) return fail(group[r]->ctx, HML_ERR_INVALID, "every rank of a shard group must use the same max_rot");
+    ops[r] = HoistOp{L, n_rot, ct_own[r], rotkeys_own ? rotkeys_own + (size_t)r * n_rot : nullptr, galois_elts, outs_own + (size_t)r * n_rot};
+    if ((rc = hoist_check(group[r], ops[r]))) return rc;
+  }
+  for (uint32_t r = 0; r < world; ++r)  // before the first exchange: nothing may allocate or synchronise while a rank waits
+    if ((rc = hoist_prepare(group[r], L))) return rc;
+  for (const HoistStep &st : hoist_steps(n_rot, group[0]->max_rot)) {
+    if (st.kind == HS_X0 || st.kind == HS_X1) {
+      if ((rc = group_exchange(group, world, emulate, streams, st.kind == HS_X0 ? 0 : 1))) return rc;
+      continue;
+    }
+    for (uint32_t r = 0; r < world; ++r) {
+      cudaSetDevice(group[r]->ctx->device);
+      if ((rc = hoist_phase(group[r], ops[r], st, group_stream(streams, r)))) return rc;
+    }
+  }
+  for (uint32_t r = 0; r < world; ++r) group[r]->rb_dirty = false;
   return HML_OK;
 }

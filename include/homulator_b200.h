@@ -213,6 +213,12 @@ int hml_ipc_close(hml_ctx *ctx, uint64_t *ptr);
  * Every rank of the group must issue the same sequence of sharded calls. */
 typedef struct hml_shard hml_shard;
 int hml_shard_create(hml_ctx *ctx, uint32_t max_L, uint32_t rank, uint32_t world, hml_shard **out);
+/* The same with room for max_rot (1..16) hoisted rotations per exchange (hml_hrotate_hoisted_sharded): gather buffer 2 holds
+ * max_rot slots of the key switch's size, back to back (about 2 * alpha * N * 8 bytes per slot and rank), and
+ * hml_shard_prepare sizes the workspace for max_rot rotations.  hml_shard_create is max_rot = 1.  Every rank of a group must
+ * use the same max_rot (the slots are addressed at the same offsets in every rank's buffer): hml_shard_connect_local rejects
+ * mixed values; IPC groups must agree on it before they exchange handles. */
+int hml_shard_create_ex(hml_ctx *ctx, uint32_t max_L, uint32_t rank, uint32_t world, uint32_t max_rot, hml_shard **out);
 int hml_shard_destroy(hml_shard *sh);
 int hml_shard_handles(hml_shard *sh, unsigned char *out_4x64);
 int hml_shard_connect_ipc(hml_shard *sh, const unsigned char *handles_world_4x64);
@@ -237,6 +243,19 @@ int hml_ew_sharded(hml_shard *sh, uint32_t L, int kind, const uint64_t *a_own, c
  * with separate signal / wait launches, so no kernel ever spins on a flag a not-yet-launched kernel has to write. */
 int hml_group_op(hml_shard *const *group, uint32_t world, int op_kind, uint32_t L, const uint64_t *const *a, const uint64_t *const *b,
                  const uint64_t *const *key, uint64_t *const *out0, uint64_t *const *out1, uint64_t galois_elt, void *const *streams);
+/* Hoisted rotations of ONE limb-sharded ciphertext (one call per rank, like hml_hrotate_sharded): ct_own [2][nq][N] ->
+ * outs_own[r] [2][nq][N] = (sigma_r(c0) + ks0, ks1) on the owned limbs, bit-identical to the owned rows of hml_hrotate_hoisted.
+ * One ModUp of c1 and its two exchanges serve all n_rot rotations; groups of up to max_rot rotations (hml_shard_create_ex)
+ * share one inner-product launch, one P-limb INTT and one exchange.  rotkeys_own / galois_elts / outs_own are HOST arrays of
+ * n_rot entries (owned key slices, word keys); a key may be null on a rank that owns no extended limb.  n_rot = 0 is a no-op;
+ * no output may alias the input. */
+int hml_hrotate_hoisted_sharded(hml_shard *sh, uint32_t L, const uint64_t *ct_own, uint32_t n_rot, const uint64_t *const *rotkeys_own,
+                                const uint64_t *galois_elts, uint64_t *const *outs_own, void *stream);
+/* The same for all ranks of a local group from one host thread (as hml_group_op): ct_own and streams are indexed by rank,
+ * rotkeys_own and outs_own rank-major ([rank * n_rot + i]). */
+int hml_group_hrotate_hoisted(hml_shard *const *group, uint32_t world, uint32_t L, const uint64_t *const *ct_own, uint32_t n_rot,
+                              const uint64_t *const *rotkeys_own, const uint64_t *galois_elts, uint64_t *const *outs_own,
+                              void *const *streams);
 
 /* ------------------------------------------------------------------ operations (reference include/Operation.h) */
 /* HMULT (reference src/Operation.cpp:913-1023): tensor + keyswitch(relinearise) + add + rescale x2.
@@ -306,7 +325,8 @@ int hml_host_free_pinned(hml_ctx *ctx, uint64_t *ptr);
  *   HROTATE dst = rotate(a, 5^b)   (needs the key bound for rotation amount b)      PMULT / PADD dst = a (*|+) plaintext[b]
  *   HADD    dst = a + slot b                                                     HMULT dst = rescale(relin(a * slot b))
  * flags: HML_REPLAY_GRAPH — the whole sequence is captured once into a CUDA graph (after a warm-up run) and every run is one
- * graph launch; HML_REPLAY_HOIST — consecutive rotations of one source share a ModUp (hml_hrotate_hoisted; sh == NULL only).
+ * graph launch; HML_REPLAY_HOIST — consecutive rotations of one source share a ModUp (hml_hrotate_hoisted, or
+ * hml_hrotate_hoisted_sharded when sh != NULL).
  * With sh != NULL the trace runs limb-sharded: every pointer is the rank's owned-limb slice (see the sharded layouts above). */
 enum { HML_OP_HROTATE = 0, HML_OP_PMULT = 1, HML_OP_HADD = 2, HML_OP_PADD = 3, HML_OP_HMULT = 4 };
 enum { HML_REPLAY_GRAPH = 1, HML_REPLAY_HOIST = 2 };
