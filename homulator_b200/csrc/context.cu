@@ -15,6 +15,32 @@
 
 using namespace hml;
 
+// Strided view of `nb` independent polynomials / ciphertext halves: item b lives at ptr + b * stride (words).
+struct BatchPtr {
+  const u64 *ptr;
+  long long stride;
+};
+struct BatchOut {
+  u64 *ptr;
+  long long stride;
+};
+
+// hrotate on two-pass rings: the automorphism rides on the key switch's loads instead of a kernel of its own.  d and add0 are
+// the RAW polynomials; the ModUp INTT reads d through sigma_g and leaves sigma_g(d) in sigma_d (item b at + b * sigma_stride)
+// for the inner product's own-digit term; the ModDown epilogue reads add0 through sigma_g.
+struct KsAuto {
+  u64 g;
+  u64 *sigma_d;
+  long long sigma_stride;
+};
+
+// hmult's merged ModDown + Rescale: the addend d_c[L-1] of u[L-1] = acc_c[L-1] * P^-1 + d_c[L-1] (packed limbs; component c at
+// add + c * comp_stride, ciphertext b at + b * batch_stride)
+struct MergedU {
+  const u64 *add;
+  long long comp_stride, batch_stride;
+};
+
 static thread_local std::string g_create_err;
 
 #define CU_TRY(ctx, call)                                                                          \
@@ -142,6 +168,101 @@ static void run_bconv(hml_ctx *ctx, const hml::HostBConv &hb, const LimbMap &src
   prof_mark(ctx, HML_CLS_BCONV, s);
   ctx->exec.kernel_launches++;
   ctx->exec.bconv_limb_macs += (uint64_t)hb.n_src * hb.n_dst * a.n_batches;
+}
+
+// A forward or inverse transform and its counters: n_batch x the (poly, limb) pairs that the map does not skip
+static void run_ntt(hml_ctx *ctx, bool inverse, const LimbMap &lm, const NttLaunch &l, cudaStream_t s) {
+  if (inverse) launch_ntt_inverse(ctx->tabs, ctx->p.logN, lm, l, s);
+  else launch_ntt_forward(ctx->tabs, ctx->p.logN, lm, l, s);
+  prof_mark(ctx, inverse ? HML_CLS_INTT : HML_CLS_NTT, s);
+  uint64_t limbs = 0;
+  for (int poly = 0; poly < l.n_polys; ++poly)
+    for (int k = 0; k < l.n_limbs; ++k) limbs += lm.skip[k] != poly;
+  (inverse ? ctx->exec.intt_limbs : ctx->exec.ntt_limbs) += limbs * l.n_batch;
+  ctx->exec.kernel_launches += ctx->p.logN <= NTT_SMALL_LOG ? 1 : 2;
+}
+
+// K9 + K10 of a ModDown, and the transform + subtract of a rescale: the forward transform of l, then for every poly
+// p = b * n_c + c of it  dst_c[b] = (x_c[b] - NTT(in)_p) * cst (+ z_c[b] when bit c of z_mask is set), as l.fuse describes.
+// Two-pass rings run it as the transform's fused epilogue.  Single-pass rings store the transform in l.out and run
+// k_sub_mul_add over the same description: one launch when n_b = 1 (the components are its polys), else one per component.
+static int ntt_sub_mul(hml_ctx *ctx, const LimbMap &lm, NttLaunch l, cudaStream_t s) {
+  const NttFuse f = l.fuse;
+  if (ctx->p.logN > NTT_SMALL_LOG) {
+    run_ntt(ctx, false, lm, l, s);
+    return HML_OK;
+  }
+  if (f.z_galois) return fail(ctx, HML_ERR_INVALID, "automorphism on the addend needs the fused ModDown epilogue");
+  l.fuse = NttFuse{};
+  run_ntt(ctx, false, lm, l, s);
+  SubMulArgs a{};
+  a.cst = f.cst; a.N = ctx->p.N; a.n_limbs = l.n_limbs; a.x_packed = f.x_packed; a.z_packed = f.z_packed;
+  const int n_b = l.n_polys / f.n_c;
+  if (n_b == 1) {
+    a.x = f.x; a.x_poly_stride = f.x_c_stride;
+    a.y = l.out; a.y_poly_stride = l.out_poly_stride;
+    a.z = f.z_mask ? f.z : nullptr; a.z_poly_stride = f.z_c_stride; a.z_mask = f.z_mask;
+    a.out = f.dst; a.out_poly_stride = f.dst_c_stride; a.n_polys = f.n_c;
+    launch_sub_mul_add(ctx->mc, lm, a, s);
+    prof_mark(ctx, HML_CLS_EWE, s);
+    ctx->exec.kernel_launches++;
+    return HML_OK;
+  }
+  for (int c = 0; c < f.n_c; ++c) {
+    a.x = f.x + c * f.x_c_stride; a.x_poly_stride = f.x_b_stride;
+    a.y = l.out + c * l.out_poly_stride; a.y_poly_stride = f.n_c * l.out_poly_stride;
+    a.z = (f.z_mask >> c) & 1u ? f.z + c * f.z_c_stride : nullptr; a.z_poly_stride = f.z_b_stride;
+    a.out = f.dst + c * f.dst_c_stride; a.out_poly_stride = f.dst_b_stride; a.n_polys = n_b;
+    launch_sub_mul_add(ctx->mc, lm, a, s);
+    prof_mark(ctx, HML_CLS_EWE, s);
+    ctx->exec.kernel_launches++;
+  }
+  return HML_OK;
+}
+
+// Device job table of the one-launch ModUp: digit j reads its sources at in + j * in_step (slots 0.., or through
+// (*src_off)[j]) and writes at out + j * out_step.  Left null for one digit or a digit the multi-conversion form cannot take.
+static int upload_up_jobs(hml_ctx *ctx, const std::vector<HostBConv> &up, long long in_step, long long out_step,
+                          const std::vector<long long *> *src_off, BConvJob **out) {
+  *out = nullptr;
+  if (up.size() < 2) return HML_OK;
+  std::vector<BConvJob> jobs(up.size());
+  for (size_t j = 0; j < up.size(); ++j) {
+    const HostBConv &hb = up[j];
+    if (!hb.d_img || hb.n_src > 48 || hb.n_dst > 48) return HML_OK;
+    BConvJob &jb = jobs[j];
+    memset(&jb, 0, sizeof(jb));
+    for (int i = 0; i < hb.n_src; ++i) jb.src_pos[i] = (uint16_t)i;
+    for (int t = 0; t < hb.n_dst; ++t) { jb.dst_mod[t] = hb.dst_lm.mod[t]; jb.dst_pos[t] = hb.dst_lm.pos[t]; }
+    jb.img = hb.d_img; jb.K = hb.im.K; jb.NP = hb.im.NP; jb.ND = hb.im.ND; jb.n_src = hb.n_src; jb.n_dst = hb.n_dst;
+    jb.in_off = (long long)j * in_step; jb.out_off = (long long)j * out_step; jb.src_off = src_off ? (*src_off)[j] : nullptr;
+  }
+  return upload(ctx, jobs, out);
+}
+
+// The ModUp conversions (K3) of every digit j: up[j] from `a.in + j * in_step` (source map src_lm[j], offsets (*src_off)[j]
+// when given) to `a.out + j * out_step`.  ONE launch for all digits when a job table is given and the tcgen05 kernel's
+// multi-conversion form takes it (every CTA serves one digit), else one launch per digit that has targets.
+static void run_modup_bconv(hml_ctx *ctx, const std::vector<HostBConv> &up, const std::vector<LimbMap> &src_lm, const BConvJob *jobs,
+                            const std::vector<long long *> *src_off, const BConvArgs &a, long long in_step, long long out_step, cudaStream_t s) {
+  const int beta = (int)up.size();
+  if (jobs) {
+    std::vector<BConvImage> ims(beta);
+    std::vector<int> nd(beta);
+    for (int j = 0; j < beta; ++j) { ims[j] = up[j].im; nd[j] = up[j].n_dst; }
+    if (launch_bconv_umma_multi(ctx->mc, jobs, ims.data(), nd.data(), beta, a, s)) {
+      prof_mark(ctx, HML_CLS_BCONV, s);
+      ctx->exec.kernel_launches++;
+      for (int j = 0; j < beta; ++j) ctx->exec.bconv_limb_macs += (uint64_t)up[j].n_src * up[j].n_dst * a.n_batches;
+      return;
+    }
+  }
+  for (int j = 0; j < beta; ++j) {
+    if (up[j].empty()) continue;
+    BConvArgs aj = a;
+    aj.in = a.in + j * in_step; aj.out = a.out + j * out_step; aj.src_off = src_off ? (*src_off)[j] : nullptr;
+    run_bconv(ctx, up[j], src_lm[j], aj, s);
+  }
 }
 
 // ------------------------------------------------------------------------------------------------ creation
@@ -306,24 +427,24 @@ int ensure_ws(hml_ctx *ctx, size_t words) {
   return HML_OK;
 }
 
-int check_launch(hml_ctx *ctx, const char *what) {
+static int check_launch(hml_ctx *ctx, const char *what) {
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { ctx->err = std::string(what) + ": " + cudaGetErrorString(e); return HML_ERR_CUDA; }
   return HML_OK;
 }
 
-void clear_map(LimbMap &lm) {
+static void clear_map(LimbMap &lm) {
   memset(&lm, 0, sizeof(lm));
   memset(lm.skip, 0xFF, sizeof(lm.skip));
 }
 
-void id_map(LimbMap &lm, const uint32_t *mod_idx, uint32_t n) {
+static void id_map(LimbMap &lm, const uint32_t *mod_idx, uint32_t n) {
   clear_map(lm);
   for (uint32_t i = 0; i < n; ++i) { lm.mod[i] = (uint16_t)mod_idx[i]; lm.pos[i] = (uint16_t)i; }
 }
 
 // ------------------------------------------------------------------------------------------------ per-level constants
-int get_level(hml_ctx *ctx, uint32_t L, LevelConsts **out) {
+static int get_level(hml_ctx *ctx, uint32_t L, LevelConsts **out) {
   auto it = ctx->levels.find(L);
   if (it != ctx->levels.end()) { *out = &it->second; return HML_OK; }
   const Params &p = ctx->p;
@@ -336,6 +457,7 @@ int get_level(hml_ctx *ctx, uint32_t L, LevelConsts **out) {
   int rc;
   // ---- ModUp
   std::vector<double2> up_scale(L);
+  for (uint32_t i = 0; i < L; ++i) up_scale[i] = mk_cst(p.modup_scale(L, i), p.mod[i]);
   for (uint32_t e = 0; e < E; ++e) {
     lc.ext_lm.mod[e] = p.ext_mod(L, e); lc.ext_lm.pos[e] = e;
     lc.ext_lm.skip[e] = e < L ? (uint8_t)(e / A) : 0xFF;  // digit j owns limbs [j*alpha, j*alpha + a_j)
@@ -351,30 +473,13 @@ int get_level(hml_ctx *ctx, uint32_t L, LevelConsts **out) {
     }
     BConvTable bt;
     make_bconv_table(p, src, dst, bt);
-    for (uint32_t i = 0; i < aj; ++i) {
-      const u64 q = p.mod[lo + i];
-      up_scale[lo + i] = mk_cst(h_mulmod(p.n_inv[lo + i], bt.hat_inv[i], q), q);
-    }
     lc.up.emplace_back();
+    lc.up_src.push_back(lc.q_lm);
     if ((rc = prepare_bconv(ctx, bt, dst_pos, lc.up.back()))) return rc;
   }
   if ((rc = upload(ctx, up_scale, &lc.modup_scale))) return rc;
-  {  // job table of the merged ModUp launch (sources at yb + j * alpha limbs, targets at ext + j * E limbs)
-    std::vector<BConvJob> jobs(beta);
-    bool ok = beta >= 2;
-    for (uint32_t j = 0; j < beta && ok; ++j) {
-      const HostBConv &hb = lc.up[j];
-      ok = hb.d_img != nullptr && hb.n_src <= 48 && hb.n_dst <= 48;
-      if (!ok) break;
-      BConvJob &jb = jobs[j];
-      memset(&jb, 0, sizeof(jb));
-      for (int i = 0; i < hb.n_src; ++i) jb.src_pos[i] = (uint16_t)i;
-      for (int t = 0; t < hb.n_dst; ++t) { jb.dst_mod[t] = hb.dst_lm.mod[t]; jb.dst_pos[t] = hb.dst_lm.pos[t]; }
-      jb.img = hb.d_img; jb.K = hb.im.K; jb.NP = hb.im.NP; jb.ND = hb.im.ND; jb.n_src = hb.n_src; jb.n_dst = hb.n_dst;
-      jb.in_off = (long long)j * A * p.N; jb.out_off = (long long)j * E * p.N;
-    }
-    if (ok && (rc = upload(ctx, jobs, &lc.up_jobs))) return rc;
-  }
+  // the merged ModUp launch: sources at yb + j * alpha limbs, targets at ext + j * E limbs
+  if ((rc = upload_up_jobs(ctx, lc.up, (long long)A * p.N, (long long)E * p.N, nullptr, &lc.up_jobs))) return rc;
   // ---- ModDown
   {
     std::vector<uint32_t> src, dst;
@@ -383,16 +488,8 @@ int get_level(hml_ctx *ctx, uint32_t L, LevelConsts **out) {
     BConvTable bt;
     make_bconv_table(p, src, dst, bt);
     std::vector<double2> sc(A), pinv(L);
-    for (uint32_t j = 0; j < A; ++j) {
-      const u64 q = p.mod[p.max_level + j];
-      sc[j] = mk_cst(h_mulmod(p.n_inv[p.max_level + j], bt.hat_inv[j], q), q);
-    }
-    for (uint32_t i = 0; i < L; ++i) {
-      const u64 q = p.mod[i];
-      u64 P = 1;
-      for (uint32_t j = 0; j < A; ++j) P = h_mulmod(P, p.mod[p.max_level + j] % q, q);
-      pinv[i] = mk_cst(h_invmod(P, q), q);
-    }
+    for (uint32_t j = 0; j < A; ++j) sc[j] = mk_cst(p.moddown_scale(j), p.mod[p.max_level + j]);
+    for (uint32_t i = 0; i < L; ++i) pinv[i] = mk_cst(p.p_inv(i), p.mod[i]);
     if ((rc = prepare_bconv(ctx, bt, dst, lc.down))) return rc;
     if ((rc = upload(ctx, sc, &lc.moddown_scale))) return rc;
     if ((rc = upload(ctx, pinv, &lc.pinv))) return rc;
@@ -411,12 +508,7 @@ int get_level(hml_ctx *ctx, uint32_t L, LevelConsts **out) {
     BConvTable bt;
     make_bconv_table(p, src, dst, bt);
     std::vector<u64> pinv_i(L);
-    for (uint32_t i = 0; i < L; ++i) {
-      const u64 q = p.mod[i];
-      u64 P = 1;
-      for (uint32_t j = 0; j < A; ++j) P = h_mulmod(P, p.mod[p.max_level + j] % q, q);
-      pinv_i[i] = h_invmod(P, q);
-    }
+    for (uint32_t i = 0; i < L; ++i) pinv_i[i] = p.p_inv(i);
     clear_map(lc.merged_src); clear_map(lc.last_lm);
     for (uint32_t j = 0; j < A; ++j) { lc.merged_src.mod[j] = p.max_level + j; lc.merged_src.pos[j] = L + j; }
     lc.merged_src.mod[A] = L - 1; lc.merged_src.pos[A] = E;  // the extra source lives in slot E of the accumulator
@@ -444,7 +536,7 @@ int get_level(hml_ctx *ctx, uint32_t L, LevelConsts **out) {
   // ---- Rescale
   {
     std::vector<double2> ql(L > 1 ? L - 1 : 0);
-    for (uint32_t l = 0; l + 1 < L; ++l) ql[l] = mk_cst(h_invmod(p.mod[L - 1] % p.mod[l], p.mod[l]), p.mod[l]);
+    for (uint32_t l = 0; l + 1 < L; ++l) ql[l] = mk_cst(p.ql_inv(L, l), p.mod[l]);
     if ((rc = upload(ctx, ql, &lc.qlinv))) return rc;
   }
   auto ins = ctx->levels.emplace(L, lc);
@@ -475,12 +567,8 @@ static int ntt_api(hml_ctx *ctx, bool inverse, const uint64_t *in, uint64_t *out
     l.n_batch = 1;
     l.in = (const u64 *)in + off * N; l.out = (u64 *)out + off * N;
     l.in_limb_stride = l.out_limb_stride = N; l.n_limbs = n; l.n_polys = 1; l.post_scale = nullptr;
-    if (inverse) launch_ntt_inverse(ctx->tabs, ctx->p.logN, lm, l, (cudaStream_t)stream);
-    else launch_ntt_forward(ctx->tabs, ctx->p.logN, lm, l, (cudaStream_t)stream);
-    prof_mark(ctx, inverse ? HML_CLS_INTT : HML_CLS_NTT, (cudaStream_t)stream);
-    ctx->exec.kernel_launches += ctx->p.logN <= NTT_SMALL_LOG ? 1 : 2;
+    run_ntt(ctx, inverse, lm, l, (cudaStream_t)stream);
   }
-  (inverse ? ctx->exec.intt_limbs : ctx->exec.ntt_limbs) += n_limbs;
   return check_launch(ctx, inverse ? "intt" : "ntt");
 }
 extern "C" int hml_ntt(hml_ctx *ctx, const uint64_t *in, uint64_t *out, const uint32_t *mod_idx, uint32_t n, void *s) {
@@ -509,12 +597,8 @@ static int ntt_batch_api(hml_ctx *ctx, bool inverse, const uint64_t *in, uint64_
     l.in = (const u64 *)in + (size_t)b0 * n_limbs * N; l.out = (u64 *)out + (size_t)b0 * n_limbs * N;
     l.in_limb_stride = l.out_limb_stride = N; l.n_limbs = n_limbs; l.n_polys = 1; l.post_scale = nullptr;
     l.n_batch = std::min(per, n_batch - b0); l.in_batch_stride = l.out_batch_stride = (long long)n_limbs * N;
-    if (inverse) launch_ntt_inverse(ctx->tabs, ctx->p.logN, lm, l, (cudaStream_t)stream);
-    else launch_ntt_forward(ctx->tabs, ctx->p.logN, lm, l, (cudaStream_t)stream);
-    prof_mark(ctx, inverse ? HML_CLS_INTT : HML_CLS_NTT, (cudaStream_t)stream);
-    ctx->exec.kernel_launches += ctx->p.logN <= NTT_SMALL_LOG ? 1 : 2;
+    run_ntt(ctx, inverse, lm, l, (cudaStream_t)stream);
   }
-  (inverse ? ctx->exec.intt_limbs : ctx->exec.ntt_limbs) += (uint64_t)n_limbs * n_batch;
   return check_launch(ctx, inverse ? "intt batch" : "ntt batch");
 }
 extern "C" int hml_ntt_batch(hml_ctx *ctx, const uint64_t *in, uint64_t *out, const uint32_t *mod_idx, uint32_t n, uint32_t nb, void *s) {
@@ -600,7 +684,7 @@ extern "C" int hml_bconv(hml_ctx *ctx, const uint64_t *in, const uint32_t *src_i
 }
 
 // ------------------------------------------------------------------------------------------------ key switch
-size_t ks_ws_words(const Params &p, uint32_t L) {
+static size_t ks_ws_words(const Params &p, uint32_t L) {
   const size_t N = p.N, E = L + p.alpha;
   return N * (L + (size_t)p.beta(L) * E + 2 * E + 2 * (size_t)L);
 }
@@ -611,15 +695,16 @@ size_t ks_ws_words(const Params &p, uint32_t L) {
 // hmult 245 -> 233 us, hrotate 249 -> 227 us): there the stand-alone inner product is latency-bound on the 150 MB key.  In a
 // 32-ciphertext chunk the key is read once per chunk and k_inner streams at the HBM rate, while the row pass is bound by the
 // FP64 pipe and the fused multiply-accumulates (+45 % FP64 work) land exactly there: 168 -> 178 us per hmult.
-bool ks_uses_hpip(const hml_ctx *ctx, uint32_t L, uint32_t nb) {
+static bool ks_uses_hpip(const hml_ctx *ctx, uint32_t L, uint32_t nb) {
   return ctx->p.logN > NTT_SMALL_LOG && ctx->p.beta(L) >= 2 && nb == 1;
 }
 
-int ks_modup(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, u64 *yb, u64 *ext, cudaStream_t s, const NttMac *mac, const KsAuto *au) {
+static int ks_modup(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, u64 *yb, u64 *ext, cudaStream_t s, const NttMac *mac = nullptr,
+                    const KsAuto *au = nullptr) {
   const Params &p = ctx->p;
   const size_t N = p.N;
   const uint32_t A = p.alpha, E = L + A, beta = lc->beta;
-  const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
+  const bool two_pass = p.logN > NTT_SMALL_LOG;
   // K1 + K2 (reference :63-135): INTT of the input, digit scaling folded into the N^-1 multiply
   {
     NttLaunch l{};
@@ -632,34 +717,16 @@ int ks_modup(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d,
       l.in_galois = (unsigned)(au->g & (2ull * N - 1)); l.in_ginv8 = gi & 255u;
       l.side_out = au->sigma_d; l.side_batch_stride = au->sigma_stride;
     }
-    launch_ntt_inverse(ctx->tabs, logN, lc->q_lm, l, s);
-    prof_mark(ctx, HML_CLS_INTT, s);
-    ctx->exec.intt_limbs += (uint64_t)nb * L; ctx->exec.kernel_launches += npass;
+    run_ntt(ctx, true, lc->q_lm, l, s);
   }
-  // K3 (reference :137-188): convert every digit to the limbs of the extended basis it does not own — ONE launch for all
-  // digits when they fit the tcgen05 kernel's multi-conversion form (every CTA serves one digit), else one launch per digit
-  bool merged_up = false;
-  if (lc->up_jobs && beta >= 2 && nb <= 4) {  // big chunks amortise the per-launch set-up anyway and run 3 % faster digit by digit
+  // K3 (reference :137-188): convert every digit to the limbs of the extended basis it does not own
+  {
     BConvArgs a{};
     a.in = yb; a.out = ext; a.step1 = nullptr; a.N = N; a.n_batches = nb;
-    a.in_batch_stride = (long long)L * N; a.out_batch_stride = (long long)beta * E * N; a.out_f64 = npass == 2;
-    std::vector<BConvImage> ims(beta);
-    std::vector<int> nd(beta);
-    for (uint32_t j = 0; j < beta; ++j) { ims[j] = lc->up[j].im; nd[j] = lc->up[j].n_dst; }
-    merged_up = launch_bconv_umma_multi(ctx->mc, lc->up_jobs, ims.data(), nd.data(), (int)beta, a, s);
-    if (merged_up) {
-      prof_mark(ctx, HML_CLS_BCONV, s);
-      ctx->exec.kernel_launches++;
-      for (uint32_t j = 0; j < beta; ++j) ctx->exec.bconv_limb_macs += (uint64_t)lc->up[j].n_src * lc->up[j].n_dst * nb;
-    }
-  }
-  for (uint32_t j = 0; j < beta && !merged_up; ++j) {
-    const uint32_t lo = j * A;
-    BConvArgs a{};
-    a.in = yb + (size_t)lo * N; a.out = ext + (size_t)j * E * N; a.step1 = nullptr;
-    a.N = N; a.n_batches = nb; a.in_batch_stride = (long long)L * N; a.out_batch_stride = (long long)beta * E * N;
-    a.out_f64 = npass == 2;  // hand-off to the forward NTT as doubles
-    run_bconv(ctx, lc->up[j], lc->q_lm, a, s);
+    a.in_batch_stride = (long long)L * N; a.out_batch_stride = (long long)beta * E * N;
+    a.out_f64 = two_pass;  // hand-off to the forward NTT as doubles
+    // the one-launch form only for small chunks: big ones amortise the per-launch set-up anyway and run 3 % faster digit by digit
+    run_modup_bconv(ctx, lc->up, lc->up_src, nb <= 4 ? lc->up_jobs : nullptr, nullptr, a, (long long)A * N, (long long)E * N, s);
   }
   // K4 (reference :190-292): NTT of the converted limbs.  The digit's own limbs are the untouched input
   // (delta D3: the reference also counts an NTT for those).
@@ -668,22 +735,20 @@ int ks_modup(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d,
     l.in = ext; l.out = ext; l.in_limb_stride = l.out_limb_stride = N; l.in_poly_stride = l.out_poly_stride = (long long)E * N;
     l.n_limbs = E; l.n_polys = beta;  // digit j skips the limbs it owns (LimbMap::skip)
     l.n_batch = nb; l.in_batch_stride = l.out_batch_stride = (long long)beta * E * N;
-    l.in_f64 = l.out_f64 = npass == 2;  // doubles in from the conversion, raw lazy doubles out to the inner product
+    l.in_f64 = l.out_f64 = two_pass;  // doubles in from the conversion, raw lazy doubles out to the inner product
     if (mac) {  // K5 rides in the row pass (HPIP analogue): the transformed digits are multiplied by the key and never stored
       l.mac = *mac;
       ctx->exec.ewe_limbs += 2ull * nb * E * beta;
     }
-    launch_ntt_forward(ctx->tabs, logN, lc->ext_lm, l, s);
-    prof_mark(ctx, HML_CLS_NTT, s);
-    ctx->exec.ntt_limbs += (uint64_t)nb * ((uint64_t)beta * E - L); ctx->exec.kernel_launches += npass;
+    run_ntt(ctx, false, lc->ext_lm, l, s);
   }
   return HML_OK;
 }
 
 // K5..K7: inner product with the key, INTT (+ step-1 scaling) of the P-limbs of both accumulators.  acc [nb][2][AL], AL >= E.
 // galois != 0: the digits are read through the automorphism X -> X^galois (hoisted rotation, see InnerArgs::galois).
-int ks_inner(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, const u64 *evk, uint32_t evk_q_limbs, const u64 *ext, u64 *acc,
-             uint32_t AL, u64 galois, cudaStream_t s, const MergedU *mu, bool ip_done) {
+static int ks_inner(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, const u64 *evk, uint32_t evk_q_limbs, const u64 *ext, u64 *acc,
+                    uint32_t AL, u64 galois, cudaStream_t s, const MergedU *mu = nullptr, bool ip_done = false) {
   const Params &p = ctx->p;
   const size_t N = p.N;
   const uint32_t A = p.alpha, E = L + A, beta = lc->beta;
@@ -736,9 +801,7 @@ int ks_inner(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d,
     l.in = acc; l.out = acc; l.in_limb_stride = l.out_limb_stride = N; l.in_poly_stride = l.out_poly_stride = (long long)AL * N;
     l.n_limbs = A + (mu ? 1 : 0); l.n_polys = 2 * nb; l.post_scale = mu ? lc->moddown_scale_u : lc->moddown_scale;  // acc is [nb][2][AL][N]
     l.n_batch = 1;
-    launch_ntt_inverse(ctx->tabs, logN, mu ? lc->pu_lm : lc->p_lm, l, s);
-    prof_mark(ctx, HML_CLS_INTT, s);
-    ctx->exec.intt_limbs += 2ull * nb * l.n_limbs; ctx->exec.kernel_launches += npass;
+    run_ntt(ctx, true, mu ? lc->pu_lm : lc->p_lm, l, s);
   }
   return HML_OK;
 }
@@ -746,8 +809,8 @@ int ks_inner(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d,
 // K1..K7.  Buffers: yb [nb][L] | ext [nb][beta][E] | acc [nb][2][AL] with AL >= E limbs per accumulator.
 // Two-pass rings with at least two digits fuse the inner product into the ModUp transform (NttMac): the Q-limb accumulators are
 // then 8-byte words (not packed limbs); ks_uses_hpip() tells the consumers.
-int ks_front(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, const u64 *evk, uint32_t evk_q_limbs, u64 *yb,
-             u64 *ext, u64 *acc, uint32_t AL, cudaStream_t s, const MergedU *mu, const KsAuto *au) {
+static int ks_front(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, const u64 *evk, uint32_t evk_q_limbs, u64 *yb,
+                    u64 *ext, u64 *acc, uint32_t AL, cudaStream_t s, const MergedU *mu = nullptr, const KsAuto *au = nullptr) {
   const Params &p = ctx->p;
   const size_t N = p.N;
   const uint32_t A = p.alpha, E = L + A;
@@ -774,66 +837,51 @@ int ks_front(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d,
   return ks_inner(ctx, lc, L, nb, d, evk, evk_flagged, ext, acc, AL, 0, s, mu, hpip);
 }
 
-// K8..K10 (+ the caller's addends): ModDown of nb accumulator pairs acc [nb][2][E] -> out_c[b] = (acc_c - NTT(BConv(acc_c; P -> Q))) * P^-1 (+ add_c[b])
-int ks_tail(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, u64 *acc, u64 *vb, BatchOut out0, BatchOut out1, BatchPtr add0, BatchPtr add1,
-            cudaStream_t s, bool acc_packed, u64 add0_galois) {
+// The addends of a ModDown epilogue: component 0 reads z0, component 1 reads z1 (either may be null)
+static void set_addends(NttFuse &f, const u64 *z0, const u64 *z1) {
+  f.z = z0 ? z0 : z1;
+  f.z_c_stride = z0 && z1 ? (long long)(z1 - z0) : 0;
+  f.z_mask = (z0 ? 1u : 0u) | (z1 ? 2u : 0u);
+}
+
+// K8..K10 (+ the caller's addends): ModDown of nb accumulator pairs acc [nb][2][E] -> out_c[b] = (acc_c - NTT(BConv(acc_c; P -> Q))) * P^-1 (+ add_c[b]).
+// out0 / out1 and add0 / add1 share one batch stride.
+static int ks_tail(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, u64 *acc, u64 *vb, BatchOut out0, BatchOut out1, BatchPtr add0, BatchPtr add1,
+                   cudaStream_t s, bool acc_packed, u64 add0_galois) {
   const Params &p = ctx->p;
   const size_t N = p.N;
   const uint32_t A = p.alpha, E = L + A;
-  const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
+  const bool two_pass = p.logN > NTT_SMALL_LOG;
   // K8 (reference :489-519): P -> Q_L
   {
     BConvArgs a{};
     a.in = acc; a.out = vb; a.in_batch_stride = (long long)E * N; a.out_batch_stride = (long long)L * N;  // p_lm.pos = L + j
-    a.step1 = nullptr; a.N = N; a.n_batches = 2 * nb; a.out_f64 = npass == 2;
+    a.step1 = nullptr; a.N = N; a.n_batches = 2 * nb; a.out_f64 = two_pass;
     run_bconv(ctx, lc->down, lc->p_lm, a, s);
   }
+  if (add0_galois && (!add0.ptr || add1.ptr)) return fail(ctx, HML_ERR_INVALID, "automorphism on the addend needs the fused ModDown epilogue");
   // K9 (reference :521-546, emitted with opcode INTT — delta D1): forward NTT of the converted limbs, and
-  // K10 (reference :548-590) (+ the caller's addend: HMULT add :967-1005 / HROTATE add :1339-1357).
-  // Two-pass rings fuse K10 into the transform's row pass (NttFuse): v-hat never reaches HBM.
-  const bool fuse = npass == 2 && out0.stride == out1.stride && (!add0.ptr || !add1.ptr || add0.stride == add1.stride);
-  if (add0_galois && (!fuse || !add0.ptr || add1.ptr)) return fail(ctx, HML_ERR_INVALID, "automorphism on the addend needs the fused ModDown epilogue");
-  {
-    NttLaunch l{};
-    l.in = vb; l.out = vb; l.in_limb_stride = l.out_limb_stride = N; l.in_poly_stride = l.out_poly_stride = (long long)L * N;
-    l.n_limbs = L; l.n_polys = 2 * nb; l.n_batch = 1; l.in_f64 = npass == 2;
-    if (fuse) {
-      NttFuse &f = l.fuse;
-      f.x = acc; f.x_c_stride = (long long)E * N; f.x_b_stride = 2ll * E * N; f.x_packed = acc_packed ? 1 : 0;
-      const BatchPtr zb = add0.ptr ? add0 : add1;  // component c reads zb.ptr + c * z_c_stride; only masked components are touched
-      f.z = zb.ptr; f.z_b_stride = zb.stride;
-      f.z_c_stride = (add0.ptr && add1.ptr) ? (long long)(add1.ptr - add0.ptr) : 0;
-      if (!add0.ptr && add1.ptr) f.z = add1.ptr;
-      f.z_mask = (add0.ptr ? 1u : 0u) | (add1.ptr ? 2u : 0u);
-      f.dst = out0.ptr; f.dst_c_stride = (long long)(out1.ptr - out0.ptr); f.dst_b_stride = out0.stride;
-      f.cst = lc->pinv; f.n_c = 2;
-      f.z_galois = (unsigned)(add0_galois & (2ull * N - 1));
-    }
-    launch_ntt_forward(ctx->tabs, logN, lc->q_lm, l, s);
-    prof_mark(ctx, HML_CLS_NTT, s);
-    ctx->exec.ntt_limbs += 2ull * nb * L; ctx->exec.kernel_launches += npass;
-    if (fuse) ctx->exec.ewe_limbs += (uint64_t)nb * (2 * L + (add0.ptr ? L : 0) + (add1.ptr ? L : 0));
-  }
-  for (int c = 0; c < 2 && !fuse; ++c) {
-    const BatchPtr add = c ? add1 : add0;
-    const BatchOut out = c ? out1 : out0;
-    SubMulArgs a{};
-    a.x = acc + (size_t)c * E * N; a.x_poly_stride = 2ll * E * N;
-    a.y = vb + (size_t)c * L * N; a.y_poly_stride = 2ll * L * N;
-    a.z = add.ptr; a.z_poly_stride = add.stride;
-    a.out = out.ptr; a.out_poly_stride = out.stride;
-    a.cst = lc->pinv; a.N = N; a.n_limbs = L; a.n_polys = nb; a.x_packed = acc_packed ? 1 : 0;
-    launch_sub_mul_add(ctx->mc, lc->q_lm, a, s);
-    prof_mark(ctx, HML_CLS_EWE, s);
-    ctx->exec.ewe_limbs += (uint64_t)nb * (L + (a.z ? L : 0)); ctx->exec.kernel_launches++;
-  }
+  // K10 (reference :548-590) (+ the caller's addend: HMULT add :967-1005 / HROTATE add :1339-1357)
+  NttLaunch l{};
+  l.in = vb; l.out = vb; l.in_limb_stride = l.out_limb_stride = N; l.in_poly_stride = l.out_poly_stride = (long long)L * N;
+  l.n_limbs = L; l.n_polys = 2 * nb; l.n_batch = 1; l.in_f64 = two_pass;
+  NttFuse &f = l.fuse;
+  f.x = acc; f.x_c_stride = (long long)E * N; f.x_b_stride = 2ll * E * N; f.x_packed = acc_packed ? 1 : 0;
+  set_addends(f, add0.ptr, add1.ptr);
+  f.z_b_stride = add0.ptr ? add0.stride : add1.stride;
+  f.dst = out0.ptr; f.dst_c_stride = (long long)(out1.ptr - out0.ptr); f.dst_b_stride = out0.stride;
+  f.cst = lc->pinv; f.n_c = 2;
+  f.z_galois = (unsigned)(add0_galois & (2ull * N - 1));
+  int rc = ntt_sub_mul(ctx, lc->q_lm, l, s);
+  if (rc) return rc;
+  ctx->exec.ewe_limbs += (uint64_t)nb * (2 * L + (add0.ptr ? L : 0) + (add1.ptr ? L : 0));
   return check_launch(ctx, "keyswitch");
 }
 
 // nb independent key switches sharing one key, one kernel launch per stage:
 // d[b] [L][N] -> out_c[b] = KS_c(d[b]) (+ add_c[b]).  `ws` must hold nb * ks_ws_words().
-int ks_run(hml_ctx *ctx, uint32_t L, uint32_t nb, BatchPtr d, const u64 *evk, uint32_t evk_q_limbs, BatchOut out0,
-           BatchOut out1, BatchPtr add0, BatchPtr add1, u64 *ws, cudaStream_t s, const KsAuto *au) {
+static int ks_run(hml_ctx *ctx, uint32_t L, uint32_t nb, BatchPtr d, const u64 *evk, uint32_t evk_q_limbs, BatchOut out0,
+                  BatchOut out1, BatchPtr add0, BatchPtr add1, u64 *ws, cudaStream_t s, const KsAuto *au = nullptr) {
   const Params &p = ctx->p;
   if ((evk_q_limbs & ~HML_KEY_PACKED) < L || (evk_q_limbs & ~HML_KEY_PACKED) > p.max_level) return fail(ctx, HML_ERR_INVALID, "evk_q_limbs must be in [L, maxLevel]");
   LevelConsts *lc;
@@ -885,7 +933,7 @@ extern "C" int hml_keyswitch(hml_ctx *ctx, uint32_t L, const uint64_t *d, const 
 //   end:    BConv P -> owned Q-limbs, NTT, (acc - v) * P^-1 for the owned Q-limbs
 // The collective itself is issued by the caller (NCCL all-gather on the same stream; homulator_b200/api.py uses
 // torch.distributed) so the library stays free of a communicator dependency.
-int get_shard_plan(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, ShardPlan **out) {
+static int get_shard_plan(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, ShardPlan **out) {
   const uint64_t key = ((uint64_t)L << 32) | ((uint64_t)world << 16) | rank;
   auto it = ctx->shard_plans.find(key);
   if (it != ctx->shard_plans.end()) { *out = &it->second; return HML_OK; }
@@ -902,25 +950,17 @@ int get_shard_plan(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, Shar
   clear_map(sp.q_lm); clear_map(sp.p_lm); clear_map(sp.e_lm);
   std::vector<double2> s1(nq), s2(np), pinv(nq);
   for (uint32_t k = 0; k < nq; ++k) {
-    const uint32_t i = sp.own_q[k], j = i / A, lo = j * A, aj = p.digit_size(L, j);
-    const u64 q = p.mod[i];
+    const uint32_t i = sp.own_q[k];
     sp.q_lm.mod[k] = i; sp.q_lm.pos[k] = k;
-    sp.e_lm.mod[k] = i; sp.e_lm.pos[k] = k; sp.e_lm.skip[k] = (uint8_t)j;
-    u64 hat = 1;  // (D_j / q_i)^-1 mod q_i
-    for (uint32_t t = lo; t < lo + aj; ++t) if (t != i) hat = h_mulmod(hat, p.mod[t] % q, q);
-    s1[k] = mk_cst(h_mulmod(p.n_inv[i], h_invmod(hat, q), q), q);
-    u64 P = 1;
-    for (uint32_t t = 0; t < A; ++t) P = h_mulmod(P, p.mod[p.max_level + t] % q, q);
-    pinv[k] = mk_cst(h_invmod(P, q), q);
+    sp.e_lm.mod[k] = i; sp.e_lm.pos[k] = k; sp.e_lm.skip[k] = (uint8_t)(i / A);
+    s1[k] = mk_cst(p.modup_scale(L, i), p.mod[i]);
+    pinv[k] = mk_cst(p.p_inv(i), p.mod[i]);
   }
   for (uint32_t k = 0; k < np; ++k) {
     const uint32_t j = sp.own_p[k], mi = p.max_level + j;
-    const u64 q = p.mod[mi];
     sp.p_lm.mod[k] = mi; sp.p_lm.pos[k] = nq + k;
     sp.e_lm.mod[nq + k] = mi; sp.e_lm.pos[nq + k] = nq + k;
-    u64 hat = 1;  // (P / p_j)^-1 mod p_j
-    for (uint32_t t = 0; t < A; ++t) if (t != j) hat = h_mulmod(hat, p.mod[p.max_level + t] % q, q);
-    s2[k] = mk_cst(h_mulmod(p.n_inv[mi], h_invmod(hat, q), q), q);
+    s2[k] = mk_cst(p.moddown_scale(j), p.mod[mi]);
   }
   int rc;
   if ((rc = upload(ctx, s1, &sp.scale1))) return rc;
@@ -930,7 +970,7 @@ int get_shard_plan(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, Shar
     std::vector<double2> ql;
     for (uint32_t k = 0; k < nq; ++k) {
       const uint32_t i = sp.own_q[k];
-      if (i + 1 < L) ql.push_back(mk_cst(h_invmod(p.mod[L - 1] % p.mod[i], p.mod[i]), p.mod[i]));
+      if (i + 1 < L) ql.push_back(mk_cst(p.ql_inv(L, i), p.mod[i]));
     }
     if ((rc = upload(ctx, ql, &sp.qlinv_own))) return rc;
   }
@@ -969,7 +1009,7 @@ int get_shard_plan(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, Shar
   return HML_OK;
 }
 
-size_t shard_ws_words(const Params &p, const ShardPlan &sp) {
+static size_t shard_ws_words(const Params &p, const ShardPlan &sp) {
   const size_t ne = sp.own_q.size() + sp.own_p.size(), nq = sp.own_q.size();
   return (size_t)p.N * ((size_t)sp.beta * ne + 2 * ne + 2 * nq);
 }
@@ -1014,9 +1054,7 @@ extern "C" int hml_keyswitch_shard_begin(hml_ctx *ctx, uint32_t L, uint32_t rank
     l.n_batch = 1;
     l.in = (const u64 *)d_own; l.out = (u64 *)gather1 + (size_t)rank * sp->gq * N;
     l.in_limb_stride = l.out_limb_stride = N; l.n_limbs = nq; l.n_polys = 1; l.post_scale = sp->scale1;
-    launch_ntt_inverse(ctx->tabs, ctx->p.logN, sp->q_lm, l, (cudaStream_t)stream);
-    prof_mark(ctx, HML_CLS_INTT, (cudaStream_t)stream);
-    ctx->exec.intt_limbs += nq; ctx->exec.kernel_launches += ctx->p.logN <= NTT_SMALL_LOG ? 1 : 2;
+    run_ntt(ctx, true, sp->q_lm, l, (cudaStream_t)stream);
   }
   return check_launch(ctx, "keyswitch shard begin");
 }
@@ -1026,13 +1064,12 @@ extern "C" int hml_keyswitch_shard_begin(hml_ctx *ctx, uint32_t L, uint32_t rank
 static void shard_ext_ntt(hml_ctx *ctx, ShardPlan *sp, u64 *ext, bool hpip, const u64 *d_own, const u64 *evk_own, u64 *acc, cudaStream_t s) {
   const Params &p = ctx->p;
   const size_t N = p.N;
-  const uint32_t nq = sp->own_q.size(), ne = nq + sp->own_p.size(), beta = sp->beta;
-  const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
+  const uint32_t ne = sp->own_q.size() + sp->own_p.size(), beta = sp->beta;
   NttLaunch l{};
   l.n_batch = 1;
   l.in = ext; l.out = ext; l.in_limb_stride = l.out_limb_stride = N; l.in_poly_stride = l.out_poly_stride = (long long)ne * N;
   l.n_limbs = ne; l.n_polys = beta;
-  l.in_f64 = l.out_f64 = npass == 2;
+  l.in_f64 = l.out_f64 = p.logN > NTT_SMALL_LOG;
   if (hpip) {
     NttMac &m = l.mac;
     m.evk = evk_own; m.d = d_own; m.acc = acc; m.d_batch_stride = 0; m.acc_batch_stride = 0; m.acc_comp_stride = (long long)ne * N;
@@ -1040,9 +1077,7 @@ static void shard_ext_ntt(hml_ctx *ctx, ShardPlan *sp, u64 *ext, bool hpip, cons
     for (uint32_t k = 0; k < ne; ++k) m.key_pos[k] = (uint16_t)k;
     ctx->exec.ewe_limbs += 2ull * ne * beta;
   }
-  launch_ntt_forward(ctx->tabs, logN, sp->e_lm, l, s);
-  prof_mark(ctx, HML_CLS_NTT, s);
-  ctx->exec.ntt_limbs += (uint64_t)beta * ne - nq; ctx->exec.kernel_launches += npass;
+  run_ntt(ctx, false, sp->e_lm, l, s);
 }
 
 // everything of the middle phase after the ModUp conversions: NTT of the extended digits, inner product with the owned key
@@ -1051,7 +1086,6 @@ static int shard_mid_tail(hml_ctx *ctx, ShardPlan *sp, uint32_t rank, const u64 
   const Params &p = ctx->p;
   const size_t N = p.N;
   const uint32_t nq = sp->own_q.size(), np = sp->own_p.size(), ne = nq + np, beta = sp->beta;
-  const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
   u64 *ext = ctx->ws, *acc = ext + (size_t)beta * ne * N;
   // one ciphertext's slice per rank: the inner product rides in the ModUp transform's row pass (NttMac) whenever it can
   const bool hpip = ks_uses_hpip(ctx, sp->L, 1);
@@ -1059,7 +1093,7 @@ static int shard_mid_tail(hml_ctx *ctx, ShardPlan *sp, uint32_t rank, const u64 
   if (!hpip) {
     InnerArgs a{};
     a.d = d_own; a.ext = ext; a.evk = evk_own; a.acc = acc; a.N = N; a.n_ext = ne; a.beta = beta;
-    a.evk_limbs = ne; a.n_batch = 1; a.u_limb = -1; a.ext_f64 = npass == 2;
+    a.evk_limbs = ne; a.n_batch = 1; a.u_limb = -1; a.ext_f64 = p.logN > NTT_SMALL_LOG;
     launch_inner_product(ctx->mc, sp->e_lm, a, s);
     prof_mark(ctx, HML_CLS_EWE, s);
     ctx->exec.ewe_limbs += 2ull * ne * beta; ctx->exec.kernel_launches++;
@@ -1072,9 +1106,7 @@ static int shard_mid_tail(hml_ctx *ctx, ShardPlan *sp, uint32_t rank, const u64 
     l.in = acc; l.in_limb_stride = N; l.in_poly_stride = (long long)ne * N;
     l.out = gather2 + (size_t)rank * 2 * sp->gp * N - (size_t)nq * N; l.out_limb_stride = N; l.out_poly_stride = (long long)sp->gp * N;
     l.n_limbs = np; l.n_polys = 2; l.post_scale = sp->scale2;
-    launch_ntt_inverse(ctx->tabs, logN, sp->p_lm, l, s);
-    prof_mark(ctx, HML_CLS_INTT, s);
-    ctx->exec.intt_limbs += 2 * np; ctx->exec.kernel_launches += npass;
+    run_ntt(ctx, true, sp->p_lm, l, s);
   }
   return check_launch(ctx, "keyswitch shard mid");
 }
@@ -1089,79 +1121,50 @@ extern "C" int hml_keyswitch_shard_mid(hml_ctx *ctx, uint32_t L, uint32_t rank, 
   if ((rc = get_shard_plan(ctx, L, rank, world, &sp))) return rc;
   if ((rc = ensure_ws(ctx, shard_ws_words(ctx->p, *sp)))) return rc;
   ws_enter(ctx, (cudaStream_t)stream);
-  const size_t N = ctx->p.N;
-  const uint32_t ne = sp->own_q.size() + sp->own_p.size(), beta = sp->beta;
+  const uint32_t ne = sp->own_q.size() + sp->own_p.size();
   cudaStream_t s = (cudaStream_t)stream;
-  u64 *ext = ctx->ws;
   if (ne == 0) return HML_OK;
-  for (uint32_t j = 0; j < beta; ++j) {
-    if (sp->up[j].empty()) continue;
-    BConvArgs a{};
-    a.in = (const u64 *)gather1; a.out = ext + (size_t)j * ne * N; a.step1 = nullptr; a.N = N; a.n_batches = 1;
-    a.out_f64 = ctx->p.logN > NTT_SMALL_LOG;
-    run_bconv(ctx, sp->up[j], sp->up_src[j], a, s);
-  }
+  BConvArgs a{};
+  a.in = (const u64 *)gather1; a.out = ctx->ws; a.step1 = nullptr; a.N = ctx->p.N; a.n_batches = 1; a.out_f64 = ctx->p.logN > NTT_SMALL_LOG;
+  run_modup_bconv(ctx, sp->up, sp->up_src, nullptr, nullptr, a, 0, (long long)ne * ctx->p.N, s);
   return shard_mid_tail(ctx, sp, rank, (const u64 *)d_own, (const u64 *)evk_own, (u64 *)gather2, s);
 }
 
-// last phase: BConv P -> owned Q-limbs (sources in `gather2`, or at src_off relative to it), NTT, (acc - v) * P^-1.
-// acc_in / vb_in: the accumulator pair [2][ne] and the conversion output [2][nq] (null: the workspace positions of the key
-// switch).  add0_galois != 0 reads add0 through that automorphism (fused epilogue, two-pass rings only).
+// last phase: BConv P -> owned Q-limbs (sources in `gather2`, or at src_off relative to it), NTT, (acc - v) * P^-1 (+ the
+// caller's addends: HROTATE add, component 0 only; HMULT add, both; owned limbs [nq][N]).  The accumulator pair is r of the
+// workspace [beta][ne] | acc [H][2][ne] | vb [2][nq] (r = 0, H = 1: the key switch's layout).  add0_galois != 0 reads add0
+// through that automorphism (fused epilogue, two-pass rings only).
 static int shard_end_run(hml_ctx *ctx, ShardPlan *sp, const u64 *gather2, const long long *src_off, u64 *out0_own, u64 *out1_own, cudaStream_t s,
-                         const u64 *add0_own = nullptr, const u64 *add1_own = nullptr, const u64 *acc_in = nullptr, u64 *vb_in = nullptr,
-                         u64 add0_galois = 0) {
+                         const u64 *add0_own = nullptr, const u64 *add1_own = nullptr, uint32_t r = 0, uint32_t H = 1, u64 add0_galois = 0) {
   int rc;
   if ((rc = ensure_ws(ctx, shard_ws_words(ctx->p, *sp)))) return rc;
   ws_enter(ctx, s);
   const Params &p = ctx->p;
   const size_t N = p.N;
-  const uint32_t nq = sp->own_q.size(), np = sp->own_p.size(), ne = nq + np, beta = sp->beta;
-  const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
+  const uint32_t nq = sp->own_q.size(), np = sp->own_p.size(), ne = nq + np;
+  const bool two_pass = p.logN > NTT_SMALL_LOG;
   if (nq == 0) return HML_OK;
-  const u64 *acc = acc_in ? acc_in : ctx->ws + (size_t)beta * ne * N;
-  u64 *vb = vb_in ? vb_in : ctx->ws + (size_t)beta * ne * N + 2 * (size_t)ne * N;
-  if (add0_galois && (npass != 2 || !add0_own || add1_own)) return fail(ctx, HML_ERR_INVALID, "automorphism on the addend needs the fused ModDown epilogue");
+  const u64 *acc0 = ctx->ws + (size_t)sp->beta * ne * N;
+  u64 *vb = (u64 *)acc0 + 2 * (size_t)H * ne * N;
+  if (add0_galois && (!add0_own || add1_own)) return fail(ctx, HML_ERR_INVALID, "automorphism on the addend needs the fused ModDown epilogue");
   {
     BConvArgs a{};
     a.in = gather2; a.out = vb; a.in_batch_stride = (long long)sp->gp * N; a.out_batch_stride = (long long)nq * N;
-    a.step1 = nullptr; a.N = N; a.n_batches = 2; a.src_off = src_off; a.out_f64 = npass == 2;
+    a.step1 = nullptr; a.N = N; a.n_batches = 2; a.src_off = src_off; a.out_f64 = two_pass;
     run_bconv(ctx, sp->down, sp->down_src, a, s);
   }
-  const bool fuse = npass == 2;  // two-pass rings: K10 (+ the caller's addends) is the transform's epilogue, as in ks_tail
-  {
-    NttLaunch l{};
-    l.n_batch = 1;
-    l.in = vb; l.out = vb; l.in_limb_stride = l.out_limb_stride = N; l.in_poly_stride = l.out_poly_stride = (long long)nq * N;
-    l.n_limbs = nq; l.n_polys = 2; l.in_f64 = npass == 2;
-    if (fuse) {
-      NttFuse &f = l.fuse;
-      f.x = acc; f.x_c_stride = (long long)ne * N; f.x_b_stride = 0; f.x_packed = 0;
-      f.z = add0_own ? add0_own : add1_own; f.z_b_stride = 0;
-      f.z_c_stride = (add0_own && add1_own) ? (long long)(add1_own - add0_own) : 0;
-      f.z_mask = (add0_own ? 1u : 0u) | (add1_own ? 2u : 0u);
-      f.dst = out0_own; f.dst_c_stride = (long long)(out1_own - out0_own); f.dst_b_stride = 0;
-      f.cst = sp->pinv; f.n_c = 2;
-      f.z_galois = (unsigned)(add0_galois & (2ull * N - 1));
-      ctx->exec.ewe_limbs += 2 * nq;
-    }
-    launch_ntt_forward(ctx->tabs, logN, sp->q_lm, l, s);
-    prof_mark(ctx, HML_CLS_NTT, s);
-    ctx->exec.ntt_limbs += 2 * nq; ctx->exec.kernel_launches += npass;
-  }
-  if (!fuse) {  // both outputs in one launch: the "poly" stride of the output is simply the distance between the two buffers
-    SubMulArgs a{};
-    a.x = acc; a.x_poly_stride = (long long)ne * N; a.y = vb; a.y_poly_stride = (long long)nq * N; a.z = nullptr;
-    a.out = out0_own; a.out_poly_stride = (long long)(out1_own - out0_own);
-    a.cst = sp->pinv; a.N = N; a.n_limbs = nq; a.n_polys = 2;
-    if (add0_own || add1_own) {  // the caller's addends (HROTATE add: component 0 only; HMULT add: both), owned limbs [nq][N]
-      a.z = add0_own ? add0_own : add1_own;
-      a.z_poly_stride = (add0_own && add1_own) ? (long long)(add1_own - add0_own) : 0;
-      a.z_mask = (add0_own ? 1u : 0u) | (add1_own ? 2u : 0u);  // a single addend is read with stride 0
-    }
-    launch_sub_mul_add(ctx->mc, sp->q_lm, a, s);
-    prof_mark(ctx, HML_CLS_EWE, s);
-    ctx->exec.ewe_limbs += 2 * nq; ctx->exec.kernel_launches++;
-  }
+  NttLaunch l{};
+  l.n_batch = 1;
+  l.in = vb; l.out = vb; l.in_limb_stride = l.out_limb_stride = N; l.in_poly_stride = l.out_poly_stride = (long long)nq * N;
+  l.n_limbs = nq; l.n_polys = 2; l.in_f64 = two_pass;
+  NttFuse &f = l.fuse;
+  f.x = acc0 + 2 * (size_t)r * ne * N; f.x_c_stride = (long long)ne * N;
+  set_addends(f, add0_own, add1_own);
+  f.dst = out0_own; f.dst_c_stride = (long long)(out1_own - out0_own);
+  f.cst = sp->pinv; f.n_c = 2;
+  f.z_galois = (unsigned)(add0_galois & (2ull * N - 1));
+  if ((rc = ntt_sub_mul(ctx, sp->q_lm, l, s))) return rc;
+  ctx->exec.ewe_limbs += 2 * nq;
   return check_launch(ctx, "keyswitch shard end");
 }
 
@@ -1328,23 +1331,8 @@ static int shard_peer_offsets(hml_ctx *ctx, ShardPlan *sp, const uint64_t *const
       sp->d_off1.push_back(d);
     }
     // the one-launch form of the ModUp conversions: every CTA serves one digit and reads its sources from the owners' buffers
-    cudaFree(sp->up_jobs); sp->up_jobs = nullptr;
-    {
-      const uint32_t ne = sp->own_q.size() + sp->own_p.size();
-      std::vector<BConvJob> jobs(sp->beta);
-      bool ok = sp->beta >= 2;
-      for (uint32_t j = 0; j < sp->beta && ok; ++j) {
-        const HostBConv &hb = sp->up[j];
-        ok = !hb.empty() && hb.d_img != nullptr && hb.n_src <= 48 && hb.n_dst <= 48;
-        if (!ok) break;
-        BConvJob &jb = jobs[j];
-        memset(&jb, 0, sizeof(jb));
-        for (int t = 0; t < hb.n_dst; ++t) { jb.dst_mod[t] = hb.dst_lm.mod[t]; jb.dst_pos[t] = hb.dst_lm.pos[t]; }
-        jb.img = hb.d_img; jb.K = hb.im.K; jb.NP = hb.im.NP; jb.ND = hb.im.ND; jb.n_src = hb.n_src; jb.n_dst = hb.n_dst;
-        jb.in_off = 0; jb.out_off = (long long)j * ne * N; jb.src_off = sp->d_off1[j];
-      }
-      if (ok && (rc = upload(ctx, jobs, &sp->up_jobs))) return rc;
-    }
+    cudaFree(sp->up_jobs);
+    if ((rc = upload_up_jobs(ctx, sp->up, 0, (long long)(sp->own_q.size() + sp->own_p.size()) * N, &sp->d_off1, &sp->up_jobs))) return rc;
   } else {
     cudaFree(sp->d_off2); sp->d_off2 = nullptr;
     std::vector<long long> off(A);
@@ -1365,29 +1353,17 @@ static int shard_p2p_check(hml_ctx *ctx, const HostBConv &hb) {
 // the ModUp conversions of the peer-direct middle phase: every digit (its limbs read from the owners' gather buffers 1, at the
 // offsets built by shard_peer_offsets relative to this rank's own buffer g1_own) -> owned extended limbs, ext [beta][ne]
 static void shard_modup_p2p(hml_ctx *ctx, ShardPlan *sp, const uint64_t *g1_own, u64 *ext, cudaStream_t s) {
-  const size_t N = ctx->p.N;
-  const uint32_t ne = sp->own_q.size() + sp->own_p.size(), beta = sp->beta;
-  bool merged_up = false;
-  if (sp->up_jobs) {
-    BConvArgs a{};
-    a.in = (const u64 *)g1_own; a.out = ext; a.step1 = nullptr; a.N = N; a.n_batches = 1; a.out_f64 = ctx->p.logN > NTT_SMALL_LOG;
-    std::vector<BConvImage> ims(beta);
-    std::vector<int> nd(beta);
-    for (uint32_t j = 0; j < beta; ++j) { ims[j] = sp->up[j].im; nd[j] = sp->up[j].n_dst; }
-    merged_up = launch_bconv_umma_multi(ctx->mc, sp->up_jobs, ims.data(), nd.data(), (int)beta, a, s);
-    if (merged_up) {
-      prof_mark(ctx, HML_CLS_BCONV, s);
-      ctx->exec.kernel_launches++;
-      for (uint32_t j = 0; j < beta; ++j) ctx->exec.bconv_limb_macs += (uint64_t)sp->up[j].n_src * sp->up[j].n_dst;
-    }
-  }
-  for (uint32_t j = 0; j < beta && !merged_up; ++j) {
-    if (sp->up[j].empty()) continue;
-    BConvArgs a{};
-    a.in = (const u64 *)g1_own; a.out = ext + (size_t)j * ne * N; a.step1 = nullptr; a.N = N; a.n_batches = 1;
-    a.src_off = sp->d_off1[j]; a.out_f64 = ctx->p.logN > NTT_SMALL_LOG;
-    run_bconv(ctx, sp->up[j], sp->up_src[j], a, s);
-  }
+  BConvArgs a{};
+  a.in = (const u64 *)g1_own; a.out = ext; a.step1 = nullptr; a.N = ctx->p.N; a.n_batches = 1; a.out_f64 = ctx->p.logN > NTT_SMALL_LOG;
+  run_modup_bconv(ctx, sp->up, sp->up_src, sp->up_jobs, &sp->d_off1, a, 0, (long long)(sp->own_q.size() + sp->own_p.size()) * ctx->p.N, s);
+}
+
+// the preamble of the internal sharded functions: rank / level checks, the context's device, the plan
+static int shard_plan_on_device(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, ShardPlan **sp) {
+  int rc = shard_check(ctx, L, rank, world);
+  if (rc) return rc;
+  HML_CU_TRY(ctx, cudaSetDevice(ctx->device));
+  return get_shard_plan(ctx, L, rank, world, sp);
 }
 
 extern "C" int hml_keyswitch_shard_mid_p2p(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *d_own,
@@ -1409,45 +1385,34 @@ extern "C" int hml_keyswitch_shard_mid_p2p(hml_ctx *ctx, uint32_t L, uint32_t ra
   return shard_mid_tail(ctx, sp, rank, (const u64 *)d_own, (const u64 *)evk_own, (u64 *)gather2_own, (cudaStream_t)stream);
 }
 
+// the peer-direct ModDown of accumulator pair r (shard_end_run): its sources read from slot r (slot_words apart) of the owners'
+// gather buffers 2
+int shard_end_p2p(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *const *peers2, uint64_t *out0_own, uint64_t *out1_own,
+                  const uint64_t *add0_own, const uint64_t *add1_own, cudaStream_t s, uint32_t r, uint32_t H, size_t slot_words, uint64_t add0_galois) {
+  ShardPlan *sp;
+  int rc = shard_plan_on_device(ctx, L, rank, world, &sp);
+  if (rc) return rc;
+  if ((rc = shard_p2p_check(ctx, sp->down))) return rc;
+  if ((rc = shard_peer_offsets(ctx, sp, peers2, true))) return rc;
+  return shard_end_run(ctx, sp, (const u64 *)peers2[rank] + (size_t)r * slot_words, sp->d_off2, (u64 *)out0_own, (u64 *)out1_own, s,
+                       (const u64 *)add0_own, (const u64 *)add1_own, r, H, add0_galois);
+}
+
 extern "C" int hml_keyswitch_shard_end_p2p(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *const *peers2,
                                            uint64_t *out0_own, uint64_t *out1_own, void *stream) {
   int rc = shard_check(ctx, L, rank, world);
   if (rc) return rc;
   if (!peers2 || !out0_own || !out1_own) return fail(ctx, HML_ERR_INVALID, "null buffer");
   for (uint32_t r = 0; r < world; ++r) if (!peers2[r]) return fail(ctx, HML_ERR_INVALID, "null peer buffer");
-  CU_TRY(ctx, cudaSetDevice(ctx->device));
-  ShardPlan *sp;
-  if ((rc = get_shard_plan(ctx, L, rank, world, &sp))) return rc;
-  if ((rc = shard_p2p_check(ctx, sp->down))) return rc;
-  if ((rc = shard_peer_offsets(ctx, sp, peers2, true))) return rc;
-  return shard_end_run(ctx, sp, (const u64 *)peers2[rank], sp->d_off2, (u64 *)out0_own, (u64 *)out1_own, (cudaStream_t)stream);
-}
-
-int shard_end_p2p_add(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *const *peers2, uint64_t *out0_own,
-                      uint64_t *out1_own, const uint64_t *add0_own, const uint64_t *add1_own, cudaStream_t s) {
-  int rc = shard_check(ctx, L, rank, world);
-  if (rc) return rc;
-  HML_CU_TRY(ctx, cudaSetDevice(ctx->device));
-  ShardPlan *sp;
-  if ((rc = get_shard_plan(ctx, L, rank, world, &sp))) return rc;
-  if ((rc = shard_p2p_check(ctx, sp->down))) return rc;
-  if ((rc = shard_peer_offsets(ctx, sp, peers2, true))) return rc;
-  return shard_end_run(ctx, sp, (const u64 *)peers2[rank], sp->d_off2, (u64 *)out0_own, (u64 *)out1_own, s, (const u64 *)add0_own, (const u64 *)add1_own);
+  return shard_end_p2p(ctx, L, rank, world, peers2, out0_own, out1_own, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 // ---- hoisted rotations of one limb-sharded ciphertext (shard.cu, hml_hrotate_hoisted_sharded).  One ModUp of c1 serves every
 // rotation; a group of up to H rotations shares one inner-product launch, one P-limb INTT and one exchange.  Workspace:
 //   ext [beta][ne] | acc [H][2][ne] | vb [2][nq]        (H = 1: the key switch's layout)
-size_t shard_hoist_ws_words(const Params &p, const ShardPlan &sp, uint32_t H) {
+static size_t shard_hoist_ws_words(const Params &p, const ShardPlan &sp, uint32_t H) {
   const size_t ne = sp.own_q.size() + sp.own_p.size(), nq = sp.own_q.size();
   return (size_t)p.N * ((size_t)sp.beta * ne + 2 * (size_t)H * ne + 2 * nq);
-}
-
-static int shard_plan_on_device(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, ShardPlan **sp) {
-  int rc = shard_check(ctx, L, rank, world);
-  if (rc) return rc;
-  HML_CU_TRY(ctx, cudaSetDevice(ctx->device));
-  return get_shard_plan(ctx, L, rank, world, sp);
 }
 
 // phase 1 of a group of n <= H rotations.  peers1 != null (the op's first group): the ModUp conversions from the owners' gather
@@ -1496,7 +1461,6 @@ int shard_hoist_intt(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, ui
   const Params &p = ctx->p;
   const size_t N = p.N;
   const uint32_t nq = sp->own_q.size(), np = sp->own_p.size(), ne = nq + np;
-  const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
   if (np == 0) return HML_OK;
   NttLaunch l{};
   l.in = ctx->ws + (size_t)sp->beta * ne * N; l.in_limb_stride = N; l.in_poly_stride = (long long)ne * N; l.in_batch_stride = 2ll * ne * N;
@@ -1504,25 +1468,8 @@ int shard_hoist_intt(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, ui
   l.out = (u64 *)g2_own + (size_t)rank * 2 * sp->gp * N - (size_t)nq * N; l.out_limb_stride = N; l.out_poly_stride = (long long)sp->gp * N;
   l.out_batch_stride = (long long)slot_words;
   l.n_limbs = np; l.n_polys = 2; l.n_batch = (int)n; l.post_scale = sp->scale2;
-  launch_ntt_inverse(ctx->tabs, logN, sp->p_lm, l, s);
-  prof_mark(ctx, HML_CLS_INTT, s);
-  ctx->exec.intt_limbs += 2ull * n * np; ctx->exec.kernel_launches += npass;
+  run_ntt(ctx, true, sp->p_lm, l, s);
   return check_launch(ctx, "hoisted shard P-limb INTT");
-}
-
-// phase 2 of rotation r of the group: ModDown from slot r of the owners' gather buffers 2, plus add0 (read through add0_galois
-// when it is not 0) on component 0
-int shard_hoist_end(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uint32_t H, const uint64_t *const *peers2, size_t slot_words,
-                    uint32_t r, const uint64_t *add0, uint64_t add0_galois, uint64_t *out0, uint64_t *out1, cudaStream_t s) {
-  ShardPlan *sp;
-  int rc = shard_plan_on_device(ctx, L, rank, world, &sp);
-  if (rc) return rc;
-  if ((rc = shard_p2p_check(ctx, sp->down))) return rc;
-  if ((rc = shard_peer_offsets(ctx, sp, peers2, true))) return rc;
-  const size_t N = ctx->p.N, ne = sp->own_q.size() + sp->own_p.size();
-  u64 *acc = ctx->ws + (size_t)sp->beta * ne * N;
-  return shard_end_run(ctx, sp, (const u64 *)peers2[rank] + (size_t)r * slot_words, sp->d_off2, (u64 *)out0, (u64 *)out1, s, (const u64 *)add0, nullptr,
-                       acc + 2 * (size_t)r * ne * N, acc + 2 * (size_t)H * ne * N, add0_galois);
 }
 
 // everything a sharded op at level L needs that costs host time or synchronises the device (plans, conversion images, offset
@@ -1530,11 +1477,9 @@ int shard_hoist_end(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uin
 // while a peer is still preparing
 int shard_prepare(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *const *peers1, const uint64_t *const *peers2,
                   uint32_t max_rot) {
-  int rc = shard_check(ctx, L, rank, world);
-  if (rc) return rc;
-  HML_CU_TRY(ctx, cudaSetDevice(ctx->device));
   ShardPlan *sp;
-  if ((rc = get_shard_plan(ctx, L, rank, world, &sp))) return rc;
+  int rc = shard_plan_on_device(ctx, L, rank, world, &sp);
+  if (rc) return rc;
   for (auto &u : sp->up) if ((rc = shard_p2p_check(ctx, u))) return rc;
   if ((rc = shard_p2p_check(ctx, sp->down))) return rc;
   if ((rc = shard_peer_offsets(ctx, sp, peers1, false))) return rc;
@@ -1544,17 +1489,16 @@ int shard_prepare(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const
 }
 
 // ------------------------------------------------------------------------------------------------ rescale
-size_t rs_ws_words(const Params &p, uint32_t L, uint32_t n_polys) { return (size_t)p.N * n_polys * L; }
+static size_t rs_ws_words(const Params &p, uint32_t L, uint32_t n_polys) { return (size_t)p.N * n_polys * L; }
 
 // in: n_polys polys of L limbs (uniform stride in_poly_stride) -> out: n_polys polys of L-1 limbs
-int rescale_run(hml_ctx *ctx, uint32_t L, const u64 *in, long long in_poly_stride, uint32_t n_polys, u64 *out,
+static int rescale_run(hml_ctx *ctx, uint32_t L, const u64 *in, long long in_poly_stride, uint32_t n_polys, u64 *out,
                        long long out_poly_stride, u64 *ws, cudaStream_t s) {
   const Params &p = ctx->p;
   LevelConsts *lc;
   int rc = get_level(ctx, L, &lc);
   if (rc) return rc;
   const size_t N = p.N;
-  const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
   u64 *rb = ws, *rh = ws + (size_t)n_polys * N;  // rb [n_polys][N], rh [n_polys][L-1][N]
   {  // INTT of the dropped limb (reference :766-805)
     LimbMap lm; clear_map(lm);
@@ -1563,34 +1507,17 @@ int rescale_run(hml_ctx *ctx, uint32_t L, const u64 *in, long long in_poly_strid
     l.n_batch = 1;
     l.in = in + (size_t)(L - 1) * N; l.out = rb; l.in_limb_stride = l.out_limb_stride = N;
     l.in_poly_stride = in_poly_stride; l.out_poly_stride = N; l.n_limbs = 1; l.n_polys = n_polys;
-    launch_ntt_inverse(ctx->tabs, logN, lm, l, s);
-    prof_mark(ctx, HML_CLS_INTT, s);
-    ctx->exec.intt_limbs += n_polys; ctx->exec.kernel_launches += npass;
+    run_ntt(ctx, true, lm, l, s);
   }
-  const bool fuse = npass == 2;
-  {  // NTT of that polynomial under each remaining modulus (reference :807-822 counts ONE; delta D2); on two-pass rings
-     // the sub + mul (reference :825-911) is the transform's fused epilogue
-    NttLaunch l{};
-    l.n_batch = 1;
-    l.in = rb; l.out = rh; l.in_limb_stride = 0; l.out_limb_stride = N; l.in_poly_stride = N;
-    l.out_poly_stride = (long long)(L - 1) * N; l.n_limbs = L - 1; l.n_polys = n_polys;
-    if (fuse) {
-      NttFuse &f = l.fuse;
-      f.x = in; f.x_c_stride = in_poly_stride; f.x_b_stride = 0; f.z = nullptr; f.z_mask = 0;
-      f.dst = out; f.dst_c_stride = out_poly_stride; f.dst_b_stride = 0; f.cst = lc->qlinv; f.n_c = (int)n_polys;
-    }
-    launch_ntt_forward(ctx->tabs, logN, lc->q_lm, l, s);
-    prof_mark(ctx, HML_CLS_NTT, s);
-    ctx->exec.ntt_limbs += (uint64_t)n_polys * (L - 1); ctx->exec.kernel_launches += npass;
-  }
-  if (!fuse) {  // sub + mul (reference :825-911), one fused pass
-    SubMulArgs a{};
-    a.x = in; a.y = rh; a.z = nullptr; a.out = out; a.x_poly_stride = in_poly_stride; a.y_poly_stride = (long long)(L - 1) * N;
-    a.out_poly_stride = out_poly_stride; a.cst = lc->qlinv; a.N = N; a.n_limbs = L - 1; a.n_polys = n_polys;
-    launch_sub_mul_add(ctx->mc, lc->q_lm, a, s);
-    prof_mark(ctx, HML_CLS_EWE, s);
-    ctx->exec.kernel_launches++;
-  }
+  // NTT of that polynomial under each remaining modulus (reference :807-822 counts ONE; delta D2), then the sub + mul
+  // (reference :825-911)
+  NttLaunch l{};
+  l.n_batch = 1;
+  l.in = rb; l.out = rh; l.in_limb_stride = 0; l.out_limb_stride = N; l.in_poly_stride = N;
+  l.out_poly_stride = (long long)(L - 1) * N; l.n_limbs = L - 1; l.n_polys = n_polys;
+  NttFuse &f = l.fuse;
+  f.x = in; f.x_c_stride = in_poly_stride; f.dst = out; f.dst_c_stride = out_poly_stride; f.cst = lc->qlinv; f.n_c = (int)n_polys;
+  if ((rc = ntt_sub_mul(ctx, lc->q_lm, l, s))) return rc;
   ctx->exec.ewe_limbs += 2ull * n_polys * (L - 1);
   return check_launch(ctx, "rescale");
 }
@@ -1632,9 +1559,7 @@ extern "C" int hml_rescale_shard_begin(hml_ctx *ctx, uint32_t L, uint32_t rank, 
   l.in = (const u64 *)x_own; l.in_limb_stride = N; l.in_poly_stride = (long long)nq * N;
   l.out = (u64 *)r_own - (size_t)(nq - 1) * N; l.out_limb_stride = N; l.out_poly_stride = N;  // position nq-1 lands on r_own
   l.n_limbs = 1; l.n_polys = 2;
-  launch_ntt_inverse(ctx->tabs, ctx->p.logN, lm, l, (cudaStream_t)stream);
-  prof_mark(ctx, HML_CLS_INTT, (cudaStream_t)stream);
-  ctx->exec.intt_limbs += 2; ctx->exec.kernel_launches += ctx->p.logN <= NTT_SMALL_LOG ? 1 : 2;
+  run_ntt(ctx, true, lm, l, (cudaStream_t)stream);
   return check_launch(ctx, "rescale shard begin");
 }
 
@@ -1654,34 +1579,16 @@ extern "C" int hml_rescale_shard_end(hml_ctx *ctx, uint32_t L, uint32_t rank, ui
   if (nk == 0) return HML_OK;
   if ((rc = ensure_ws(ctx, std::max(shard_ws_words(p, *sp), (size_t)2 * nk * N)))) return rc;
   ws_enter(ctx, (cudaStream_t)stream);
-  const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
-  cudaStream_t s = (cudaStream_t)stream;
   LimbMap lm; clear_map(lm);
   for (uint32_t k = 0; k < nk; ++k) { lm.mod[k] = sp->own_q[k]; lm.pos[k] = k; }
-  u64 *rh = ctx->ws;  // [2][nk][N]
-  const bool fuse = npass == 2;
-  {
-    NttLaunch l{};
-    l.n_batch = 1;
-    l.in = (const u64 *)r_src; l.in_limb_stride = 0; l.in_poly_stride = N;
-    l.out = rh; l.out_limb_stride = N; l.out_poly_stride = (long long)nk * N; l.n_limbs = nk; l.n_polys = 2;
-    if (fuse) {
-      NttFuse &f = l.fuse;
-      f.x = (const u64 *)x_own; f.x_c_stride = (long long)nq * N; f.x_b_stride = 0; f.z = nullptr; f.z_mask = 0;
-      f.dst = (u64 *)out_own; f.dst_c_stride = (long long)nk * N; f.dst_b_stride = 0; f.cst = sp->qlinv_own; f.n_c = 2;
-    }
-    launch_ntt_forward(ctx->tabs, logN, lm, l, s);
-    prof_mark(ctx, HML_CLS_NTT, s);
-    ctx->exec.ntt_limbs += 2ull * nk; ctx->exec.kernel_launches += npass;
-  }
-  if (!fuse) {
-    SubMulArgs a{};
-    a.x = (const u64 *)x_own; a.y = rh; a.z = nullptr; a.out = (u64 *)out_own; a.x_poly_stride = (long long)nq * N;
-    a.y_poly_stride = (long long)nk * N; a.out_poly_stride = (long long)nk * N; a.cst = sp->qlinv_own; a.N = N; a.n_limbs = nk; a.n_polys = 2;
-    launch_sub_mul_add(ctx->mc, lm, a, s);
-    prof_mark(ctx, HML_CLS_EWE, s);
-    ctx->exec.kernel_launches++;
-  }
+  NttLaunch l{};
+  l.n_batch = 1;
+  l.in = (const u64 *)r_src; l.in_limb_stride = 0; l.in_poly_stride = N;
+  l.out = ctx->ws; l.out_limb_stride = N; l.out_poly_stride = (long long)nk * N; l.n_limbs = nk; l.n_polys = 2;  // ws: [2][nk][N]
+  NttFuse &f = l.fuse;
+  f.x = (const u64 *)x_own; f.x_c_stride = (long long)nq * N;
+  f.dst = (u64 *)out_own; f.dst_c_stride = (long long)nk * N; f.cst = sp->qlinv_own; f.n_c = 2;
+  if ((rc = ntt_sub_mul(ctx, lm, l, (cudaStream_t)stream))) return rc;
   ctx->exec.ewe_limbs += 4ull * nk;
   return check_launch(ctx, "rescale shard end");
 }
@@ -1743,7 +1650,6 @@ int hmult_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct_a, const u64 
   // (reference Rescale INTT :766-805) rides in the launch that transforms the P-limbs: no extra launches, no re-reads
   const MergedU mu{d0, (long long)(d1 - d0), (long long)PL};
   if ((rc = ks_front(ctx, lc, L, nb, {d2, (long long)PL}, evk, evk_q_limbs, yb, ext, acc, AL, s, &mu))) return rc;
-  const int logN = p.logN;
   {  // w_l = v_l * P^-1 + [r]_{q_l}, l < L-1, with r = slot_E - v[L-1] * P^-1 folded on the staged tile (reference K8 :489-519)
     BConvArgs a{};
     a.in = acc; a.in_batch_stride = (long long)AL * N; a.out = wb; a.out_batch_stride = (long long)(L - 1) * N;
@@ -1759,9 +1665,7 @@ int hmult_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct_a, const u64 
     f.z = d0; f.z_c_stride = (long long)(d1 - d0); f.z_b_stride = (long long)PL; f.z_mask = 3;
     f.dst = ct_out; f.dst_c_stride = (long long)(L - 1) * N; f.dst_b_stride = 2ll * (L - 1) * N;
     f.cst = lc->pinv; f.cst2 = lc->qlinv; f.n_c = 2; f.x_packed = ks_uses_hpip(ctx, L, nb) ? 0 : 1; f.z_packed = 1;
-    launch_ntt_forward(ctx->tabs, logN, lc->q_lm, l, s);
-    prof_mark(ctx, HML_CLS_NTT, s);
-    ctx->exec.ntt_limbs += 2ull * nb * (L - 1); ctx->exec.kernel_launches += 2;
+    run_ntt(ctx, false, lc->q_lm, l, s);
     ctx->exec.ewe_limbs += 2ull * nb * 4 * (L - 1);
   }
   return check_launch(ctx, "hmult");
@@ -1824,8 +1728,8 @@ extern "C" int hml_hrotate(hml_ctx *ctx, uint32_t L, const uint64_t *ct, const u
 // (ModUp(sigma(c1)) and sigma(ModUp(c1)) differ by multiples of the digit's modulus product), both are valid key-switch
 // inputs; the oracle defines this op separately (oracle/oracle.c orc_hrotate_hoisted).  Reference: the rotation it replaces is
 // src/Operation.cpp:1271-1358 run n_rot times; the reference itself cannot chain or share work between ops (:636,:675,:714).
-int hrot_hoisted_run(hml_ctx *ctx, uint32_t L, const u64 *ct, uint32_t n_rot, const uint64_t *const *rotkeys, uint32_t evk_q_limbs,
-                     const uint64_t *galois, uint64_t *const *outs, u64 *ws, cudaStream_t s) {
+static int hrot_hoisted_run(hml_ctx *ctx, uint32_t L, const u64 *ct, uint32_t n_rot, const uint64_t *const *rotkeys, uint32_t evk_q_limbs,
+                            const uint64_t *galois, uint64_t *const *outs, u64 *ws, cudaStream_t s) {
   const Params &p = ctx->p;
   if ((evk_q_limbs & ~HML_KEY_PACKED) < L || (evk_q_limbs & ~HML_KEY_PACKED) > p.max_level) return fail(ctx, HML_ERR_INVALID, "evk_q_limbs must be in [L, maxLevel]");
   LevelConsts *lc;

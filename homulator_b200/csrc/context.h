@@ -32,6 +32,7 @@ struct LevelConsts {
   double2 *modup_scale = nullptr;            // [L]
   // K3: per digit, the conversion to the E - a_j other limbs (matrix in 12-bit pieces, kernel-parameter resident)
   std::vector<HostBConv> up;                 // [beta]
+  std::vector<LimbMap> up_src;               // [beta] source map of each digit's conversion (q_lm: the digit sits at yb + j * alpha)
   BConvJob *up_jobs = nullptr;               // [beta] device table of the one-launch form (null: digits launch one by one)
   // K4: limbs = the E extended limbs, polys = the beta digits, skip = the digit that owns the limb
   LimbMap ext_lm;

@@ -85,6 +85,32 @@ void Params::twiddles(uint32_t mi, bool inverse, std::vector<u64> &out) const {
   }
 }
 
+u64 Params::p_inv(uint32_t i) const {
+  const u64 q = mod[i];
+  u64 P = 1;
+  for (uint32_t j = 0; j < alpha; ++j) P = h_mulmod(P, mod[max_level + j] % q, q);
+  return h_invmod(P, q);
+}
+
+u64 Params::modup_scale(uint32_t L, uint32_t i) const {
+  const uint32_t lo = i / alpha * alpha, hi = lo + digit_size(L, i / alpha);
+  const u64 q = mod[i];
+  u64 hat = 1;
+  for (uint32_t t = lo; t < hi; ++t)
+    if (t != i) hat = h_mulmod(hat, mod[t] % q, q);
+  return h_mulmod(n_inv[i], h_invmod(hat, q), q);
+}
+
+u64 Params::moddown_scale(uint32_t j) const {
+  const u64 q = mod[max_level + j];
+  u64 hat = 1;
+  for (uint32_t t = 0; t < alpha; ++t)
+    if (t != j) hat = h_mulmod(hat, mod[max_level + t] % q, q);
+  return h_mulmod(n_inv[max_level + j], h_invmod(hat, q), q);
+}
+
+u64 Params::ql_inv(uint32_t L, uint32_t l) const { return h_invmod(mod[L - 1] % mod[l], mod[l]); }
+
 void make_bconv_table(const Params &p, const std::vector<uint32_t> &src, const std::vector<uint32_t> &dst, BConvTable &out) {
   out.src = src; out.dst = dst;
   const size_t ns = src.size(), nd = dst.size();

@@ -36,6 +36,12 @@ struct Params {
 
   // psi^bitrev(i) (forward) or psi^-bitrev(i) (inverse), i < N, for modulus index mi
   void twiddles(uint32_t mi, bool inverse, std::vector<u64> &out) const;
+
+  // Constants of the key switch and the rescale at level L (SURVEY.md Appendix A), P = p_0 * .. * p_{alpha-1}:
+  u64 p_inv(uint32_t i) const;                    // P^-1 mod q_i
+  u64 modup_scale(uint32_t L, uint32_t i) const;  // N^-1 * (D_j / q_i)^-1 mod q_i, D_j the product of the digit j = i / alpha
+  u64 moddown_scale(uint32_t j) const;            // N^-1 * (P / p_j)^-1 mod p_j
+  u64 ql_inv(uint32_t L, uint32_t l) const;       // q_{L-1}^-1 mod q_l
 };
 
 // Base-conversion constants for source moduli S (product D) and destination moduli T:

@@ -230,7 +230,7 @@ static int run_phase(hml_shard *sh, const ShardOp &op, int ph, cudaStream_t s) {
       }
       if (ph == 1) return own_ext ? hml_keyswitch_shard_mid_p2p(ctx, L, rank, world, sig + (size_t)nq * N, peers(sh->p1), op.key, sh->g2, st) : HML_OK;
       // (sigma(c0) + ks0, ks1): the addend rides in the ModDown epilogue
-      return shard_end_p2p_add(ctx, L, rank, world, peers(sh->p2), op.out0, op.out0 + (size_t)nq * N, sig, nullptr, s);
+      return shard_end_p2p(ctx, L, rank, world, peers(sh->p2), op.out0, op.out0 + (size_t)nq * N, sig, nullptr, s);
     }
     case SOP_HMULT: {
       uint64_t *d0 = sc, *d1 = d0 + (size_t)nq * N, *d2 = d1 + (size_t)nq * N, *c = d2 + (size_t)nq * N;  // c [2][nq][N]
@@ -245,7 +245,7 @@ static int run_phase(hml_shard *sh, const ShardOp &op, int ph, cudaStream_t s) {
       }
       if (ph == 1) return own_ext ? hml_keyswitch_shard_mid_p2p(ctx, L, rank, world, d2, peers(sh->p1), op.key, sh->g2, st) : HML_OK;
       if (ph == 2) {
-        if ((rc = shard_end_p2p_add(ctx, L, rank, world, peers(sh->p2), c, c + PL, d0, d1, s))) return rc;
+        if ((rc = shard_end_p2p(ctx, L, rank, world, peers(sh->p2), c, c + PL, d0, d1, s))) return rc;
         return hml_rescale_shard_begin(ctx, L, rank, world, c, sh->rb, st);
       }
       return hml_rescale_shard_end(ctx, L, rank, world, c, sh->pr[(L - 1) % world], op.out0, st);
@@ -403,7 +403,7 @@ static int hoist_phase(hml_shard *sh, const HoistOp &op, const HoistStep &st, cu
           if (rc) return rc;
           add = sh->scratch;
         }
-        int rc = shard_hoist_end(ctx, L, rank, world, H, peers(sh->p2), sh->n2, r, add, add_g, o, o + (size_t)nq * N, s);
+        int rc = shard_end_p2p(ctx, L, rank, world, peers(sh->p2), o, o + (size_t)nq * N, add, nullptr, s, r, H, sh->n2, add_g);
         if (rc) return rc;
       }
       return HML_OK;
