@@ -69,7 +69,7 @@ EXPORTS = [
     "hml_shard_connect_local", "hml_shard_prepare", "hml_shard_check", "hml_shard_own_limbs", "hml_keyswitch_sharded",
     "hml_hrotate_sharded", "hml_hmult_sharded", "hml_rescale_sharded", "hml_ew_sharded", "hml_group_op", "hml_hrotate_hoisted",
     "hml_replay_create", "hml_replay_bind", "hml_replay_run", "hml_replay_slot", "hml_replay_slot_level", "hml_replay_destroy",
-    "hml_shard_create_ex", "hml_hrotate_hoisted_sharded", "hml_group_hrotate_hoisted",
+    "hml_shard_create_ex", "hml_hrotate_hoisted_sharded", "hml_group_hrotate_hoisted", "hml_hrotate_sum_hoisted",
 ]
 
 
@@ -164,6 +164,7 @@ def load_library():
     L.hml_group_op.argtypes = [C.POINTER(vp), u32, i32, u32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), u64,
                                C.POINTER(vp)]
     L.hml_hrotate_hoisted.argtypes = [vp, u32, vp, u32, C.POINTER(vp), u32, C.POINTER(u64), C.POINTER(vp), vp]
+    L.hml_hrotate_sum_hoisted.argtypes = [vp, u32, vp, u32, C.POINTER(vp), u32, C.POINTER(u64), C.POINTER(vp), u32, vp, vp]
     L.hml_hrotate_hoisted_sharded.argtypes = [vp, u32, vp, u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(vp), vp]
     L.hml_group_hrotate_hoisted.argtypes = [C.POINTER(vp), u32, u32, C.POINTER(vp), u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(vp),
                                             C.POINTER(vp)]
@@ -386,6 +387,20 @@ class Context:
         gs = (C.c_uint64 * n)(*[int(g) for g in galois_elts])
         self._chk(self.lib.hml_hrotate_hoisted(self.h, L, _ptr(ct), n, keys, evk_q_limbs or L, gs, po, self._stream()))
         return outs
+
+    def hrotate_sum_hoisted(self, L, ct, rotkeys, galois_elts, pts, evk_q_limbs=None, pt_q_limbs=None, out=None):
+        """sum_i pts[i] * rotate(ct, galois_elts[i]) with one ModUp and one ModDown (hml_hrotate_sum_hoisted).  pts[i] is
+        [pt_q_limbs + alpha][N]: Q-limbs first, P-limb j at row pt_q_limbs + j (pt_q_limbs defaults to L)."""
+        n = len(galois_elts)
+        if len(rotkeys) != n or len(pts) != n:
+            raise ValueError("one key and one plaintext per galois element")
+        out = self.empty(2, L, self.N) if out is None else out
+        keys = (C.c_void_p * max(n, 1))(*[_ptr(k) for k in rotkeys])
+        pa = (C.c_void_p * max(n, 1))(*[_ptr(p) for p in pts])
+        gs = (C.c_uint64 * max(n, 1))(*[int(g) for g in galois_elts])
+        self._chk(self.lib.hml_hrotate_sum_hoisted(self.h, L, _ptr(ct), n, keys, evk_q_limbs or L, gs, pa, pt_q_limbs or L, _ptr(out),
+                                                   self._stream()))
+        return out
 
     def hadd(self, L, a, b, out=None):
         out = self.empty(2, L, self.N) if out is None else out
@@ -699,10 +714,12 @@ def group_hrotate_hoisted(group, L, ct_own, keys, galois_elts, outs=None, stream
 class Replay:
     """hml_replay: a trace of (kind, dst, a, b) tuples over named ciphertexts, run through the C ABI (optionally as one CUDA
     graph, optionally with hoisted rotations, optionally limb-sharded).  `trace` uses the tuple format of
-    homulator_b200.replay; names are mapped to slots here ("x" = slot 0 = the input)."""
+    homulator_b200.replay; names are mapped to slots here ("x" = slot 0 = the input).  hoist_sum=True turns a hoistable run of
+    rotations whose outputs are summed with plaintext weights into one double-hoisted sum (HML_REPLAY_HOIST_SUM); the
+    plaintexts are then bound as [L + alpha][N] (P-limbs at rows L..)."""
     KINDS = {"hrotate": 0, "pmult": 1, "hadd": 2, "padd": 3, "hmult": 4}
 
-    def __init__(self, ctx, L, trace, shard=None, graph=False, hoist=False):
+    def __init__(self, ctx, L, trace, shard=None, graph=False, hoist=False, hoist_sum=False):
         self.ctx, self.L, self.shard = ctx, L, shard
         self.names = {"x": 0}
         ops = []
@@ -721,7 +738,7 @@ class Replay:
             ops.append((self.KINDS[kind], self.names[dst], self.names[a], bb))
         arr = (_TraceOp * len(ops))(*[_TraceOp(*o) for o in ops])
         self.h = C.c_void_p()
-        flags = (1 if graph else 0) | (2 if hoist else 0)
+        flags = (1 if graph else 0) | (2 if hoist else 0) | (4 if hoist_sum else 0)
         ctx._chk(ctx.lib.hml_replay_create(ctx.h, shard.h if shard is not None else None, L, arr, len(ops), flags, C.byref(self.h)))
         self._keep = None
 

@@ -1776,6 +1776,74 @@ extern "C" int hml_hrotate_hoisted(hml_ctx *ctx, uint32_t L, const uint64_t *ct,
   return hrot_hoisted_run(ctx, L, (const u64 *)ct, n_rot, rotkeys, evk_q_limbs, galois_elts, ct_outs, ctx->ws, (cudaStream_t)stream);
 }
 
+// Double-hoisted rotation sum (Bossuat et al., Eurocrypt 2021):  out = sum_r pt_r * rotate_r(ct) with ONE ModUp and ONE ModDown.
+// With t = ModUp(c1) (K1..K4, once), the inner products stay in the extended basis, are weighted by the plaintexts there and
+// summed (k_inner_rot_sum, one launch per group of IP_MAX_ROT rotations, later groups adding to the stored sums):
+//   acc_c = sum_r pt_r * sum_j sigma_r(t_j) * rk_r[j][c],   z = sum_r pt_r * sigma_r(c0)   (Q-limbs)
+//   out   = (ModDown(acc_0) + z, ModDown(acc_1))            (the P-limb INTT of ks_inner, then ks_tail, once)
+// Not bit-identical to sum_r pt_r * hml_hrotate_hoisted_r: ModDown of a sum differs from the sum of ModDowns by the
+// approximate conversion's overflow terms; the oracle defines the op itself (tests/orc_rotsum.py).  n = 1 with pt = 1 on every
+// limb of the extended basis is hml_hrotate_hoisted bit for bit.
+static int hrot_sum_hoisted_run(hml_ctx *ctx, uint32_t L, const u64 *ct, uint32_t n_rot, const uint64_t *const *rotkeys, uint32_t evk_q_limbs,
+                                const uint64_t *galois, const uint64_t *const *pts, uint32_t pt_q_limbs, u64 *ct_out, u64 *ws, cudaStream_t s) {
+  const Params &p = ctx->p;
+  const uint32_t kq = evk_q_limbs & ~HML_KEY_PACKED;
+  if (kq < L || kq > p.max_level) return fail(ctx, HML_ERR_INVALID, "evk_q_limbs must be in [L, maxLevel]");
+  if (pt_q_limbs < L || pt_q_limbs > p.max_level) return fail(ctx, HML_ERR_INVALID, "pt_q_limbs must be in [L, maxLevel]");
+  LevelConsts *lc;
+  int rc = get_level(ctx, L, &lc);
+  if (rc) return rc;
+  const size_t N = p.N, PL = N * L;
+  const uint32_t A = p.alpha, E = L + A, beta = lc->beta;
+  if (beta > 8) return fail(ctx, HML_ERR_UNSUPPORTED, "more than 8 key-switch digits (ceil(L/alpha) > 8)");
+  // the workspace of hrot_hoisted_run: zb [L] (of 2L) | yb [L] | ext [beta][E] | acc [2][E] | vb [2][L]
+  u64 *zb = ws, *yb = zb + 2 * PL, *ext = yb + PL, *acc = ext + (size_t)beta * E * N, *vb = acc + 2 * (size_t)E * N;
+  const BatchPtr c1{ct + PL, 0};
+  if ((rc = ks_modup(ctx, lc, L, 1, c1, yb, ext, s, nullptr))) return rc;
+  LimbMap ip = lc->ext_lm;  // pos = limb index inside the key, as in ks_inner
+  for (uint32_t e = 0; e < E; ++e) ip.pos[e] = (uint16_t)(e < L ? e : kq + (e - L));
+  InnerRotSumArgs a{};
+  a.d = c1.ptr; a.ext = ext; a.c0 = ct; a.acc = acc; a.z = zb;
+  a.N = (int)N; a.n_ext = (int)E; a.L = (int)L; a.beta = (int)beta; a.evk_limbs = (int)(kq + A); a.pt_q_limbs = (int)pt_q_limbs; a.logN = p.logN;
+  a.ext_f64 = p.logN > NTT_SMALL_LOG; a.evk_packed = (evk_q_limbs & HML_KEY_PACKED) ? 1 : 0;
+  for (uint32_t r0 = 0; r0 < n_rot; r0 += IP_MAX_ROT) {
+    const uint32_t n = std::min<uint32_t>(IP_MAX_ROT, n_rot - r0);
+    a.accumulate = r0 > 0; a.n_rot = (int)n;
+    for (uint32_t k = 0; k < n; ++k) {
+      const unsigned g = (unsigned)(galois[r0 + k] & (2ull * N - 1));
+      a.evk[k] = (const u64 *)rotkeys[r0 + k]; a.pt[k] = (const u64 *)pts[r0 + k]; a.galois[k] = g == 1 ? 0 : g;
+    }
+    launch_inner_product_rot_sum(ctx->mc, ip, a, s);
+    prof_mark(ctx, HML_CLS_EWE, s);
+    ctx->exec.kernel_launches++;
+    ctx->exec.ewe_limbs += (uint64_t)n * (2ull * E * beta + 2ull * E + L);
+    ctx->exec.automorph_limbs += (uint64_t)n * L;  // sigma_r(c0), applied on load
+  }
+  if ((rc = ks_inner(ctx, lc, L, 1, c1, nullptr, evk_q_limbs, ext, acc, E, 0, s, nullptr, true))) return rc;
+  if ((rc = ks_tail(ctx, lc, L, 1, acc, vb, {ct_out, 0}, {ct_out + PL, 0}, {zb, 0}, {nullptr, 0}, s, false, 0))) return rc;
+  return check_launch(ctx, "hrotate sum hoisted");
+}
+
+extern "C" int hml_hrotate_sum_hoisted(hml_ctx *ctx, uint32_t L, const uint64_t *ct, uint32_t n_rot, const uint64_t *const *rotkeys,
+                                       uint32_t evk_q_limbs, const uint64_t *galois_elts, const uint64_t *const *pts, uint32_t pt_q_limbs,
+                                       uint64_t *ct_out, void *stream) {
+  int rc = check_level(ctx, L, 1);
+  if (rc) return rc;
+  if (n_rot == 0) return fail(ctx, HML_ERR_INVALID, "n_rot must be at least 1");
+  if (!ct || !rotkeys || !galois_elts || !pts || !ct_out) return fail(ctx, HML_ERR_INVALID, "null buffer");
+  const size_t w = 2 * (size_t)ctx->p.N * L;
+  if (ct_out < ct + w && ct < ct_out + w) return fail(ctx, HML_ERR_INVALID, "the output overlaps the input");
+  for (uint32_t r = 0; r < n_rot; ++r) {
+    if (!rotkeys[r] || !pts[r]) return fail(ctx, HML_ERR_INVALID, "null key or plaintext");
+    if (!(galois_elts[r] & 1)) return fail(ctx, HML_ERR_INVALID, "galois element must be odd");
+  }
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  if ((rc = ensure_ws(ctx, hrot_ws_words(ctx->p, L, 1)))) return rc;
+  ws_enter(ctx, (cudaStream_t)stream);
+  return hrot_sum_hoisted_run(ctx, L, (const u64 *)ct, n_rot, rotkeys, evk_q_limbs, galois_elts, pts, pt_q_limbs, (u64 *)ct_out, ctx->ws,
+                              (cudaStream_t)stream);
+}
+
 static int ew_ct_op(hml_ctx *ctx, uint32_t L, const uint64_t *a, const uint64_t *b, bool b_is_pt, bool mul, uint64_t *out, void *stream) {
   int rc = check_level(ctx, L, 1);
   if (rc) return rc;

@@ -309,6 +309,127 @@ void launch_inner_product_rot(const ModConst *mc, const LimbMap &lm, const Inner
   else launch_pdl(k_inner_rot<8>, g, EW_THREADS, 0, s, mc, lm, a);
 }
 
+// Double-hoisted rotation sum (ewe.cuh InnerRotSumArgs).  The body of k_inner_rot once per rotation, then the two component
+// sums are weighted by the plaintext and kept in registers: the op is bound by reading the keys, and every rotation's key,
+// plaintext and c0 loads are issued before its first use.  The argument table is read in place (grid constant), so the
+// rotation index may be a loop variable.  Exact: |sum_j| <= 8 * 0.51 q, each weighted term <= 0.51 q, 16 terms + one stored
+// word stay far below 2^51.  PACKED (the key's load path) is a template argument: with both paths in one body four digits
+// spilled at 128 registers.  Up to three digits fit three CTAs per SM (76 registers), four digits two (108-128), five to eight
+// digits one (229-237).
+template <int IP_MAX_BETA, bool PACKED>
+__global__ void __launch_bounds__(EW_THREADS, IP_MAX_BETA > 4 ? 1 : IP_MAX_BETA > 3 ? 2 : 3)
+    k_inner_rot_sum(const ModConst *__restrict__ mc, LimbMap lm, const __grid_constant__ InnerRotSumArgs a) {
+  pdl_wait();
+  const int i2 = blockIdx.x * EW_THREADS + threadIdx.x;
+  if (i2 >= a.N / 2) return;
+  const int e = blockIdx.y;
+  const ModConst m = mc[lm.mod[e]];
+  const int kl = lm.pos[e], own = lm.skip[e];
+  const size_t n2 = a.N / 2;
+  const bool q_limb = e < a.L;  // uniform per CTA
+  const size_t prow = q_limb ? (size_t)e : (size_t)a.pt_q_limbs + (e - a.L);
+  double a00 = 0, a01 = 0, a10 = 0, a11 = 0, z0 = 0, z1 = 0;  // [component][coefficient], z = the c0 term
+#pragma unroll 1
+  for (int r = 0; r < a.n_rot; ++r) {
+    const unsigned g = a.galois[r];
+    unsigned s0 = 2u * i2, s1 = 2u * i2 + 1u;
+    if (g) {  // the index formula of k_inner
+      const unsigned sh = 32 - a.logN, m2n = (2u << a.logN) - 1u;
+      s0 = __brev((((g * (2u * (__brev(s0) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
+      s1 = __brev((((g * (2u * (__brev(s1) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
+    }
+    ulonglong2 t[IP_MAX_BETA];
+#pragma unroll
+    for (int j = 0; j < IP_MAX_BETA; ++j)
+      if (j < a.beta) {
+        const u64 *p = j == own ? a.d + (size_t)e * a.N : a.ext + ((size_t)j * a.n_ext + e) * a.N;
+        t[j] = g ? make_ulonglong2(__ldg(p + s0), __ldg(p + s1)) : ld2(p, i2);
+      }
+    const u64 *evk = a.evk[r];
+    ulonglong2 kraw[IP_MAX_BETA][2];
+    if constexpr (PACKED) {  // the packed load path of k_inner (kraw.x = the pair's low words, kraw.y = its two high bytes)
+#pragma unroll
+      for (int j = 0; j < IP_MAX_BETA; ++j)
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {
+          const u64 *slot = evk + (((size_t)j * 2 + c) * a.evk_limbs + kl) * a.N;
+          kraw[j][c] = j < a.beta ? make_ulonglong2(__ldg(slot + i2),
+                                                    __ldg(reinterpret_cast<const unsigned short *>(reinterpret_cast<const unsigned char *>(slot) + 4 * (size_t)a.N) + i2))
+                                  : make_ulonglong2(0, 0);
+        }
+    } else {
+#pragma unroll
+      for (int j = 0; j < IP_MAX_BETA; ++j)
+#pragma unroll
+        for (int c = 0; c < 2; ++c)
+          kraw[j][c] = j < a.beta ? ld2(evk, (((size_t)j * 2 + c) * a.evk_limbs + kl) * n2 + i2) : make_ulonglong2(0, 0);
+    }
+    ulonglong2 w = ld2(a.pt[r] + prow * a.N, i2), x = make_ulonglong2(0, 0);
+    if (q_limb) {
+      const u64 *p = a.c0 + (size_t)e * a.N;
+      x = g ? make_ulonglong2(__ldg(p + s0), __ldg(p + s1)) : ld2(p, i2);
+    }
+    pin_loads(kraw);
+    asm volatile("" : "+l"(w.x), "+l"(w.y), "+l"(x.x), "+l"(x.y));
+    if constexpr (PACKED) {
+#pragma unroll
+      for (int j = 0; j < IP_MAX_BETA; ++j)
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {
+          const u64 lo = kraw[j][c].x, hi = kraw[j][c].y;
+          kraw[j][c] = make_ulonglong2(((hi & 0xFFull) << 32) | (lo & 0xFFFFFFFFull), ((hi >> 8) << 32) | (lo >> 32));
+        }
+    }
+    double s00 = 0, s01 = 0, s10 = 0, s11 = 0;
+#pragma unroll
+    for (int j = 0; j < IP_MAX_BETA; ++j)
+      if (j < a.beta) {
+        const bool f64 = a.ext_f64 && j != own;
+        const double t0 = f64 ? __longlong_as_double((long long)t[j].x) : u64_to_f64(t[j].x);
+        const double t1 = f64 ? __longlong_as_double((long long)t[j].y) : u64_to_f64(t[j].y);
+        s00 += mulmod_var(t0, u64_to_f64(kraw[j][0].x), m.q, m.qinv);
+        s01 += mulmod_var(t1, u64_to_f64(kraw[j][0].y), m.q, m.qinv);
+        s10 += mulmod_var(t0, u64_to_f64(kraw[j][1].x), m.q, m.qinv);
+        s11 += mulmod_var(t1, u64_to_f64(kraw[j][1].y), m.q, m.qinv);
+      }
+    const double w0 = u64_to_f64(w.x), w1 = u64_to_f64(w.y);
+    a00 += mulmod_var(s00, w0, m.q, m.qinv);
+    a01 += mulmod_var(s01, w1, m.q, m.qinv);
+    a10 += mulmod_var(s10, w0, m.q, m.qinv);
+    a11 += mulmod_var(s11, w1, m.q, m.qinv);
+    if (q_limb) {
+      z0 += mulmod_var(u64_to_f64(x.x), w0, m.q, m.qinv);
+      z1 += mulmod_var(u64_to_f64(x.y), w1, m.q, m.qinv);
+    }
+  }
+  const size_t o0 = (size_t)e * n2 + i2, o1 = (size_t)(a.n_ext + e) * n2 + i2;
+  if (a.accumulate) {  // uniform: a later group of the same op
+    const ulonglong2 p0 = ld2(a.acc, o0), p1 = ld2(a.acc, o1);
+    a00 += u64_to_f64(p0.x); a01 += u64_to_f64(p0.y); a10 += u64_to_f64(p1.x); a11 += u64_to_f64(p1.y);
+    if (q_limb) {
+      const ulonglong2 pz = ld2(a.z, o0);
+      z0 += u64_to_f64(pz.x); z1 += u64_to_f64(pz.y);
+    }
+  }
+  st2(a.acc, o0, finish(a00, m), finish(a01, m));
+  st2(a.acc, o1, finish(a10, m), finish(a11, m));
+  if (q_limb) st2(a.z, o0, finish(z0, m), finish(z1, m));
+}
+
+template <bool PACKED>
+static void launch_inner_rot_sum_t(const ModConst *mc, const LimbMap &lm, const InnerRotSumArgs &a, cudaStream_t s) {
+  const dim3 g = ew_grid(a.N, a.n_ext);
+  if (a.beta <= 1) launch_pdl(k_inner_rot_sum<1, PACKED>, g, EW_THREADS, 0, s, mc, lm, a);
+  else if (a.beta <= 2) launch_pdl(k_inner_rot_sum<2, PACKED>, g, EW_THREADS, 0, s, mc, lm, a);
+  else if (a.beta <= 3) launch_pdl(k_inner_rot_sum<3, PACKED>, g, EW_THREADS, 0, s, mc, lm, a);
+  else if (a.beta <= 4) launch_pdl(k_inner_rot_sum<4, PACKED>, g, EW_THREADS, 0, s, mc, lm, a);
+  else launch_pdl(k_inner_rot_sum<8, PACKED>, g, EW_THREADS, 0, s, mc, lm, a);
+}
+void launch_inner_product_rot_sum(const ModConst *mc, const LimbMap &lm, const InnerRotSumArgs &a, cudaStream_t s) {
+  if (a.evk_packed) launch_inner_rot_sum_t<true>(mc, lm, a, s);
+  else launch_inner_rot_sum_t<false>(mc, lm, a, s);
+}
+
 // ------------------------------------------------------------------------------------------------ (x - y) * c (+ z)
 __global__ void __launch_bounds__(EW_THREADS) k_sub_mul_add(const ModConst *__restrict__ mc, LimbMap lm, SubMulArgs a) {
   pdl_wait();

@@ -71,6 +71,28 @@ struct InnerRotArgs {
 };
 void launch_inner_product_rot(const ModConst *mc, const LimbMap &lm, const InnerRotArgs &a, int n_rot, cudaStream_t s);
 
+// Double-hoisted rotation sum (context.cu, hrot_sum_hoisted_run): the inner product of up to IP_MAX_ROT rotations of one
+// ciphertext, each weighted by its plaintext in the extended basis and summed before any ModDown.  One thread serves one
+// coefficient pair of extended limb e (grid (N/2/256, n_ext)) and loops over the rotations r < n_rot:
+//   acc[c][e] (+)= sum_r pt_r[e] * sum_j sigma_r(t_j)[e] * evk_r[j][c][lm.pos[e]]        (words, [2][n_ext][N])
+//   z[e]      (+)= sum_r pt_r[e] * sigma_r(c0)[e]                          for e < L      (words, [L][N])
+// t_j as in InnerArgs (d for the digit's own limbs, else ext), read through sigma_r like InnerRotArgs.  pt_r[e] is row
+// e < L ? e : pt_q_limbs + (e - L) of pt[r].  accumulate = 1 adds to what acc / z hold (the later groups of one op).
+struct InnerRotSumArgs {
+  const u64 *d;                    // [>= number of owned Q-limbs][N] (c1)
+  const u64 *ext;                  // [beta][n_ext][N]
+  const u64 *c0;                   // [L][N]
+  u64 *acc, *z;
+  int N, n_ext, L, beta, evk_limbs, pt_q_limbs, logN;  // beta <= 8
+  int ext_f64;                     // as InnerArgs::ext_f64
+  int evk_packed;                  // as InnerArgs::evk_packed
+  int accumulate, n_rot;           // n_rot <= IP_MAX_ROT
+  const u64 *evk[IP_MAX_ROT];      // [beta][2][evk_limbs][N] per rotation
+  const u64 *pt[IP_MAX_ROT];       // [pt_q_limbs + alpha][N] per rotation
+  unsigned galois[IP_MAX_ROT];     // galois element mod 2N per rotation; 0 = identity
+};
+void launch_inner_product_rot_sum(const ModConst *mc, const LimbMap &lm, const InnerRotSumArgs &a, cudaStream_t s);
+
 // out = (x - y) * c (+ z) per limb:  ModDownSub (+ HMULT add)  reference src/Operation.cpp:548-590, :967-1005
 // and Rescale sub+mul  reference src/Operation.cpp:825-911.  cst[limb] = (c, RN(c/q)).  n_polys via strides.
 struct SubMulArgs {

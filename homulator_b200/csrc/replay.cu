@@ -7,7 +7,8 @@
 // layout with evk_q_limbs >= L serve every level; a plaintext's first limbs serve the lower levels).  A trace runs on one GPU
 // (hml_ctx) or limb-sharded over a group (hml_shard), as plain launches or as ONE captured CUDA graph,
 // and optionally with hoisted rotations: consecutive hrotate ops that read the same slot share one ModUp
-// (hml_hrotate_hoisted on one GPU, hml_hrotate_hoisted_sharded over a shard group).
+// (hml_hrotate_hoisted on one GPU, hml_hrotate_hoisted_sharded over a shard group).  On one GPU such a run whose outputs are
+// summed with plaintext weights right after it may also become one double-hoisted sum (hml_hrotate_sum_hoisted).
 #include <algorithm>
 #include <cstring>
 #include <map>
@@ -57,6 +58,7 @@ extern "C" int hml_replay_create(hml_ctx *ctx, hml_shard *sh, uint32_t L, const 
   *out = nullptr;
   int rc = check_level(ctx, L, 1);
   if (rc) return rc;
+  if (sh && (flags & HML_REPLAY_HOIST_SUM)) return fail(ctx, HML_ERR_UNSUPPORTED, "HML_REPLAY_HOIST_SUM has no limb-sharded op");
   hml_replay *rp = new hml_replay();
   rp->ctx = ctx; rp->sh = sh; rp->L = L; rp->flags = flags;
   rp->ops.assign(ops, ops + n_ops);
@@ -154,6 +156,57 @@ static uint64_t galois_of(const hml_ctx *ctx, uint32_t r) {
   return g;
 }
 
+// true when `slot` is dead from op `from` on: its next access, if any, is a write
+static bool dead_from(const std::vector<hml_trace_op> &ops, size_t from, uint32_t slot) {
+  for (size_t k = from; k < ops.size(); ++k) {
+    const hml_trace_op &q = ops[k];
+    if (q.a == slot || ((q.kind == HML_OP_HADD || q.kind == HML_OP_HMULT) && q.b == slot)) return false;
+    if (q.dst == slot) return true;
+  }
+  return true;
+}
+
+// HML_REPLAY_HOIST_SUM: the rotations ops[i, j) of one source are followed directly by
+//   pmult(y, d, pt), then n - 1 times  pmult(t, d, pt); hadd(y, y, t) (or hadd(y, t, y)),
+// consuming every rotation output d exactly once, with y neither the source nor a rotation output, t none of y, the source or
+// a rotation output, and every d and t dead afterwards.  On a match: *end = the op after the chain, *y = its slot and
+// pt_of[k] = the plaintext that weights rotation i + k.
+static bool match_rot_sum(const std::vector<hml_trace_op> &ops, size_t i, size_t j, size_t *end, uint32_t *y, std::vector<uint32_t> &pt_of) {
+  const size_t n = j - i;
+  const uint32_t src = ops[i].a, none = ~0u;
+  auto rot_of = [&](uint32_t slot) -> size_t {
+    for (size_t k = 0; k < n; ++k)
+      if (ops[i + k].dst == slot) return k;
+    return n;
+  };
+  pt_of.assign(n, none);
+  size_t k = j;
+  if (k >= ops.size() || ops[k].kind != HML_OP_PMULT) return false;
+  const uint32_t acc = ops[k].dst;
+  size_t r = rot_of(ops[k].a);
+  if (r == n || acc == src || rot_of(acc) != n) return false;
+  pt_of[r] = ops[k].b;
+  std::vector<uint32_t> temps;
+  for (k = j + 1; temps.size() + 1 < n; k += 2) {
+    if (k + 1 >= ops.size()) return false;
+    const hml_trace_op &pm = ops[k], &ad = ops[k + 1];
+    if (pm.kind != HML_OP_PMULT || ad.kind != HML_OP_HADD) return false;
+    const uint32_t t = pm.dst;
+    r = rot_of(pm.a);
+    if (r == n || pt_of[r] != none || t == acc || t == src || rot_of(t) != n) return false;
+    if (ad.dst != acc || !((ad.a == acc && ad.b == t) || (ad.a == t && ad.b == acc))) return false;
+    pt_of[r] = pm.b;
+    temps.push_back(t);
+  }
+  for (size_t q = 0; q < n; ++q)
+    if (!dead_from(ops, k, ops[i + q].dst)) return false;
+  for (uint32_t t : temps)
+    if (!dead_from(ops, k, t)) return false;
+  *end = k;
+  *y = acc;
+  return true;
+}
+
 static int enqueue(hml_replay *rp, cudaStream_t s) {
   hml_ctx *ctx = rp->ctx;
   void *st = (void *)s;
@@ -165,7 +218,7 @@ static int enqueue(hml_replay *rp, cudaStream_t s) {
     const uint64_t *a = rp->slot[o.a];
     switch (o.kind) {
       case HML_OP_HROTATE: {
-        if (rp->flags & HML_REPLAY_HOIST) {
+        if (rp->flags & (HML_REPLAY_HOIST | HML_REPLAY_HOIST_SUM)) {
           // the run of consecutive rotations of the same source (none of which overwrites it) shares one ModUp
           size_t j = i;
           std::vector<const uint64_t *> keys;
@@ -180,7 +233,18 @@ static int enqueue(hml_replay *rp, cudaStream_t s) {
             outs.push_back(rp->slot[rp->ops[j].dst]);
             ++j;
           }
-          if (outs.size() >= 2) {
+          size_t end;
+          uint32_t y;
+          std::vector<uint32_t> pt_of;
+          if (outs.size() >= 2 && (rp->flags & HML_REPLAY_HOIST_SUM) && match_rot_sum(rp->ops, i, j, &end, &y, pt_of)) {
+            std::vector<const uint64_t *> pts;
+            for (uint32_t b : pt_of) pts.push_back(rp->pts[b]);
+            rc = hml_hrotate_sum_hoisted(ctx, L, a, (uint32_t)outs.size(), keys.data(), rp->evk_q_limbs, gs.data(), pts.data(), rp->L,
+                                         rp->slot[y], st);
+            i = end - 1;
+            break;
+          }
+          if (outs.size() >= 2 && (rp->flags & HML_REPLAY_HOIST)) {
             rc = rp->sh ? hml_hrotate_hoisted_sharded(rp->sh, L, a, (uint32_t)outs.size(), keys.data(), gs.data(), outs.data(), st)
                         : hml_hrotate_hoisted(ctx, L, a, (uint32_t)outs.size(), keys.data(), rp->evk_q_limbs, gs.data(), outs.data(), st);
             i = j - 1;
@@ -198,14 +262,7 @@ static int enqueue(hml_replay *rp, cudaStream_t s) {
         if (i + 1 < rp->ops.size()) {
           const hml_trace_op &n = rp->ops[i + 1];
           const bool pair = n.kind == HML_OP_HADD && n.dst != o.dst && rp->op_level[i + 1] == L && ((n.a == n.dst && n.b == o.dst) || (n.b == n.dst && n.a == o.dst)) && o.a != n.dst;
-          bool dead = pair;
-          for (size_t k = i + 2; k < rp->ops.size() && dead; ++k) {
-            const hml_trace_op &q = rp->ops[k];
-            const bool reads = q.a == o.dst || ((q.kind == HML_OP_HADD || q.kind == HML_OP_HMULT) && q.b == o.dst);
-            if (reads) dead = false;
-            else if (q.dst == o.dst) break;  // overwritten before any read
-          }
-          if (pair && dead) {
+          if (pair && dead_from(rp->ops, i + 2, o.dst)) {
             uint64_t *acc = rp->slot[n.dst];
             rc = rp->sh ? hml_ew_sharded(rp->sh, L, 3, a, rp->pts[o.b], acc, st) : hml_pmult_add(ctx, L, a, rp->pts[o.b], acc, acc, st);
             ++i;

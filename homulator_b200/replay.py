@@ -9,7 +9,7 @@ tuples over the five operations the reference's CLI accepts (reference bench_tes
     ("padd",    dst, src, pt)       dst = src + plaintext[pt]
     ("hmult",   dst, a, b)          dst = rescale(relin(a * b))       (drops one level; final)
 Execution lives in the library (homulator_b200/csrc/replay.cu: hml_replay_*): plain launches or one captured CUDA graph,
-textbook or hoisted rotations, one GPU or limb-sharded over a group.  This module only defines the synthetic traces and maps
+textbook, hoisted or (one GPU) double-hoisted rotation sums, one GPU or limb-sharded over a group.  This module only defines the synthetic traces and maps
 names to slots (homulator_b200.api.Replay).
 """
 from collections import Counter
@@ -58,10 +58,11 @@ def trace_counts(trace):
     return dict(Counter(op[0] for op in trace))
 
 
-def replay(ctx, L, trace, x, plaintexts, rot_keys, evk, graph=False, hoist=False, names=("y", "z")):
-    """Run `trace` once at level L through hml_replay_* and return {name: tensor} for `names` (copies)."""
+def replay(ctx, L, trace, x, plaintexts, rot_keys, evk, graph=False, hoist=False, hoist_sum=False, names=("y", "z")):
+    """Run `trace` once at level L through hml_replay_* and return {name: tensor} for `names` (copies).  With hoist_sum=True
+    the plaintexts are [L + alpha][N] (see homulator_b200.api.Replay)."""
     from .api import Replay
-    rp = Replay(ctx, L, trace, graph=graph, hoist=hoist).bind(x, plaintexts, rot_keys, evk)
+    rp = Replay(ctx, L, trace, graph=graph, hoist=hoist, hoist_sum=hoist_sum).bind(x, plaintexts, rot_keys, evk)
     rp.run()
     out = {n: rp.result(n).clone() for n in names if n in rp.names}
     rp.close()

@@ -277,6 +277,26 @@ int hml_hrotate(hml_ctx *ctx, uint32_t L, const uint64_t *ct, const uint64_t *ro
  * ct_outs are HOST arrays of n_rot entries; no output may alias the input. */
 int hml_hrotate_hoisted(hml_ctx *ctx, uint32_t L, const uint64_t *ct, uint32_t n_rot, const uint64_t *const *rotkeys,
                         uint32_t evk_q_limbs, const uint64_t *galois_elts, uint64_t *const *ct_outs, void *stream);
+/* Double-hoisted rotation sum (Bossuat et al., Eurocrypt 2021): ct_out = sum_i pts[i] * rotate(ct, galois_elts[i]) with ONE
+ * ModUp of c1 and ONE ModDown.  With t = ModUp(c1) and E = (q_0..q_{L-1}, p_0..p_{alpha-1}):
+ *   acc_c[m] = sum_i pt_i[m] * sum_j sigma_i(t_j)[m] * rotkeys[i][j][c][m]     (m in E, c = 0, 1)
+ *   z[l]     = sum_i pt_i[l] * sigma_i(c0)[l]                                  (l < L)
+ *   ct_out   = (z + ModDown(acc_0), ModDown(acc_1))
+ * sigma_i is applied to every digit limb, as in hml_hrotate_hoisted; galois element 1 is the identity (with a key).  With
+ * n_rot = 1 and pt = 1 on every limb of E the result is hml_hrotate_hoisted's bit for bit.  In general it is NOT
+ * sum_i pt_i * hml_hrotate_hoisted_i bit for bit (ModDown of a sum differs from the sum of ModDowns through the approximate base
+ * conversion) and an equally valid result, pinned by its own oracle definition (tests/orc_rotsum.py).
+ * ct, ct_out [2][L][N], not overlapping.  rotkeys / galois_elts / pts are HOST arrays of n_rot entries; pts[i] is
+ * [pt_q_limbs + alpha][N] in the key's convention (Q-limbs first, P-limb j at row pt_q_limbs + j), so a plaintext laid out for
+ * a higher level serves every level from L up to pt_q_limbs.  evk_q_limbs and pt_q_limbs lie in [L, maxLevel] (keys may be
+ * packed: HML_KEY_PACKED).  HML_ERR_INVALID: n_rot = 0, a null key / plaintext / output, an even galois element, overlapping
+ * ct / ct_out, limbs out of range; HML_ERR_UNSUPPORTED: more than 8 digits.
+ * Executed counts: per call the key switch's ModUp, the P-limb INTT of both accumulators and one ModDown (as hml_keyswitch),
+ * and one kernel launch per group of 16 rotations; per rotation ewe_limbs += 2 * beta * E + 2 * E + L and
+ * automorph_limbs += L (the automorphism rides on the loads).  No transform or conversion grows with n_rot. */
+int hml_hrotate_sum_hoisted(hml_ctx *ctx, uint32_t L, const uint64_t *ct, uint32_t n_rot, const uint64_t *const *rotkeys,
+                            uint32_t evk_q_limbs, const uint64_t *galois_elts, const uint64_t *const *pts, uint32_t pt_q_limbs,
+                            uint64_t *ct_out, void *stream);
 /* HADD / PMULT / PADD (reference src/Operation.cpp:1114-1176, :1453-1523, :1618-1680).  pt is [L][N].
  * PADD adds the plaintext to BOTH components, as the reference's trace does (:1650-1672). */
 int hml_hadd(hml_ctx *ctx, uint32_t L, const uint64_t *ct_a, const uint64_t *ct_b, uint64_t *ct_out, void *stream);
@@ -326,10 +346,17 @@ int hml_host_free_pinned(hml_ctx *ctx, uint64_t *ptr);
  *   HADD    dst = a + slot b                                                     HMULT dst = rescale(relin(a * slot b))
  * flags: HML_REPLAY_GRAPH — the whole sequence is captured once into a CUDA graph (after a warm-up run) and every run is one
  * graph launch; HML_REPLAY_HOIST — consecutive rotations of one source share a ModUp (hml_hrotate_hoisted, or
- * hml_hrotate_hoisted_sharded when sh != NULL).
+ * hml_hrotate_hoisted_sharded when sh != NULL); HML_REPLAY_HOIST_SUM — a run of at least two such rotations (same rule)
+ * that is directly followed by a plaintext-weighted accumulation of all their outputs,
+ *   PMULT y = d_k * pt,  then  { PMULT t = d_k * pt; HADD y = y + t (or t + y) }  once for every other output d_k,
+ * becomes ONE hml_hrotate_sum_hoisted that writes y — when y is neither the source nor a rotation output and every d_k and t is
+ * dead afterwards (its next access, if any, is a write).  The fused rotation outputs and t are then left unwritten, as the t of
+ * a fused PMULT / HADD pair already is.  Anything else runs as without the flag (through HML_REPLAY_HOIST when that is set
+ * too).  With HML_REPLAY_HOIST_SUM every plaintext is bound as [L + alpha][N] (P-limb j at row L + j, L = the replay's
+ * level); PMULT and PADD read its first limbs as before.  Not available with sh != NULL (HML_ERR_UNSUPPORTED).
  * With sh != NULL the trace runs limb-sharded: every pointer is the rank's owned-limb slice (see the sharded layouts above). */
 enum { HML_OP_HROTATE = 0, HML_OP_PMULT = 1, HML_OP_HADD = 2, HML_OP_PADD = 3, HML_OP_HMULT = 4 };
-enum { HML_REPLAY_GRAPH = 1, HML_REPLAY_HOIST = 2 };
+enum { HML_REPLAY_GRAPH = 1, HML_REPLAY_HOIST = 2, HML_REPLAY_HOIST_SUM = 4 };
 typedef struct { uint32_t kind, dst, a, b; } hml_trace_op;
 typedef struct hml_replay hml_replay;
 int hml_replay_create(hml_ctx *ctx, hml_shard *sh, uint32_t L, const hml_trace_op *ops, uint32_t n_ops, uint32_t flags,
