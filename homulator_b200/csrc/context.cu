@@ -714,7 +714,7 @@ static int ks_modup(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, Batc
       unsigned gi = 1;
       const unsigned g8 = (unsigned)(au->g & 255);
       for (int i = 0; i < 7; ++i) gi = gi * (2u - g8 * gi);  // Newton: g^-1 mod 256 (g odd)
-      l.in_galois = (unsigned)(au->g & (2ull * N - 1)); l.in_ginv8 = gi & 255u;
+      l.in_galois = galois_mod(au->g, N); l.in_ginv8 = gi & 255u;
       l.side_out = au->sigma_d; l.side_batch_stride = au->sigma_stride;
     }
     run_ntt(ctx, true, lc->q_lm, l, s);
@@ -745,30 +745,45 @@ static int ks_modup(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, Batc
   return HML_OK;
 }
 
+// The evaluation key of a level-L key switch, decoded once from (evk, evk_q_limbs): q_limbs Q-limbs, then the alpha P-limbs,
+// so extended limb e (the L Q-limbs, then the P-limbs) is key limb pos(e, L).
+struct KeyDesc {
+  const u64 *evk;
+  uint32_t q_limbs;  // evk_q_limbs without HML_KEY_PACKED
+  bool packed;       // HML_KEY_PACKED: the limb slots hold packed limbs (hml_key_pack)
+  uint32_t pos(uint32_t e, uint32_t L) const { return e < L ? e : q_limbs + (e - L); }
+};
+static int key_desc(hml_ctx *ctx, uint32_t L, const u64 *evk, uint32_t evk_q_limbs, KeyDesc *k) {
+  const Params &p = ctx->p;
+  const uint32_t q = evk_q_limbs & ~HML_KEY_PACKED;
+  if (q < L || q > p.max_level) return fail(ctx, HML_ERR_INVALID, "evk_q_limbs must be in [L, maxLevel]");
+  if (p.beta(L) > 8) return fail(ctx, HML_ERR_UNSUPPORTED, "more than 8 key-switch digits (ceil(L/alpha) > 8)");
+  *k = KeyDesc{evk, q, (evk_q_limbs & HML_KEY_PACKED) != 0};
+  return HML_OK;
+}
+
 // K5..K7: inner product with the key, INTT (+ step-1 scaling) of the P-limbs of both accumulators.  acc [nb][2][AL], AL >= E.
 // galois != 0: the digits are read through the automorphism X -> X^galois (hoisted rotation, see InnerArgs::galois).
-static int ks_inner(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, const u64 *evk, uint32_t evk_q_limbs, const u64 *ext, u64 *acc,
+static int ks_inner(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, const KeyDesc &key, const u64 *ext, u64 *acc,
                     uint32_t AL, u64 galois, cudaStream_t s, const MergedU *mu = nullptr, bool ip_done = false) {
   const Params &p = ctx->p;
   const size_t N = p.N;
   const uint32_t A = p.alpha, E = L + A, beta = lc->beta;
   const int logN = p.logN, npass = logN <= NTT_SMALL_LOG ? 1 : 2;
-  const bool key_packed = (evk_q_limbs & HML_KEY_PACKED) != 0;
-  evk_q_limbs &= ~HML_KEY_PACKED;
   // K5 (reference :294-414): inner product with the key (key words loaded once per batch) — unless the ModUp transform's row
   // pass has already done it (ks_front with HPIP)
   if (!ip_done) {
-    LimbMap ip = lc->ext_lm;  // pos = limb index inside the key (Q-limbs first, then P-limbs after evk_q_limbs)
-    for (uint32_t e = 0; e < E; ++e) ip.pos[e] = (uint16_t)(e < L ? e : evk_q_limbs + (e - L));
+    LimbMap ip = lc->ext_lm;  // pos = limb index inside the key
+    for (uint32_t e = 0; e < E; ++e) ip.pos[e] = (uint16_t)key.pos(e, L);
     InnerArgs a{};
-    a.d = d.ptr; a.ext = ext; a.evk = evk; a.evk_packed = key_packed ? 1 : 0; a.acc = acc; a.N = N; a.n_ext = E; a.beta = beta; a.evk_limbs = evk_q_limbs + A;
+    a.d = d.ptr; a.ext = ext; a.evk = key.evk; a.evk_packed = key.packed ? 1 : 0; a.acc = acc; a.N = N; a.n_ext = E; a.beta = beta;
+    a.evk_limbs = key.q_limbs + A;
     a.n_batch = nb; a.d_batch_stride = d.stride; a.ext_batch_stride = (long long)beta * E * N; a.acc_batch_stride = 2ll * AL * N;
     a.acc_comp_stride = (long long)AL * N; a.ext_f64 = npass == 2;
     // Q-limb accumulators only feed element-wise epilogues: packed (5 B / coefficient) — but the HPIP path, which some other
     // call of this level may take, leaves words, and the consumers are told per call (ks_tail's acc_packed)
     a.acc_pack_limbs = npass == 2 ? (int)L : 0;
-    a.galois = (unsigned)(galois & (2ull * N - 1)); a.logN = logN;
-    if (a.galois == 1) a.galois = 0;
+    a.galois = inner_galois(galois, N); a.logN = logN;
     a.u_limb = -1;
     if (mu && nb == 1) {  // hmult: u[L-1] = acc[L-1] * P^-1 + d[L-1] lands in slot E of each accumulator (host copy of the constant)
       a.u_limb = (int)L - 1; a.u_slot = (int)E; a.u_add = mu->add; a.u_add_comp_stride = mu->comp_stride; a.u_add_batch_stride = mu->batch_stride;
@@ -809,22 +824,19 @@ static int ks_inner(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, Batc
 // K1..K7.  Buffers: yb [nb][L] | ext [nb][beta][E] | acc [nb][2][AL] with AL >= E limbs per accumulator.
 // Two-pass rings with at least two digits fuse the inner product into the ModUp transform (NttMac): the Q-limb accumulators are
 // then 8-byte words (not packed limbs); ks_uses_hpip() tells the consumers.
-static int ks_front(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, const u64 *evk, uint32_t evk_q_limbs, u64 *yb,
+static int ks_front(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, const KeyDesc &key, u64 *yb,
                     u64 *ext, u64 *acc, uint32_t AL, cudaStream_t s, const MergedU *mu = nullptr, const KsAuto *au = nullptr) {
   const Params &p = ctx->p;
   const size_t N = p.N;
   const uint32_t A = p.alpha, E = L + A;
   const bool hpip = ks_uses_hpip(ctx, L, nb);
-  const bool key_packed = (evk_q_limbs & HML_KEY_PACKED) != 0;  // ks_inner strips the flag itself
-  const uint32_t evk_flagged = evk_q_limbs;
-  evk_q_limbs &= ~HML_KEY_PACKED;
   const BatchPtr d_raw = d;
   if (au) d = {au->sigma_d, au->sigma_stride};  // what K5 reads (written by the ModUp INTT)
   NttMac mac{};
   if (hpip) {
-    mac.evk = evk; mac.evk_packed = key_packed ? 1 : 0; mac.d = d.ptr; mac.acc = acc; mac.d_batch_stride = d.stride; mac.acc_batch_stride = 2ll * AL * N;
-    mac.acc_comp_stride = (long long)AL * N; mac.evk_limbs = (int)(evk_q_limbs + A);
-    for (uint32_t e = 0; e < E; ++e) mac.key_pos[e] = (uint16_t)(e < L ? e : evk_q_limbs + (e - L));
+    mac.evk = key.evk; mac.evk_packed = key.packed ? 1 : 0; mac.d = d.ptr; mac.acc = acc; mac.d_batch_stride = d.stride; mac.acc_batch_stride = 2ll * AL * N;
+    mac.acc_comp_stride = (long long)AL * N; mac.evk_limbs = (int)(key.q_limbs + A);
+    for (uint32_t e = 0; e < E; ++e) mac.key_pos[e] = (uint16_t)key.pos(e, L);
     mac.u_limb = -1;
     if (mu) {
       mac.u_limb = (int)L - 1; mac.u_slot = (int)E; mac.u_add = mu->add; mac.u_add_comp_stride = mu->comp_stride;
@@ -834,7 +846,7 @@ static int ks_front(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, Batc
   }
   int rc = ks_modup(ctx, lc, L, nb, d_raw, yb, ext, s, hpip ? &mac : nullptr, au);
   if (rc) return rc;
-  return ks_inner(ctx, lc, L, nb, d, evk, evk_flagged, ext, acc, AL, 0, s, mu, hpip);
+  return ks_inner(ctx, lc, L, nb, d, key, ext, acc, AL, 0, s, mu, hpip);
 }
 
 // The addends of a ModDown epilogue: component 0 reads z0, component 1 reads z1 (either may be null)
@@ -871,7 +883,7 @@ static int ks_tail(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, u64 *
   f.z_b_stride = add0.ptr ? add0.stride : add1.stride;
   f.dst = out0.ptr; f.dst_c_stride = (long long)(out1.ptr - out0.ptr); f.dst_b_stride = out0.stride;
   f.cst = lc->pinv; f.n_c = 2;
-  f.z_galois = (unsigned)(add0_galois & (2ull * N - 1));
+  f.z_galois = galois_mod(add0_galois, N);
   int rc = ntt_sub_mul(ctx, lc->q_lm, l, s);
   if (rc) return rc;
   ctx->exec.ewe_limbs += (uint64_t)nb * (2 * L + (add0.ptr ? L : 0) + (add1.ptr ? L : 0));
@@ -883,16 +895,16 @@ static int ks_tail(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, u64 *
 static int ks_run(hml_ctx *ctx, uint32_t L, uint32_t nb, BatchPtr d, const u64 *evk, uint32_t evk_q_limbs, BatchOut out0,
                   BatchOut out1, BatchPtr add0, BatchPtr add1, u64 *ws, cudaStream_t s, const KsAuto *au = nullptr) {
   const Params &p = ctx->p;
-  if ((evk_q_limbs & ~HML_KEY_PACKED) < L || (evk_q_limbs & ~HML_KEY_PACKED) > p.max_level) return fail(ctx, HML_ERR_INVALID, "evk_q_limbs must be in [L, maxLevel]");
-  LevelConsts *lc;
-  int rc = get_level(ctx, L, &lc);
+  KeyDesc key;
+  int rc = key_desc(ctx, L, evk, evk_q_limbs, &key);
   if (rc) return rc;
+  LevelConsts *lc;
+  if ((rc = get_level(ctx, L, &lc))) return rc;
   const size_t N = p.N;
   const uint32_t A = p.alpha, E = L + A, beta = lc->beta;
-  if (beta > 8) return fail(ctx, HML_ERR_UNSUPPORTED, "more than 8 key-switch digits (ceil(L/alpha) > 8)");
   // workspace, every buffer batch-major: yb [nb][L] | ext [nb][beta][E] | acc [nb][2][E] | vb [nb][2][L]  (limbs of N words)
   u64 *yb = ws, *ext = yb + (size_t)nb * L * N, *acc = ext + (size_t)nb * beta * E * N, *vb = acc + (size_t)nb * 2 * E * N;
-  if ((rc = ks_front(ctx, lc, L, nb, d, evk, evk_q_limbs, yb, ext, acc, E, s, nullptr, au))) return rc;
+  if ((rc = ks_front(ctx, lc, L, nb, d, key, yb, ext, acc, E, s, nullptr, au))) return rc;
   return ks_tail(ctx, lc, L, nb, acc, vb, out0, out1, add0, add1, s, p.logN > NTT_SMALL_LOG && !ks_uses_hpip(ctx, L, nb), au ? au->g : 0);
 }
 
@@ -1162,7 +1174,7 @@ static int shard_end_run(hml_ctx *ctx, ShardPlan *sp, const u64 *gather2, const 
   set_addends(f, add0_own, add1_own);
   f.dst = out0_own; f.dst_c_stride = (long long)(out1_own - out0_own);
   f.cst = sp->pinv; f.n_c = 2;
-  f.z_galois = (unsigned)(add0_galois & (2ull * N - 1));
+  f.z_galois = galois_mod(add0_galois, N);
   if ((rc = ntt_sub_mul(ctx, sp->q_lm, l, s))) return rc;
   ctx->exec.ewe_limbs += 2 * nq;
   return check_launch(ctx, "keyswitch shard end");
@@ -1441,10 +1453,7 @@ int shard_hoist_inner(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, u
   InnerRotArgs a{};
   a.d = (const u64 *)c1_own; a.ext = ext; a.acc = acc; a.acc_rot_stride = 2ll * ne * N;
   a.N = (int)N; a.n_ext = (int)ne; a.beta = (int)beta; a.evk_limbs = (int)ne; a.logN = p.logN; a.ext_f64 = p.logN > NTT_SMALL_LOG;
-  for (uint32_t r = 0; r < n; ++r) {
-    const unsigned g = (unsigned)(galois[r] & (2ull * N - 1));
-    a.evk[r] = (const u64 *)keys[r]; a.galois[r] = g == 1 ? 0 : g;
-  }
+  for (uint32_t r = 0; r < n; ++r) { a.evk[r] = (const u64 *)keys[r]; a.galois[r] = inner_galois(galois[r], N); }
   launch_inner_product_rot(ctx->mc, sp->e_lm, a, (int)n, s);
   prof_mark(ctx, HML_CLS_EWE, s);
   ctx->exec.ewe_limbs += 2ull * n * ne * beta; ctx->exec.kernel_launches++;
@@ -1638,18 +1647,18 @@ int hmult_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct_a, const u64 
     if (rc) return rc;
     return rescale_run(ctx, L, cb, (long long)PL, 2 * nb, ct_out, (long long)(L - 1) * N, rest, s);
   }
-  if ((evk_q_limbs & ~HML_KEY_PACKED) < L || (evk_q_limbs & ~HML_KEY_PACKED) > p.max_level) return fail(ctx, HML_ERR_INVALID, "evk_q_limbs must be in [L, maxLevel]");
-  LevelConsts *lc;
-  int rc = get_level(ctx, L, &lc);
+  KeyDesc key;
+  int rc = key_desc(ctx, L, evk, evk_q_limbs, &key);
   if (rc) return rc;
+  LevelConsts *lc;
+  if ((rc = get_level(ctx, L, &lc))) return rc;
   const uint32_t A = p.alpha, E = L + A, AL = E + 1, beta = lc->beta;
-  if (beta > 8) return fail(ctx, HML_ERR_UNSUPPORTED, "more than 8 key-switch digits (ceil(L/alpha) > 8)");
   // yb [nb][L] | ext [nb][beta][E] | acc [nb][2][E+1] | wb [nb][2][L-1]; yb is free again after ModUp: ul [nb][2][N] reuses it
   u64 *yb = d2 + nb * PL, *ext = yb + (size_t)nb * L * N, *acc = ext + (size_t)nb * beta * E * N, *wb = acc + (size_t)nb * 2 * AL * N;
   // u[L-1] = d_c[L-1] + acc_c[L-1] * P^-1 is produced by the inner product itself (slot E of each accumulator) and its INTT
   // (reference Rescale INTT :766-805) rides in the launch that transforms the P-limbs: no extra launches, no re-reads
   const MergedU mu{d0, (long long)(d1 - d0), (long long)PL};
-  if ((rc = ks_front(ctx, lc, L, nb, {d2, (long long)PL}, evk, evk_q_limbs, yb, ext, acc, AL, s, &mu))) return rc;
+  if ((rc = ks_front(ctx, lc, L, nb, {d2, (long long)PL}, key, yb, ext, acc, AL, s, &mu))) return rc;
   {  // w_l = v_l * P^-1 + [r]_{q_l}, l < L-1, with r = slot_E - v[L-1] * P^-1 folded on the staged tile (reference K8 :489-519)
     BConvArgs a{};
     a.in = acc; a.in_batch_stride = (long long)AL * N; a.out = wb; a.out_batch_stride = (long long)(L - 1) * N;
@@ -1690,7 +1699,7 @@ int hrot_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct, const u64 *rk
   const size_t N = ctx->p.N, PL = N * L;
   u64 *sb = ws, *rest = sb + 2 * nb * PL;  // sb [nb][2][L][N]
   const bool in_place = ct_out < ct + 2 * nb * PL && ct < ct_out + 2 * nb * PL;  // the epilogue would gather c0 rows it has overwritten
-  if (!in_place && ctx->p.logN > NTT_SMALL_LOG && (g & (2 * N - 1)) != 1) {
+  if (!in_place && ctx->p.logN > NTT_SMALL_LOG && galois_mod(g, N) != 1) {
     // two-pass rings: no kernel for the automorphism (reference :1302-1319).  In evaluation order sigma_g maps every 256-slot
     // row onto one source row (ntt_core.cuh RowSigma), so the ModUp INTT permutes c1 while it loads it (and leaves sigma(c1)
     // in sb for the inner product's own-digit term) and the ModDown epilogue gathers sigma(c0) from the raw c0
@@ -1731,26 +1740,27 @@ extern "C" int hml_hrotate(hml_ctx *ctx, uint32_t L, const uint64_t *ct, const u
 static int hrot_hoisted_run(hml_ctx *ctx, uint32_t L, const u64 *ct, uint32_t n_rot, const uint64_t *const *rotkeys, uint32_t evk_q_limbs,
                             const uint64_t *galois, uint64_t *const *outs, u64 *ws, cudaStream_t s) {
   const Params &p = ctx->p;
-  if ((evk_q_limbs & ~HML_KEY_PACKED) < L || (evk_q_limbs & ~HML_KEY_PACKED) > p.max_level) return fail(ctx, HML_ERR_INVALID, "evk_q_limbs must be in [L, maxLevel]");
-  LevelConsts *lc;
-  int rc = get_level(ctx, L, &lc);
+  KeyDesc key;  // key.evk: rotation r's key, set in the loop
+  int rc = key_desc(ctx, L, nullptr, evk_q_limbs, &key);
   if (rc) return rc;
+  LevelConsts *lc;
+  if ((rc = get_level(ctx, L, &lc))) return rc;
   const size_t N = p.N, PL = N * L;
   const uint32_t A = p.alpha, E = L + A, beta = lc->beta;
-  if (beta > 8) return fail(ctx, HML_ERR_UNSUPPORTED, "more than 8 key-switch digits (ceil(L/alpha) > 8)");
   u64 *sb = ws, *yb = sb + 2 * PL, *ext = yb + PL, *acc = ext + (size_t)beta * E * N, *vb = acc + 2 * (size_t)E * N;
   const BatchPtr c1{ct + PL, 0};
   if ((rc = ks_modup(ctx, lc, L, 1, c1, yb, ext, s, nullptr))) return rc;
   for (uint32_t r = 0; r < n_rot; ++r) {
     // sigma_r(c0), the addend of the ModDown epilogue: gathered by the epilogue itself on two-pass rings (hrot_run), else a kernel
-    const bool gather = p.logN > NTT_SMALL_LOG && (galois[r] & (2 * N - 1)) != 1;
+    const bool gather = p.logN > NTT_SMALL_LOG && galois_mod(galois[r], N) != 1;
     if (!gather) {
       launch_automorph(p.logN, L, ct, sb, galois[r], s);
       prof_mark(ctx, HML_CLS_AUTO, s);
       ctx->exec.kernel_launches++;
     }
     ctx->exec.automorph_limbs += L;
-    if ((rc = ks_inner(ctx, lc, L, 1, c1, (const u64 *)rotkeys[r], evk_q_limbs, ext, acc, E, galois[r], s, nullptr, false))) return rc;
+    key.evk = (const u64 *)rotkeys[r];
+    if ((rc = ks_inner(ctx, lc, L, 1, c1, key, ext, acc, E, galois[r], s, nullptr, false))) return rc;
     u64 *o = (u64 *)outs[r];
     if ((rc = ks_tail(ctx, lc, L, 1, acc, vb, {o, 0}, {o + PL, 0}, {gather ? ct : sb, 0}, {nullptr, 0}, s, p.logN > NTT_SMALL_LOG,
                       gather ? galois[r] : 0)))
@@ -1787,31 +1797,29 @@ extern "C" int hml_hrotate_hoisted(hml_ctx *ctx, uint32_t L, const uint64_t *ct,
 static int hrot_sum_hoisted_run(hml_ctx *ctx, uint32_t L, const u64 *ct, uint32_t n_rot, const uint64_t *const *rotkeys, uint32_t evk_q_limbs,
                                 const uint64_t *galois, const uint64_t *const *pts, uint32_t pt_q_limbs, u64 *ct_out, u64 *ws, cudaStream_t s) {
   const Params &p = ctx->p;
-  const uint32_t kq = evk_q_limbs & ~HML_KEY_PACKED;
-  if (kq < L || kq > p.max_level) return fail(ctx, HML_ERR_INVALID, "evk_q_limbs must be in [L, maxLevel]");
+  KeyDesc key;  // one key per rotation: only the layout is shared
+  int rc = key_desc(ctx, L, nullptr, evk_q_limbs, &key);
+  if (rc) return rc;
   if (pt_q_limbs < L || pt_q_limbs > p.max_level) return fail(ctx, HML_ERR_INVALID, "pt_q_limbs must be in [L, maxLevel]");
   LevelConsts *lc;
-  int rc = get_level(ctx, L, &lc);
-  if (rc) return rc;
+  if ((rc = get_level(ctx, L, &lc))) return rc;
   const size_t N = p.N, PL = N * L;
   const uint32_t A = p.alpha, E = L + A, beta = lc->beta;
-  if (beta > 8) return fail(ctx, HML_ERR_UNSUPPORTED, "more than 8 key-switch digits (ceil(L/alpha) > 8)");
   // the workspace of hrot_hoisted_run: zb [L] (of 2L) | yb [L] | ext [beta][E] | acc [2][E] | vb [2][L]
   u64 *zb = ws, *yb = zb + 2 * PL, *ext = yb + PL, *acc = ext + (size_t)beta * E * N, *vb = acc + 2 * (size_t)E * N;
   const BatchPtr c1{ct + PL, 0};
   if ((rc = ks_modup(ctx, lc, L, 1, c1, yb, ext, s, nullptr))) return rc;
-  LimbMap ip = lc->ext_lm;  // pos = limb index inside the key, as in ks_inner
-  for (uint32_t e = 0; e < E; ++e) ip.pos[e] = (uint16_t)(e < L ? e : kq + (e - L));
+  LimbMap ip = lc->ext_lm;  // pos = limb index inside the key
+  for (uint32_t e = 0; e < E; ++e) ip.pos[e] = (uint16_t)key.pos(e, L);
   InnerRotSumArgs a{};
   a.d = c1.ptr; a.ext = ext; a.c0 = ct; a.acc = acc; a.z = zb;
-  a.N = (int)N; a.n_ext = (int)E; a.L = (int)L; a.beta = (int)beta; a.evk_limbs = (int)(kq + A); a.pt_q_limbs = (int)pt_q_limbs; a.logN = p.logN;
-  a.ext_f64 = p.logN > NTT_SMALL_LOG; a.evk_packed = (evk_q_limbs & HML_KEY_PACKED) ? 1 : 0;
+  a.N = (int)N; a.n_ext = (int)E; a.L = (int)L; a.beta = (int)beta; a.evk_limbs = (int)(key.q_limbs + A); a.pt_q_limbs = (int)pt_q_limbs; a.logN = p.logN;
+  a.ext_f64 = p.logN > NTT_SMALL_LOG; a.evk_packed = key.packed ? 1 : 0;
   for (uint32_t r0 = 0; r0 < n_rot; r0 += IP_MAX_ROT) {
     const uint32_t n = std::min<uint32_t>(IP_MAX_ROT, n_rot - r0);
     a.accumulate = r0 > 0; a.n_rot = (int)n;
     for (uint32_t k = 0; k < n; ++k) {
-      const unsigned g = (unsigned)(galois[r0 + k] & (2ull * N - 1));
-      a.evk[k] = (const u64 *)rotkeys[r0 + k]; a.pt[k] = (const u64 *)pts[r0 + k]; a.galois[k] = g == 1 ? 0 : g;
+      a.evk[k] = (const u64 *)rotkeys[r0 + k]; a.pt[k] = (const u64 *)pts[r0 + k]; a.galois[k] = inner_galois(galois[r0 + k], N);
     }
     launch_inner_product_rot_sum(ctx->mc, ip, a, s);
     prof_mark(ctx, HML_CLS_EWE, s);
@@ -1819,7 +1827,7 @@ static int hrot_sum_hoisted_run(hml_ctx *ctx, uint32_t L, const u64 *ct, uint32_
     ctx->exec.ewe_limbs += (uint64_t)n * (2ull * E * beta + 2ull * E + L);
     ctx->exec.automorph_limbs += (uint64_t)n * L;  // sigma_r(c0), applied on load
   }
-  if ((rc = ks_inner(ctx, lc, L, 1, c1, nullptr, evk_q_limbs, ext, acc, E, 0, s, nullptr, true))) return rc;
+  if ((rc = ks_inner(ctx, lc, L, 1, c1, key, ext, acc, E, 0, s, nullptr, true))) return rc;
   if ((rc = ks_tail(ctx, lc, L, 1, acc, vb, {ct_out, 0}, {ct_out + PL, 0}, {zb, 0}, {nullptr, 0}, s, false, 0))) return rc;
   return check_launch(ctx, "hrotate sum hoisted");
 }

@@ -4,6 +4,7 @@
 
 #include <algorithm>
 #include <cstdlib>
+#include <type_traits>
 
 namespace hml {
 
@@ -120,6 +121,72 @@ __device__ __forceinline__ void pin_loads(ulonglong2 (&k)[NB][2]) {
   }
 }
 
+// Source slots of coefficient pair i2 under the automorphism X -> X^g (g == 0: the identity): the slot k' the automorphism
+// kernel would fetch, 2*brv(k')+1 = g*(2*brv(k)+1) mod 2N.
+__device__ __forceinline__ uint2 gal_slots(unsigned g, int logN, int i2) {
+  unsigned s0 = 2u * i2, s1 = 2u * i2 + 1u;
+  if (g) {
+    const unsigned sh = 32 - logN, m2n = (2u << logN) - 1u;
+    s0 = __brev((((g * (2u * (__brev(s0) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
+    s1 = __brev((((g * (2u * (__brev(s1) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
+  }
+  return make_uint2(s0, s1);
+}
+// coefficient pair i2 of a digit (or c0), read through the slots src when gal
+__device__ __forceinline__ ulonglong2 ld_pair(const u64 *p, int i2, uint2 src, bool gal) {
+  return gal ? make_ulonglong2(__ldg(p + src.x), __ldg(p + src.y)) : ld2(p, i2);
+}
+// The key words of digits j < beta at key limb kl (evk [beta][2][evk_limbs][N]; a = the kernel's argument struct, n2 = N / 2);
+// padding digits are zero.  PACKED: the raw halves of packed limbs, joined by join_key after pin_loads.
+template <bool PACKED, int NB, class A>
+__device__ __forceinline__ void ld_key(ulonglong2 (&k)[NB][2], const u64 *evk, const A &a, int kl, size_t n2, int i2) {
+#pragma unroll
+  for (int j = 0; j < NB; ++j)
+#pragma unroll
+    for (int c = 0; c < 2; ++c) {
+      if constexpr (PACKED) {
+        const u64 *slot = evk + (((size_t)j * 2 + c) * a.evk_limbs + kl) * a.N;
+        k[j][c] = j < a.beta ? ld_packed2_raw(slot, a.N, i2) : make_ulonglong2(0, 0);
+      } else {
+        k[j][c] = j < a.beta ? ld2(evk, (((size_t)j * 2 + c) * a.evk_limbs + kl) * n2 + i2) : make_ulonglong2(0, 0);
+      }
+    }
+}
+template <int NB>
+__device__ __forceinline__ void join_key(ulonglong2 (&k)[NB][2]) {
+#pragma unroll
+  for (int j = 0; j < NB; ++j)
+#pragma unroll
+    for (int c = 0; c < 2; ++c) k[j][c] = packed2_join(k[j][c]);
+}
+// s[c][h] += t_j[h] * key_j[c][h] over the digits j < beta (key words as loaded)
+template <int NB>
+__device__ __forceinline__ void mac_digits(double &s00, double &s01, double &s10, double &s11, const ulonglong2 (&t)[NB],
+                                           const ulonglong2 (&k)[NB][2], int beta, int ext_f64, int own, const ModConst &m) {
+#pragma unroll
+  for (int j = 0; j < NB; ++j)
+    if (j < beta) {
+      // converted digits may arrive as raw lazy doubles straight from the transform (own-digit limbs are always words)
+      const bool f64 = ext_f64 && j != own;
+      const double t0 = f64 ? __longlong_as_double((long long)t[j].x) : u64_to_f64(t[j].x);
+      const double t1 = f64 ? __longlong_as_double((long long)t[j].y) : u64_to_f64(t[j].y);
+      s00 += mulmod_var(t0, u64_to_f64(k[j][0].x), m.q, m.qinv);
+      s01 += mulmod_var(t1, u64_to_f64(k[j][0].y), m.q, m.qinv);
+      s10 += mulmod_var(t0, u64_to_f64(k[j][1].x), m.q, m.qinv);
+      s11 += mulmod_var(t1, u64_to_f64(k[j][1].y), m.q, m.qinv);
+    }
+}
+
+// calls f(std::integral_constant<int, NB>()) with the digit bound NB in {1, 2, 3, 4, 8} of the kernels for beta <= 8
+template <class F>
+static void with_max_beta(int beta, F &&f) {
+  if (beta <= 1) f(std::integral_constant<int, 1>());
+  else if (beta <= 2) f(std::integral_constant<int, 2>());
+  else if (beta <= 3) f(std::integral_constant<int, 3>());
+  else if (beta <= 4) f(std::integral_constant<int, 4>());
+  else f(std::integral_constant<int, 8>());
+}
+
 // MULTI: more than one ciphertext per launch (the next ciphertext's digits are prefetched while this one is multiplied)
 template <int IP_MAX_BETA, bool MULTI>
 __global__ void __launch_bounds__(EW_THREADS, 3) k_inner(const ModConst *__restrict__ mc, LimbMap lm, InnerArgs a) {
@@ -136,45 +203,32 @@ __global__ void __launch_bounds__(EW_THREADS, 3) k_inner(const ModConst *__restr
     return j == own ? a.d + (size_t)b * a.d_batch_stride + (size_t)e * a.N
                     : a.ext + (size_t)b * a.ext_batch_stride + ((size_t)j * a.n_ext + e) * a.N;
   };
-  // source slots of this thread's two coefficients under the automorphism (identity when galois == 0)
-  unsigned s0 = 2u * i2, s1 = 2u * i2 + 1u;
   const bool gal = !MULTI && a.galois != 0;  // the batched variant stays lean: no automorphism on load, no u side output
-  if (gal) {
-    const unsigned sh = 32 - a.logN, m2n = (2u << a.logN) - 1u;
-    s0 = __brev((((a.galois * (2u * (__brev(s0) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
-    s1 = __brev((((a.galois * (2u * (__brev(s1) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
-  }
+  const uint2 src = gal_slots(gal ? a.galois : 0u, a.logN, i2);
   auto ld_digit = [&](int b, int j) -> ulonglong2 {
     const u64 *p = digit_ptr(b, j);
     if (!gal) return ld2(p, i2);
-    return make_ulonglong2(__ldg(p + s0), __ldg(p + s1));
+    return make_ulonglong2(__ldg(p + src.x), __ldg(p + src.y));
   };
   ulonglong2 tn[IP_MAX_BETA];
 #pragma unroll
   for (int j = 0; j < IP_MAX_BETA; ++j)
     if (j < a.beta) tn[j] = ld_digit(0, j);
   // every key word of the thread is requested before the first one is used: ONE memory round trip for the 3 * beta loads
-  // (converting inside the load loop made ptxas wait for each digit's pair before issuing the next)
+  // (converting inside the load loop made ptxas wait for each digit's pair before issuing the next).  The key loads, the
+  // digit loads and the product stay spelled out here: through ld_key, ld_pair or mac_digits ptxas schedules this kernel
+  // differently.
   ulonglong2 kraw[IP_MAX_BETA][2];
-  if (a.evk_packed) {  // uniform: packed key limbs — the raw halves are all requested first, then assembled (kraw.x = the pair's low
-    // words, kraw.y = its two high bytes until the loop below)
+  if (a.evk_packed) {  // uniform
 #pragma unroll
     for (int j = 0; j < IP_MAX_BETA; ++j)
 #pragma unroll
       for (int c = 0; c < 2; ++c) {
         const u64 *slot = a.evk + (((size_t)j * 2 + c) * a.evk_limbs + kl) * a.N;
-        kraw[j][c] = j < a.beta ? make_ulonglong2(__ldg(reinterpret_cast<const u64 *>(slot) + i2),
-                                                  __ldg(reinterpret_cast<const unsigned short *>(reinterpret_cast<const unsigned char *>(slot) + 4 * (size_t)a.N) + i2))
-                                : make_ulonglong2(0, 0);
+        kraw[j][c] = j < a.beta ? ld_packed2_raw(slot, a.N, i2) : make_ulonglong2(0, 0);
       }
     pin_loads(kraw);
-#pragma unroll
-    for (int j = 0; j < IP_MAX_BETA; ++j)
-#pragma unroll
-      for (int c = 0; c < 2; ++c) {
-        const u64 lo = kraw[j][c].x, hi = kraw[j][c].y;
-        kraw[j][c] = make_ulonglong2(((hi & 0xFFull) << 32) | (lo & 0xFFFFFFFFull), ((hi >> 8) << 32) | (lo >> 32));
-      }
+    join_key(kraw);
   } else {
 #pragma unroll
     for (int j = 0; j < IP_MAX_BETA; ++j)
@@ -204,7 +258,6 @@ __global__ void __launch_bounds__(EW_THREADS, 3) k_inner(const ModConst *__restr
 #pragma unroll
     for (int j = 0; j < IP_MAX_BETA; ++j)
       if (j < a.beta) {
-        // converted digits may arrive as raw lazy doubles straight from the transform (own-digit limbs are always words)
         const bool f64 = a.ext_f64 && j != own;
         const double t0 = f64 ? __longlong_as_double((long long)t[j].x) : u64_to_f64(t[j].x);
         const double t1 = f64 ? __longlong_as_double((long long)t[j].y) : u64_to_f64(t[j].y);
@@ -234,18 +287,12 @@ __global__ void __launch_bounds__(EW_THREADS, 3) k_inner(const ModConst *__restr
   }
 }
 
-template <bool MULTI>
-static void launch_inner_t(const ModConst *mc, const LimbMap &lm, const InnerArgs &a, cudaStream_t s) {
-  const dim3 g = ew_grid(a.N, a.n_ext);
-  if (a.beta <= 1) launch_pdl(k_inner<1, MULTI>, g, EW_THREADS, 0, s, mc, lm, a);
-  else if (a.beta <= 2) launch_pdl(k_inner<2, MULTI>, g, EW_THREADS, 0, s, mc, lm, a);
-  else if (a.beta <= 3) launch_pdl(k_inner<3, MULTI>, g, EW_THREADS, 0, s, mc, lm, a);
-  else if (a.beta <= 4) launch_pdl(k_inner<4, MULTI>, g, EW_THREADS, 0, s, mc, lm, a);
-  else launch_pdl(k_inner<8, MULTI>, g, EW_THREADS, 0, s, mc, lm, a);
-}
 void launch_inner_product(const ModConst *mc, const LimbMap &lm, const InnerArgs &a, cudaStream_t s) {
-  if (a.n_batch > 1) launch_inner_t<true>(mc, lm, a, s);
-  else launch_inner_t<false>(mc, lm, a, s);
+  with_max_beta(a.beta, [&](auto nb) {
+    constexpr int NB = decltype(nb)::value;
+    if (a.n_batch > 1) launch_pdl(k_inner<NB, true>, ew_grid(a.N, a.n_ext), EW_THREADS, 0, s, mc, lm, a);
+    else launch_pdl(k_inner<NB, false>, ew_grid(a.N, a.n_ext), EW_THREADS, 0, s, mc, lm, a);
+  });
 }
 
 // Hoisted rotations of one ciphertext (limb-sharded, shard.cu): k_inner's single-ciphertext body with the automorphism on
@@ -263,50 +310,28 @@ __global__ void __launch_bounds__(EW_THREADS, IP_MAX_BETA > 4 ? 2 : 3) k_inner_r
   const size_t n2 = a.N / 2;
   const unsigned g = a.galois[r];
   const u64 *evk = a.evk[r];
-  unsigned s0 = 2u * i2, s1 = 2u * i2 + 1u;
-  if (g) {  // the index formula of k_inner
-    const unsigned sh = 32 - a.logN, m2n = (2u << a.logN) - 1u;
-    s0 = __brev((((g * (2u * (__brev(s0) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
-    s1 = __brev((((g * (2u * (__brev(s1) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
-  }
+  const uint2 src = gal_slots(g, a.logN, i2);
   ulonglong2 t[IP_MAX_BETA];
 #pragma unroll
   for (int j = 0; j < IP_MAX_BETA; ++j)
     if (j < a.beta) {
       const u64 *p = j == own ? a.d + (size_t)e * a.N : a.ext + ((size_t)j * a.n_ext + e) * a.N;
-      t[j] = g ? make_ulonglong2(__ldg(p + s0), __ldg(p + s1)) : ld2(p, i2);
+      t[j] = ld_pair(p, i2, src, g != 0);
     }
-  ulonglong2 kraw[IP_MAX_BETA][2];  // every key word requested before the first use, as in k_inner
-#pragma unroll
-  for (int j = 0; j < IP_MAX_BETA; ++j)
-#pragma unroll
-    for (int c = 0; c < 2; ++c)
-      kraw[j][c] = j < a.beta ? ld2(evk, (((size_t)j * 2 + c) * a.evk_limbs + kl) * n2 + i2) : make_ulonglong2(0, 0);
+  ulonglong2 kraw[IP_MAX_BETA][2];  // every key word requested before the first use
+  ld_key<false>(kraw, evk, a, kl, n2, i2);
   pin_loads(kraw);
   double s00 = 0, s01 = 0, s10 = 0, s11 = 0;  // [component][coefficient]
-#pragma unroll
-  for (int j = 0; j < IP_MAX_BETA; ++j)
-    if (j < a.beta) {
-      const bool f64 = a.ext_f64 && j != own;
-      const double t0 = f64 ? __longlong_as_double((long long)t[j].x) : u64_to_f64(t[j].x);
-      const double t1 = f64 ? __longlong_as_double((long long)t[j].y) : u64_to_f64(t[j].y);
-      s00 += mulmod_var(t0, u64_to_f64(kraw[j][0].x), m.q, m.qinv);
-      s01 += mulmod_var(t1, u64_to_f64(kraw[j][0].y), m.q, m.qinv);
-      s10 += mulmod_var(t0, u64_to_f64(kraw[j][1].x), m.q, m.qinv);
-      s11 += mulmod_var(t1, u64_to_f64(kraw[j][1].y), m.q, m.qinv);
-    }
+  mac_digits(s00, s01, s10, s11, t, kraw, a.beta, a.ext_f64, own, m);
   u64 *acc = a.acc + (size_t)r * a.acc_rot_stride;
   st2(acc, (size_t)e * n2 + i2, finish(s00, m), finish(s01, m));
   st2(acc, (size_t)(a.n_ext + e) * n2 + i2, finish(s10, m), finish(s11, m));
 }
 
 void launch_inner_product_rot(const ModConst *mc, const LimbMap &lm, const InnerRotArgs &a, int n_rot, cudaStream_t s) {
-  const dim3 g = ew_grid(a.N, a.n_ext, n_rot);
-  if (a.beta <= 1) launch_pdl(k_inner_rot<1>, g, EW_THREADS, 0, s, mc, lm, a);
-  else if (a.beta <= 2) launch_pdl(k_inner_rot<2>, g, EW_THREADS, 0, s, mc, lm, a);
-  else if (a.beta <= 3) launch_pdl(k_inner_rot<3>, g, EW_THREADS, 0, s, mc, lm, a);
-  else if (a.beta <= 4) launch_pdl(k_inner_rot<4>, g, EW_THREADS, 0, s, mc, lm, a);
-  else launch_pdl(k_inner_rot<8>, g, EW_THREADS, 0, s, mc, lm, a);
+  with_max_beta(a.beta, [&](auto nb) {
+    launch_pdl(k_inner_rot<decltype(nb)::value>, ew_grid(a.N, a.n_ext, n_rot), EW_THREADS, 0, s, mc, lm, a);
+  });
 }
 
 // Double-hoisted rotation sum (ewe.cuh InnerRotSumArgs).  The body of k_inner_rot once per rotation, then the two component
@@ -332,66 +357,23 @@ __global__ void __launch_bounds__(EW_THREADS, IP_MAX_BETA > 4 ? 1 : IP_MAX_BETA 
 #pragma unroll 1
   for (int r = 0; r < a.n_rot; ++r) {
     const unsigned g = a.galois[r];
-    unsigned s0 = 2u * i2, s1 = 2u * i2 + 1u;
-    if (g) {  // the index formula of k_inner
-      const unsigned sh = 32 - a.logN, m2n = (2u << a.logN) - 1u;
-      s0 = __brev((((g * (2u * (__brev(s0) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
-      s1 = __brev((((g * (2u * (__brev(s1) >> sh) + 1u)) & m2n) - 1u) >> 1) >> sh;
-    }
+    const uint2 src = gal_slots(g, a.logN, i2);
     ulonglong2 t[IP_MAX_BETA];
 #pragma unroll
     for (int j = 0; j < IP_MAX_BETA; ++j)
       if (j < a.beta) {
         const u64 *p = j == own ? a.d + (size_t)e * a.N : a.ext + ((size_t)j * a.n_ext + e) * a.N;
-        t[j] = g ? make_ulonglong2(__ldg(p + s0), __ldg(p + s1)) : ld2(p, i2);
+        t[j] = ld_pair(p, i2, src, g != 0);
       }
-    const u64 *evk = a.evk[r];
     ulonglong2 kraw[IP_MAX_BETA][2];
-    if constexpr (PACKED) {  // the packed load path of k_inner (kraw.x = the pair's low words, kraw.y = its two high bytes)
-#pragma unroll
-      for (int j = 0; j < IP_MAX_BETA; ++j)
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          const u64 *slot = evk + (((size_t)j * 2 + c) * a.evk_limbs + kl) * a.N;
-          kraw[j][c] = j < a.beta ? make_ulonglong2(__ldg(slot + i2),
-                                                    __ldg(reinterpret_cast<const unsigned short *>(reinterpret_cast<const unsigned char *>(slot) + 4 * (size_t)a.N) + i2))
-                                  : make_ulonglong2(0, 0);
-        }
-    } else {
-#pragma unroll
-      for (int j = 0; j < IP_MAX_BETA; ++j)
-#pragma unroll
-        for (int c = 0; c < 2; ++c)
-          kraw[j][c] = j < a.beta ? ld2(evk, (((size_t)j * 2 + c) * a.evk_limbs + kl) * n2 + i2) : make_ulonglong2(0, 0);
-    }
+    ld_key<PACKED>(kraw, a.evk[r], a, kl, n2, i2);
     ulonglong2 w = ld2(a.pt[r] + prow * a.N, i2), x = make_ulonglong2(0, 0);
-    if (q_limb) {
-      const u64 *p = a.c0 + (size_t)e * a.N;
-      x = g ? make_ulonglong2(__ldg(p + s0), __ldg(p + s1)) : ld2(p, i2);
-    }
+    if (q_limb) x = ld_pair(a.c0 + (size_t)e * a.N, i2, src, g != 0);
     pin_loads(kraw);
     asm volatile("" : "+l"(w.x), "+l"(w.y), "+l"(x.x), "+l"(x.y));
-    if constexpr (PACKED) {
-#pragma unroll
-      for (int j = 0; j < IP_MAX_BETA; ++j)
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          const u64 lo = kraw[j][c].x, hi = kraw[j][c].y;
-          kraw[j][c] = make_ulonglong2(((hi & 0xFFull) << 32) | (lo & 0xFFFFFFFFull), ((hi >> 8) << 32) | (lo >> 32));
-        }
-    }
+    if constexpr (PACKED) join_key(kraw);
     double s00 = 0, s01 = 0, s10 = 0, s11 = 0;
-#pragma unroll
-    for (int j = 0; j < IP_MAX_BETA; ++j)
-      if (j < a.beta) {
-        const bool f64 = a.ext_f64 && j != own;
-        const double t0 = f64 ? __longlong_as_double((long long)t[j].x) : u64_to_f64(t[j].x);
-        const double t1 = f64 ? __longlong_as_double((long long)t[j].y) : u64_to_f64(t[j].y);
-        s00 += mulmod_var(t0, u64_to_f64(kraw[j][0].x), m.q, m.qinv);
-        s01 += mulmod_var(t1, u64_to_f64(kraw[j][0].y), m.q, m.qinv);
-        s10 += mulmod_var(t0, u64_to_f64(kraw[j][1].x), m.q, m.qinv);
-        s11 += mulmod_var(t1, u64_to_f64(kraw[j][1].y), m.q, m.qinv);
-      }
+    mac_digits(s00, s01, s10, s11, t, kraw, a.beta, a.ext_f64, own, m);
     const double w0 = u64_to_f64(w.x), w1 = u64_to_f64(w.y);
     a00 += mulmod_var(s00, w0, m.q, m.qinv);
     a01 += mulmod_var(s01, w1, m.q, m.qinv);
@@ -416,18 +398,12 @@ __global__ void __launch_bounds__(EW_THREADS, IP_MAX_BETA > 4 ? 1 : IP_MAX_BETA 
   if (q_limb) st2(a.z, o0, finish(z0, m), finish(z1, m));
 }
 
-template <bool PACKED>
-static void launch_inner_rot_sum_t(const ModConst *mc, const LimbMap &lm, const InnerRotSumArgs &a, cudaStream_t s) {
-  const dim3 g = ew_grid(a.N, a.n_ext);
-  if (a.beta <= 1) launch_pdl(k_inner_rot_sum<1, PACKED>, g, EW_THREADS, 0, s, mc, lm, a);
-  else if (a.beta <= 2) launch_pdl(k_inner_rot_sum<2, PACKED>, g, EW_THREADS, 0, s, mc, lm, a);
-  else if (a.beta <= 3) launch_pdl(k_inner_rot_sum<3, PACKED>, g, EW_THREADS, 0, s, mc, lm, a);
-  else if (a.beta <= 4) launch_pdl(k_inner_rot_sum<4, PACKED>, g, EW_THREADS, 0, s, mc, lm, a);
-  else launch_pdl(k_inner_rot_sum<8, PACKED>, g, EW_THREADS, 0, s, mc, lm, a);
-}
 void launch_inner_product_rot_sum(const ModConst *mc, const LimbMap &lm, const InnerRotSumArgs &a, cudaStream_t s) {
-  if (a.evk_packed) launch_inner_rot_sum_t<true>(mc, lm, a, s);
-  else launch_inner_rot_sum_t<false>(mc, lm, a, s);
+  with_max_beta(a.beta, [&](auto nb) {
+    constexpr int NB = decltype(nb)::value;
+    if (a.evk_packed) launch_pdl(k_inner_rot_sum<NB, true>, ew_grid(a.N, a.n_ext), EW_THREADS, 0, s, mc, lm, a);
+    else launch_pdl(k_inner_rot_sum<NB, false>, ew_grid(a.N, a.n_ext), EW_THREADS, 0, s, mc, lm, a);
+  });
 }
 
 // ------------------------------------------------------------------------------------------------ (x - y) * c (+ z)

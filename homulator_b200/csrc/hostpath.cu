@@ -19,24 +19,21 @@ using namespace hml;
 // chunk's kernels and copy-out, which nothing overlaps — grows with it.
 constexpr uint32_t HOST_CHUNK = 2;
 
-// packed [n_limbs][5N] <-> words [n_limbs][N]; two coefficients per thread
+// packed [n_limbs][5N] <-> words [n_limbs][N]; two coefficients per thread.  The packed limbs of the device (modarith.cuh)
+// with a 5N-byte slot stride: 5N is a multiple of 80, so every slot stays 8-byte aligned.
 __global__ void __launch_bounds__(256) k_unpack(const unsigned char *__restrict__ in, u64 *__restrict__ out, size_t N) {
   pdl_wait();
   const size_t i2 = (size_t)blockIdx.x * 256 + threadIdx.x;
   if (i2 >= N / 2) return;
-  const unsigned char *limb = in + (size_t)blockIdx.y * 5 * N;
-  const uint2 lo = __ldg(reinterpret_cast<const uint2 *>(limb) + i2);
-  const unsigned hi = __ldg(reinterpret_cast<const unsigned short *>(limb + 4 * N) + i2);
-  reinterpret_cast<ulonglong2 *>(out + (size_t)blockIdx.y * N)[i2] = make_ulonglong2(((u64)(hi & 0xFFu) << 32) | lo.x, ((u64)(hi >> 8) << 32) | lo.y);
+  const u64 *limb = reinterpret_cast<const u64 *>(in + (size_t)blockIdx.y * 5 * N);
+  reinterpret_cast<ulonglong2 *>(out + (size_t)blockIdx.y * N)[i2] = ld_packed2(limb, N, i2);
 }
 __global__ void __launch_bounds__(256) k_pack(const u64 *__restrict__ in, unsigned char *__restrict__ out, size_t N) {
   pdl_wait();
   const size_t i2 = (size_t)blockIdx.x * 256 + threadIdx.x;
   if (i2 >= N / 2) return;
   const ulonglong2 v = __ldg(reinterpret_cast<const ulonglong2 *>(in + (size_t)blockIdx.y * N) + i2);
-  unsigned char *limb = out + (size_t)blockIdx.y * 5 * N;
-  reinterpret_cast<uint2 *>(limb)[i2] = make_uint2((unsigned)v.x, (unsigned)v.y);
-  reinterpret_cast<unsigned short *>(limb + 4 * N)[i2] = (unsigned short)((unsigned)(v.x >> 32) | ((unsigned)(v.y >> 32) << 8));
+  st_packed2(reinterpret_cast<u64 *>(out + (size_t)blockIdx.y * 5 * N), N, i2, v.x, v.y);
 }
 
 extern "C" uint64_t hml_packed_bytes(const hml_ctx *ctx, uint64_t n_limbs) { return ctx ? 5ull * ctx->p.N * n_limbs : 0; }

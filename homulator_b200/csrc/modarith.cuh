@@ -94,10 +94,25 @@ __device__ __forceinline__ void st_packed2(u64 *limb_slot, size_t N, size_t i2, 
   reinterpret_cast<unsigned short *>(reinterpret_cast<unsigned char *>(limb_slot) + 4 * N)[i2] =
       (unsigned short)((unsigned)(a >> 32) | ((unsigned)(b >> 32) << 8));
 }
+// Joins a pair's low words and its two high bytes.  hi is 32 bits wide where the loads are joined right away and 64 bits
+// after pin_loads: the casts keep the same instructions for both, with no wider shifts for the 32-bit callers.
+template <class H>
+__device__ __forceinline__ ulonglong2 packed2_join(uint2 lo, H hi) {
+  return make_ulonglong2((u64)(unsigned)(hi & 0xFFu) << 32 | lo.x, (u64)(unsigned)(hi >> 8) << 32 | lo.y);
+}
 __device__ __forceinline__ ulonglong2 ld_packed2(const u64 *limb_slot, size_t N, size_t i2) {
   const uint2 lo = __ldg(reinterpret_cast<const uint2 *>(limb_slot) + i2);
   const unsigned hi = __ldg(reinterpret_cast<const unsigned short *>(reinterpret_cast<const unsigned char *>(limb_slot) + 4 * N) + i2);
-  return make_ulonglong2(((u64)(hi & 0xFFu) << 32) | lo.x, ((u64)(hi >> 8) << 32) | lo.y);
+  return packed2_join(lo, hi);
+}
+// The same two loads, not yet joined, in one 16-byte value (x = the pair's low words, y = its two high bytes): kernels that
+// must have every load in flight before the first use hold these in pin_loads, then join them.
+__device__ __forceinline__ ulonglong2 ld_packed2_raw(const u64 *limb_slot, size_t N, size_t i2) {
+  return make_ulonglong2(__ldg(limb_slot + i2),
+                         __ldg(reinterpret_cast<const unsigned short *>(reinterpret_cast<const unsigned char *>(limb_slot) + 4 * N) + i2));
+}
+__device__ __forceinline__ ulonglong2 packed2_join(ulonglong2 raw) {
+  return packed2_join(make_uint2((unsigned)raw.x, (unsigned)(raw.x >> 32)), raw.y);
 }
 
 // per-modulus constants kept in device memory

@@ -482,20 +482,11 @@ __global__ void __launch_bounds__(NTT_THREADS, 2) ntt_rows(NttTables t, int logN
         for (int h = 0; h < 2; ++h) {  // four chunks at a time: every load of the half is in flight before the first product
           ulonglong2 kv0[4], kv1[4];
           double2 old0[4], old1[4];
-          // packed key limbs (NttMac::evk_packed): the pair's low words and its two high bytes, assembled after all loads are out
-          auto ld_key_raw = [&](const u64 *kp, int mm) -> ulonglong2 {
-            const u64 *slot = kp - ci;
-            const size_t i2 = (ci >> 1) + 16 * mm;
-            return make_ulonglong2(__ldg(slot + i2), __ldg(reinterpret_cast<const unsigned short *>(reinterpret_cast<const unsigned char *>(slot) + 4 * nn) + i2));
-          };
-          auto key_join = [](ulonglong2 r) {
-            return make_ulonglong2(((r.y & 0xFFull) << 32) | (r.x & 0xFFFFFFFFull), ((r.y >> 8) << 32) | (r.x >> 32));
-          };
-          if constexpr (KPK) {
+          if constexpr (KPK) {  // packed key limbs (NttMac::evk_packed): joined after all loads are out
 #pragma unroll
             for (int m = 0; m < 4; ++m) {
-              kv0[m] = ld_key_raw(k0, 4 * h + m);
-              kv1[m] = ld_key_raw(k1, 4 * h + m);
+              kv0[m] = ld_packed2_raw(k0 - ci, nn, (ci >> 1) + 16 * (4 * h + m));
+              kv1[m] = ld_packed2_raw(k1 - ci, nn, (ci >> 1) + 16 * (4 * h + m));
             }
           } else {
 #pragma unroll
@@ -514,8 +505,8 @@ __global__ void __launch_bounds__(NTT_THREADS, 2) ntt_rows(NttTables t, int logN
 #pragma unroll
             for (int m = 0; m < 4; ++m) {
               const ulonglong2 dv = __ldg(reinterpret_cast<const ulonglong2 *>(dd + 32 * (4 * h + m)));
-              const ulonglong2 w0 = KPK ? key_join(ld_key_raw(o0, 4 * h + m)) : __ldg(reinterpret_cast<const ulonglong2 *>(o0 + 32 * (4 * h + m)));
-              const ulonglong2 w1 = KPK ? key_join(ld_key_raw(o1, 4 * h + m)) : __ldg(reinterpret_cast<const ulonglong2 *>(o1 + 32 * (4 * h + m)));
+              const ulonglong2 w0 = KPK ? packed2_join(ld_packed2_raw(o0 - ci, nn, (ci >> 1) + 16 * (4 * h + m))) : __ldg(reinterpret_cast<const ulonglong2 *>(o0 + 32 * (4 * h + m)));
+              const ulonglong2 w1 = KPK ? packed2_join(ld_packed2_raw(o1 - ci, nn, (ci >> 1) + 16 * (4 * h + m))) : __ldg(reinterpret_cast<const ulonglong2 *>(o1 + 32 * (4 * h + m)));
               const double dx = u64_to_f64(dv.x), dy = u64_to_f64(dv.y);
               old0[m] = make_double2(mulmod_var(dx, u64_to_f64(w0.x), q, qinv), mulmod_var(dy, u64_to_f64(w0.y), q, qinv));
               old1[m] = make_double2(mulmod_var(dx, u64_to_f64(w1.x), q, qinv), mulmod_var(dy, u64_to_f64(w1.y), q, qinv));
@@ -526,7 +517,7 @@ __global__ void __launch_bounds__(NTT_THREADS, 2) ntt_rows(NttTables t, int logN
           }
           if constexpr (KPK) {
 #pragma unroll
-            for (int m = 0; m < 4; ++m) { kv0[m] = key_join(kv0[m]); kv1[m] = key_join(kv1[m]); }
+            for (int m = 0; m < 4; ++m) { kv0[m] = packed2_join(kv0[m]); kv1[m] = packed2_join(kv1[m]); }
           }
 #pragma unroll
           for (int m = 0; m < 4; ++m) {

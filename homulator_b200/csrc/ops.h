@@ -18,6 +18,10 @@ int ensure_ws(hml_ctx *ctx, size_t words);
 int check_level(hml_ctx *ctx, uint32_t L, uint32_t min_level);
 int shard_check(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world);
 
+// A galois element mod 2N, and the inner-product kernels' form of it: 0 for the identity (InnerArgs::galois)
+inline unsigned galois_mod(uint64_t g, size_t N) { return (unsigned)(g & (2ull * N - 1)); }
+inline unsigned inner_galois(uint64_t g, size_t N) { const unsigned r = galois_mod(g, N); return r == 1 ? 0 : r; }
+
 size_t hmult_ws_words(const hml::Params &p, uint32_t L, uint32_t nb);
 size_t hrot_ws_words(const hml::Params &p, uint32_t L, uint32_t nb);
 

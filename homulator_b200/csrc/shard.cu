@@ -391,7 +391,7 @@ static int hoist_phase(hml_shard *sh, const HoistOp &op, const HoistStep &st, cu
     case HS_INTT: return shard_hoist_intt(ctx, L, rank, world, n, sh->g2, sh->n2, s);
     case HS_END:
       for (uint32_t r = 0; r < n && nq; ++r) {
-        const uint64_t g = op.galois[lo + r] & (2 * N - 1);
+        const uint64_t g = galois_mod(op.galois[lo + r], N);
         uint64_t *o = op.outs[lo + r];
         const uint64_t *add = op.ct;  // g = 1: sigma(c0) is c0 itself
         uint64_t add_g = 0;
