@@ -70,6 +70,7 @@ EXPORTS = [
     "hml_hrotate_sharded", "hml_hmult_sharded", "hml_rescale_sharded", "hml_ew_sharded", "hml_group_op", "hml_hrotate_hoisted",
     "hml_replay_create", "hml_replay_bind", "hml_replay_run", "hml_replay_slot", "hml_replay_slot_level", "hml_replay_destroy",
     "hml_shard_create_ex", "hml_hrotate_hoisted_sharded", "hml_group_hrotate_hoisted", "hml_hrotate_sum_hoisted",
+    "hml_hrotate_bsgs_hoisted",
 ]
 
 
@@ -165,6 +166,8 @@ def load_library():
                                C.POINTER(vp)]
     L.hml_hrotate_hoisted.argtypes = [vp, u32, vp, u32, C.POINTER(vp), u32, C.POINTER(u64), C.POINTER(vp), vp]
     L.hml_hrotate_sum_hoisted.argtypes = [vp, u32, vp, u32, C.POINTER(vp), u32, C.POINTER(u64), C.POINTER(vp), u32, vp, vp]
+    L.hml_hrotate_bsgs_hoisted.argtypes = [vp, u32, vp, u32, C.POINTER(u64), C.POINTER(vp), u32, C.POINTER(u64), C.POINTER(vp), u32,
+                                           C.POINTER(vp), u32, vp, vp]
     L.hml_hrotate_hoisted_sharded.argtypes = [vp, u32, vp, u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(vp), vp]
     L.hml_group_hrotate_hoisted.argtypes = [C.POINTER(vp), u32, u32, C.POINTER(vp), u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(vp),
                                             C.POINTER(vp)]
@@ -400,6 +403,24 @@ class Context:
         gs = (C.c_uint64 * max(n, 1))(*[int(g) for g in galois_elts])
         self._chk(self.lib.hml_hrotate_sum_hoisted(self.h, L, _ptr(ct), n, keys, evk_q_limbs or L, gs, pa, pt_q_limbs or L, _ptr(out),
                                                    self._stream()))
+        return out
+
+    def hrotate_bsgs_hoisted(self, L, ct, baby_galois, baby_keys, giant_galois, giant_keys, pts, evk_q_limbs=None, pt_q_limbs=None,
+                             out=None):
+        """sum_j rotate(sum_i pts[j][i] * rotate(ct, baby_galois[i]), giant_galois[j]) with one ModUp for every baby step and one
+        final ModDown (hml_hrotate_bsgs_hoisted).  pts is n2 lists of n1 plaintexts [pt_q_limbs + alpha][N] (P-limb m at row
+        pt_q_limbs + m); a key may be None for an identity element (galois 1)."""
+        n1, n2 = len(baby_galois), len(giant_galois)
+        if len(baby_keys) != n1 or len(giant_keys) != n2 or len(pts) != n2 or any(len(row) != n1 for row in pts):
+            raise ValueError("one key per galois element and n2 rows of n1 plaintexts")
+        out = self.empty(2, L, self.N) if out is None else out
+        bk = (C.c_void_p * max(n1, 1))(*[_ptr(k) for k in baby_keys])
+        gk = (C.c_void_p * max(n2, 1))(*[_ptr(k) for k in giant_keys])
+        bg = (C.c_uint64 * max(n1, 1))(*[int(g) for g in baby_galois])
+        gg = (C.c_uint64 * max(n2, 1))(*[int(g) for g in giant_galois])
+        pa = (C.c_void_p * max(n1 * n2, 1))(*[_ptr(p) for row in pts for p in row])
+        self._chk(self.lib.hml_hrotate_bsgs_hoisted(self.h, L, _ptr(ct), n1, bg, bk, n2, gg, gk, evk_q_limbs or L, pa, pt_q_limbs or L,
+                                                    _ptr(out), self._stream()))
         return out
 
     def hadd(self, L, a, b, out=None):

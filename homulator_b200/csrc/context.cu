@@ -1852,6 +1852,116 @@ extern "C" int hml_hrotate_sum_hoisted(hml_ctx *ctx, uint32_t L, const uint64_t 
                               (cudaStream_t)stream);
 }
 
+// Z [2][L] | yb [L] | ext [beta][E] | A [2][E] | vb [2][L] | acc_j [2][E] | z_j [2][L] | ct_j [2][L] | ext_j [beta][E]
+static size_t bsgs_ws_words(const Params &p, uint32_t L) {
+  const size_t N = p.N, E = L + p.alpha;
+  return N * (9 * (size_t)L + 4 * E + 2 * (size_t)p.beta(L) * E);
+}
+
+// Double-hoisted baby-step / giant-step linear transform (Bossuat et al., Eurocrypt 2021):
+//   out = sum_j rotate( sum_i pt_{j,i} * rotate(ct, b_i), G_j )
+// with the ModUp of c1 shared by every baby step and ONE final ModDown.  IP_g(c) = sum_d sigma_g(ModUp(c)_d) * rk_g[d] (in Q*P):
+//   inner sum j:  acc_j = sum_{b_i != 1} pt_{j,i} * IP_{b_i}(c1),  z0_j = sum_i pt_{j,i} * sigma_{b_i}(c0),  z1_j = sum_{b_i = 1} pt_{j,i} * c1
+//   giant j != 1: ct_j = (ModDown(acc_j) + (z0_j, z1_j)), then A += IP_{G_j}(ct_j.c1) and Z0 += sigma_{G_j}(ct_j.c0)
+//   giant j  = 1: A += acc_j, Z0 += z0_j, Z1 += z1_j
+//   out   = ModDown(A) + (Z0, Z1)
+// Identity elements (g = 1 mod 2N) pay no key switch.  ModUps: 1 + k, ModDowns: k + 1 (k = non-identity giant steps), whatever
+// n1.  The oracle defines the op (tests/orc_bsgs.py).
+static int hrot_bsgs_hoisted_run(hml_ctx *ctx, uint32_t L, const u64 *ct, uint32_t n1, const uint64_t *baby_galois,
+                                 const uint64_t *const *baby_keys, uint32_t n2, const uint64_t *giant_galois, const uint64_t *const *giant_keys,
+                                 uint32_t evk_q_limbs, const uint64_t *const *pts, uint32_t pt_q_limbs, u64 *ct_out, u64 *ws, cudaStream_t s) {
+  const Params &p = ctx->p;
+  KeyDesc key;  // one key per rotation: only the layout is shared
+  int rc = key_desc(ctx, L, nullptr, evk_q_limbs, &key);
+  if (rc) return rc;
+  if (pt_q_limbs < L || pt_q_limbs > p.max_level) return fail(ctx, HML_ERR_INVALID, "pt_q_limbs must be in [L, maxLevel]");
+  LevelConsts *lc;
+  if ((rc = get_level(ctx, L, &lc))) return rc;
+  const size_t N = p.N, PL = N * L;
+  const uint32_t A = p.alpha, E = L + A, beta = lc->beta;
+  u64 *Z = ws, *yb = Z + 2 * PL, *ext = yb + PL, *acc = ext + (size_t)beta * E * N, *vb = acc + 2 * (size_t)E * N;
+  u64 *acc_j = vb + 2 * PL, *z_j = acc_j + 2 * (size_t)E * N, *ct_j = z_j + 2 * PL, *ext_j = ct_j + 2 * PL;
+  const BatchPtr c1{ct + PL, 0};
+  if ((rc = ks_modup(ctx, lc, L, 1, c1, yb, ext, s, nullptr))) return rc;
+  LimbMap ip = lc->ext_lm;  // pos = limb index inside the key
+  for (uint32_t e = 0; e < E; ++e) ip.pos[e] = (uint16_t)key.pos(e, L);
+  InnerBsgsArgs a{};
+  a.d = c1.ptr; a.ext = ext; a.c0 = ct;
+  a.N = (int)N; a.n_ext = (int)E; a.L = (int)L; a.beta = (int)beta; a.evk_limbs = (int)(key.q_limbs + A); a.pt_q_limbs = (int)pt_q_limbs; a.logN = p.logN;
+  a.ext_f64 = p.logN > NTT_SMALL_LOG; a.evk_packed = key.packed ? 1 : 0;
+  // the inner sum of giant step j into (out_acc, z0, z1), in launches of IP_MAX_ROT baby steps
+  auto inner_sum = [&](uint32_t j, u64 *out_acc, u64 *z0, u64 *z1, bool accumulate) {
+    a.acc = out_acc; a.z = z0; a.z1 = z1;
+    for (uint32_t i0 = 0; i0 < n1; i0 += IP_MAX_ROT) {
+      const uint32_t n = std::min<uint32_t>(IP_MAX_ROT, n1 - i0);
+      a.accumulate = accumulate || i0 > 0; a.n_rot = (int)n;
+      uint32_t n_id = 0;
+      for (uint32_t k = 0; k < n; ++k) {
+        const unsigned g = inner_galois(baby_galois[i0 + k], N);
+        a.galois[k] = g; a.evk[k] = g ? (const u64 *)baby_keys[i0 + k] : nullptr; a.pt[k] = (const u64 *)pts[(size_t)j * n1 + i0 + k];
+        n_id += g ? 0 : 1;
+      }
+      launch_inner_product_bsgs(ctx->mc, ip, a, false, s);
+      prof_mark(ctx, HML_CLS_EWE, s);
+      ctx->exec.kernel_launches++;
+      ctx->exec.ewe_limbs += (uint64_t)(n - n_id) * (2ull * E * beta + 2ull * E + L) + 2ull * n_id * L;
+      ctx->exec.automorph_limbs += (uint64_t)(n - n_id) * L;  // sigma(c0), applied on load
+    }
+  };
+  bool have_acc = false;  // A / Z0 hold a sum (later launches add to it); Z1 is used only by identity giant steps
+  for (uint32_t j = 0; j < n2; ++j)
+    if (!inner_galois(giant_galois[j], N)) { inner_sum(j, acc, Z, Z + PL, have_acc); have_acc = true; }
+  const bool z1_used = have_acc;
+  for (uint32_t j = 0; j < n2; ++j) {
+    const unsigned g = inner_galois(giant_galois[j], N);
+    if (!g) continue;
+    inner_sum(j, acc_j, z_j, z_j + PL, false);
+    if ((rc = ks_inner(ctx, lc, L, 1, c1, key, ext, acc_j, E, 0, s, nullptr, true))) return rc;
+    if ((rc = ks_tail(ctx, lc, L, 1, acc_j, vb, {ct_j, 0}, {ct_j + PL, 0}, {z_j, 0}, {z_j + PL, 0}, s, false, 0))) return rc;
+    // the baby digits in ext serve every later giant step: ct_j's digits get their own buffer
+    if ((rc = ks_modup(ctx, lc, L, 1, {ct_j + PL, 0}, yb, ext_j, s, nullptr))) return rc;
+    InnerBsgsArgs ga = a;
+    ga.d = ct_j + PL; ga.ext = ext_j; ga.c0 = ct_j; ga.acc = acc; ga.z = Z; ga.z1 = nullptr;
+    ga.accumulate = have_acc; ga.n_rot = 1; ga.evk[0] = (const u64 *)giant_keys[j]; ga.pt[0] = nullptr; ga.galois[0] = g;
+    launch_inner_product_bsgs(ctx->mc, ip, ga, true, s);
+    prof_mark(ctx, HML_CLS_EWE, s);
+    ctx->exec.kernel_launches++;
+    ctx->exec.ewe_limbs += 2ull * E * beta + L;
+    ctx->exec.automorph_limbs += L;
+    have_acc = true;
+  }
+  if ((rc = ks_inner(ctx, lc, L, 1, c1, key, ext, acc, E, 0, s, nullptr, true))) return rc;
+  if ((rc = ks_tail(ctx, lc, L, 1, acc, vb, {ct_out, 0}, {ct_out + PL, 0}, {Z, 0}, {z1_used ? Z + PL : nullptr, 0}, s, false, 0))) return rc;
+  return check_launch(ctx, "hrotate bsgs hoisted");
+}
+
+extern "C" int hml_hrotate_bsgs_hoisted(hml_ctx *ctx, uint32_t L, const uint64_t *ct, uint32_t n1, const uint64_t *baby_galois,
+                                        const uint64_t *const *baby_keys, uint32_t n2, const uint64_t *giant_galois,
+                                        const uint64_t *const *giant_keys, uint32_t evk_q_limbs, const uint64_t *const *pts,
+                                        uint32_t pt_q_limbs, uint64_t *ct_out, void *stream) {
+  int rc = check_level(ctx, L, 1);
+  if (rc) return rc;
+  if (n1 == 0 || n2 == 0) return fail(ctx, HML_ERR_INVALID, "n1 and n2 must be at least 1");
+  if (!ct || !baby_galois || !giant_galois || !pts || !ct_out) return fail(ctx, HML_ERR_INVALID, "null buffer");
+  const size_t N = ctx->p.N, w = 2 * N * L;
+  if (ct_out < ct + w && ct < ct_out + w) return fail(ctx, HML_ERR_INVALID, "the output overlaps the input");
+  for (int giant = 0; giant < 2; ++giant) {
+    const uint64_t *gs = giant ? giant_galois : baby_galois;
+    const uint64_t *const *keys = giant ? giant_keys : baby_keys;
+    for (uint32_t i = 0; i < (giant ? n2 : n1); ++i) {
+      if (!(gs[i] & 1)) return fail(ctx, HML_ERR_INVALID, "galois element must be odd");
+      if (inner_galois(gs[i], N) && !(keys && keys[i])) return fail(ctx, HML_ERR_INVALID, "null key for a non-identity galois element");
+    }
+  }
+  for (size_t k = 0; k < (size_t)n1 * n2; ++k)
+    if (!pts[k]) return fail(ctx, HML_ERR_INVALID, "null plaintext");
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  if ((rc = ensure_ws(ctx, bsgs_ws_words(ctx->p, L)))) return rc;
+  ws_enter(ctx, (cudaStream_t)stream);
+  return hrot_bsgs_hoisted_run(ctx, L, (const u64 *)ct, n1, baby_galois, baby_keys, n2, giant_galois, giant_keys, evk_q_limbs, pts,
+                               pt_q_limbs, (u64 *)ct_out, ctx->ws, (cudaStream_t)stream);
+}
+
 static int ew_ct_op(hml_ctx *ctx, uint32_t L, const uint64_t *a, const uint64_t *b, bool b_is_pt, bool mul, uint64_t *out, void *stream) {
   int rc = check_level(ctx, L, 1);
   if (rc) return rc;

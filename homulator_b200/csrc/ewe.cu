@@ -341,12 +341,10 @@ void launch_inner_product_rot(const ModConst *mc, const LimbMap &lm, const Inner
 // word stay far below 2^51.  PACKED (the key's load path) is a template argument: with both paths in one body four digits
 // spilled at 128 registers.  Up to three digits fit three CTAs per SM (76 registers), four digits two (108-128), five to eight
 // digits one (229-237).
-template <int IP_MAX_BETA, bool PACKED>
-__global__ void __launch_bounds__(EW_THREADS, IP_MAX_BETA > 4 ? 1 : IP_MAX_BETA > 3 ? 2 : 3)
-    k_inner_rot_sum(const ModConst *__restrict__ mc, LimbMap lm, const __grid_constant__ InnerRotSumArgs a) {
-  pdl_wait();
-  const int i2 = blockIdx.x * EW_THREADS + threadIdx.x;
-  if (i2 >= a.N / 2) return;
+// MODE selects the kernel the body serves: RS_SUM k_inner_rot_sum; RS_BABY and RS_GIANT k_inner_bsgs (ewe.cuh InnerBsgsArgs).
+enum { RS_SUM, RS_BABY, RS_GIANT };
+template <int IP_MAX_BETA, bool PACKED, int MODE, class A>
+__device__ __forceinline__ void rot_sum_body(const ModConst *__restrict__ mc, const LimbMap &lm, const A &a, int i2) {
   const int e = blockIdx.y;
   const ModConst m = mc[lm.mod[e]];
   const int kl = lm.pos[e], own = lm.skip[e];
@@ -354,8 +352,22 @@ __global__ void __launch_bounds__(EW_THREADS, IP_MAX_BETA > 4 ? 1 : IP_MAX_BETA 
   const bool q_limb = e < a.L;  // uniform per CTA
   const size_t prow = q_limb ? (size_t)e : (size_t)a.pt_q_limbs + (e - a.L);
   double a00 = 0, a01 = 0, a10 = 0, a11 = 0, z0 = 0, z1 = 0;  // [component][coefficient], z = the c0 term
+  double y0 = 0, y1 = 0;                                       // RS_BABY: the c1 term of the identity entries
 #pragma unroll 1
   for (int r = 0; r < a.n_rot; ++r) {
+    if constexpr (MODE == RS_BABY) {
+      if (!a.evk[r]) {  // uniform: the identity without a key switch, nothing on the P-limbs
+        if (q_limb) {
+          const ulonglong2 w = ld2(a.pt[r] + prow * a.N, i2), x = ld2(a.c0 + (size_t)e * a.N, i2), y = ld2(a.d + (size_t)e * a.N, i2);
+          const double w0 = u64_to_f64(w.x), w1 = u64_to_f64(w.y);
+          z0 += mulmod_var(u64_to_f64(x.x), w0, m.q, m.qinv);
+          z1 += mulmod_var(u64_to_f64(x.y), w1, m.q, m.qinv);
+          y0 += mulmod_var(u64_to_f64(y.x), w0, m.q, m.qinv);
+          y1 += mulmod_var(u64_to_f64(y.y), w1, m.q, m.qinv);
+        }
+        continue;
+      }
+    }
     const unsigned g = a.galois[r];
     const uint2 src = gal_slots(g, a.logN, i2);
     ulonglong2 t[IP_MAX_BETA];
@@ -367,21 +379,28 @@ __global__ void __launch_bounds__(EW_THREADS, IP_MAX_BETA > 4 ? 1 : IP_MAX_BETA 
       }
     ulonglong2 kraw[IP_MAX_BETA][2];
     ld_key<PACKED>(kraw, a.evk[r], a, kl, n2, i2);
-    ulonglong2 w = ld2(a.pt[r] + prow * a.N, i2), x = make_ulonglong2(0, 0);
+    ulonglong2 w = make_ulonglong2(0, 0), x = make_ulonglong2(0, 0);
+    if constexpr (MODE != RS_GIANT) w = ld2(a.pt[r] + prow * a.N, i2);
     if (q_limb) x = ld_pair(a.c0 + (size_t)e * a.N, i2, src, g != 0);
     pin_loads(kraw);
-    asm volatile("" : "+l"(w.x), "+l"(w.y), "+l"(x.x), "+l"(x.y));
+    if constexpr (MODE != RS_GIANT) asm volatile("" : "+l"(w.x), "+l"(w.y), "+l"(x.x), "+l"(x.y));
+    else asm volatile("" : "+l"(x.x), "+l"(x.y));
     if constexpr (PACKED) join_key(kraw);
     double s00 = 0, s01 = 0, s10 = 0, s11 = 0;
     mac_digits(s00, s01, s10, s11, t, kraw, a.beta, a.ext_f64, own, m);
-    const double w0 = u64_to_f64(w.x), w1 = u64_to_f64(w.y);
-    a00 += mulmod_var(s00, w0, m.q, m.qinv);
-    a01 += mulmod_var(s01, w1, m.q, m.qinv);
-    a10 += mulmod_var(s10, w0, m.q, m.qinv);
-    a11 += mulmod_var(s11, w1, m.q, m.qinv);
-    if (q_limb) {
-      z0 += mulmod_var(u64_to_f64(x.x), w0, m.q, m.qinv);
-      z1 += mulmod_var(u64_to_f64(x.y), w1, m.q, m.qinv);
+    if constexpr (MODE == RS_GIANT) {  // unweighted: one term of at most 8 * 0.51 q per rotation
+      a00 += s00; a01 += s01; a10 += s10; a11 += s11;
+      if (q_limb) { z0 += u64_to_f64(x.x); z1 += u64_to_f64(x.y); }
+    } else {
+      const double w0 = u64_to_f64(w.x), w1 = u64_to_f64(w.y);
+      a00 += mulmod_var(s00, w0, m.q, m.qinv);
+      a01 += mulmod_var(s01, w1, m.q, m.qinv);
+      a10 += mulmod_var(s10, w0, m.q, m.qinv);
+      a11 += mulmod_var(s11, w1, m.q, m.qinv);
+      if (q_limb) {
+        z0 += mulmod_var(u64_to_f64(x.x), w0, m.q, m.qinv);
+        z1 += mulmod_var(u64_to_f64(x.y), w1, m.q, m.qinv);
+      }
     }
   }
   const size_t o0 = (size_t)e * n2 + i2, o1 = (size_t)(a.n_ext + e) * n2 + i2;
@@ -391,11 +410,26 @@ __global__ void __launch_bounds__(EW_THREADS, IP_MAX_BETA > 4 ? 1 : IP_MAX_BETA 
     if (q_limb) {
       const ulonglong2 pz = ld2(a.z, o0);
       z0 += u64_to_f64(pz.x); z1 += u64_to_f64(pz.y);
+      if constexpr (MODE == RS_BABY) {
+        const ulonglong2 py = ld2(a.z1, o0);
+        y0 += u64_to_f64(py.x); y1 += u64_to_f64(py.y);
+      }
     }
   }
   st2(a.acc, o0, finish(a00, m), finish(a01, m));
   st2(a.acc, o1, finish(a10, m), finish(a11, m));
   if (q_limb) st2(a.z, o0, finish(z0, m), finish(z1, m));
+  if constexpr (MODE == RS_BABY)
+    if (q_limb) st2(a.z1, o0, finish(y0, m), finish(y1, m));
+}
+
+template <int IP_MAX_BETA, bool PACKED>
+__global__ void __launch_bounds__(EW_THREADS, IP_MAX_BETA > 4 ? 1 : IP_MAX_BETA > 3 ? 2 : 3)
+    k_inner_rot_sum(const ModConst *__restrict__ mc, LimbMap lm, const __grid_constant__ InnerRotSumArgs a) {
+  pdl_wait();
+  const int i2 = blockIdx.x * EW_THREADS + threadIdx.x;
+  if (i2 >= a.N / 2) return;
+  rot_sum_body<IP_MAX_BETA, PACKED, RS_SUM>(mc, lm, a, i2);
 }
 
 void launch_inner_product_rot_sum(const ModConst *mc, const LimbMap &lm, const InnerRotSumArgs &a, cudaStream_t s) {
@@ -403,6 +437,31 @@ void launch_inner_product_rot_sum(const ModConst *mc, const LimbMap &lm, const I
     constexpr int NB = decltype(nb)::value;
     if (a.evk_packed) launch_pdl(k_inner_rot_sum<NB, true>, ew_grid(a.N, a.n_ext), EW_THREADS, 0, s, mc, lm, a);
     else launch_pdl(k_inner_rot_sum<NB, false>, ew_grid(a.N, a.n_ext), EW_THREADS, 0, s, mc, lm, a);
+  });
+}
+
+// The two inner products of a double-hoisted BSGS linear transform (ewe.cuh InnerBsgsArgs), k_inner_rot_sum's body with
+// identity entries (GIANT = false) or without the plaintext (GIANT = true)
+template <int IP_MAX_BETA, bool PACKED, bool GIANT>
+__global__ void __launch_bounds__(EW_THREADS, IP_MAX_BETA > 4 ? 1 : IP_MAX_BETA > 3 ? 2 : 3)
+    k_inner_bsgs(const ModConst *__restrict__ mc, LimbMap lm, const __grid_constant__ InnerBsgsArgs a) {
+  pdl_wait();
+  const int i2 = blockIdx.x * EW_THREADS + threadIdx.x;
+  if (i2 >= a.N / 2) return;
+  rot_sum_body<IP_MAX_BETA, PACKED, GIANT ? RS_GIANT : RS_BABY>(mc, lm, a, i2);
+}
+
+void launch_inner_product_bsgs(const ModConst *mc, const LimbMap &lm, const InnerBsgsArgs &a, bool giant, cudaStream_t s) {
+  with_max_beta(a.beta, [&](auto nb) {
+    constexpr int NB = decltype(nb)::value;
+    const dim3 grid = ew_grid(a.N, a.n_ext);
+    if (giant) {
+      if (a.evk_packed) launch_pdl(k_inner_bsgs<NB, true, true>, grid, EW_THREADS, 0, s, mc, lm, a);
+      else launch_pdl(k_inner_bsgs<NB, false, true>, grid, EW_THREADS, 0, s, mc, lm, a);
+    } else {
+      if (a.evk_packed) launch_pdl(k_inner_bsgs<NB, true, false>, grid, EW_THREADS, 0, s, mc, lm, a);
+      else launch_pdl(k_inner_bsgs<NB, false, false>, grid, EW_THREADS, 0, s, mc, lm, a);
+    }
   });
 }
 

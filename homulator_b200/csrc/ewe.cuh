@@ -93,6 +93,17 @@ struct InnerRotSumArgs {
 };
 void launch_inner_product_rot_sum(const ModConst *mc, const LimbMap &lm, const InnerRotSumArgs &a, cudaStream_t s);
 
+// The two inner products of a double-hoisted baby-step / giant-step linear transform (context.cu, hrot_bsgs_hoisted_run), as
+// InnerRotSumArgs with:
+//   baby  (giant = false): an entry with evk[r] == null is the identity without a key switch.  It loads no digit and no key
+//         and adds pt_r[e] * c0[e] to z and pt_r[e] * d[e] (c1) to z1, on the Q-limbs only.  z1 is stored like z.
+//   giant (giant = true):  no plaintext is read and the sums are unweighted, acc (+)= sum_j sigma_r(t_j) * evk_r[j],
+//         z (+)= sigma_r(c0); z1 is not touched.
+struct InnerBsgsArgs : InnerRotSumArgs {
+  u64 *z1;                         // [L][N] (baby only)
+};
+void launch_inner_product_bsgs(const ModConst *mc, const LimbMap &lm, const InnerBsgsArgs &a, bool giant, cudaStream_t s);
+
 // out = (x - y) * c (+ z) per limb:  ModDownSub (+ HMULT add)  reference src/Operation.cpp:548-590, :967-1005
 // and Rescale sub+mul  reference src/Operation.cpp:825-911.  cst[limb] = (c, RN(c/q)).  n_polys via strides.
 struct SubMulArgs {

@@ -297,6 +297,30 @@ int hml_hrotate_hoisted(hml_ctx *ctx, uint32_t L, const uint64_t *ct, uint32_t n
 int hml_hrotate_sum_hoisted(hml_ctx *ctx, uint32_t L, const uint64_t *ct, uint32_t n_rot, const uint64_t *const *rotkeys,
                             uint32_t evk_q_limbs, const uint64_t *galois_elts, const uint64_t *const *pts, uint32_t pt_q_limbs,
                             uint64_t *ct_out, void *stream);
+/* Double-hoisted baby-step / giant-step linear transform (Bossuat et al., Eurocrypt 2021), the form of CoeffToSlot /
+ * SlotToCoeff and of any plaintext-matrix x encrypted-vector product:
+ *   ct_out = sum_j rotate( sum_i pts[j * n1 + i] * rotate(ct, baby_galois[i]), giant_galois[j] )     i < n1, j < n2
+ * with ONE ModUp of c1 for every baby step, one ModUp per non-identity giant step and ONE final ModDown.  With
+ * IP_g(c) = sum_d sigma_g(ModUp(c)_d) * rk_g[d], a pair of accumulators over E = (q_0..q_{L-1}, p_0..p_{alpha-1}):
+ *   1. per giant step j:  acc_j = sum_{b_i != 1} pt_{j,i} * IP_{b_i}(c1),  z0_j = sum_i pt_{j,i} * sigma_{b_i}(c0),
+ *                         z1_j  = sum_{b_i = 1} pt_{j,i} * c1
+ *   2. per G_j != 1:      ct_j  = (ModDown(acc_j, 0) + z0_j, ModDown(acc_j, 1) + z1_j)
+ *   3. A  = sum_{G_j = 1} acc_j + sum_{G_j != 1} IP_{G_j}(ct_j.c1),   Z0 = sum_{G_j = 1} z0_j + sum_{G_j != 1} sigma_{G_j}(ct_j.c0),
+ *      Z1 = sum_{G_j = 1} z1_j
+ *   4. ct_out = (ModDown(A, 0) + Z0, ModDown(A, 1) + Z1)
+ * Identity elements (g = 1 mod 2N) pay no key switch and their key entry may be NULL; every other element needs its rotation
+ * key.  Keys follow hml_hrotate_sum_hoisted: one layout for all (evk_q_limbs, optionally | HML_KEY_PACKED).  pts[j * n1 + i]
+ * (j-major) is [pt_q_limbs + alpha][N], P-limb m at row pt_q_limbs + m.  With n2 = 1, G_0 = 1 and no identity baby step the
+ * result is hml_hrotate_sum_hoisted's bit for bit.  The oracle defines the op (tests/orc_bsgs.py).
+ * ct, ct_out [2][L][N], not overlapping.  The key, galois and plaintext arrays are HOST arrays.  HML_ERR_INVALID: n1 = 0 or
+ * n2 = 0, a null ct / ct_out / galois array / plaintext, a null key for a non-identity element, an even galois element,
+ * overlapping ct / ct_out, evk_q_limbs or pt_q_limbs outside [L, maxLevel]; HML_ERR_UNSUPPORTED: more than 8 digits.
+ * Executed counts: with k non-identity giant steps, the transforms and conversions of (k + 1) hml_hrotate_sum_hoisted calls
+ * of one rotation, whatever n1; one kernel launch per group of 16 baby steps of every giant step and one per non-identity
+ * giant step.  After the workspace exists the call neither allocates nor synchronises (it can be captured in a CUDA graph). */
+int hml_hrotate_bsgs_hoisted(hml_ctx *ctx, uint32_t L, const uint64_t *ct, uint32_t n1, const uint64_t *baby_galois,
+                             const uint64_t *const *baby_keys, uint32_t n2, const uint64_t *giant_galois, const uint64_t *const *giant_keys,
+                             uint32_t evk_q_limbs, const uint64_t *const *pts, uint32_t pt_q_limbs, uint64_t *ct_out, void *stream);
 /* HADD / PMULT / PADD (reference src/Operation.cpp:1114-1176, :1453-1523, :1618-1680).  pt is [L][N].
  * PADD adds the plaintext to BOTH components, as the reference's trace does (:1650-1672). */
 int hml_hadd(hml_ctx *ctx, uint32_t L, const uint64_t *ct_a, const uint64_t *ct_b, uint64_t *ct_out, void *stream);
