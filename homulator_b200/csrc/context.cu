@@ -41,6 +41,14 @@ struct MergedU {
   long long comp_stride, batch_stride;
 };
 
+// The batched hmult's ciphertext pairs (a, b), component c of pair b at a + b * batch_stride + c * comp_stride: the key switch
+// squares c1 on the ModUp transform's load (d2 = a1 * b1, NttLaunch::in_mul) and forms the tensor product in the inner
+// product (InnerArgs::ct_a), so that d0, d1 and d2 never reach memory.
+struct KsTensor {
+  const u64 *a, *b;
+  long long comp_stride, batch_stride;
+};
+
 static thread_local std::string g_create_err;
 
 #define CU_TRY(ctx, call)                                                                          \
@@ -351,7 +359,7 @@ extern "C" int hml_ctx_create(const char *cfg_path, uint32_t max_level, uint32_t
 }
 
 static void free_level(LevelConsts &lc) {
-  cudaFree(lc.modup_scale); cudaFree(lc.moddown_scale); cudaFree(lc.moddown_scale_u); cudaFree(lc.pinv); cudaFree(lc.qlinv);
+  cudaFree(lc.modup_scale); cudaFree(lc.moddown_scale); cudaFree(lc.moddown_scale_u); cudaFree(lc.pinv); cudaFree(lc.pmod); cudaFree(lc.qlinv);
   for (auto &u : lc.up) { cudaFree(u.d_mat); cudaFree(u.d_img); }
   cudaFree(lc.down.d_mat); cudaFree(lc.merged_rest.d_mat); cudaFree(lc.merged_fold);
   cudaFree(lc.down.d_img); cudaFree(lc.merged_rest.d_img); cudaFree(lc.up_jobs);
@@ -489,10 +497,17 @@ static int get_level(hml_ctx *ctx, uint32_t L, LevelConsts **out) {
     make_bconv_table(p, src, dst, bt);
     std::vector<double2> sc(A), pinv(L);
     for (uint32_t j = 0; j < A; ++j) sc[j] = mk_cst(p.moddown_scale(j), p.mod[p.max_level + j]);
-    for (uint32_t i = 0; i < L; ++i) pinv[i] = mk_cst(p.p_inv(i), p.mod[i]);
+    std::vector<double2> pmod(L);
+    for (uint32_t i = 0; i < L; ++i) {
+      pinv[i] = mk_cst(p.p_inv(i), p.mod[i]);
+      u64 pm = 1;
+      for (uint32_t j = 0; j < A; ++j) pm = h_mulmod(pm, p.mod[p.max_level + j] % p.mod[i], p.mod[i]);
+      pmod[i] = mk_cst(pm, p.mod[i]);
+    }
     if ((rc = prepare_bconv(ctx, bt, dst, lc.down))) return rc;
     if ((rc = upload(ctx, sc, &lc.moddown_scale))) return rc;
     if ((rc = upload(ctx, pinv, &lc.pinv))) return rc;
+    if ((rc = upload(ctx, pmod, &lc.pmod))) return rc;
     // hmult's merged path: the P-limbs plus slot E (modulus q_{L-1}, plain N^-1) in one INTT launch
     lc.pu_lm = lc.p_lm;
     lc.pu_lm.mod[A] = (uint16_t)(L - 1); lc.pu_lm.pos[A] = (uint16_t)E;
@@ -700,7 +715,7 @@ static bool ks_uses_hpip(const hml_ctx *ctx, uint32_t L, uint32_t nb) {
 }
 
 static int ks_modup(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, u64 *yb, u64 *ext, cudaStream_t s, const NttMac *mac = nullptr,
-                    const KsAuto *au = nullptr) {
+                    const KsAuto *au = nullptr, const KsTensor *ten = nullptr) {
   const Params &p = ctx->p;
   const size_t N = p.N;
   const uint32_t A = p.alpha, E = L + A, beta = lc->beta;
@@ -716,6 +731,9 @@ static int ks_modup(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, Batc
       for (int i = 0; i < 7; ++i) gi = gi * (2u - g8 * gi);  // Newton: g^-1 mod 256 (g odd)
       l.in_galois = galois_mod(au->g, N); l.in_ginv8 = gi & 255u;
       l.side_out = au->sigma_d; l.side_batch_stride = au->sigma_stride;
+    }
+    if (ten) {  // d = a1 * b1, formed on load (tallied with the tensor product in ks_inner)
+      l.in = ten->a + ten->comp_stride; l.in_mul = ten->b + ten->comp_stride; l.in_batch_stride = ten->batch_stride;
     }
     run_ntt(ctx, true, lc->q_lm, l, s);
   }
@@ -765,7 +783,7 @@ static int key_desc(hml_ctx *ctx, uint32_t L, const u64 *evk, uint32_t evk_q_lim
 // K5..K7: inner product with the key, INTT (+ step-1 scaling) of the P-limbs of both accumulators.  acc [nb][2][AL], AL >= E.
 // galois != 0: the digits are read through the automorphism X -> X^galois (hoisted rotation, see InnerArgs::galois).
 static int ks_inner(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, const KeyDesc &key, const u64 *ext, u64 *acc,
-                    uint32_t AL, u64 galois, cudaStream_t s, const MergedU *mu = nullptr, bool ip_done = false) {
+                    uint32_t AL, u64 galois, cudaStream_t s, const MergedU *mu = nullptr, bool ip_done = false, const KsTensor *ten = nullptr) {
   const Params &p = ctx->p;
   const size_t N = p.N;
   const uint32_t A = p.alpha, E = L + A, beta = lc->beta;
@@ -790,17 +808,37 @@ static int ks_inner(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, Batc
       a.u_cst = lc->pinv_last;
       ctx->exec.ewe_limbs += 4ull * nb;
     }
-    launch_inner_product(ctx->mc, ip, a, s);
-    prof_mark(ctx, HML_CLS_EWE, s);
-    ctx->exec.ewe_limbs += 2ull * nb * E * beta; ctx->exec.kernel_launches++;
+    if (!ten) {
+      launch_inner_product(ctx->mc, ip, a, s);
+      prof_mark(ctx, HML_CLS_EWE, s);
+      ctx->exec.kernel_launches++;
+    } else {
+      // the Q-limbs form d0, d1, d2 (the tensor product, reference :592-739) and carry d0 * P, d1 * P; the P-limbs need none of
+      // it and run in the lean kernel (78 registers, three CTAs per SM, instead of 128 and two), as a launch of their own
+      InnerArgs aq = a;
+      aq.ct_a = ten->a; aq.ct_b = ten->b; aq.ct_comp_stride = ten->comp_stride; aq.ct_batch_stride = ten->batch_stride;
+      aq.tensor_pmod = lc->pmod;
+      launch_inner_product(ctx->mc, ip, aq, s, (int)L);
+      prof_mark(ctx, HML_CLS_EWE, s);
+      ctx->exec.ewe_limbs += 3ull * nb * L; ctx->exec.kernel_launches++;
+      LimbMap pl = ip;  // extended limbs L.. renumbered from 0; ext and acc start at limb L
+      for (uint32_t j = 0; j < A; ++j) { pl.mod[j] = ip.mod[L + j]; pl.pos[j] = ip.pos[L + j]; pl.skip[j] = ip.skip[L + j]; }
+      InnerArgs ap = a;
+      ap.ext = ext + (size_t)L * N; ap.acc = acc + (size_t)L * N; ap.acc_pack_limbs = 0;
+      launch_inner_product(ctx->mc, pl, ap, s, (int)A);
+      prof_mark(ctx, HML_CLS_EWE, s);
+      ctx->exec.kernel_launches++;
+    }
+    ctx->exec.ewe_limbs += 2ull * nb * E * beta;
     if (mu && nb > 1) {
-      // batches keep the inner product's kernel lean (78 registers): u[L-1] = acc[L-1] * P^-1 + d[L-1] -> slot E is two small
-      // element-wise launches per chunk (one per component, every ciphertext of the chunk) instead of a side output
+      // batches keep the inner product's kernel lean: u[L-1] = acc[L-1] * P^-1 + d[L-1] -> slot E is two small element-wise
+      // launches per chunk (one per component, every ciphertext of the chunk) instead of a side output.  With the tensor
+      // product in the inner product (mu->add null) acc[L-1] already holds the d term.
       for (int c = 0; c < 2; ++c) {
         SubMulArgs u{};
         u.x = acc + ((size_t)c * AL + (L - 1)) * N; u.x_poly_stride = 2ll * AL * N;
         u.y = nullptr;
-        u.z = mu->add + c * mu->comp_stride + (size_t)(L - 1) * N; u.z_poly_stride = mu->batch_stride;
+        u.z = mu->add ? mu->add + c * mu->comp_stride + (size_t)(L - 1) * N : nullptr; u.z_poly_stride = mu->batch_stride;
         u.out = acc + ((size_t)c * AL + E) * N; u.out_poly_stride = 2ll * AL * N;
         u.cst = lc->pinv + (L - 1); u.N = N; u.n_limbs = 1; u.n_polys = nb; u.x_packed = u.z_packed = 1;
         launch_sub_mul_add(ctx->mc, lc->last_lm, u, s);
@@ -825,7 +863,8 @@ static int ks_inner(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, Batc
 // Two-pass rings with at least two digits fuse the inner product into the ModUp transform (NttMac): the Q-limb accumulators are
 // then 8-byte words (not packed limbs); ks_uses_hpip() tells the consumers.
 static int ks_front(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, BatchPtr d, const KeyDesc &key, u64 *yb,
-                    u64 *ext, u64 *acc, uint32_t AL, cudaStream_t s, const MergedU *mu = nullptr, const KsAuto *au = nullptr) {
+                    u64 *ext, u64 *acc, uint32_t AL, cudaStream_t s, const MergedU *mu = nullptr, const KsAuto *au = nullptr,
+                    const KsTensor *ten = nullptr) {
   const Params &p = ctx->p;
   const size_t N = p.N;
   const uint32_t A = p.alpha, E = L + A;
@@ -844,9 +883,9 @@ static int ks_front(hml_ctx *ctx, LevelConsts *lc, uint32_t L, uint32_t nb, Batc
       ctx->exec.ewe_limbs += 4ull * nb;
     }
   }
-  int rc = ks_modup(ctx, lc, L, nb, d_raw, yb, ext, s, hpip ? &mac : nullptr, au);
+  int rc = ks_modup(ctx, lc, L, nb, d_raw, yb, ext, s, hpip ? &mac : nullptr, au, ten);
   if (rc) return rc;
-  return ks_inner(ctx, lc, L, nb, d, key, ext, acc, AL, 0, s, mu, hpip);
+  return ks_inner(ctx, lc, L, nb, d, key, ext, acc, AL, 0, s, mu, hpip, ten);
 }
 
 // The addends of a ModDown epilogue: component 0 reads z0, component 1 reads z1 (either may be null)
@@ -1637,9 +1676,14 @@ int hmult_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct_a, const u64 
   // d0 | d1 | d2 each [nb][L][N], cb [nb][2][L][N], then the key-switch / rescale workspace
   u64 *d0 = ws, *d1 = d0 + nb * PL, *d2 = d1 + nb * PL;
   const int merged = p.logN > NTT_SMALL_LOG;  // d0 / d1 then only feed element-wise epilogues: stored packed
-  launch_tensor3(ctx->mc, (int)N, (int)L, ct_a, ct_a + PL, ct_b, ct_b + PL, d0, d1, d2, (int)nb, (long long)(2 * PL), (long long)PL, s, merged);  // reference :592-739
-  prof_mark(ctx, HML_CLS_EWE, s);
-  ctx->exec.ewe_limbs += 3ull * nb * L; ctx->exec.kernel_launches++;
+  // batches on two-pass rings form the tensor product (reference :592-739) inside the key switch (KsTensor): d2 on the ModUp
+  // transform's load, d0 / d1 folded into the accumulators by the inner product, so neither is stored nor read back
+  const bool in_ks = merged && nb > 1;
+  if (!in_ks) {
+    launch_tensor3(ctx->mc, (int)N, (int)L, ct_a, ct_a + PL, ct_b, ct_b + PL, d0, d1, d2, (int)nb, (long long)(2 * PL), (long long)PL, s, merged);
+    prof_mark(ctx, HML_CLS_EWE, s);
+    ctx->exec.ewe_limbs += 3ull * nb * L; ctx->exec.kernel_launches++;
+  }
   if (!merged) {  // single-pass rings: the textbook sequence
     u64 *cb = d2 + nb * PL, *rest = cb + 2 * nb * PL;
     int rc = ks_run(ctx, L, nb, {d2, (long long)PL}, evk, evk_q_limbs, {cb, (long long)(2 * PL)}, {cb + PL, (long long)(2 * PL)}, {d0, (long long)PL},
@@ -1657,25 +1701,27 @@ int hmult_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct_a, const u64 
   u64 *yb = d2 + nb * PL, *ext = yb + (size_t)nb * L * N, *acc = ext + (size_t)nb * beta * E * N, *wb = acc + (size_t)nb * 2 * AL * N;
   // u[L-1] = d_c[L-1] + acc_c[L-1] * P^-1 is produced by the inner product itself (slot E of each accumulator) and its INTT
   // (reference Rescale INTT :766-805) rides in the launch that transforms the P-limbs: no extra launches, no re-reads
-  const MergedU mu{d0, (long long)(d1 - d0), (long long)PL};
-  if ((rc = ks_front(ctx, lc, L, nb, {d2, (long long)PL}, key, yb, ext, acc, AL, s, &mu))) return rc;
+  const MergedU mu{in_ks ? nullptr : d0, (long long)(d1 - d0), (long long)PL};
+  const KsTensor ten{ct_a, ct_b, (long long)PL, (long long)(2 * PL)};
+  if ((rc = ks_front(ctx, lc, L, nb, {d2, (long long)PL}, key, yb, ext, acc, AL, s, &mu, nullptr, in_ks ? &ten : nullptr))) return rc;
   {  // w_l = v_l * P^-1 + [r]_{q_l}, l < L-1, with r = slot_E - v[L-1] * P^-1 folded on the staged tile (reference K8 :489-519)
     BConvArgs a{};
     a.in = acc; a.in_batch_stride = (long long)AL * N; a.out = wb; a.out_batch_stride = (long long)(L - 1) * N;
     a.step1 = nullptr; a.N = N; a.n_batches = 2 * nb; a.fold = lc->merged_fold; a.fold_mod = (int)(L - 1); a.out_f64 = 1;
     run_bconv(ctx, lc->merged_rest, lc->merged_src, a, s);
   }
-  {  // out[l] = ((acc[l] * P^-1 + d[l]) - NTT_l(w_l)) * q_{L-1}^-1  (K9, K10, HMULT add and Rescale in one transform)
+  {  // out[l] = ((acc[l] * P^-1 + d[l]) - NTT_l(w_l)) * q_{L-1}^-1  (K9, K10, HMULT add and Rescale in one transform); with the
+     // tensor product in the key switch acc[l] * P^-1 already holds d[l]
     NttLaunch l{};
     l.in = wb; l.out = wb; l.in_limb_stride = l.out_limb_stride = N; l.in_poly_stride = l.out_poly_stride = (long long)(L - 1) * N;
     l.n_limbs = L - 1; l.n_polys = 2 * nb; l.n_batch = 1; l.in_f64 = 1;
     NttFuse &f = l.fuse;
     f.x = acc; f.x_c_stride = (long long)AL * N; f.x_b_stride = 2ll * AL * N;
-    f.z = d0; f.z_c_stride = (long long)(d1 - d0); f.z_b_stride = (long long)PL; f.z_mask = 3;
+    if (!in_ks) { f.z = d0; f.z_c_stride = (long long)(d1 - d0); f.z_b_stride = (long long)PL; f.z_mask = 3; }
     f.dst = ct_out; f.dst_c_stride = (long long)(L - 1) * N; f.dst_b_stride = 2ll * (L - 1) * N;
     f.cst = lc->pinv; f.cst2 = lc->qlinv; f.n_c = 2; f.x_packed = ks_uses_hpip(ctx, L, nb) ? 0 : 1; f.z_packed = 1;
     run_ntt(ctx, false, lc->q_lm, l, s);
-    ctx->exec.ewe_limbs += 2ull * nb * 4 * (L - 1);
+    ctx->exec.ewe_limbs += 2ull * nb * 4 * (L - 1);  // (+ d: with the tensor product in the key switch, the inner product's fold)
   }
   return check_launch(ctx, "hmult");
 }

@@ -43,6 +43,7 @@ struct LevelConsts {
   double2 pinv_last{};                       // P^-1 mod q_{L-1} (host copy, kernel parameter of the inner product)
   HostBConv down;
   double2 *pinv = nullptr;                   // [L]
+  double2 *pmod = nullptr;                   // [L]: P mod q_i (the batched hmult's tensor fold, InnerArgs::tensor_pmod)
   // Rescale: q_{L-1}^-1 mod q_l
   double2 *qlinv = nullptr;                  // [L-1]
   // hmult only (L >= 2): ModDown merged with Rescale by linearity of the NTT (context.cu, hmult_run).  Sources = the alpha

@@ -188,8 +188,9 @@ static void with_max_beta(int beta, F &&f) {
 }
 
 // MULTI: more than one ciphertext per launch (the next ciphertext's digits are prefetched while this one is multiplied)
-template <int IP_MAX_BETA, bool MULTI>
-__global__ void __launch_bounds__(EW_THREADS, 3) k_inner(const ModConst *__restrict__ mc, LimbMap lm, InnerArgs a) {
+// TENSOR (MULTI only, Q-limbs only): the tensor product (InnerArgs::ct_a); a1 travels as the own digit, a0, b0, b1 beside it
+template <int IP_MAX_BETA, bool MULTI, bool TENSOR>
+__global__ void __launch_bounds__(EW_THREADS, TENSOR ? 2 : 3) k_inner(const ModConst *__restrict__ mc, LimbMap lm, InnerArgs a) {
   pdl_wait();
   const int i2 = blockIdx.x * EW_THREADS + threadIdx.x;
   if (i2 >= a.N / 2) return;
@@ -197,12 +198,20 @@ __global__ void __launch_bounds__(EW_THREADS, 3) k_inner(const ModConst *__restr
   const ModConst m = mc[lm.mod[e]];
   const int kl = lm.pos[e], own = lm.skip[e];
   const size_t n2 = a.N / 2;
+  constexpr bool tq = TENSOR;
   // all loads of the first ciphertext (digits + key words) are issued together; afterwards the next ciphertext's
   // digits are in flight while the current one is multiplied
   auto digit_ptr = [&](int b, int j) {
+    if (tq && j == own) return a.ct_a + (size_t)b * a.ct_batch_stride + a.ct_comp_stride + (size_t)e * a.N;  // a1
     return j == own ? a.d + (size_t)b * a.d_batch_stride + (size_t)e * a.N
                     : a.ext + (size_t)b * a.ext_batch_stride + ((size_t)j * a.n_ext + e) * a.N;
   };
+  ulonglong2 xn[3];  // TENSOR: a0, b0, b1 of the ciphertext the digits in flight belong to
+  auto ld_tensor = [&](int b) {
+    const size_t o = (size_t)b * a.ct_batch_stride + (size_t)e * a.N;
+    xn[0] = ld2(a.ct_a + o, i2); xn[1] = ld2(a.ct_b + o, i2); xn[2] = ld2(a.ct_b + o + a.ct_comp_stride, i2);
+  };
+  if constexpr (tq) ld_tensor(0);
   const bool gal = !MULTI && a.galois != 0;  // the batched variant stays lean: no automorphism on load, no u side output
   const uint2 src = gal_slots(gal ? a.galois : 0u, a.logN, i2);
   auto ld_digit = [&](int b, int j) -> ulonglong2 {
@@ -244,23 +253,40 @@ __global__ void __launch_bounds__(EW_THREADS, 3) k_inner(const ModConst *__restr
     for (int c = 0; c < 2; ++c) {
       k[j][c][0] = u64_to_f64(kraw[j][c].x); k[j][c][1] = u64_to_f64(kraw[j][c].y);
     }
+  const double2 pm = tq ? a.tensor_pmod[e] : make_double2(0.0, 0.0);  // P mod q_e
   for (int b = 0; b < a.n_batch; ++b) {
     u64 *acc = a.acc + (size_t)b * a.acc_batch_stride;
     ulonglong2 t[IP_MAX_BETA];
 #pragma unroll
     for (int j = 0; j < IP_MAX_BETA; ++j) t[j] = tn[j];
+    double s00 = 0, s01 = 0, s10 = 0, s11 = 0;  // [component][coefficient]
+    double o0 = 0, o1 = 0;                      // TENSOR: the own-digit term d2 = a1 * b1
+    if constexpr (tq) {  // d2, and the accumulators start at d0 * P, d1 * P (before the next loads: xn is refilled below)
+      ulonglong2 a1 = t[0];
+#pragma unroll
+      for (int j = 1; j < IP_MAX_BETA; ++j)
+        if (j == own) a1 = t[j];
+      const double a0x = u64_to_f64(xn[0].x), a0y = u64_to_f64(xn[0].y), a1x = u64_to_f64(a1.x), a1y = u64_to_f64(a1.y);
+      const double b0x = u64_to_f64(xn[1].x), b0y = u64_to_f64(xn[1].y), b1x = u64_to_f64(xn[2].x), b1y = u64_to_f64(xn[2].y);
+      o0 = mulmod_var(a1x, b1x, m.q, m.qinv);
+      o1 = mulmod_var(a1y, b1y, m.q, m.qinv);
+      s00 = mulmod_const(mulmod_var(a0x, b0x, m.q, m.qinv), pm.x, pm.y, m.q);
+      s01 = mulmod_const(mulmod_var(a0y, b0y, m.q, m.qinv), pm.x, pm.y, m.q);
+      s10 = mulmod_const(mulmod_var(a0x, b1x, m.q, m.qinv) + mulmod_var(a1x, b0x, m.q, m.qinv), pm.x, pm.y, m.q);
+      s11 = mulmod_const(mulmod_var(a0y, b1y, m.q, m.qinv) + mulmod_var(a1y, b0y, m.q, m.qinv), pm.x, pm.y, m.q);
+    }
     if (MULTI && b + 1 < a.n_batch) {
 #pragma unroll
       for (int j = 0; j < IP_MAX_BETA; ++j)
         if (j < a.beta) tn[j] = ld_digit(b + 1, j);
+      if constexpr (tq) ld_tensor(b + 1);
     }
-    double s00 = 0, s01 = 0, s10 = 0, s11 = 0;  // [component][coefficient]
 #pragma unroll
     for (int j = 0; j < IP_MAX_BETA; ++j)
       if (j < a.beta) {
-        const bool f64 = a.ext_f64 && j != own;
-        const double t0 = f64 ? __longlong_as_double((long long)t[j].x) : u64_to_f64(t[j].x);
-        const double t1 = f64 ? __longlong_as_double((long long)t[j].y) : u64_to_f64(t[j].y);
+        const bool f64 = a.ext_f64 && j != own, sq = tq && j == own;
+        const double t0 = sq ? o0 : f64 ? __longlong_as_double((long long)t[j].x) : u64_to_f64(t[j].x);
+        const double t1 = sq ? o1 : f64 ? __longlong_as_double((long long)t[j].y) : u64_to_f64(t[j].y);
         s00 += mulmod_var(t0, k[j][0][0], m.q, m.qinv);
         s01 += mulmod_var(t1, k[j][0][1], m.q, m.qinv);
         s10 += mulmod_var(t0, k[j][1][0], m.q, m.qinv);
@@ -287,11 +313,13 @@ __global__ void __launch_bounds__(EW_THREADS, 3) k_inner(const ModConst *__restr
   }
 }
 
-void launch_inner_product(const ModConst *mc, const LimbMap &lm, const InnerArgs &a, cudaStream_t s) {
+void launch_inner_product(const ModConst *mc, const LimbMap &lm, const InnerArgs &a, cudaStream_t s, int n_limbs) {
+  const dim3 grid = ew_grid(a.N, n_limbs ? n_limbs : a.n_ext);
   with_max_beta(a.beta, [&](auto nb) {
     constexpr int NB = decltype(nb)::value;
-    if (a.n_batch > 1) launch_pdl(k_inner<NB, true>, ew_grid(a.N, a.n_ext), EW_THREADS, 0, s, mc, lm, a);
-    else launch_pdl(k_inner<NB, false>, ew_grid(a.N, a.n_ext), EW_THREADS, 0, s, mc, lm, a);
+    if (a.n_batch > 1 && a.ct_a) launch_pdl(k_inner<NB, true, true>, grid, EW_THREADS, 0, s, mc, lm, a);
+    else if (a.n_batch > 1) launch_pdl(k_inner<NB, true, false>, grid, EW_THREADS, 0, s, mc, lm, a);
+    else launch_pdl(k_inner<NB, false, false>, grid, EW_THREADS, 0, s, mc, lm, a);
   });
 }
 

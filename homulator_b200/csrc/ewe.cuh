@@ -51,8 +51,17 @@ struct InnerArgs {
   const u64 *u_add;
   long long u_add_comp_stride, u_add_batch_stride;
   double2 u_cst;
+  // the batched hmult's tensor product (context.cu, hmult_run), n_batch > 1 and ct_a != null: the launch covers Q-limbs
+  // only; the kernel reads the ciphertext pair instead of d and forms d0 = a0*b0, d1 = a0*b1 + a1*b0 and d2 = a1*b1
+  // itself.  d2 is the own-digit term, and the stored accumulators are acc_c + d_c * P mod q_e
+  // (tensor_pmod[e] = (P mod q_e, RN(that / q_e))), so a consumer's acc * P^-1 already holds the d_c term.
+  // a_c = ct_a + b * ct_batch_stride + c * ct_comp_stride (limb slots of N words), likewise b_c.  d is not read.
+  const u64 *ct_a, *ct_b;
+  long long ct_comp_stride, ct_batch_stride;
+  const double2 *tensor_pmod;
 };
-void launch_inner_product(const ModConst *mc, const LimbMap &lm, const InnerArgs &a, cudaStream_t s);
+// n_limbs > 0: only the extended limbs e < n_limbs of lm (grid.y = n_limbs instead of n_ext)
+void launch_inner_product(const ModConst *mc, const LimbMap &lm, const InnerArgs &a, cudaStream_t s, int n_limbs = 0);
 
 // The same inner product for up to IP_MAX_ROT hoisted rotations of one ciphertext in ONE launch (grid.z = rotation): every
 // rotation reads the same digits d / ext, through its own automorphism (as InnerArgs::galois), and multiplies them by its own

@@ -321,10 +321,13 @@ struct RowItemsB {
 };
 
 // MODE 0: plain transform; 1: fused element-wise epilogue (NttFuse); 2: fused key-switch inner product (NttMac); 3: the same
-// with a packed key
+// with a packed key; 4 (inverse only): the input multiplied by NttLaunch::in_mul on load; 5: MODE 1 with cst2 and without z
+// (the batched hmult's epilogue, whose addend is already in x)
 template <bool INV, int MODE>
 __global__ void __launch_bounds__(NTT_THREADS, 2) ntt_rows(NttTables t, int logN, LimbMap lm, NttLaunch l) {
-  constexpr bool FUSE = MODE == 1, MAC = MODE >= 2, KPK = MODE == 3;  // MODE 3: MAC with packed key limbs (NttMac::evk_packed)
+  constexpr bool FUSE = MODE == 1 || MODE == 5, MAC = MODE == 2 || MODE == 3, KPK = MODE == 3;  // MODE 3: MAC with packed key limbs (NttMac::evk_packed)
+  constexpr bool NOZ = MODE == 5;
+  constexpr bool MUL = INV && MODE == 4;
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ __align__(8) unsigned long long bar;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -362,10 +365,17 @@ __global__ void __launch_bounds__(NTT_THREADS, 2) ntt_rows(NttTables t, int logN
   if constexpr (MAC) cur = RowItem{zi, items.first_p()};
   else cur = items.next(RowItem{0, zi - zn});
   RowItem nxt = items.valid(cur) ? items.next(cur) : cur;
+  // the multiplier's share of item i (NttLaunch::in_mul), addressed like `in`
+  auto mul_of = [&](const RowItem &i) -> const u64 * {
+    return l.in_mul + (long long)i.b * l.in_batch_stride + (long long)i.p * l.in_poly_stride + slot * l.in_limb_stride + tile_off;
+  };
   // inverse rows may load through an automorphism (NttLaunch::in_galois)
   auto issue = [&](const RowItem &i, unsigned stage) {
     if constexpr (INV && MODE == 0) {
       if (l.in_galois) { row_issue_sigma(src_of(i) - tile_off, stage, lane, warp, tile_i, l.in_galois, l.in_ginv8, logN); return; }
+    }
+    if constexpr (MUL) {  // the multiplier's 4 KB for this warp's rows start their trip to L2 with the tile (one line per lane)
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(mul_of(i) + (size_t)warp * 512 + (size_t)lane * 16));
     }
     row_issue(src_of(i), stage, lane, warp);
   };
@@ -587,11 +597,11 @@ __global__ void __launch_bounds__(NTT_THREADS, 2) ntt_rows(NttTables t, int logN
         ulonglong2 xv[8];
 #pragma unroll
         for (int m = 0; m < 8; ++m) xv[m] = load_chunk(xs, f.x_packed, m);
-        if (f.cst2 != nullptr) {  // ((x * c + z) - y) * c2: z is mandatory
+        if (f.cst2 != nullptr) {  // ((x * c + z) - y) * c2: z is mandatory, except in MODE 5
           const double2 cst2 = f.cst2[limb];
           ulonglong2 zv[8];
 #pragma unroll
-          for (int m = 0; m < 8; ++m) zv[m] = load_chunk(zs, f.z_packed, m);
+          for (int m = 0; m < 8; ++m) zv[m] = NOZ ? make_ulonglong2(0, 0) : load_chunk(zs, f.z_packed, m);
 #pragma unroll
           for (int m = 0; m < 8; ++m) {
             const double2 y = *reinterpret_cast<const double2 *>(data + ad.C(m));
@@ -642,10 +652,30 @@ __global__ void __launch_bounds__(NTT_THREADS, 2) ntt_rows(NttTables t, int logN
 #pragma unroll
         for (int m = 0; m < 8; ++m) *reinterpret_cast<ulonglong2 *>(so + 32 * m) = *reinterpret_cast<const ulonglong2 *>(data + ad.C(m));
       }
+      if constexpr (MUL) {
+        // in * in_mul on the chunks this lane would store (coalesced loads, 256 B per half-warp); the centred products
+        // (|v| <= 0.51 q) go back into the tile as doubles
+        const u64 *mp = mul_of(cur) + (size_t)rr * 256 + (l16 >> 3) * 16 + (l16 & 7) * 2;
+        ulonglong2 mv[8];
+#pragma unroll
+        for (int m = 0; m < 8; ++m) mv[m] = __ldg(reinterpret_cast<const ulonglong2 *>(mp + 32 * m));
+#pragma unroll
+        for (int m = 0; m < 8; ++m) {
+          const ulonglong2 v = *reinterpret_cast<const ulonglong2 *>(data + ad.C(m));
+          *reinterpret_cast<double2 *>(data + ad.C(m)) = make_double2(mulmod_var(u64_to_f64(v.x), u64_to_f64(mv[m].x), q, qinv),
+                                                                      mulmod_var(u64_to_f64(v.y), u64_to_f64(mv[m].y), q, qinv));
+        }
+        __syncwarp();
+      }
 #pragma unroll
       for (int m = 0; m < 8; ++m) {
-        const ulonglong2 v = *reinterpret_cast<const ulonglong2 *>(data + ad.B(m));
-        a[2 * m] = u64_to_f64(v.x); a[2 * m + 1] = u64_to_f64(v.y);
+        if constexpr (MUL) {
+          const double2 v = *reinterpret_cast<const double2 *>(data + ad.B(m));
+          a[2 * m] = v.x; a[2 * m + 1] = v.y;
+        } else {
+          const ulonglong2 v = *reinterpret_cast<const ulonglong2 *>(data + ad.B(m));
+          a[2 * m] = u64_to_f64(v.x); a[2 * m + 1] = u64_to_f64(v.y);
+        }
       }
 #pragma unroll
       for (int m = 0; m < 4; ++m) {
@@ -831,9 +861,11 @@ static void launch_rows(bool inverse, const NttTables &t, int logN, const LimbMa
   if (once.first()) {
     allow_smem(ntt_rows<false, 0>, ROW_SMEM_BYTES);
     allow_smem(ntt_rows<false, 1>, ROW_SMEM_BYTES);
+    allow_smem(ntt_rows<false, 5>, ROW_SMEM_BYTES);
     allow_smem(ntt_rows<false, 2>, ROW_SMEM_BYTES);
     allow_smem(ntt_rows<false, 3>, ROW_SMEM_BYTES);
     allow_smem(ntt_rows<true, 0>, ROW_SMEM_BYTES);
+    allow_smem(ntt_rows<true, 4>, ROW_SMEM_BYTES);
   }
   const int tiles = 1 << (logN - NTT_ROW_LOG - 4);
   if (!inverse && l.mac.evk) {  // the grid splits the ciphertexts; every CTA walks all digits of its (ciphertext, limb, tile)
@@ -845,7 +877,9 @@ static void launch_rows(bool inverse, const NttTables &t, int logN, const LimbMa
     return;
   }
   const dim3 grid(tiles * row_split(l.n_polys * l.n_batch, tiles * l.n_limbs), l.n_limbs);
-  if (inverse) launch_pdl(ntt_rows<true, 0>, grid, NTT_THREADS, ROW_SMEM_BYTES, s, t, logN, lm, l);
+  if (inverse && l.in_mul) launch_pdl(ntt_rows<true, 4>, grid, NTT_THREADS, ROW_SMEM_BYTES, s, t, logN, lm, l);
+  else if (inverse) launch_pdl(ntt_rows<true, 0>, grid, NTT_THREADS, ROW_SMEM_BYTES, s, t, logN, lm, l);
+  else if (l.fuse.x && l.fuse.cst2 && !l.fuse.z) launch_pdl(ntt_rows<false, 5>, grid, NTT_THREADS, ROW_SMEM_BYTES, s, t, logN, lm, l);
   else if (l.fuse.x) launch_pdl(ntt_rows<false, 1>, grid, NTT_THREADS, ROW_SMEM_BYTES, s, t, logN, lm, l);
   else launch_pdl(ntt_rows<false, 0>, grid, NTT_THREADS, ROW_SMEM_BYTES, s, t, logN, lm, l);
 }

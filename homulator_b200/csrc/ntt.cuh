@@ -123,6 +123,9 @@ struct NttLaunch {
   int in_f64;                 // forward only, two-pass rings: `in` holds signed doubles |v| <= q (BConvArgs::out_f64)
   int out_f64;                // forward only, two-pass rings, no fused epilogue: leave the raw lazy sums (|v| < 10 q) as doubles
                               // in `out` instead of canonical words (consumer: InnerArgs::ext_f64)
+  // inverse only, two-pass rings, n_polys == 1, no in_galois: the row pass transforms in * in_mul mod q (canonical words,
+  // same limb and batch strides as `in`) — the batched hmult squares its ciphertexts' c1 (d2 = a1 * b1) on load.  null: off.
+  const u64 *in_mul;
 };
 
 void launch_ntt_forward(const NttTables &t, int logN, const LimbMap &lm, const NttLaunch &l, cudaStream_t s);
