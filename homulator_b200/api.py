@@ -70,7 +70,7 @@ EXPORTS = [
     "hml_hrotate_sharded", "hml_hmult_sharded", "hml_rescale_sharded", "hml_ew_sharded", "hml_group_op", "hml_hrotate_hoisted",
     "hml_replay_create", "hml_replay_bind", "hml_replay_run", "hml_replay_slot", "hml_replay_slot_level", "hml_replay_destroy",
     "hml_shard_create_ex", "hml_hrotate_hoisted_sharded", "hml_group_hrotate_hoisted", "hml_hrotate_sum_hoisted",
-    "hml_hrotate_bsgs_hoisted",
+    "hml_hrotate_bsgs_hoisted", "hml_hmult_sum",
 ]
 
 
@@ -116,6 +116,7 @@ def load_library():
         getattr(L, f).argtypes = [vp, u32, vp, vp, vp, vp]
     L.hml_pmult_add.argtypes = [vp, u32, vp, vp, vp, vp, vp]
     L.hml_hmult_batch.argtypes = [vp, u32, u32, vp, vp, vp, u32, vp, vp]
+    L.hml_hmult_sum.argtypes = [vp, u32, u32, C.POINTER(vp), C.POINTER(vp), u32, vp, u32, vp, vp]
     L.hml_hrotate_batch.argtypes = [vp, u32, u32, vp, vp, u32, u64, vp, vp]
     L.hml_hmult_host.argtypes = [vp, u32, u32, vp, vp, vp, u32, vp]
     L.hml_hrotate_host.argtypes = [vp, u32, u32, vp, vp, u32, u64, vp]
@@ -449,6 +450,24 @@ class Context:
         self._chk(self.lib.hml_hmult_batch(self.h, L, n, _ptr(ct_a), _ptr(ct_b), _ptr(evk), evk_q_limbs or L, _ptr(out), self._stream()))
         return out
 
+    def hmult_sum(self, L, cts_a, cts_b, evk, evk_q_limbs=None, out=None):
+        """sum_i cts_a[i] * cts_b[i] with one key switch and one rescale per output (hml_hmult_sum).  cts_a / cts_b are equally long
+        lists of [2][L][N] tensors (one output, [2][L-1][N]) or of [n_out][2][L][N] tensors (n_out outputs, [n_out][2][L-1][N]);
+        passing the same tensor as cts_a[i] and cts_b[i] squares it and reads it once."""
+        n = len(cts_a)
+        if len(cts_b) != n or n == 0:
+            raise ValueError("cts_a and cts_b must be equally long and not empty")
+        shape = tuple(cts_a[0].shape)
+        if len(shape) not in (3, 4) or any(tuple(t.shape) != shape for t in list(cts_a) + list(cts_b)):
+            raise ValueError("every term must have the shape [2][L][N] or the same [n_out][2][L][N]")
+        n_out = shape[0] if len(shape) == 4 else 1
+        if out is None:
+            out = self.empty(*shape[:-3], 2, L - 1, self.N)
+        pa = (C.c_void_p * n)(*[_ptr(t) for t in cts_a])
+        pb = (C.c_void_p * n)(*[_ptr(t) for t in cts_b])
+        self._chk(self.lib.hml_hmult_sum(self.h, L, n, pa, pb, n_out, _ptr(evk), evk_q_limbs or L, _ptr(out), self._stream()))
+        return out
+
     def hrotate_batch(self, L, ct, rotkey, galois_elt=5, evk_q_limbs=None, out=None):
         n = ct.shape[0]
         out = self.empty(n, 2, L, self.N) if out is None else out
@@ -737,10 +756,11 @@ class Replay:
     graph, optionally with hoisted rotations, optionally limb-sharded).  `trace` uses the tuple format of
     homulator_b200.replay; names are mapped to slots here ("x" = slot 0 = the input).  hoist_sum=True turns a hoistable run of
     rotations whose outputs are summed with plaintext weights into one double-hoisted sum (HML_REPLAY_HOIST_SUM); the
-    plaintexts are then bound as [L + alpha][N] (P-limbs at rows L..)."""
+    plaintexts are then bound as [L + alpha][N] (P-limbs at rows L..).  hmult_sum=True turns a chain of products summed as they
+    are formed into one lazily relinearised sum (HML_REPLAY_HMULT_SUM, hml_hmult_sum)."""
     KINDS = {"hrotate": 0, "pmult": 1, "hadd": 2, "padd": 3, "hmult": 4}
 
-    def __init__(self, ctx, L, trace, shard=None, graph=False, hoist=False, hoist_sum=False):
+    def __init__(self, ctx, L, trace, shard=None, graph=False, hoist=False, hoist_sum=False, hmult_sum=False):
         self.ctx, self.L, self.shard = ctx, L, shard
         self.names = {"x": 0}
         ops = []
@@ -759,7 +779,7 @@ class Replay:
             ops.append((self.KINDS[kind], self.names[dst], self.names[a], bb))
         arr = (_TraceOp * len(ops))(*[_TraceOp(*o) for o in ops])
         self.h = C.c_void_p()
-        flags = (1 if graph else 0) | (2 if hoist else 0) | (4 if hoist_sum else 0)
+        flags = (1 if graph else 0) | (2 if hoist else 0) | (4 if hoist_sum else 0) | (8 if hmult_sum else 0)
         ctx._chk(ctx.lib.hml_replay_create(ctx.h, shard.h if shard is not None else None, L, arr, len(ops), flags, C.byref(self.h)))
         self._keep = None
 

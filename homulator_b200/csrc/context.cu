@@ -1669,21 +1669,17 @@ size_t hmult_ws_words(const Params &p, uint32_t L, uint32_t nb) {
 // straight out of the base conversion: P^-1 is folded into the matrix on the host, r is computed by the conversion kernel on
 // its staged tile (a 15-term dot product per coefficient) and rides in the otherwise padded 16th source row with matrix
 // entry 1 (exact: it only adds one term < 2^36 to the 16-term sums).
-int hmult_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct_a, const u64 *ct_b, const u64 *evk, uint32_t evk_q_limbs,
-                     u64 *ct_out, u64 *ws, cudaStream_t s) {
+//
+// Everything after the tensor product: ten == null reads d0 | d1 | d2 from the workspace (each [nb][L][N]; d0 / d1 packed limbs
+// on two-pass rings), ten != null (two-pass rings only) forms the tensor product inside the key switch.
+static int hmult_tail(hml_ctx *ctx, uint32_t L, uint32_t nb, const KsTensor *ten, const u64 *evk, uint32_t evk_q_limbs, u64 *ct_out,
+                      u64 *ws, cudaStream_t s) {
   const Params &p = ctx->p;
   const size_t N = p.N, PL = N * L;
   // d0 | d1 | d2 each [nb][L][N], cb [nb][2][L][N], then the key-switch / rescale workspace
   u64 *d0 = ws, *d1 = d0 + nb * PL, *d2 = d1 + nb * PL;
-  const int merged = p.logN > NTT_SMALL_LOG;  // d0 / d1 then only feed element-wise epilogues: stored packed
-  // batches on two-pass rings form the tensor product (reference :592-739) inside the key switch (KsTensor): d2 on the ModUp
-  // transform's load, d0 / d1 folded into the accumulators by the inner product, so neither is stored nor read back
-  const bool in_ks = merged && nb > 1;
-  if (!in_ks) {
-    launch_tensor3(ctx->mc, (int)N, (int)L, ct_a, ct_a + PL, ct_b, ct_b + PL, d0, d1, d2, (int)nb, (long long)(2 * PL), (long long)PL, s, merged);
-    prof_mark(ctx, HML_CLS_EWE, s);
-    ctx->exec.ewe_limbs += 3ull * nb * L; ctx->exec.kernel_launches++;
-  }
+  const int merged = p.logN > NTT_SMALL_LOG;
+  const bool in_ks = ten != nullptr;
   if (!merged) {  // single-pass rings: the textbook sequence
     u64 *cb = d2 + nb * PL, *rest = cb + 2 * nb * PL;
     int rc = ks_run(ctx, L, nb, {d2, (long long)PL}, evk, evk_q_limbs, {cb, (long long)(2 * PL)}, {cb + PL, (long long)(2 * PL)}, {d0, (long long)PL},
@@ -1702,8 +1698,7 @@ int hmult_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct_a, const u64 
   // u[L-1] = d_c[L-1] + acc_c[L-1] * P^-1 is produced by the inner product itself (slot E of each accumulator) and its INTT
   // (reference Rescale INTT :766-805) rides in the launch that transforms the P-limbs: no extra launches, no re-reads
   const MergedU mu{in_ks ? nullptr : d0, (long long)(d1 - d0), (long long)PL};
-  const KsTensor ten{ct_a, ct_b, (long long)PL, (long long)(2 * PL)};
-  if ((rc = ks_front(ctx, lc, L, nb, {d2, (long long)PL}, key, yb, ext, acc, AL, s, &mu, nullptr, in_ks ? &ten : nullptr))) return rc;
+  if ((rc = ks_front(ctx, lc, L, nb, {d2, (long long)PL}, key, yb, ext, acc, AL, s, &mu, nullptr, ten))) return rc;
   {  // w_l = v_l * P^-1 + [r]_{q_l}, l < L-1, with r = slot_E - v[L-1] * P^-1 folded on the staged tile (reference K8 :489-519)
     BConvArgs a{};
     a.in = acc; a.in_batch_stride = (long long)AL * N; a.out = wb; a.out_batch_stride = (long long)(L - 1) * N;
@@ -1724,6 +1719,49 @@ int hmult_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct_a, const u64 
     ctx->exec.ewe_limbs += 2ull * nb * 4 * (L - 1);  // (+ d: with the tensor product in the key switch, the inner product's fold)
   }
   return check_launch(ctx, "hmult");
+}
+
+int hmult_run(hml_ctx *ctx, uint32_t L, uint32_t nb, const u64 *ct_a, const u64 *ct_b, const u64 *evk, uint32_t evk_q_limbs,
+                     u64 *ct_out, u64 *ws, cudaStream_t s) {
+  const Params &p = ctx->p;
+  const size_t N = p.N, PL = N * L;
+  const int merged = p.logN > NTT_SMALL_LOG;  // d0 / d1 then only feed element-wise epilogues: stored packed
+  // batches on two-pass rings form the tensor product (reference :592-739) inside the key switch (KsTensor): d2 on the ModUp
+  // transform's load, d0 / d1 folded into the accumulators by the inner product, so neither is stored nor read back
+  const KsTensor ten{ct_a, ct_b, (long long)PL, (long long)(2 * PL)};
+  const bool in_ks = merged && nb > 1;
+  if (!in_ks) {
+    u64 *d0 = ws, *d1 = d0 + nb * PL, *d2 = d1 + nb * PL;
+    launch_tensor3(ctx->mc, (int)N, (int)L, ct_a, ct_a + PL, ct_b, ct_b + PL, d0, d1, d2, (int)nb, (long long)(2 * PL), (long long)PL, s, merged);
+    prof_mark(ctx, HML_CLS_EWE, s);
+    ctx->exec.ewe_limbs += 3ull * nb * L; ctx->exec.kernel_launches++;
+  }
+  return hmult_tail(ctx, L, nb, in_ks ? &ten : nullptr, evk, evk_q_limbs, ct_out, ws, s);
+}
+
+// Lazy relinearisation: out[b] = Rescale(Relin(sum_k a_k[b] (x) b_k[b])) for the nb outputs of a chunk, with ONE key switch and
+// ONE rescale per output.  The tensor products are summed over Q (k_tensor_sum, one launch per group of IP_MAX_ROT pairs, later
+// groups adding to the stored sums) into hmult_tail's d0 | d1 | d2, which then runs unchanged on them.  n_terms = 1 is
+// hmult_run bit for bit; for n_terms >= 2 the result is not the sum of the products' hmults bit for bit (the approximate ModUp
+// conversion and the rescale's lift are not additive) and the oracle defines the op (tests/orc_hmult_sum.py).  Input pointers
+// advance by `off` words (the chunk's first output).
+static int hmult_sum_run(hml_ctx *ctx, uint32_t L, uint32_t nb, uint32_t n_terms, const uint64_t *const *cts_a, const uint64_t *const *cts_b,
+                         size_t off, const u64 *evk, uint32_t evk_q_limbs, u64 *ct_out, u64 *ws, cudaStream_t s) {
+  const Params &p = ctx->p;
+  const size_t N = p.N, PL = N * L;
+  TensorSumArgs a{};
+  a.d0 = ws; a.d1 = a.d0 + nb * PL; a.d2 = a.d1 + nb * PL;
+  a.comp_stride = (long long)PL; a.in_stride = (long long)(2 * PL); a.out_stride = (long long)PL;
+  a.N = (int)N; a.pack01 = p.logN > NTT_SMALL_LOG;
+  for (uint32_t k0 = 0; k0 < n_terms; k0 += IP_MAX_ROT) {
+    const uint32_t n = std::min<uint32_t>(IP_MAX_ROT, n_terms - k0);
+    a.accumulate = k0 > 0; a.n_pairs = (int)n;
+    for (uint32_t k = 0; k < n; ++k) { a.a[k] = (const u64 *)cts_a[k0 + k] + off; a.b[k] = (const u64 *)cts_b[k0 + k] + off; }
+    launch_tensor_sum(ctx->mc, (int)L, (int)nb, a, s);
+    prof_mark(ctx, HML_CLS_EWE, s);
+    ctx->exec.ewe_limbs += 3ull * n * nb * L; ctx->exec.kernel_launches++;
+  }
+  return hmult_tail(ctx, L, nb, nullptr, evk, evk_q_limbs, ct_out, ws, s);
 }
 
 extern "C" int hml_hmult(hml_ctx *ctx, uint32_t L, const uint64_t *ct_a, const uint64_t *ct_b, const uint64_t *evk,
@@ -2081,6 +2119,28 @@ extern "C" int hml_hmult_batch(hml_ctx *ctx, uint32_t L, uint32_t n, const uint6
   return run_batch_chunks(ctx, n, hmult_ws_words(ctx->p, L, 1), (cudaStream_t)stream, [&](uint32_t i, uint32_t nb, u64 *ws, cudaStream_t s) {
     return hmult_run(ctx, L, nb, (const u64 *)ct_a + i * in_w, (const u64 *)ct_b + i * in_w, (const u64 *)evk, evk_q_limbs,
                      (u64 *)ct_out + i * out_w, ws, s);
+  });
+}
+
+extern "C" int hml_hmult_sum(hml_ctx *ctx, uint32_t L, uint32_t n_terms, const uint64_t *const *cts_a, const uint64_t *const *cts_b,
+                             uint32_t n_out, const uint64_t *evk, uint32_t evk_q_limbs, uint64_t *ct_out, void *stream) {
+  int rc = check_level(ctx, L, 2);
+  if (rc) return rc;
+  if (n_out == 0) return HML_OK;  // an empty batch is a no-op whatever the pointers are, as for hml_hmult_batch
+  if (n_terms == 0) return fail(ctx, HML_ERR_INVALID, "n_terms must be at least 1");
+  if (!cts_a || !cts_b || !evk || !ct_out) return fail(ctx, HML_ERR_INVALID, "null buffer");
+  const size_t N = ctx->p.N, in_w = 2 * N * L, out_w = 2 * N * (L - 1);
+  const uint64_t *out_end = ct_out + n_out * out_w;
+  for (uint32_t k = 0; k < n_terms; ++k) {
+    if (!cts_a[k] || !cts_b[k]) return fail(ctx, HML_ERR_INVALID, "null ciphertext");
+    for (const uint64_t *in : {cts_a[k], cts_b[k]})
+      if (ct_out < in + n_out * in_w && in < out_end) return fail(ctx, HML_ERR_INVALID, "the output overlaps an input");
+  }
+  KeyDesc key;  // checked before anything is enqueued
+  if ((rc = key_desc(ctx, L, (const u64 *)evk, evk_q_limbs, &key))) return rc;
+  CU_TRY(ctx, cudaSetDevice(ctx->device));
+  return run_batch_chunks(ctx, n_out, hmult_ws_words(ctx->p, L, 1), (cudaStream_t)stream, [&](uint32_t i, uint32_t nb, u64 *ws, cudaStream_t s) {
+    return hmult_sum_run(ctx, L, nb, n_terms, cts_a, cts_b, i * in_w, (const u64 *)evk, evk_q_limbs, (u64 *)ct_out + i * out_w, ws, s);
   });
 }
 

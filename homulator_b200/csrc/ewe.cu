@@ -103,6 +103,56 @@ void launch_tensor3(const ModConst *mc, int N, int L, const u64 *a0, const u64 *
   launch_pdl(k_tensor3, ew_grid(N, L, n_batch), EW_THREADS, 0, s, mc, N, a0, a1, b0, b1, d0, d1, d2, in_stride, out_stride, pack01);
 }
 
+// Sum of tensor products (ewe.cuh TensorSumArgs), k_tensor3's layout with a loop over the pairs; the pair table is read in place
+// (grid constant).  The sums stay lazy doubles and each output is reduced once.  Exact: every mulmod_var product lies in
+// (-0.51q, 0.51q), so with 16 pairs d1 sums 32 products plus one stored canonical word: |v| < 17.4q < 2^41 (q < 2^36), far
+// inside reduce_signed's |v| < 2^51.
+__global__ void __launch_bounds__(EW_THREADS) k_tensor_sum(const ModConst *__restrict__ mc, const __grid_constant__ TensorSumArgs a) {
+  pdl_wait();
+  const int i2 = blockIdx.x * EW_THREADS + threadIdx.x;
+  if (i2 >= a.N / 2) return;
+  const int limb = blockIdx.y;  // limbs 0..L-1 are moduli q_0..q_{L-1}
+  const ModConst m = mc[limb];
+  const size_t o = (size_t)limb * (a.N / 2) + i2;
+  const long long bi = (long long)blockIdx.z * a.in_stride, bo = (long long)blockIdx.z * a.out_stride;
+  double s0[2] = {0, 0}, s1[2] = {0, 0}, s2[2] = {0, 0};
+  for (int k = 0; k < a.n_pairs; ++k) {
+    const u64 *pa = a.a[k] + bi, *pb = a.b[k] + bi;
+    const ulonglong2 A0 = ld2(pa, o), A1 = ld2(pa + a.comp_stride, o);
+    const bool sq = pa == pb;  // uniform: a square reads one ciphertext
+    const ulonglong2 B0 = sq ? A0 : ld2(pb, o), B1 = sq ? A1 : ld2(pb + a.comp_stride, o);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const double x0 = u64_to_f64(h ? A0.y : A0.x), x1 = u64_to_f64(h ? A1.y : A1.x);
+      const double y0 = u64_to_f64(h ? B0.y : B0.x), y1 = u64_to_f64(h ? B1.y : B1.x);
+      s0[h] += mulmod_var(x0, y0, m.q, m.qinv);
+      s1[h] += mulmod_var(x0, y1, m.q, m.qinv) + mulmod_var(x1, y0, m.q, m.qinv);
+      s2[h] += mulmod_var(x1, y1, m.q, m.qinv);
+    }
+  }
+  u64 *d0 = a.d0 + bo, *d1 = a.d1 + bo, *d2 = a.d2 + bo;
+  if (a.accumulate) {  // uniform: a later group of the same op
+    const ulonglong2 p0 = a.pack01 ? ld_packed2(d0 + (size_t)limb * a.N, a.N, i2) : ld2(d0, o);
+    const ulonglong2 p1 = a.pack01 ? ld_packed2(d1 + (size_t)limb * a.N, a.N, i2) : ld2(d1, o);
+    const ulonglong2 p2 = ld2(d2, o);
+    s0[0] += u64_to_f64(p0.x); s0[1] += u64_to_f64(p0.y);
+    s1[0] += u64_to_f64(p1.x); s1[1] += u64_to_f64(p1.y);
+    s2[0] += u64_to_f64(p2.x); s2[1] += u64_to_f64(p2.y);
+  }
+  if (a.pack01) {
+    st_packed2(d0 + (size_t)limb * a.N, a.N, i2, finish(s0[0], m), finish(s0[1], m));
+    st_packed2(d1 + (size_t)limb * a.N, a.N, i2, finish(s1[0], m), finish(s1[1], m));
+  } else {
+    st2(d0, o, finish(s0[0], m), finish(s0[1], m));
+    st2(d1, o, finish(s1[0], m), finish(s1[1], m));
+  }
+  st2(d2, o, finish(s2[0], m), finish(s2[1], m));
+}
+
+void launch_tensor_sum(const ModConst *mc, int L, int n_batch, const TensorSumArgs &a, cudaStream_t s) {
+  launch_pdl(k_tensor_sum, ew_grid(a.N, L, n_batch), EW_THREADS, 0, s, mc, a);
+}
+
 // ------------------------------------------------------------------------------------------------ key-switch inner product
 // The key words of a (limb, coefficient pair) are loaded once and reused for every ciphertext of the batch
 // (the key is 60% of the traffic of an unbatched inner product).

@@ -8,7 +8,8 @@
 // (hml_ctx) or limb-sharded over a group (hml_shard), as plain launches or as ONE captured CUDA graph,
 // and optionally with hoisted rotations: consecutive hrotate ops that read the same slot share one ModUp
 // (hml_hrotate_hoisted on one GPU, hml_hrotate_hoisted_sharded over a shard group).  On one GPU such a run whose outputs are
-// summed with plaintext weights right after it may also become one double-hoisted sum (hml_hrotate_sum_hoisted).
+// summed with plaintext weights right after it may also become one double-hoisted sum (hml_hrotate_sum_hoisted), and a chain
+// of products summed as they are formed one lazily relinearised sum (hml_hmult_sum).
 #include <algorithm>
 #include <cstring>
 #include <map>
@@ -59,6 +60,7 @@ extern "C" int hml_replay_create(hml_ctx *ctx, hml_shard *sh, uint32_t L, const 
   int rc = check_level(ctx, L, 1);
   if (rc) return rc;
   if (sh && (flags & HML_REPLAY_HOIST_SUM)) return fail(ctx, HML_ERR_UNSUPPORTED, "HML_REPLAY_HOIST_SUM has no limb-sharded op");
+  if (sh && (flags & HML_REPLAY_HMULT_SUM)) return fail(ctx, HML_ERR_UNSUPPORTED, "HML_REPLAY_HMULT_SUM has no limb-sharded op");
   hml_replay *rp = new hml_replay();
   rp->ctx = ctx; rp->sh = sh; rp->L = L; rp->flags = flags;
   rp->ops.assign(ops, ops + n_ops);
@@ -207,6 +209,35 @@ static bool match_rot_sum(const std::vector<hml_trace_op> &ops, size_t i, size_t
   return true;
 }
 
+// HML_REPLAY_HMULT_SUM: ops[i] = hmult(y, a_0, b_0) is followed by n - 1 >= 1 pairs  hmult(t, a_k, b_k); hadd(y, y, t) (or
+// hadd(y, t, y)), every product at the level of the first, y and every t neither a source of any product of the chain nor each
+// other, and every t dead afterwards.  On a match: *end = the op after the chain and srcs[k] = the sources of product k.
+static bool match_hmult_sum(const std::vector<hml_trace_op> &ops, const std::vector<uint32_t> &level, size_t i, size_t *end,
+                            std::vector<std::pair<uint32_t, uint32_t>> &srcs) {
+  const uint32_t y = ops[i].dst;
+  srcs.assign(1, {ops[i].a, ops[i].b});
+  std::vector<uint32_t> temps;
+  size_t k = i + 1;
+  for (; k + 1 < ops.size(); k += 2) {
+    const hml_trace_op &mu = ops[k], &ad = ops[k + 1];
+    if (mu.kind != HML_OP_HMULT || ad.kind != HML_OP_HADD || level[k] != level[i]) break;
+    const uint32_t t = mu.dst;
+    if (t == y || ad.dst != y || !((ad.a == y && ad.b == t) || (ad.a == t && ad.b == y))) break;
+    srcs.push_back({mu.a, mu.b});
+    temps.push_back(t);
+  }
+  if (temps.empty()) return false;
+  for (const auto &s : srcs) {
+    if (s.first == y || s.second == y) return false;
+    for (uint32_t t : temps)
+      if (s.first == t || s.second == t) return false;
+  }
+  for (uint32_t t : temps)
+    if (!dead_from(ops, k, t)) return false;
+  *end = k;
+  return true;
+}
+
 static int enqueue(hml_replay *rp, cudaStream_t s) {
   hml_ctx *ctx = rp->ctx;
   void *st = (void *)s;
@@ -278,10 +309,20 @@ static int enqueue(hml_replay *rp, cudaStream_t s) {
       case HML_OP_HADD:
         rc = rp->sh ? hml_ew_sharded(rp->sh, L, 0, a, rp->slot[o.b], dst, st) : hml_hadd(ctx, L, a, rp->slot[o.b], dst, st);
         break;
-      case HML_OP_HMULT:
+      case HML_OP_HMULT: {
+        size_t end;
+        std::vector<std::pair<uint32_t, uint32_t>> srcs;
+        if ((rp->flags & HML_REPLAY_HMULT_SUM) && match_hmult_sum(rp->ops, rp->op_level, i, &end, srcs)) {
+          std::vector<const uint64_t *> as, bs;
+          for (const auto &s : srcs) { as.push_back(rp->slot[s.first]); bs.push_back(rp->slot[s.second]); }
+          rc = hml_hmult_sum(ctx, L, (uint32_t)srcs.size(), as.data(), bs.data(), 1, rp->evk, rp->evk_q_limbs, dst, st);
+          i = end - 1;
+          break;
+        }
         rc = rp->sh ? hml_hmult_sharded(rp->sh, L, a, rp->slot[o.b], rp->evk, dst, st)
                     : hml_hmult(ctx, L, a, rp->slot[o.b], rp->evk, rp->evk_q_limbs, dst, st);
         break;
+      }
       default: rc = HML_ERR_INVALID;
     }
   }

@@ -9,7 +9,7 @@ tuples over the five operations the reference's CLI accepts (reference bench_tes
     ("padd",    dst, src, pt)       dst = src + plaintext[pt]
     ("hmult",   dst, a, b)          dst = rescale(relin(a * b))       (drops one level; final)
 Execution lives in the library (homulator_b200/csrc/replay.cu: hml_replay_*): plain launches or one captured CUDA graph,
-textbook, hoisted or (one GPU) double-hoisted rotation sums, one GPU or limb-sharded over a group.  This module only defines the synthetic traces and maps
+textbook, hoisted or (one GPU) double-hoisted rotation sums and lazily relinearised product sums, one GPU or limb-sharded over a group.  This module only defines the synthetic traces and maps
 names to slots (homulator_b200.api.Replay).
 """
 from collections import Counter
@@ -51,6 +51,18 @@ def rotsum_trace(n=16):
             t.append(("pmult", "m", "r%d" % i, i))
             t.append(("hadd", "y", "y", "m"))
     t.append(("hmult", "z", "y", "y"))
+    return t
+
+
+def dot_trace(n=16):
+    """y = sum_{i<n} x * rotate(x, i): n - 1 hoistable rotations of x, then the chain of products summed as they are formed
+    (one square x * x, n - 1 products and n - 1 hadd).  The rotation-plus-product shape of an encrypted inner product; with
+    hmult_sum=True the chain is one hml_hmult_sum."""
+    t = [("hrotate", "r%d" % i, "x", i) for i in range(1, n)]
+    t.append(("hmult", "y", "x", "x"))
+    for i in range(1, n):
+        t.append(("hmult", "m", "x", "r%d" % i))
+        t.append(("hadd", "y", "y", "m"))
     return t
 
 

@@ -335,6 +335,24 @@ int hml_pmult_add(hml_ctx *ctx, uint32_t L, const uint64_t *ct, const uint64_t *
  * ct_a, ct_b [n][2][L][N]; ct_out [n][2][L-1][N] (hmult) / [n][2][L][N] (hrotate). */
 int hml_hmult_batch(hml_ctx *ctx, uint32_t L, uint32_t n, const uint64_t *ct_a, const uint64_t *ct_b,
                     const uint64_t *evk, uint32_t evk_q_limbs, uint64_t *ct_out, void *stream);
+/* out_k = Rescale(Relin(sum_i cts_a[i][k] (x) cts_b[i][k])), k < n_out: one key switch and one rescale per output.
+ * Sums of ciphertext products (dot products, sums of squares, the inner sums of polynomial evaluation) with lazy
+ * relinearisation: for each output k, over the Q-limbs l < L,
+ *   D0 = sum_i a_i0 * b_i0,   D1 = sum_i (a_i0 * b_i1 + a_i1 * b_i0),   D2 = sum_i a_i1 * b_i1      (mod q_l)
+ *   out_k = Rescale( D0 + KS0(D2), D1 + KS1(D2) )                                                    [2][L-1][N]
+ * with the hybrid key switch and the rescale hml_hmult runs after its tensor product.  n_terms = 1 is hml_hmult (n_out = 1) and
+ * hml_hmult_batch (n_out > 1) bit for bit.  For n_terms >= 2 it is NOT sum_i hml_hmult(a_i, b_i) bit for bit (the approximate
+ * ModUp conversion of a sum differs from the sum of the conversions, and the rescale's lift is not additive) and an equally
+ * valid result, decrypting to sum_i m_ai * m_bi / q_{L-1} within the noise; the oracle defines the op (tests/orc_hmult_sum.py).
+ * cts_a / cts_b are HOST arrays of n_terms device pointers, each to [n_out][2][L][N]; a term with cts_a[i] == cts_b[i] is a
+ * square and reads its ciphertext once.  ct_out [n_out][2][L-1][N] overlaps no input.  evk as in hml_hmult (evk_q_limbs in
+ * [L, maxLevel], optionally | HML_KEY_PACKED).  n_out = 0 is a no-op.  HML_ERR_INVALID: L < 2, n_terms = 0, a null array,
+ * entry, key or output, ct_out overlapping an input, evk_q_limbs out of range; HML_ERR_UNSUPPORTED: more than 8 digits.
+ * Executed counts: the transforms and conversions of hml_hmult (n_out = 1) or hml_hmult_batch (n_out > 1) whatever n_terms;
+ * ewe_limbs += 3L per term and output, and one kernel launch per group of 16 terms and chunk of outputs.  After the workspace
+ * exists the call neither allocates nor synchronises (it can be captured in a CUDA graph). */
+int hml_hmult_sum(hml_ctx *ctx, uint32_t L, uint32_t n_terms, const uint64_t *const *cts_a, const uint64_t *const *cts_b,
+                  uint32_t n_out, const uint64_t *evk, uint32_t evk_q_limbs, uint64_t *ct_out, void *stream);
 int hml_hrotate_batch(hml_ctx *ctx, uint32_t L, uint32_t n, const uint64_t *ct, const uint64_t *rotkey,
                       uint32_t evk_q_limbs, uint64_t galois_elt, uint64_t *ct_out, void *stream);
 
@@ -378,9 +396,14 @@ int hml_host_free_pinned(hml_ctx *ctx, uint64_t *ptr);
  * a fused PMULT / HADD pair already is.  Anything else runs as without the flag (through HML_REPLAY_HOIST when that is set
  * too).  With HML_REPLAY_HOIST_SUM every plaintext is bound as [L + alpha][N] (P-limb j at row L + j, L = the replay's
  * level); PMULT and PADD read its first limbs as before.  Not available with sh != NULL (HML_ERR_UNSUPPORTED).
+ * HML_REPLAY_HMULT_SUM — a chain of products summed right after they are formed,
+ *   HMULT y = a_0 * b_0,  then  { HMULT t = a_k * b_k; HADD y = y + t (or t + y) }  for k = 1 .. n-1  (n >= 2),
+ * becomes ONE hml_hmult_sum (n_out = 1) that writes y — when every product runs at the same level, y and every t are neither
+ * sources of any product of the chain nor each other, and every t is dead afterwards (its next access, if any, is a write); t
+ * is then left unwritten.  Anything else runs as without the flag.  Not available with sh != NULL (HML_ERR_UNSUPPORTED).
  * With sh != NULL the trace runs limb-sharded: every pointer is the rank's owned-limb slice (see the sharded layouts above). */
 enum { HML_OP_HROTATE = 0, HML_OP_PMULT = 1, HML_OP_HADD = 2, HML_OP_PADD = 3, HML_OP_HMULT = 4 };
-enum { HML_REPLAY_GRAPH = 1, HML_REPLAY_HOIST = 2, HML_REPLAY_HOIST_SUM = 4 };
+enum { HML_REPLAY_GRAPH = 1, HML_REPLAY_HOIST = 2, HML_REPLAY_HOIST_SUM = 4, HML_REPLAY_HMULT_SUM = 8 };
 typedef struct { uint32_t kind, dst, a, b; } hml_trace_op;
 typedef struct hml_replay hml_replay;
 int hml_replay_create(hml_ctx *ctx, hml_shard *sh, uint32_t L, const hml_trace_op *ops, uint32_t n_ops, uint32_t flags,
