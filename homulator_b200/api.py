@@ -70,7 +70,8 @@ EXPORTS = [
     "hml_hrotate_sharded", "hml_hmult_sharded", "hml_rescale_sharded", "hml_ew_sharded", "hml_group_op", "hml_hrotate_hoisted",
     "hml_replay_create", "hml_replay_bind", "hml_replay_run", "hml_replay_slot", "hml_replay_slot_level", "hml_replay_destroy",
     "hml_shard_create_ex", "hml_hrotate_hoisted_sharded", "hml_group_hrotate_hoisted", "hml_hrotate_sum_hoisted",
-    "hml_hrotate_bsgs_hoisted", "hml_hmult_sum",
+    "hml_hrotate_bsgs_hoisted", "hml_hmult_sum", "hml_hrotate_sum_hoisted_sharded", "hml_group_hrotate_sum_hoisted",
+    "hml_hmult_sum_sharded", "hml_group_hmult_sum",
 ]
 
 
@@ -172,6 +173,11 @@ def load_library():
     L.hml_hrotate_hoisted_sharded.argtypes = [vp, u32, vp, u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(vp), vp]
     L.hml_group_hrotate_hoisted.argtypes = [C.POINTER(vp), u32, u32, C.POINTER(vp), u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(vp),
                                             C.POINTER(vp)]
+    L.hml_hrotate_sum_hoisted_sharded.argtypes = [vp, u32, vp, u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(vp), vp, vp]
+    L.hml_group_hrotate_sum_hoisted.argtypes = [C.POINTER(vp), u32, u32, C.POINTER(vp), u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(vp),
+                                                C.POINTER(vp), C.POINTER(vp)]
+    L.hml_hmult_sum_sharded.argtypes = [vp, u32, u32, C.POINTER(vp), C.POINTER(vp), vp, vp, vp]
+    L.hml_group_hmult_sum.argtypes = [C.POINTER(vp), u32, u32, u32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]
     L.hml_replay_create.argtypes = [vp, vp, u32, C.POINTER(_TraceOp), u32, u32, C.POINTER(vp)]
     L.hml_replay_bind.argtypes = [vp, vp, C.POINTER(vp), u32, C.POINTER(u32), C.POINTER(vp), u32, vp, u32]
     L.hml_replay_run.argtypes = [vp, vp]
@@ -679,6 +685,37 @@ class Shard:
         c._chk(c.lib.hml_hrotate_hoisted_sharded(self.h, L, _ptr(ct_own), n, keys, gs, po, c._stream()))
         return outs
 
+    def hrotate_sum_hoisted(self, L, ct_own, rk_owns, galois_elts, pt_owns, out=None):
+        """sum_i pt_owns[i] * rotate(ct, galois_elts[i]) on this rank's limbs with one ModUp, one ModDown and two exchanges
+        (hml_hrotate_sum_hoisted_sharded).  rk_owns[i] / pt_owns[i] are this rank's key and plaintext slices (the plaintext's
+        owned rows of the extended basis, own_ext(L) order: replay.shard_plaintexts); None on a rank that owns no extended limb.
+        Returns the output [2][nq][N]."""
+        c = self.ctx
+        nq, _ = self.own(L)
+        n = len(galois_elts)
+        if len(rk_owns) != n or len(pt_owns) != n:
+            raise ValueError("one key slice and one plaintext slice per galois element")
+        out = c.empty(2, max(nq, 1), c.N) if out is None else out
+        keys = (C.c_void_p * max(n, 1))(*[(_ptr(k) if k is not None else None) for k in rk_owns])
+        pa = (C.c_void_p * max(n, 1))(*[(_ptr(p) if p is not None else None) for p in pt_owns])
+        gs = (C.c_uint64 * max(n, 1))(*[int(g) for g in galois_elts])
+        c._chk(c.lib.hml_hrotate_sum_hoisted_sharded(self.h, L, _ptr(ct_own), n, keys, gs, pa, _ptr(out), c._stream()))
+        return out
+
+    def hmult_sum(self, L, a_owns, b_owns, evk_own, out=None):
+        """sum_i a_owns[i] * b_owns[i] on this rank's limbs with one key switch and one rescale (hml_hmult_sum_sharded); the
+        same tensor as a_owns[i] and b_owns[i] squares it.  Returns the output [2][nk][N] (the owned limbs below L-1)."""
+        c = self.ctx
+        _, nk = self.own(L)
+        n = len(a_owns)
+        if len(b_owns) != n:
+            raise ValueError("a_owns and b_owns must be equally long")
+        out = c.empty(2, max(nk, 1), c.N) if out is None else out
+        pa = (C.c_void_p * max(n, 1))(*[_ptr(t) for t in a_owns])
+        pb = (C.c_void_p * max(n, 1))(*[_ptr(t) for t in b_owns])
+        c._chk(c.lib.hml_hmult_sum_sharded(self.h, L, n, pa, pb, _ptr(evk_own), _ptr(out), c._stream()))
+        return out
+
     def hmult(self, L, a_own, b_own, evk_own, out=None):
         c = self.ctx
         _, nk = self.own(L)
@@ -748,6 +785,58 @@ def group_hrotate_hoisted(group, L, ct_own, keys, galois_elts, outs=None, stream
     if rc:
         msgs = [g.ctx.lib.hml_last_error(g.ctx.h).decode() for g in group]
         raise HmlError(rc, next((m for m in msgs if m), "group hoisted rotation failed"))
+    return outs
+
+
+def _group_call(group, streams, fn, what):
+    """fn(group handle array, stream array) -> return code of a hml_group_* call; raises with the first rank's message"""
+    import torch
+    world = len(group)
+    if streams is None:
+        streams = [torch.cuda.current_stream(group[0].ctx.device).cuda_stream] * world
+    rc = fn((C.c_void_p * world)(*[g.h for g in group]), (C.c_void_p * world)(*streams))
+    if rc:
+        msgs = [g.ctx.lib.hml_last_error(g.ctx.h).decode() for g in group]
+        raise HmlError(rc, next((m for m in msgs if m), what + " failed"))
+
+
+def group_hrotate_sum_hoisted(group, L, ct_own, keys, galois_elts, pts, outs=None, streams=None):
+    """hml_group_hrotate_sum_hoisted: Shard.hrotate_sum_hoisted on every rank of a local group from one host thread.  ct_own[r]
+    is rank r's ciphertext slice, keys[r][i] / pts[r][i] its key and plaintext slices for galois_elts[i] (None where the rank owns
+    no extended limb); returns outs[r] (allocated when not given)."""
+    world, n = len(group), len(galois_elts)
+    if len(ct_own) != world or len(keys) != world or len(pts) != world or any(len(k) != n for k in keys) or any(len(p) != n for p in pts):
+        raise ValueError("ct_own needs one entry per rank, keys and pts one list of len(galois_elts) slices per rank")
+    if outs is None:
+        outs = [g.ctx.empty(2, max(g.own(L)[0], 1), g.ctx.N) for g in group]
+    opt = lambda t: _ptr(t) if t is not None else None  # noqa: E731
+    ca = (C.c_void_p * world)(*[opt(t) for t in ct_own])
+    ka = (C.c_void_p * max(world * n, 1))(*[opt(k) for r in range(world) for k in keys[r]])
+    pa = (C.c_void_p * max(world * n, 1))(*[opt(p) for r in range(world) for p in pts[r]])
+    oa = (C.c_void_p * world)(*[opt(o) for o in outs])
+    gs = (C.c_uint64 * max(n, 1))(*[int(g) for g in galois_elts])
+    lib = group[0].ctx.lib
+    _group_call(group, streams, lambda gh, sa: lib.hml_group_hrotate_sum_hoisted(gh, world, L, ca, n, ka, gs, pa, oa, sa), "group rotation sum")
+    return outs
+
+
+def group_hmult_sum(group, L, a_own, b_own, evk_own, outs=None, streams=None):
+    """hml_group_hmult_sum: Shard.hmult_sum on every rank of a local group from one host thread.  a_own[r][i] / b_own[r][i] are
+    rank r's slices of term i, evk_own[r] its key slice (None where the rank owns no extended limb); returns outs[r]
+    [2][nk][N] (allocated when not given)."""
+    world = len(group)
+    n = len(a_own[0]) if a_own else 0
+    if len(a_own) != world or len(b_own) != world or len(evk_own) != world or any(len(x) != n for x in list(a_own) + list(b_own)):
+        raise ValueError("a_own / b_own need one list of n_terms slices per rank, evk_own one key slice per rank")
+    if outs is None:
+        outs = [g.ctx.empty(2, max(g.own(L)[1], 1), g.ctx.N) for g in group]
+    opt = lambda t: _ptr(t) if t is not None else None  # noqa: E731
+    pa = (C.c_void_p * max(world * n, 1))(*[opt(t) for r in range(world) for t in a_own[r]])
+    pb = (C.c_void_p * max(world * n, 1))(*[opt(t) for r in range(world) for t in b_own[r]])
+    ea = (C.c_void_p * world)(*[opt(k) for k in evk_own])
+    oa = (C.c_void_p * world)(*[opt(o) for o in outs])
+    lib = group[0].ctx.lib
+    _group_call(group, streams, lambda gh, sa: lib.hml_group_hmult_sum(gh, world, L, n, pa, pb, ea, oa, sa), "group product sum")
     return outs
 
 

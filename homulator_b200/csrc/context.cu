@@ -1466,6 +1466,17 @@ static size_t shard_hoist_ws_words(const Params &p, const ShardPlan &sp, uint32_
   return (size_t)p.N * ((size_t)sp.beta * ne + 2 * (size_t)H * ne + 2 * nq);
 }
 
+// the ModUp of the hoisted ops: the conversions from the owners' gather buffers 1 and the forward NTT of the owned extended
+// digits into ext [beta][ne], stored for the inner products (no fused inner product)
+static int shard_hoist_modup(hml_ctx *ctx, ShardPlan *sp, const uint64_t *const *peers1, u64 *ext, cudaStream_t s) {
+  int rc;
+  for (auto &u : sp->up) if ((rc = shard_p2p_check(ctx, u))) return rc;
+  if ((rc = shard_peer_offsets(ctx, sp, peers1, false))) return rc;
+  shard_modup_p2p(ctx, sp, peers1[sp->rank], ext, s);
+  shard_ext_ntt(ctx, sp, ext, false, nullptr, nullptr, nullptr, s);
+  return HML_OK;
+}
+
 // phase 1 of a group of n <= H rotations.  peers1 != null (the op's first group): the ModUp conversions from the owners' gather
 // buffers 1 and the forward NTT of the owned extended digits, stored for the later groups (no fused inner product).  Then ONE
 // launch of the inner product for all n rotations: acc[r] = sum_j sigma_r(t_j) * keys[r][j]; the own-digit term reads c1_own
@@ -1483,12 +1494,7 @@ int shard_hoist_inner(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, u
   const uint32_t ne = sp->own_q.size() + sp->own_p.size(), beta = sp->beta;
   if (ne == 0) return HML_OK;
   u64 *ext = ctx->ws, *acc = ext + (size_t)beta * ne * N;
-  if (peers1) {
-    for (auto &u : sp->up) if ((rc = shard_p2p_check(ctx, u))) return rc;
-    if ((rc = shard_peer_offsets(ctx, sp, peers1, false))) return rc;
-    shard_modup_p2p(ctx, sp, peers1[rank], ext, s);
-    shard_ext_ntt(ctx, sp, ext, false, nullptr, nullptr, nullptr, s);
-  }
+  if (peers1 && (rc = shard_hoist_modup(ctx, sp, peers1, ext, s))) return rc;
   InnerRotArgs a{};
   a.d = (const u64 *)c1_own; a.ext = ext; a.acc = acc; a.acc_rot_stride = 2ll * ne * N;
   a.N = (int)N; a.n_ext = (int)ne; a.beta = (int)beta; a.evk_limbs = (int)ne; a.logN = p.logN; a.ext_f64 = p.logN > NTT_SMALL_LOG;
@@ -1497,6 +1503,69 @@ int shard_hoist_inner(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, u
   prof_mark(ctx, HML_CLS_EWE, s);
   ctx->exec.ewe_limbs += 2ull * n * ne * beta; ctx->exec.kernel_launches++;
   return check_launch(ctx, "hoisted shard inner product");
+}
+
+// phase 1 of the sharded double-hoisted rotation sum (shard.cu, hml_hrotate_sum_hoisted_sharded) before its P-limb INTT: the
+// ModUp of c1, then k_inner_rot_sum on the owned extended limbs, one launch per group of IP_MAX_ROT rotations (later groups
+// add to the stored sums).  The kernel's limb index is the position in the owned layout (Q-limbs first), so L = nq and
+// pt_q_limbs = nq make it read Q-limb rows and P-limb rows of the owned plaintext slices [nq + np][N] alike.  acc [2][ne]
+// lands where shard_hoist_intt reads accumulator pair 0; z [nq][N] = sum_r pt_r * sigma_r(c0) on the owned Q-limbs.
+int shard_rot_sum_inner(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *const *peers1, const uint64_t *ct_own,
+                        uint32_t n_rot, const uint64_t *const *keys, const uint64_t *galois, const uint64_t *const *pts, uint64_t *z_own,
+                        cudaStream_t s) {
+  ShardPlan *sp;
+  int rc = shard_plan_on_device(ctx, L, rank, world, &sp);
+  if (rc) return rc;
+  if ((rc = ensure_ws(ctx, shard_hoist_ws_words(ctx->p, *sp, 1)))) return rc;
+  ws_enter(ctx, s);
+  const Params &p = ctx->p;
+  const size_t N = p.N;
+  const uint32_t nq = sp->own_q.size(), ne = nq + sp->own_p.size(), beta = sp->beta;
+  if (ne == 0) return HML_OK;
+  u64 *ext = ctx->ws, *acc = ext + (size_t)beta * ne * N;
+  if ((rc = shard_hoist_modup(ctx, sp, peers1, ext, s))) return rc;
+  InnerRotSumArgs a{};
+  a.d = (const u64 *)ct_own + (size_t)nq * N; a.ext = ext; a.c0 = (const u64 *)ct_own; a.acc = acc; a.z = (u64 *)z_own;
+  a.N = (int)N; a.n_ext = (int)ne; a.L = (int)nq; a.beta = (int)beta; a.evk_limbs = (int)ne; a.pt_q_limbs = (int)nq; a.logN = p.logN;
+  a.ext_f64 = p.logN > NTT_SMALL_LOG; a.evk_packed = 0;
+  for (uint32_t r0 = 0; r0 < n_rot; r0 += IP_MAX_ROT) {
+    const uint32_t n = std::min<uint32_t>(IP_MAX_ROT, n_rot - r0);
+    a.accumulate = r0 > 0; a.n_rot = (int)n;
+    for (uint32_t k = 0; k < n; ++k) {
+      a.evk[k] = (const u64 *)keys[r0 + k]; a.pt[k] = (const u64 *)pts[r0 + k]; a.galois[k] = inner_galois(galois[r0 + k], N);
+    }
+    launch_inner_product_rot_sum(ctx->mc, sp->e_lm, a, s);
+    prof_mark(ctx, HML_CLS_EWE, s);
+    ctx->exec.kernel_launches++;
+    ctx->exec.ewe_limbs += (uint64_t)n * (2ull * ne * beta + 2ull * ne + nq);
+    ctx->exec.automorph_limbs += (uint64_t)n * nq;  // sigma_r(c0), applied on load
+  }
+  return check_launch(ctx, "sharded rotation sum inner product");
+}
+
+// phase 0 of the sharded product sum (shard.cu, hml_hmult_sum_sharded): d0 | d1 | d2 [nq][N] words = the sums of the n tensor
+// products a[k] (x) b[k] on the owned Q-limbs, k_tensor_sum once per group of IP_MAX_ROT terms
+int shard_tensor_sum(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uint32_t n, const uint64_t *const *a_own,
+                     const uint64_t *const *b_own, uint64_t *d0, uint64_t *d1, uint64_t *d2, cudaStream_t s) {
+  ShardPlan *sp;
+  int rc = shard_plan_on_device(ctx, L, rank, world, &sp);
+  if (rc) return rc;
+  ws_enter(ctx, s);
+  const uint32_t nq = sp->own_q.size();
+  if (nq == 0) return HML_OK;
+  TensorSumArgs a{};
+  a.d0 = (u64 *)d0; a.d1 = (u64 *)d1; a.d2 = (u64 *)d2;
+  a.comp_stride = (long long)nq * ctx->p.N; a.in_stride = 0; a.out_stride = 0;
+  a.N = (int)ctx->p.N; a.pack01 = 0; a.mod0 = (int)rank; a.mod_step = (int)world;  // the sharded ModDown adds d0 / d1 as words
+  for (uint32_t k0 = 0; k0 < n; k0 += IP_MAX_ROT) {
+    const uint32_t m = std::min<uint32_t>(IP_MAX_ROT, n - k0);
+    a.accumulate = k0 > 0; a.n_pairs = (int)m;
+    for (uint32_t k = 0; k < m; ++k) { a.a[k] = (const u64 *)a_own[k0 + k]; a.b[k] = (const u64 *)b_own[k0 + k]; }
+    launch_tensor_sum(ctx->mc, (int)nq, 1, a, s);
+    prof_mark(ctx, HML_CLS_EWE, s);
+    ctx->exec.ewe_limbs += 3ull * m * nq; ctx->exec.kernel_launches++;
+  }
+  return check_launch(ctx, "sharded tensor product sum");
 }
 
 // the rest of phase 1: ONE inverse NTT (+ scaling) of the owned P-limbs of all 2n accumulators, rotation r into this rank's
@@ -1752,7 +1821,7 @@ static int hmult_sum_run(hml_ctx *ctx, uint32_t L, uint32_t nb, uint32_t n_terms
   TensorSumArgs a{};
   a.d0 = ws; a.d1 = a.d0 + nb * PL; a.d2 = a.d1 + nb * PL;
   a.comp_stride = (long long)PL; a.in_stride = (long long)(2 * PL); a.out_stride = (long long)PL;
-  a.N = (int)N; a.pack01 = p.logN > NTT_SMALL_LOG;
+  a.N = (int)N; a.pack01 = p.logN > NTT_SMALL_LOG; a.mod0 = 0; a.mod_step = 1;
   for (uint32_t k0 = 0; k0 < n_terms; k0 += IP_MAX_ROT) {
     const uint32_t n = std::min<uint32_t>(IP_MAX_ROT, n_terms - k0);
     a.accumulate = k0 > 0; a.n_pairs = (int)n;

@@ -111,8 +111,8 @@ __global__ void __launch_bounds__(EW_THREADS) k_tensor_sum(const ModConst *__res
   pdl_wait();
   const int i2 = blockIdx.x * EW_THREADS + threadIdx.x;
   if (i2 >= a.N / 2) return;
-  const int limb = blockIdx.y;  // limbs 0..L-1 are moduli q_0..q_{L-1}
-  const ModConst m = mc[limb];
+  const int limb = blockIdx.y;  // limb slot; its modulus is q_{mod0 + limb * mod_step}
+  const ModConst m = mc[a.mod0 + limb * a.mod_step];
   const size_t o = (size_t)limb * (a.N / 2) + i2;
   const long long bi = (long long)blockIdx.z * a.in_stride, bo = (long long)blockIdx.z * a.out_stride;
   double s0[2] = {0, 0}, s1[2] = {0, 0}, s2[2] = {0, 0};

@@ -113,16 +113,19 @@ struct InnerBsgsArgs : InnerRotSumArgs {
 };
 void launch_inner_product_bsgs(const ModConst *mc, const LimbMap &lm, const InnerBsgsArgs &a, bool giant, cudaStream_t s);
 
-// A sum of up to IP_MAX_ROT tensor products (context.cu, hmult_sum_run), limbs 0..L-1, grid (N/2/256, L, n_batch):
+// A sum of up to IP_MAX_ROT tensor products (context.cu, hmult_sum_run and shard_tensor_sum), L limb slots, grid
+// (N/2/256, L, n_batch):
 //   d0 (+)= sum_k a_k0*b_k0,   d1 (+)= sum_k (a_k0*b_k1 + a_k1*b_k0),   d2 (+)= sum_k a_k1*b_k1        k < n_pairs
 // a[k] / b[k] are [n_batch][2][L][N]: component c at + c * comp_stride, batch entry z at + z * in_stride; d0 / d1 / d2 advance
-// by out_stride per batch entry.  A pair with a[k] == b[k] (a square) loads one ciphertext.  The outputs have launch_tensor3's
+// by out_stride per batch entry.  Limb slot l has modulus q_{mod0 + l * mod_step}: 0 and 1 for a whole ciphertext, rank and
+// world for a limb-sharded one.  A pair with a[k] == b[k] (a square) loads one ciphertext.  The outputs have launch_tensor3's
 // formats (pack01: d0 / d1 packed limbs); accumulate = 1 adds to what d0 / d1 / d2 hold (the later groups of one op).
 struct TensorSumArgs {
   const u64 *a[IP_MAX_ROT], *b[IP_MAX_ROT];
   u64 *d0, *d1, *d2;
   long long comp_stride, in_stride, out_stride;
   int N, n_pairs, accumulate, pack01;
+  int mod0, mod_step;
 };
 void launch_tensor_sum(const ModConst *mc, int L, int n_batch, const TensorSumArgs &a, cudaStream_t s);
 

@@ -42,3 +42,10 @@ int shard_prepare(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const
 int shard_hoist_inner(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uint32_t H, const uint64_t *const *peers1, const uint64_t *c1_own,
                       uint32_t n, const uint64_t *const *keys, const uint64_t *galois, cudaStream_t s);
 int shard_hoist_intt(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uint32_t n, uint64_t *g2_own, size_t slot_words, cudaStream_t s);
+// the sharded sums' limb-local stages (context.cu): the rotation sum's ModUp + weighted inner product (z_own [nq][N] = the c0
+// term), and the product sum's tensor-product sum into d0 | d1 | d2 [nq][N]
+int shard_rot_sum_inner(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, const uint64_t *const *peers1, const uint64_t *ct_own,
+                        uint32_t n_rot, const uint64_t *const *keys, const uint64_t *galois, const uint64_t *const *pts, uint64_t *z_own,
+                        cudaStream_t s);
+int shard_tensor_sum(hml_ctx *ctx, uint32_t L, uint32_t rank, uint32_t world, uint32_t n, const uint64_t *const *a_own,
+                     const uint64_t *const *b_own, uint64_t *d0, uint64_t *d1, uint64_t *d2, cudaStream_t s);

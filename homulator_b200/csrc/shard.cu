@@ -40,15 +40,22 @@ struct hml_shard {
   bool rb_dirty = false;                   // peers may still be reading the rescale buffer of the previous rescale
 };
 
-enum ShardOpKind { SOP_KEYSWITCH = 0, SOP_HROTATE = 1, SOP_HMULT = 2, SOP_RESCALE = 3 };
+// SOP_ROT_SUM and SOP_HMULT_SUM are internal kinds (hml_group_op serves 0..3): the double-hoisted rotation sum has the key
+// switch's phases, the product sum hmult's
+enum ShardOpKind { SOP_KEYSWITCH = 0, SOP_HROTATE = 1, SOP_HMULT = 2, SOP_RESCALE = 3, SOP_ROT_SUM = 4, SOP_HMULT_SUM = 5 };
 struct ShardOp {
   int kind;
   uint32_t L;
-  const uint64_t *a, *b, *key;   // keyswitch: a = d_own; hrotate: a = ct_own; hmult: a, b = ct_own; rescale: a = x_own
+  const uint64_t *a, *b, *key;   // keyswitch: a = d_own; hrotate, rotation sum: a = ct_own; hmult: a, b = ct_own; rescale: a = x_own
   uint64_t *out0, *out1;         // keyswitch: both outputs; others: out0 = the result ciphertext
   uint64_t g;
+  // the term table of the sums (n entries): rotation sum ta = key slices, tb = plaintext slices, gs = galois elements;
+  // product sum ta[i] (x) tb[i]
+  uint32_t n = 0;
+  const uint64_t *const *ta = nullptr, *const *tb = nullptr;
+  const uint64_t *gs = nullptr;
 };
-static int op_phases(int kind) { return kind == SOP_HMULT ? 4 : kind == SOP_RESCALE ? 2 : 3; }
+static int op_phases(int kind) { return kind == SOP_HMULT || kind == SOP_HMULT_SUM ? 4 : kind == SOP_RESCALE ? 2 : 3; }
 // exchange group (= flag slot group) after phase `ph`
 static int op_exchange(int kind, int ph) { return kind == SOP_RESCALE ? 2 : ph; }
 
@@ -196,12 +203,39 @@ extern "C" int hml_shard_own_limbs(const hml_shard *sh, uint32_t L, uint32_t *n_
 }
 
 // ------------------------------------------------------------------------------------------------ phases
+// the sums' operands, checked on every rank before anything is enqueued
+static int sum_check(hml_shard *sh, const ShardOp &op) {
+  const bool rot = op.kind == SOP_ROT_SUM;
+  if (op.n == 0) return sfail(sh, HML_ERR_INVALID, rot ? "n_rot must be at least 1" : "n_terms must be at least 1");
+  if (!op.out0 || (rot && (!op.a || !op.gs)) || (!rot && (!op.ta || !op.tb))) return sfail(sh, HML_ERR_INVALID, "null buffer");
+  const size_t N = sh->ctx->p.N;
+  const uint32_t nq = own_q_count(op.L, sh->rank, sh->world);
+  const bool own_ext = nq > 0 || own_q_count(op.L + sh->ctx->p.alpha, sh->rank, sh->world) > 0;
+  const uint32_t n_out = rot ? nq : nq - ((op.L - 1) % sh->world == sh->rank ? 1 : 0);
+  const size_t in_w = 2 * (size_t)std::max<uint32_t>(nq, 1) * N, out_w = 2 * (size_t)std::max<uint32_t>(n_out, 1) * N;
+  auto overlaps = [&](const uint64_t *in) { return op.out0 < in + in_w && in < op.out0 + out_w; };
+  if (rot && overlaps(op.a)) return sfail(sh, HML_ERR_INVALID, "the output overlaps the input");
+  if (!rot && own_ext && !op.key) return sfail(sh, HML_ERR_INVALID, "null key on a rank that owns extended limbs");
+  for (uint32_t i = 0; i < op.n; ++i) {
+    if (rot) {
+      if (!(op.gs[i] & 1)) return sfail(sh, HML_ERR_INVALID, "galois element must be odd");
+      if (own_ext && (!op.ta || !op.ta[i])) return sfail(sh, HML_ERR_INVALID, "null rotation key on a rank that owns extended limbs");
+      if (own_ext && (!op.tb || !op.tb[i])) return sfail(sh, HML_ERR_INVALID, "null plaintext on a rank that owns extended limbs");
+    } else {
+      if (!op.ta[i] || !op.tb[i]) return sfail(sh, HML_ERR_INVALID, "null ciphertext");
+      if (overlaps(op.ta[i]) || overlaps(op.tb[i])) return sfail(sh, HML_ERR_INVALID, "the output overlaps an input");
+    }
+  }
+  return HML_OK;
+}
+
 static int op_check(hml_shard *sh, const ShardOp &op) {
   if (!sh->connected) return sfail(sh, HML_ERR_INVALID, "shard group not connected");
-  int rc = check_level(sh->ctx, op.L, op.kind == SOP_HMULT || op.kind == SOP_RESCALE ? 2 : 1);
+  int rc = check_level(sh->ctx, op.L, op.kind == SOP_HMULT || op.kind == SOP_RESCALE || op.kind == SOP_HMULT_SUM ? 2 : 1);
   if (rc) return rc;
   if (op.L > sh->max_L) return sfail(sh, HML_ERR_INVALID, "level above the shard's maximum");
   if (op.kind == SOP_HROTATE && !(op.g & 1)) return sfail(sh, HML_ERR_INVALID, "galois element must be odd");
+  if (op.kind == SOP_ROT_SUM || op.kind == SOP_HMULT_SUM) return sum_check(sh, op);
   return HML_OK;
 }
 
@@ -232,11 +266,25 @@ static int run_phase(hml_shard *sh, const ShardOp &op, int ph, cudaStream_t s) {
       // (sigma(c0) + ks0, ks1): the addend rides in the ModDown epilogue
       return shard_end_p2p(ctx, L, rank, world, peers(sh->p2), op.out0, op.out0 + (size_t)nq * N, sig, nullptr, s);
     }
-    case SOP_HMULT: {
+    case SOP_ROT_SUM: {
+      // begin(c1) | X0 | ModUp, weighted inner products, P-limb INTT | X1 | one ModDown with addend z = sum_r pt_r * sigma_r(c0)
+      uint64_t *z = sc;  // [nq][N]
+      if (ph == 0) return hml_keyswitch_shard_begin(ctx, L, rank, world, op.a + (size_t)nq * N, sh->g1, st);
+      if (ph == 1) {
+        if (!own_ext) return HML_OK;
+        if ((rc = shard_rot_sum_inner(ctx, L, rank, world, peers(sh->p1), op.a, op.n, op.ta, op.gs, op.tb, z, s))) return rc;
+        return shard_hoist_intt(ctx, L, rank, world, 1, sh->g2, sh->n2, s);
+      }
+      return shard_end_p2p(ctx, L, rank, world, peers(sh->p2), op.out0, op.out0 + (size_t)nq * N, z, nullptr, s);
+    }
+    case SOP_HMULT:
+    case SOP_HMULT_SUM: {
       uint64_t *d0 = sc, *d1 = d0 + (size_t)nq * N, *d2 = d1 + (size_t)nq * N, *c = d2 + (size_t)nq * N;  // c [2][nq][N]
       const size_t PL = (size_t)nq * N;
       if (ph == 0) {
-        if (nq) {  // TensorCompute on the owned limbs (reference src/Operation.cpp:592-739)
+        if (op.kind == SOP_HMULT_SUM) {  // the sums of the terms' tensor products: everything after them is hmult's
+          if ((rc = shard_tensor_sum(ctx, L, rank, world, op.n, op.ta, op.tb, d0, d1, d2, s))) return rc;
+        } else if (nq) {  // TensorCompute on the owned limbs (reference src/Operation.cpp:592-739)
           if ((rc = hml_ewe(ctx, op.a, op.b, nullptr, nullptr, 0, d0, own.data(), nq, st))) return rc;
           if ((rc = hml_ewe(ctx, op.a, op.b + PL, op.a + PL, op.b, 0, d1, own.data(), nq, st))) return rc;
           if ((rc = hml_ewe(ctx, op.a + PL, op.b + PL, nullptr, nullptr, 0, d2, own.data(), nq, st))) return rc;
@@ -261,11 +309,14 @@ static int fused_sync(hml_shard *sh, int grp, cudaStream_t s) {
   return hml_shard_sync(sh->ctx, (uint64_t *const *)sh->pf_dev, grp * sh->world + sh->rank, sh->fl, grp * sh->world, 0, sh->world, (void *)s);
 }
 
+static int hoist_prepare(hml_shard *sh, uint32_t L);
+
 // one rank per GPU: phases with one fused exchange launch between them
 static int run_op(hml_shard *sh, const ShardOp &op, cudaStream_t s) {
   int rc = op_check(sh, op);
   if (rc) return rc;
   HML_CU_TRY(sh->ctx, cudaSetDevice(sh->ctx->device));
+  if (op.kind >= SOP_ROT_SUM && (rc = hoist_prepare(sh, op.L))) return rc;  // a no-op after hml_shard_prepare(L)
   if ((op.kind == SOP_RESCALE) && sh->rb_dirty && (rc = fused_sync(sh, 2, s))) return rc;  // write-after-read on the rescale buffer
   const int n = op_phases(op.kind);
   for (int ph = 0; ph < n; ++ph) {
@@ -469,19 +520,17 @@ static int group_exchange(hml_shard *const *group, uint32_t world, bool emulate,
   return HML_OK;
 }
 
-// op: 0 keyswitch (a = d_own, out0/out1), 1 hrotate (a = ct_own, out0), 2 hmult (a, b, out0), 3 rescale (a, out0).
-extern "C" int hml_group_op(hml_shard *const *group, uint32_t world, int op_kind, uint32_t L, const uint64_t *const *a, const uint64_t *const *b,
-                            const uint64_t *const *key, uint64_t *const *out0, uint64_t *const *out1, uint64_t galois_elt, void *const *streams) {
-  if (!group || world == 0 || !a || !out0 || op_kind < 0 || op_kind > 3) return HML_ERR_INVALID;
+// ops[r] (one kind) on every rank of the group, phase by phase
+static int group_run(hml_shard *const *group, uint32_t world, void *const *streams, const std::vector<ShardOp> &ops) {
   bool emulate;
   int rc = group_setup(group, world, streams, &emulate);
   if (rc) return rc;
-  std::vector<ShardOp> ops(world);
-  for (uint32_t r = 0; r < world; ++r) {
-    ops[r] = ShardOp{op_kind, L, (const uint64_t *)a[r], b ? (const uint64_t *)b[r] : nullptr, key ? (const uint64_t *)key[r] : nullptr, (uint64_t *)out0[r],
-                     out1 ? (uint64_t *)out1[r] : nullptr, galois_elt};
+  const int op_kind = ops[0].kind;
+  for (uint32_t r = 0; r < world; ++r)
     if ((rc = op_check(group[r], ops[r]))) return rc;
-  }
+  if (op_kind >= SOP_ROT_SUM)  // before the first exchange: nothing may allocate or synchronise while a rank waits
+    for (uint32_t r = 0; r < world; ++r)
+      if ((rc = hoist_prepare(group[r], ops[r].L))) return rc;
   if (op_kind == SOP_RESCALE && group[0]->rb_dirty && (rc = group_exchange(group, world, emulate, streams, 2))) return rc;
   const int n = op_phases(op_kind);
   for (int ph = 0; ph < n; ++ph) {
@@ -493,6 +542,17 @@ extern "C" int hml_group_op(hml_shard *const *group, uint32_t world, int op_kind
   }
   for (uint32_t r = 0; r < world; ++r) group[r]->rb_dirty = op_kind == SOP_RESCALE;
   return HML_OK;
+}
+
+// op: 0 keyswitch (a = d_own, out0/out1), 1 hrotate (a = ct_own, out0), 2 hmult (a, b, out0), 3 rescale (a, out0).
+extern "C" int hml_group_op(hml_shard *const *group, uint32_t world, int op_kind, uint32_t L, const uint64_t *const *a, const uint64_t *const *b,
+                            const uint64_t *const *key, uint64_t *const *out0, uint64_t *const *out1, uint64_t galois_elt, void *const *streams) {
+  if (!group || world == 0 || !a || !out0 || op_kind < 0 || op_kind > 3) return HML_ERR_INVALID;
+  std::vector<ShardOp> ops(world);
+  for (uint32_t r = 0; r < world; ++r)
+    ops[r] = ShardOp{op_kind, L, (const uint64_t *)a[r], b ? (const uint64_t *)b[r] : nullptr, key ? (const uint64_t *)key[r] : nullptr, (uint64_t *)out0[r],
+                     out1 ? (uint64_t *)out1[r] : nullptr, galois_elt};
+  return group_run(group, world, streams, ops);
 }
 
 // hml_hrotate_hoisted_sharded for every rank of a local group; rotkeys_own / outs_own are rank-major ([rank * n_rot + i])
@@ -525,4 +585,48 @@ extern "C" int hml_group_hrotate_hoisted(hml_shard *const *group, uint32_t world
   }
   for (uint32_t r = 0; r < world; ++r) group[r]->rb_dirty = false;
   return HML_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ sums
+// The double-hoisted rotation sum and the lazily relinearised product sum on the owned limbs, with the exchanges of ONE key
+// switch (rotation sum) or ONE hmult (product sum) whatever the number of terms: every term's work is limb-local.
+extern "C" int hml_hrotate_sum_hoisted_sharded(hml_shard *sh, uint32_t L, const uint64_t *ct_own, uint32_t n_rot, const uint64_t *const *rotkeys_own,
+                                               const uint64_t *galois_elts, const uint64_t *const *pts_own, uint64_t *out_own, void *stream) {
+  if (!sh) return HML_ERR_INVALID;
+  ShardOp op{SOP_ROT_SUM, L, ct_own, nullptr, nullptr, out_own, nullptr, 0};
+  op.n = n_rot; op.ta = rotkeys_own; op.tb = pts_own; op.gs = galois_elts;
+  return run_op(sh, op, (cudaStream_t)stream);
+}
+
+extern "C" int hml_group_hrotate_sum_hoisted(hml_shard *const *group, uint32_t world, uint32_t L, const uint64_t *const *ct_own, uint32_t n_rot,
+                                             const uint64_t *const *rotkeys_own, const uint64_t *galois_elts, const uint64_t *const *pts_own,
+                                             uint64_t *const *out_own, void *const *streams) {
+  if (!group || world == 0 || !ct_own || !out_own) return HML_ERR_INVALID;
+  std::vector<ShardOp> ops(world);
+  for (uint32_t r = 0; r < world; ++r) {
+    ops[r] = ShardOp{SOP_ROT_SUM, L, ct_own[r], nullptr, nullptr, out_own[r], nullptr, 0};
+    ops[r].n = n_rot; ops[r].gs = galois_elts;
+    ops[r].ta = rotkeys_own ? rotkeys_own + (size_t)r * n_rot : nullptr;
+    ops[r].tb = pts_own ? pts_own + (size_t)r * n_rot : nullptr;
+  }
+  return group_run(group, world, streams, ops);
+}
+
+extern "C" int hml_hmult_sum_sharded(hml_shard *sh, uint32_t L, uint32_t n_terms, const uint64_t *const *a_own, const uint64_t *const *b_own,
+                                     const uint64_t *evk_own, uint64_t *out_own, void *stream) {
+  if (!sh) return HML_ERR_INVALID;
+  ShardOp op{SOP_HMULT_SUM, L, nullptr, nullptr, evk_own, out_own, nullptr, 0};
+  op.n = n_terms; op.ta = a_own; op.tb = b_own;
+  return run_op(sh, op, (cudaStream_t)stream);
+}
+
+extern "C" int hml_group_hmult_sum(hml_shard *const *group, uint32_t world, uint32_t L, uint32_t n_terms, const uint64_t *const *a_own,
+                                   const uint64_t *const *b_own, const uint64_t *const *evk_own, uint64_t *const *out_own, void *const *streams) {
+  if (!group || world == 0 || !a_own || !b_own || !out_own) return HML_ERR_INVALID;
+  std::vector<ShardOp> ops(world);
+  for (uint32_t r = 0; r < world; ++r) {
+    ops[r] = ShardOp{SOP_HMULT_SUM, L, nullptr, nullptr, evk_own ? evk_own[r] : nullptr, out_own[r], nullptr, 0};
+    ops[r].n = n_terms; ops[r].ta = a_own + (size_t)r * n_terms; ops[r].tb = b_own + (size_t)r * n_terms;
+  }
+  return group_run(group, world, streams, ops);
 }

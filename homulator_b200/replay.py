@@ -88,3 +88,14 @@ def shard_operands(sh, L, x, plaintexts, rot_keys, evk):
     oe = torch.tensor(sh.own_ext(L), device=x.device, dtype=torch.long)
     cut = lambda k: k[:, :, oe].contiguous() if k is not None else None  # noqa: E731
     return (x[:, oi].contiguous(), {i: p[oi].contiguous() for i, p in plaintexts.items()}, {r: cut(k) for r, k in rot_keys.items()}, cut(evk))
+
+
+def shard_plaintexts(sh, L, plaintexts):
+    """This rank's slices of extended-basis plaintexts [L + alpha][N] (P-limb j at row L + j), as the sharded rotation sum takes
+    them: the owned rows in own_ext(L) order, [nq + np][N]; None where the rank owns no extended limb."""
+    import torch
+    own = sh.own_ext(L)
+    if not own:
+        return [None for _ in plaintexts]
+    oe = torch.tensor(own, device=plaintexts[0].device, dtype=torch.long) if plaintexts else None
+    return [p[oe].contiguous() for p in plaintexts]

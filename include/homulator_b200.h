@@ -256,6 +256,45 @@ int hml_hrotate_hoisted_sharded(hml_shard *sh, uint32_t L, const uint64_t *ct_ow
 int hml_group_hrotate_hoisted(hml_shard *const *group, uint32_t world, uint32_t L, const uint64_t *const *ct_own, uint32_t n_rot,
                               const uint64_t *const *rotkeys_own, const uint64_t *galois_elts, uint64_t *const *outs_own,
                               void *const *streams);
+/* Double-hoisted rotation sum of ONE limb-sharded ciphertext (one call per rank): out_own [2][nq][N] =
+ * sum_i pts_own[i] * rotate(ct_own, galois_elts[i]) on the owned limbs, bit-identical to the owned rows of
+ * hml_hrotate_sum_hoisted (same formula: acc_c = sum_i pt_i * sum_j sigma_i(t_j) * rk_i[j][c] over the owned extended limbs,
+ * z = sum_i pt_i * sigma_i(c0) over the owned Q-limbs, out = (z + ModDown(acc_0), ModDown(acc_1))).
+ *   begin(c1) | X0 | ModUp + NTT of the owned digits, one inner-product launch per group of 16 rotations, P-limb INTT | X1 |
+ *   one ModDown with addend z
+ * Two exchanges per call whatever n_rot and max_rot; no slot of gather buffer 2 beyond the first is used.  ct_own, out_own
+ * [2][nq][N], not overlapping.  rotkeys_own / galois_elts / pts_own are HOST arrays of n_rot entries: word key slices
+ * [beta][2][n_own_ext][N] (no HML_KEY_PACKED) and plaintext slices [nq + np][N] holding the rank's owned rows of the extended
+ * basis (owned Q-limbs, then owned P-limbs, as the key slices).  A rank that owns no extended limb may pass null keys and
+ * plaintexts; a rank that owns only P-limbs needs both.  HML_ERR_INVALID (before anything is enqueued): n_rot = 0, a null
+ * ct / output / galois array, a null key or plaintext on a rank that owns extended limbs, an even galois element, out_own
+ * overlapping ct_own, L above the shard's maximum.  Executed counts per rank: the transforms and conversions of one
+ * hml_hrotate_hoisted_sharded rotation whatever n_rot; one kernel launch per group of 16 rotations; per rotation
+ * ewe_limbs += 2 * beta * ne + 2 * ne + nq and automorph_limbs += nq (ne = owned extended limbs).  After hml_shard_prepare(L) the
+ * call neither allocates nor synchronises (it can be captured in a CUDA graph). */
+int hml_hrotate_sum_hoisted_sharded(hml_shard *sh, uint32_t L, const uint64_t *ct_own, uint32_t n_rot, const uint64_t *const *rotkeys_own,
+                                    const uint64_t *galois_elts, const uint64_t *const *pts_own, uint64_t *out_own, void *stream);
+/* The same for all ranks of a local group from one host thread (as hml_group_op): ct_own, out_own and streams are indexed by
+ * rank, rotkeys_own and pts_own rank-major ([rank * n_rot + i]). */
+int hml_group_hrotate_sum_hoisted(hml_shard *const *group, uint32_t world, uint32_t L, const uint64_t *const *ct_own, uint32_t n_rot,
+                                  const uint64_t *const *rotkeys_own, const uint64_t *galois_elts, const uint64_t *const *pts_own,
+                                  uint64_t *const *out_own, void *const *streams);
+/* Sum of ciphertext products on limb-sharded operands (one call per rank, one output): out_own [2][nk][N] =
+ * Rescale(Relin(sum_i a_own[i] (x) b_own[i])) on the owned limbs below L-1 (nk from hml_shard_own_limbs), bit-identical to the
+ * owned rows of hml_hmult_sum with n_out = 1; with n_terms = 1 it is hml_hmult_sharded.  The phases of hml_hmult_sharded,
+ * whose tensor product becomes the sums D0 / D1 / D2 of the n_terms tensor products on the owned limbs (one launch per group of
+ * 16 terms); the key switch, the exchanges and the rescale run once.  a_own / b_own are HOST arrays of n_terms device pointers
+ * to [2][nq][N]; a_own[i] == b_own[i] is a square and reads its ciphertext once.  evk_own [beta][2][n_own_ext][N] (word key;
+ * may be null on a rank that owns no extended limb).  HML_ERR_INVALID (before anything is enqueued): n_terms = 0, L < 2, L above
+ * the shard's maximum, a null array, entry or output, a null key on a rank that owns extended limbs, out_own overlapping an
+ * input.  Executed counts per rank: the transforms and conversions of hml_hmult_sharded whatever n_terms; ewe_limbs += 3 * nq
+ * per term.  After hml_shard_prepare(L) the call neither allocates nor synchronises (it can be captured in a CUDA graph). */
+int hml_hmult_sum_sharded(hml_shard *sh, uint32_t L, uint32_t n_terms, const uint64_t *const *a_own, const uint64_t *const *b_own,
+                          const uint64_t *evk_own, uint64_t *out_own, void *stream);
+/* The same for all ranks of a local group from one host thread: evk_own, out_own and streams are indexed by rank, a_own and
+ * b_own rank-major ([rank * n_terms + i]). */
+int hml_group_hmult_sum(hml_shard *const *group, uint32_t world, uint32_t L, uint32_t n_terms, const uint64_t *const *a_own,
+                        const uint64_t *const *b_own, const uint64_t *const *evk_own, uint64_t *const *out_own, void *const *streams);
 
 /* ------------------------------------------------------------------ operations (reference include/Operation.h) */
 /* HMULT (reference src/Operation.cpp:913-1023): tensor + keyswitch(relinearise) + add + rescale x2.
