@@ -17,8 +17,10 @@
  *   - a ctx is bound to one CUDA device and is NOT thread-safe (the reference is single-threaded and
  *     not re-entrant either: globals at reference src/Instruction.cpp:3, src/Operation.cpp:7).
  *   - all polynomial buffers are DEVICE pointers to uint64_t (reference include/Context.h:8
- *     `DataType = uint64_t`), caller-owned, residues < 2^elementBitWidth, layout [.. ][limb][N],
- *     a ciphertext is [2][L][N] (c0 limbs, then c1 limbs), in EVALUATION form:
+ *     `DataType = uint64_t`), caller-owned, layout [.. ][limb][N].  Every residue of limb i must be CANONICAL,
+ *     in [0, q_i) (not merely < 2^elementBitWidth): the kernels convert words to doubles and centre them assuming it, and
+ *     a word in [q_i, 2^elementBitWidth) gives undefined results.  Every output residue is canonical too.
+ *     A ciphertext is [2][L][N] (c0 limbs, then c1 limbs), in EVALUATION form:
  *         slot k of limb i holds a(psi_i^(2*bitrev(k)+1)) mod q_i      (bitrev over log2 N bits)
  *   - `stream` is a cudaStream_t passed as void* (NULL = default stream); calls are asynchronous.  The ops of one ctx share
  *     one device workspace: calls may arrive on different streams (the library orders the workspace between them with an

@@ -171,6 +171,18 @@ def test_bconv_batch(N, ml, al, src, dst, nb):
 def test_bconv_tensor_core_kernels_agree_in_a_subprocess():
     """HML_BCONV_UMMA is read once per process: the same batched conversions and one hmult on the FP64 tensor-core kernel
     (child process, HML_BCONV_UMMA=0) must be bit-identical to the tcgen05 kernel's results here."""
+    _tensor_core_kernels_agree(36)
+
+
+def test_bconv_tensor_core_kernels_agree_in_a_subprocess_at_28_bits():
+    """the same comparison with 28-bit moduli: every residue is below 2^32, so the fifth byte plane of the tcgen05 operands is
+    zero"""
+    _tensor_core_kernels_agree(28)
+
+
+def _tensor_core_kernels_agree(w):
+    """batched conversions, hmult_batch and hrotate_batch at element width w, run once with the tcgen05 conversion and once
+    with the FP64 tensor-core conversion (one child process each): the results must be bit-identical"""
     import os
     import subprocess
     import sys
@@ -179,7 +191,7 @@ def test_bconv_tensor_core_kernels_agree_in_a_subprocess():
     body = (
         "import sys; sys.path.insert(0, %r)\n"
         "import torch, homulator_b200 as hml\n"
-        "ctx = hml.Context(N=8192, max_level=12, alpha=4)\n"
+        "ctx = hml.Context(N=8192, max_level=12, alpha=4, element_bit_width=%d)\n"
         "L = 11\n"
         "src, dst = list(range(12, 16)), list(range(L))\n"
         "x = ctx.uniform(src, 5, lead=(6,))\n"
@@ -187,7 +199,7 @@ def test_bconv_tensor_core_kernels_agree_in_a_subprocess():
         "evk = ctx.uniform(ctx.ext_mod_idx(L), 3, lead=(ctx.beta(L), 2))\n"
         "a = ctx.uniform(list(range(L)), 1, lead=(3, 2)); b = ctx.uniform(list(range(L)), 2, lead=(3, 2))\n"
         "h = ctx.hmult_batch(L, a, b, evk); r = ctx.hrotate_batch(L, a, evk, 5)\n"
-        "torch.save([y.cpu(), h.cpu(), r.cpu()], sys.argv[1])\n" % root)
+        "torch.save([y.cpu(), h.cpu(), r.cpu()], sys.argv[1])\n" % (root, w))
     outs = []
     with tempfile.TemporaryDirectory() as d:
         for flag in ("1", "0"):

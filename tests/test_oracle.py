@@ -28,7 +28,9 @@ def is_prime(n):
     return True
 
 
-@pytest.mark.parametrize("N,w,ml,al", [(16, 36, 6, 2), (256, 36, 5, 3), (65536, 36, 45, 15), (32768, 36, 28, 28)])
+@pytest.mark.parametrize("N,w,ml,al", [(16, 36, 6, 2), (256, 36, 5, 3), (65536, 36, 45, 15), (32768, 36, 28, 28),
+                                       (2048, 20, 12, 4), (256, 20, 70, 10), (8192, 24, 40, 10), (65536, 28, 45, 15), (65536, 32, 45, 15),
+                                       (4096, 33, 16, 2), (65536, 35, 45, 15)])
 def test_moduli_rule(N, w, ml, al):
     o = Oracle(N, w, ml, al)
     # independent python restatement of the rule: primes = 1 mod 2N, scanned downward from 2^w
@@ -43,9 +45,10 @@ def test_moduli_rule(N, w, ml, al):
         assert pow(psi, N, m) == m - 1  # primitive 2N-th root
 
 
-@pytest.mark.parametrize("N", [16, 64, 256])
-def test_fast_ntt_equals_definition(N):
-    o = Oracle(N, 36, 3, 2)
+@pytest.mark.parametrize("N,w", [(16, 36), (64, 36), (256, 36), (64, 20), (256, 28), (64, 33), (256, 35)],
+                         ids=["16", "64", "256", "64-w20", "256-w28", "64-w33", "256-w35"])
+def test_fast_ntt_equals_definition(N, w):
+    o = Oracle(N, w, 3, 2)
     for mi in range(o.n_mod):
         a = uniform_limbs([o.moduli[mi]], N, 7 + mi)[0]
         fast = o.ntt(mi, a)
